@@ -9,6 +9,15 @@ contiguous segment per rank, IQ-corrector state handed off through an all-gather
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference ...                     # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also save the last timed step's output
+
+`--dump-outputs DIR` writes DIR/out.npy (float64): what the timed path returned in its last timed
+step, the whole stream in rank order, or a fixed seeded sample of its columns beyond 64 MB.  The
+inputs depend only on the arguments, so two builds can be compared output for output.
+
+`--steps` is the number of timed steps of the headline measurement (`value`, `ms_per_step`,
+`gpu_launches`; the reference arm likewise).  The secondary legs keep their own counts: `e2e`
+times min(--steps, 3) steps, `simo` 24 batches and `simo_config4` 12.
 
 One JSON line on stdout (rank 0).  `value`: device-resident input, CUDA-event timed, max over
 ranks.  `e2e`: the same through the C ABI's host entry points (pinned host buffers, H2D and D2H
@@ -154,6 +163,8 @@ def run_reference_arm(args):
         dt = time.perf_counter() - t0
         if it >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {'out': out})
     t = sum(times) / len(times)
     val = nch * 32768 / t / 1e6
     sample = f'{nch} chunks ({nch * 32768} samples) per step'
@@ -274,10 +285,15 @@ def measure_cli(torch, raw_dev, nch_small: int, nch_big: int):
     streaming rate is not the difference of two process times: `steady` times the CLI's own
     `main(argv)` in THIS process (context already up) on the big file, best of two -- the same
     reader thread, page-locked chunk pool, processor and file writer, minus process start."""
+    import shutil
     import tempfile
     import signals
     res = {}
     d = '/dev/shm' if os.path.isdir('/dev/shm') else tempfile.gettempdir()
+    # the CLI caches its plan tables; keep that cache out of the (possibly read-only) source tree
+    plan_cache = tempfile.mkdtemp(prefix='sdrb_plan_cache_')
+    saved_cache = os.environ.get('SDRB_PLAN_CACHE')
+    os.environ['SDRB_PLAN_CACHE'] = plan_cache
     env = dict(os.environ, PYTHONPATH=os.path.join(ROOT, 'src'))
     times = {}
     flags = ['-c', '15k', '-w', '5k', '-d', '64', '--correct-iq']
@@ -330,6 +346,11 @@ def measure_cli(torch, raw_dev, nch_small: int, nch_big: int):
         for f in made:
             if os.path.exists(f):
                 os.unlink(f)
+        if saved_cache is None:
+            os.environ.pop('SDRB_PLAN_CACHE', None)
+        else:
+            os.environ['SDRB_PLAN_CACHE'] = saved_cache
+        shutil.rmtree(plan_cache, ignore_errors=True)
     return res
 
 
@@ -477,6 +498,11 @@ def run_cuda_arm(args):
         if i % 16 == 15:
             torch.cuda.synchronize()
     barrier()
+    if world == 1:
+        # one GPU carries the IQ corrector's offset from step to step, and how many steps ran above
+        # depends on timing: the timed steps start from a zero offset, so what they compute depends
+        # on the arguments only
+        eng.iq_state = 0j
     l0 = eng.launches
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ktimes = []
@@ -490,6 +516,14 @@ def run_cuda_arm(args):
     barrier()
     ms_total = max_over_ranks(ev0.elapsed_time(ev1))
     launches = eng.launches - l0
+    dumped = None
+    if args.dump_outputs:
+        dumped = out.clone()                # the steps below overwrite `out`
+        if world > 1:
+            parts = [torch.empty_like(dumped) for _ in range(world)]
+            dist.all_gather(parts, dumped)
+            dumped = torch.cat(parts, dim=1)
+        dumped = dumped.cpu().numpy() if rank == 0 else None
     kt = eng.kernel_times() if world == 1 else None
     # a few extra profiled steps for a steadier per-kernel average
     kavg = None
@@ -627,6 +661,8 @@ def run_cuda_arm(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if dumped is not None:
+        write_outputs(args.dump_outputs, {'out': dumped})
 
     peaks_path = os.path.join(ROOT, 'MEASURED_PEAKS.json')
     if os.path.exists(peaks_path):
@@ -718,10 +754,29 @@ def emit(line: dict) -> None:
         os.write(_JSON_FD, data)
 
 
+DUMP_BYTES = 64_000_000
+
+
+def write_outputs(d: str, arrays: dict) -> None:
+    """Save each array as d/<name>.npy in float64.  Past DUMP_BYTES in all, an array keeps the same
+    seeded sample of its last axis at every run with the same shapes."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    budget = (DUMP_BYTES - 4096 * len(arrays)) // len(arrays)          # 4096: room for the .npy header
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if a.nbytes > budget:
+            keep = budget // (8 * (a.size // a.shape[-1]))
+            cols = np.sort(np.random.default_rng(0).choice(a.shape[-1], keep, replace=False))
+            a = a[..., cols]
+        np.save(os.path.join(d, name + '.npy'), np.ascontiguousarray(a))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=5)
+    ap.add_argument('--steps', type=int, default=5,
+                    help='timed steps of the headline measurement (the e2e and SIMO legs keep their own counts)')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--chunks', type=int, default=8192, help='chunks per GPU per step')
@@ -736,7 +791,11 @@ def main():
     ap.add_argument('--ref-chunks', type=int, default=1024, help='chunks per step of the reference arm')
     ap.add_argument('--cpu-seconds', type=float, default=10.0)
     ap.add_argument('--no-cpu', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the last timed step\'s output to DIR/out.npy (float64, at most 64 MB)')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
     claim_stdout()
     if args.impl == 'reference':
         run_reference_arm(args)

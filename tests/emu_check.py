@@ -1,10 +1,11 @@
 """Developer script: the numpy twins of the kernels vs the oracle for the parity cases
 (python tests/emu_check.py [case ...]); tests/test_emulator.py runs a subset in the CPU suite."""
+import os
 import sys
 import time
 
-sys.path.insert(0, '/root/repo')
-sys.path.insert(0, '/root/repo/tests')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path[:0] = [ROOT, os.path.join(ROOT, 'tests')]
 import numpy as np
 
 from cases import CASES

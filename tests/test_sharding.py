@@ -206,6 +206,9 @@ def _bank_worker(rank, world, port, q):
             sys.path.insert(0, p)
     import ctypes
     from sdrterm_b200 import multigpu
+    # the stand-in engine reads host memory: the product classes must keep their tensors on the
+    # host, as they do on a machine without a CUDA device
+    torch.cuda.is_available = lambda: False
     os.environ.update(MASTER_ADDR='127.0.0.1', MASTER_PORT=str(port), SDRB_BCAST='nccl')
     dist.init_process_group('gloo', rank=rank, world_size=world)
 
@@ -291,6 +294,9 @@ def _chain_worker(rank, world, port, q):
             sys.path.insert(0, p)
     import ctypes
     from sdrterm_b200 import multigpu
+    # the stand-in engine writes host memory: the product class must keep its tensors on the host,
+    # as it does on a machine without a CUDA device
+    torch.cuda.is_available = lambda: False
     os.environ.update(MASTER_ADDR='127.0.0.1', MASTER_PORT=str(port))
     dist.init_process_group('gloo', rank=rank, world_size=world)
     lam = 1 - 50 / 1_024_000
