@@ -18,7 +18,7 @@
 extern "C" {
 #endif
 
-#define SDRB_ABI_VERSION 6
+#define SDRB_ABI_VERSION 7
 #define SDRB_TILE_BLOCKS 32
 #define SDRB_NPOLES 8
 #define SDRB_MAX_DECIMATION 256
@@ -48,7 +48,9 @@ typedef struct sdrb_config {
     uint8_t normalize;       /* --normalize-input (read_file.py:79-96) */
     uint8_t demod;           /* enum sdrb_demod (io_args.py:37-47) */
     uint8_t big_endian_out;  /* SIMO framing '!d' (vfo_processor.py:84) vs '@d' (dsp_processor.py:162) */
-    uint8_t reserved[2];
+    uint8_t seamless;        /* not a reference option: filter and demodulate the whole stream instead of
+                                each chunk (sdrb_stream*; DESIGN.md section 11).  Needs q | N. */
+    uint8_t reserved[1];
     int32_t q;               /* -d decimation, 2..SDRB_MAX_DECIMATION */
     int32_t N;               /* complex samples per chunk = 131072 / (2*itemsize) */
     int32_t edge;            /* sosfiltfilt pad length (27) */
@@ -121,6 +123,13 @@ typedef struct sdrb_tables {
     const double *tc_cst;    /* [R][tc_nout + 4] */
     const double *tc_rowc;   /* [R][tc_nrowc] complex: epilogue constants (plan.py RC_* layout) */
     uint8_t tc_xor[16];      /* XOR pattern of 16 consecutive stream bytes */
+    /* seamless streaming (cfg.seamless; plan.py build_plan(seamless=True)) */
+    int32_t lookahead;       /* D: a chunk's output is final once the D chunks after it exist */
+    int64_t fs;              /* sample rate in Hz (exact integer NCO phase across chunks) */
+    const int64_t *chunk_step;   /* [R] (f_r * N) mod fs: NCO phase step per chunk, in units of 2 pi / fs */
+    const double *PN;        /* [lookahead+1][8] complex: p_i^(N j) */
+    const double *sos_AM;    /* [ns][ns]: A^M of the output cascade */
+    const double *sos_CAM;   /* [M][ns]: c A^i, i < M */
 } sdrb_tables;
 
 typedef struct sdrb_handle sdrb_handle;
@@ -264,6 +273,30 @@ int sdrb_correct_iq(int device, double *z_inout, size_t nsamples, double off_ino
  * exact integers) as [chunk][row][N/q] interleaved complex128. */
 int sdrb_keep_x0(sdrb_handle *h, int on);
 int sdrb_read_x0(sdrb_handle *h, size_t nchunks, double *x0_host);
+/* Seamless streaming (not a reference option; DESIGN.md section 11).  On a handle created with
+ * cfg.seamless the chunk stream is filtered and demodulated as ONE signal, the way
+ * scipy.signal.decimate / sosfilt would treat the concatenated stream: the NCO phase runs on across
+ * chunks, the decimator's zero-phase filter sees the stream's two real ends only, the fm
+ * discriminator and the output low-pass carry their state.  The framing per chunk is unchanged
+ * (M doubles per chunk and row, [row][chunk][M], big-endian when cfg.big_endian_out).
+ *   sdrb_stream         host `raw` of nchunks whole chunks in; emits every chunk that has become final
+ *                       (a chunk is final once the lookahead D chunks after it exist), synchronously,
+ *                       into host `out` (room for nchunks + D chunks); *nchunks_out = chunks emitted
+ *   sdrb_stream_device  the same on device buffers, only enqueued on `stream` (`out_dev`: room for
+ *                       nchunks chunks)
+ *   sdrb_stream_end     end of stream: emits the chunks still held back, with the stream's real end
+ *                       as the boundary (room for D chunks), and resets the stream (IQ offset included)
+ *   sdrb_stream_end_device  the same into a device buffer, enqueued on `stream`
+ *   sdrb_stream_lookahead   D
+ * sdrb_process*, sdrb_submit, the phase entry points and sdrb_iq_gain return SDRB_ERR_STATE on such a
+ * handle; sdrb_set_smooth returns SDRB_ERR_ARG (Savitzky-Golay per chunk is chunk-local by design). */
+int sdrb_stream(sdrb_handle *h, const void *raw_host, size_t nchunks, double *out_host, size_t *nchunks_out);
+int sdrb_stream_device(sdrb_handle *h, const void *raw_dev, size_t nchunks, double *out_dev, void *stream,
+                       size_t *nchunks_out);
+int sdrb_stream_end(sdrb_handle *h, double *out_host, size_t *nchunks_out);
+int sdrb_stream_end_device(sdrb_handle *h, double *out_dev, void *stream, size_t *nchunks_out);
+int sdrb_stream_lookahead(const sdrb_handle *h);
+
 const char *sdrb_global_error(void);
 
 #ifdef __cplusplus

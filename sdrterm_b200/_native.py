@@ -14,9 +14,10 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(_HERE)
 LIB_PATH = os.environ.get('SDRB_LIB') or os.path.join(_HERE, 'libsdrterm_b200.so')   # SDRB_LIB: experiment builds
 HEADER = os.path.join(ROOT, 'include', 'sdrterm_b200.h')
-SOURCES = [os.path.join(_HERE, 'csrc', f) for f in ('sdrb_api.cu', 'sdrb_kernels.cuh', 'sdrb_device.cuh', 'sdrb_tc.cuh', 'sdrb_finish.cuh')]
+SOURCES = [os.path.join(_HERE, 'csrc', f) for f in ('sdrb_api.cu', 'sdrb_kernels.cuh', 'sdrb_device.cuh', 'sdrb_tc.cuh', 'sdrb_finish.cuh',
+                                                    'sdrb_spectrum.cuh', 'sdrb_seamless.cuh')]
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 FM, AM, RE, IM = 0, 1, 2, 3
 DEMOD_CODE = {'fm': FM, 'am': AM, 're': RE, 'im': IM}
 
@@ -28,7 +29,8 @@ class SdrbError(RuntimeError):
 class Config(C.Structure):
     _fields_ = [('abi_version', C.c_int32), ('device', C.c_int32), ('enc', C.c_char),
                 ('swap', C.c_uint8), ('correct_iq', C.c_uint8), ('normalize', C.c_uint8),
-                ('demod', C.c_uint8), ('big_endian_out', C.c_uint8), ('reserved', C.c_uint8 * 2),
+                ('demod', C.c_uint8), ('big_endian_out', C.c_uint8), ('seamless', C.c_uint8),
+                ('reserved', C.c_uint8 * 1),
                 ('q', C.c_int32), ('N', C.c_int32), ('edge', C.c_int32), ('R', C.c_int32),
                 ('n_out_sections', C.c_int32), ('max_chunks', C.c_int32), ('iq_L', C.c_double),
                 ('norm_xmin', C.c_double), ('norm_k', C.c_double)]
@@ -51,7 +53,9 @@ class Tables(C.Structure):
                 ('tc_ncol', C.c_int32), ('tc_nout', C.c_int32), ('tc_npad', C.c_int32),
                 ('tc_S', C.c_int32), ('tc_S_yl', C.c_int32), ('tc_nrowc', C.c_int32), ('tc_a_signed', C.c_int32),
                 ('tc_Bq', C.POINTER(C.c_int8)), ('tc_cst', _DP), ('tc_rowc', _DP),
-                ('tc_xor', C.c_uint8 * 16)]
+                ('tc_xor', C.c_uint8 * 16),
+                ('lookahead', C.c_int32), ('fs', C.c_int64), ('chunk_step', C.POINTER(C.c_int64)),
+                ('PN', _DP), ('sos_AM', _DP), ('sos_CAM', _DP)]
 
 
 EXPORTS = ['sdrb_create', 'sdrb_destroy', 'sdrb_last_error', 'sdrb_outputs_per_chunk',
@@ -60,7 +64,8 @@ EXPORTS = ['sdrb_create', 'sdrb_destroy', 'sdrb_last_error', 'sdrb_outputs_per_c
            'sdrb_fm_demod', 'sdrb_am_demod', 'sdrb_real_output', 'sdrb_imag_output',
            'sdrb_shift_freq', 'sdrb_power_spectrum', 'sdrb_stft_db', 'sdrb_global_error', 'sdrb_process_device_phases',
            'sdrb_set_profiling', 'sdrb_kernel_times', 'sdrb_keep_decimated', 'sdrb_read_debug', 'sdrb_iq_export_device',
-           'sdrb_iq_prefix_device', 'sdrb_decode_iq', 'sdrb_correct_iq', 'sdrb_keep_x0', 'sdrb_read_x0', 'sdrb_iq_gain', 'sdrb_set_smooth', 'sdrb_host_alloc', 'sdrb_host_free', 'sdrb_reserve_sms']
+           'sdrb_iq_prefix_device', 'sdrb_decode_iq', 'sdrb_correct_iq', 'sdrb_keep_x0', 'sdrb_read_x0', 'sdrb_iq_gain', 'sdrb_set_smooth', 'sdrb_host_alloc', 'sdrb_host_free', 'sdrb_reserve_sms',
+           'sdrb_stream', 'sdrb_stream_device', 'sdrb_stream_end', 'sdrb_stream_end_device', 'sdrb_stream_lookahead']
 
 
 def nvcc_command(out: str = LIB_PATH) -> list[str]:
@@ -130,6 +135,12 @@ def lib():
         L.sdrb_reserve_sms.argtypes = [vp, C.c_int]
         L.sdrb_set_smooth.argtypes = [vp, C.c_int, C.c_int, C.c_int, C.c_int, vp]
         L.sdrb_read_x0.argtypes = [vp, sz, vp]
+        szp = C.POINTER(sz)
+        L.sdrb_stream.argtypes = [vp, vp, sz, vp, szp]
+        L.sdrb_stream_device.argtypes = [vp, vp, sz, vp, vp, szp]
+        L.sdrb_stream_end.argtypes = [vp, vp, szp]
+        L.sdrb_stream_end_device.argtypes = [vp, vp, vp, szp]
+        L.sdrb_stream_lookahead.argtypes = [vp]
         _lib = L
     return _lib
 

@@ -15,6 +15,7 @@
 #include "sdrb_tc.cuh"
 #include "sdrb_finish.cuh"
 #include "sdrb_spectrum.cuh"
+#include "sdrb_seamless.cuh"
 
 namespace {
 
@@ -62,6 +63,11 @@ struct sdrb_handle {
     double2 *x0_buf = nullptr;      // sdrb_keep_x0
     int smooth_w = 0, smooth_nhead = 0, smooth_ntail = 0, smooth_lo = 0;   // --smooth-output (window 0 = off)
     double *smooth_S = nullptr, *smooth_tmp = nullptr;
+    // seamless streaming (cfg.seamless): window of unemitted chunks in slots 0..nwin-1 of the scratch
+    bool seamless = false;
+    SeamDev sd{};
+    long long seen = 0, emitted = 0;   // chunks of the current stream taken in / emitted
+    int nwin = 0;
 };
 
 namespace {
@@ -301,7 +307,7 @@ int launch_chain_t(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, 
     if ((phases & PH_IQSCAN) && IQ) {
         int nth = 1024;
         while (nth > 32 && (size_t)nth / 2 >= nch) nth /= 2;
-        if (h->finish_on && pl.ntiles <= 32) {
+        if (h->finish_on && pl.ntiles <= 32 && !h->seamless) {
             // whole-tile chunks: warp-parallel gains, the chunk scan; k_finish derives the offsets
             // at the tile starts itself
             const bool pdl = h->pdl && (phases & PH_MAIN);        // only right behind the front end of the same call
@@ -590,8 +596,8 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
         if (cudaFuncSetAttribute(k_demod, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->demod_smem) != cudaSuccess)
             return bail(fail(h, SDRB_ERR_CUDA, "cudaFuncSetAttribute(k_demod) failed"));
 
-    // scratch for max_chunks
-    const size_t nch = h->max_chunks;
+    // scratch for max_chunks (seamless: plus the D chunks held back between calls)
+    const size_t nch = h->max_chunks + (cfg->seamless ? (size_t)std::max(tab->lookahead, 0) : 0);
     Scratch &sc = h->sc;
     UP(dalloc(h, nch * R * pl.Mf, &sc.ypart));
     UP(dalloc(h, nch * R * nt * 16, &sc.agg));
@@ -613,6 +619,35 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
         UP(dalloc(h, nch * R * M, &sc.zrow));
     }
     UP(setup_tc(h, tab));
+    if (cfg->seamless) {
+        h->seamless = true;
+        SeamDev &sd = h->sd;
+        if (pl.rem != 0 || pl.cnt_last != SDRB_TB || tab->lookahead < 1 || !tab->PN || !tab->chunk_step ||
+            tab->fs <= 0 || tab->fs >= (1LL << 31) || (cfg->n_out_sections != 0 && cfg->n_out_sections != 2) ||
+            (cfg->n_out_sections && (!tab->sos_AM || !tab->sos_CAM || !tab->sos_AP || pl.sos_Lseg * 32 != M)) ||
+            pl.edge + 1 > 64 || pl.nend > 64)
+            return bail(fail(h, SDRB_ERR_ARG, "seamless mode needs the decimation to divide the chunk (q | N), "
+                                              "a lookahead >= 1 and its tables"));
+        sd.D = tab->lookahead; sd.fs = tab->fs; sd.nedge = pl.edge + 1 + pl.nend;
+        UP(upload(h, reinterpret_cast<const long long *>(tab->chunk_step), (size_t)R, &sd.step));
+        UP(upload(h, reinterpret_cast<const double2 *>(tab->PN), (size_t)(sd.D + 1) * 8, &sd.PN));
+        if (cfg->n_out_sections) {
+            for (int i = 0; i < SEAM_NS * SEAM_NS; i++) sd.AM[i] = tab->sos_AM[i];
+            UP(upload(h, tab->sos_CAM, (size_t)M * SEAM_NS, &sd.CAM));
+        }
+        UP(dalloc(h, nch * sd.nedge, &sd.edges));
+        UP(dalloc(h, nch * R * 16, &sd.cagg));
+        UP(dalloc(h, nch * R * 8, &sd.G));
+        UP(dalloc(h, nch * R * 24, &sd.cin));
+        UP(dalloc(h, nch * R * (M + 1), &sd.ybuf));
+        UP(dalloc(h, nch * R * SEAM_NS, &sd.echunk));
+        UP(dalloc(h, nch * R * SEAM_NS, &sd.sst));
+        UP(dalloc(h, (size_t)R * 8, &sd.fwd));
+        UP(dalloc(h, (size_t)R * SEAM_NS, &sd.sos));
+        UP(dalloc(h, (size_t)R * 16, &sd.endv));
+        if (cudaMemset(sd.sos, 0, (size_t)R * SEAM_NS * sizeof(double)) != cudaSuccess)
+            return bail(fail(h, SDRB_ERR_CUDA, "memset failed"));
+    }
 #undef UP
     for (int s = 0; s < 2; s++) {
         if (cudaStreamCreateWithFlags(&h->slot[s].stream, cudaStreamNonBlocking) != cudaSuccess ||
@@ -650,6 +685,7 @@ long long sdrb_launch_count(const sdrb_handle *h) { return h ? h->launches : 0; 
 int sdrb_process_device(sdrb_handle *h, const void *raw_dev, size_t nchunks, double *out_dev, void *stream)
 {
     if (!h || !raw_dev || !out_dev) return fail(h, SDRB_ERR_ARG, "null argument");
+    if (h->seamless) return fail(h, SDRB_ERR_STATE, "seamless handle: use sdrb_stream_device / sdrb_stream_end_device");
     if (nchunks == 0) return SDRB_OK;
     if (nchunks > h->max_chunks) return fail(h, SDRB_ERR_ARG, "nchunks %zu > max_chunks %zu", nchunks, h->max_chunks);
     CK(h, cudaSetDevice(h->cfg.device));
@@ -661,13 +697,15 @@ static int ensure_slot(sdrb_handle *h, int s)
 {
     Slot &sl = h->slot[s];
     if (!sl.raw) CK(h, cudaMalloc(&sl.raw, h->max_chunks * sdrb_chunk_bytes(h)));
-    if (!sl.out) CK(h, cudaMalloc(&sl.out, h->max_chunks * (size_t)h->pl.R * h->pl.M * sizeof(double)));
+    const size_t och = h->max_chunks + (h->seamless ? (size_t)h->sd.D : 0);
+    if (!sl.out) CK(h, cudaMalloc(&sl.out, och * (size_t)h->pl.R * h->pl.M * sizeof(double)));
     return 0;
 }
 
 int sdrb_submit(sdrb_handle *h, int s, const void *raw_host, size_t nchunks, double *out_host)
 {
     if (!h || !raw_host || !out_host || s < 0 || s > 1) return fail(h, SDRB_ERR_ARG, "bad argument");
+    if (h->seamless) return fail(h, SDRB_ERR_STATE, "seamless handle: use sdrb_stream / sdrb_stream_end");
     if (nchunks == 0 || nchunks > h->max_chunks) return fail(h, SDRB_ERR_ARG, "nchunks %zu outside 1..%zu", nchunks, h->max_chunks);
     CK(h, cudaSetDevice(h->cfg.device));
     int rc = ensure_slot(h, s);
@@ -700,6 +738,7 @@ int sdrb_wait(sdrb_handle *h, int s)
 int sdrb_process(sdrb_handle *h, const void *raw, size_t nchunks, double *out)
 {
     if (!h || (!raw && nchunks) || (!out && nchunks)) return fail(h, SDRB_ERR_ARG, "null argument");
+    if (h->seamless) return fail(h, SDRB_ERR_STATE, "seamless handle: use sdrb_stream / sdrb_stream_end");
     const size_t cb = sdrb_chunk_bytes(h), M = (size_t)h->pl.M, R = (size_t)h->pl.R;
     if (nchunks <= h->max_chunks) {
         if (nchunks == 0) return SDRB_OK;
@@ -746,13 +785,183 @@ void launch_iqchunk(sdrb_handle *h, const uint8_t *raw, size_t nch, cudaStream_t
 {
     k_iqchunk<ENC><<<(unsigned)((nch + 7) / 8), 256, 0, st>>>(h->pl, h->sc, raw, (int)nch);
 }
+
+// ------------------------------------------------------------------ seamless streaming
+template <int ENC>
+void launch_seam_edges(sdrb_handle *h, const uint8_t *raw, int slot0, size_t nch, cudaStream_t st)
+{
+    k_seam_edges<ENC><<<(unsigned)nch, 64, 0, st>>>(h->pl, h->sd, raw, slot0, (int)nch);
+}
+
+// Copy window slots [from, from + n) to [0, n) of a [slot][per] buffer (from > 0; a slot is never
+// read after it has been written when the ranges overlap).
+template <typename T>
+int seam_shift(sdrb_handle *h, T *buf, size_t per, int from, int n, cudaStream_t st)
+{
+    if (n <= 0 || from <= 0) return 0;
+    if (from >= n) {
+        CK(h, cudaMemcpyAsync(buf, buf + (size_t)from * per, (size_t)n * per * sizeof(T), cudaMemcpyDeviceToDevice, st));
+    } else {
+        for (int j = 0; j < n; j++)
+            CK(h, cudaMemcpyAsync(buf + (size_t)j * per, buf + (size_t)(from + j) * per, per * sizeof(T),
+                                  cudaMemcpyDeviceToDevice, st));
+    }
+    return 0;
+}
+
+// One seamless step: the front end and the IQ kernels over `nch` new chunks (into the window slots
+// after the held-back ones), the chunk aggregates and the forward scan; then every chunk that is
+// final (all of them when `end`) goes through carry / outputs / demodulation / SOS into `out`.
+int seam_step(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, cudaStream_t st, bool end, size_t *nout)
+{
+    const DevPlan &pl = h->pl;
+    SeamDev &sd = h->sd;
+    const int R = pl.R, nt = pl.ntiles, M = pl.M;
+    int rc = 0;
+    if (nch) {
+        const int s0 = h->nwin;
+        Scratch base = h->sc, sh = h->sc;
+        sh.ypart += (size_t)s0 * R * pl.Mf;
+        sh.agg += (size_t)s0 * R * nt * 16;
+        sh.tile_agg += (size_t)s0 * nt;
+        sh.off_tile += (size_t)s0 * (nt + 1);
+        sh.gain += s0;
+        sh.start += s0;
+        h->sc = sh;
+        rc = launch_chain(h, raw, nch, nullptr, st, PH_MAIN | PH_IQSCAN);
+        h->sc = base;
+        if (rc) return rc;
+        switch (h->enc_code) {
+        case ENC_b: launch_seam_edges<ENC_b>(h, raw, s0, nch, st); break;
+        case ENC_B: launch_seam_edges<ENC_B>(h, raw, s0, nch, st); break;
+        case ENC_h: launch_seam_edges<ENC_h>(h, raw, s0, nch, st); break;
+        case ENC_H: launch_seam_edges<ENC_H>(h, raw, s0, nch, st); break;
+        case ENC_i: launch_seam_edges<ENC_i>(h, raw, s0, nch, st); break;
+        case ENC_I: launch_seam_edges<ENC_I>(h, raw, s0, nch, st); break;
+        case ENC_f: launch_seam_edges<ENC_f>(h, raw, s0, nch, st); break;
+        case ENC_d: launch_seam_edges<ENC_d>(h, raw, s0, nch, st); break;
+        default:    launch_seam_edges<ENC_Z>(h, raw, s0, nch, st); break;
+        }
+        const size_t items = nch * (size_t)R;
+        k_seam_agg<<<(unsigned)((items + 7) / 8), 256, 0, st>>>(pl, h->sc, sd, s0, (int)nch, h->seen);
+        if (h->seen == 0) k_seam_head<<<(unsigned)((R + 63) / 64), 64, 0, st>>>(pl, h->sc, sd, s0);
+        k_seam_fscan<<<(unsigned)R, 256, 0, st>>>(pl, sd, s0, (int)nch);
+        h->launches += 3 + (h->seen == 0);
+        h->seen += (long long)nch;
+        h->nwin += (int)nch;
+    }
+    long long upto = end ? h->seen : std::max(0LL, h->seen - sd.D);
+    const int ne = (int)(upto - h->emitted);
+    const long long g0 = h->emitted;
+    if (ne > 0) {
+        if (end) {
+            k_seam_tail<<<(unsigned)((R + 63) / 64), 64, 0, st>>>(pl, h->sc, sd, h->nwin - 1, h->seen - 1);
+            h->launches++;
+        }
+        const size_t items = (size_t)ne * R;
+        const unsigned wg = (unsigned)((items + 7) / 8);
+        k_seam_carry<<<wg, 256, 0, st>>>(pl, h->sc, sd, ne, h->nwin, g0, end ? 1 : 0);
+        k_seam_y<<<wg, 256, 0, st>>>(pl, h->sc, sd, ne, h->nwin, g0, end ? 1 : 0);
+        k_seam_demod<<<wg, 256, 0, st>>>(pl, sd, out, ne, h->nwin, end ? 1 : 0);
+        h->launches += 3;
+        if (pl.nsec_out) {
+            k_seam_sscan<<<(unsigned)R, 32, 0, st>>>(pl, sd, ne);
+            const size_t total = items * M;
+            k_seam_frame<<<(unsigned)std::min<size_t>((total + 255) / 256, (size_t)h->num_sms * 16), 256, 0, st>>>(pl, sd, out, ne);
+            h->launches += 2;
+        }
+        CK(h, cudaGetLastError());
+        // the chunks still held back move to the front of the window
+        const int keep = h->nwin - ne;
+        if ((rc = seam_shift(h, h->sc.ypart, (size_t)R * pl.Mf, ne, keep, st)) ||
+            (rc = seam_shift(h, h->sc.agg, (size_t)R * nt * 16, ne, keep, st)) ||
+            (rc = seam_shift(h, h->sc.off_tile, (size_t)(nt + 1), ne, keep, st)) ||
+            (rc = seam_shift(h, sd.edges, (size_t)sd.nedge, ne, keep, st)) ||
+            (rc = seam_shift(h, sd.cagg, (size_t)R * 16, ne, keep, st)) ||
+            (rc = seam_shift(h, sd.G, (size_t)R * 8, ne, keep, st)))
+            return rc;
+        h->nwin = keep;
+        h->emitted = upto;
+    }
+    CK(h, cudaGetLastError());
+    if (nout) *nout = (size_t)std::max(ne, 0);
+    if (end) {   // a new stream starts from scratch: counters, output filter and IQ corrector
+        h->seen = h->emitted = 0;
+        h->nwin = 0;
+        CK(h, cudaMemsetAsync(sd.sos, 0, (size_t)R * SEAM_NS * sizeof(double), st));
+        CK(h, cudaMemsetAsync(h->sc.iq_state, 0, sizeof(double2), st));
+    }
+    return 0;
+}
 }  // namespace
 extern "C" {
+
+int sdrb_stream_device(sdrb_handle *h, const void *raw_dev, size_t nchunks, double *out_dev, void *stream,
+                       size_t *nchunks_out)
+{
+    if (nchunks_out) *nchunks_out = 0;
+    if (!h || (!raw_dev && nchunks) || !out_dev) return fail(h, SDRB_ERR_ARG, "null argument");
+    if (!h->seamless) return fail(h, SDRB_ERR_STATE, "sdrb_stream needs a handle created with cfg.seamless");
+    if (nchunks > h->max_chunks) return fail(h, SDRB_ERR_ARG, "nchunks %zu > max_chunks %zu", nchunks, h->max_chunks);
+    CK(h, cudaSetDevice(h->cfg.device));
+    return seam_step(h, static_cast<const uint8_t *>(raw_dev), nchunks, out_dev, static_cast<cudaStream_t>(stream), false,
+                     nchunks_out);
+}
+
+int sdrb_stream_end_device(sdrb_handle *h, double *out_dev, void *stream, size_t *nchunks_out)
+{
+    if (nchunks_out) *nchunks_out = 0;
+    if (!h || !out_dev) return fail(h, SDRB_ERR_ARG, "null argument");
+    if (!h->seamless) return fail(h, SDRB_ERR_STATE, "sdrb_stream_end needs a handle created with cfg.seamless");
+    CK(h, cudaSetDevice(h->cfg.device));
+    return seam_step(h, nullptr, 0, out_dev, static_cast<cudaStream_t>(stream), true, nchunks_out);
+}
+
+static int seam_host(sdrb_handle *h, const void *raw_host, size_t nchunks, double *out_host, size_t *nchunks_out, bool end)
+{
+    if (nchunks_out) *nchunks_out = 0;
+    if (!h || (!raw_host && nchunks) || !out_host) return fail(h, SDRB_ERR_ARG, "null argument");
+    if (!h->seamless) return fail(h, SDRB_ERR_STATE, "sdrb_stream needs a handle created with cfg.seamless");
+    if (nchunks > h->max_chunks) return fail(h, SDRB_ERR_ARG, "nchunks %zu > max_chunks %zu", nchunks, h->max_chunks);
+    CK(h, cudaSetDevice(h->cfg.device));
+    int rc = ensure_slot(h, 0);
+    if (rc) return rc;
+    Slot &sl = h->slot[0];
+    if (nchunks)
+        CK(h, cudaMemcpyAsync(sl.raw, raw_host, nchunks * sdrb_chunk_bytes(h), cudaMemcpyHostToDevice, sl.stream));
+    size_t ne = 0;
+    rc = seam_step(h, sl.raw, nchunks, sl.out, sl.stream, end, &ne);
+    if (rc) return rc;
+    if (ne)
+        CK(h, cudaMemcpyAsync(out_host, sl.out, ne * (size_t)h->pl.R * h->pl.M * sizeof(double), cudaMemcpyDeviceToHost,
+                              sl.stream));
+    CK(h, cudaStreamSynchronize(sl.stream));
+    if (nchunks_out) *nchunks_out = ne;
+    return SDRB_OK;
+}
+
+int sdrb_stream(sdrb_handle *h, const void *raw_host, size_t nchunks, double *out_host, size_t *nchunks_out)
+{
+    return seam_host(h, raw_host, nchunks, out_host, nchunks_out, false);
+}
+
+int sdrb_stream_end(sdrb_handle *h, double *out_host, size_t *nchunks_out)
+{
+    return seam_host(h, nullptr, 0, out_host, nchunks_out, true);
+}
+
+int sdrb_stream_lookahead(const sdrb_handle *h)
+{
+    if (!h) return SDRB_ERR_ARG;
+    return h->seamless ? h->sd.D : 0;
+}
 
 int sdrb_set_smooth(sdrb_handle *h, int window, int nhead, int ntail, int lo, const double *tab)
 {
     if (!h || window < 0 || (window > 0 && (!tab || nhead < 0 || ntail < 0 || nhead + ntail > h->pl.M)))
         return fail(h, SDRB_ERR_ARG, "bad argument");
+    if (h->seamless && window > 0)
+        return fail(h, SDRB_ERR_ARG, "--smooth-output is per-chunk Savitzky-Golay by definition: not available in seamless mode");
     if (window > h->pl.M) return fail(h, SDRB_ERR_ARG, "smoothing window %d longer than a chunk's %d outputs", window, h->pl.M);
     CK(h, cudaSetDevice(h->cfg.device));
     CK(h, cudaDeviceSynchronize());
@@ -776,6 +985,7 @@ int sdrb_set_smooth(sdrb_handle *h, int window, int nhead, int ntail, int lo, co
 int sdrb_iq_gain(sdrb_handle *h, const void *raw_host, size_t nchunks)
 {
     if (!h || !raw_host) return fail(h, SDRB_ERR_ARG, "null argument");
+    if (h->seamless) return fail(h, SDRB_ERR_STATE, "seamless handle: the IQ state advances with sdrb_stream");
     if (nchunks == 0 || !h->pl.correct_iq) return SDRB_OK;
     if (nchunks > h->max_chunks) return fail(h, SDRB_ERR_ARG, "nchunks %zu > max_chunks %zu", nchunks, h->max_chunks);
     CK(h, cudaSetDevice(h->cfg.device));
@@ -806,6 +1016,7 @@ int sdrb_iq_gain(sdrb_handle *h, const void *raw_host, size_t nchunks)
 int sdrb_process_device_phases(sdrb_handle *h, const void *raw_dev, size_t nchunks, double *out_dev, void *stream, int phases)
 {
     if (!h || !raw_dev || (!out_dev && (phases & PH_FINISH))) return fail(h, SDRB_ERR_ARG, "null argument");
+    if (h->seamless) return fail(h, SDRB_ERR_STATE, "seamless handle: time-segment phases are not available");
     if (nchunks == 0) return SDRB_OK;
     if (nchunks > h->max_chunks) return fail(h, SDRB_ERR_ARG, "nchunks %zu > max_chunks %zu", nchunks, h->max_chunks);
     CK(h, cudaSetDevice(h->cfg.device));
@@ -818,6 +1029,7 @@ int sdrb_process_device_phases(sdrb_handle *h, const void *raw_dev, size_t nchun
 int sdrb_iq_export_device(sdrb_handle *h, double *dst3_dev, double nsamples, void *stream)
 {
     if (!h || !dst3_dev) return fail(h, SDRB_ERR_ARG, "null argument");
+    if (h->seamless) return fail(h, SDRB_ERR_STATE, "seamless handle: time-segment phases are not available");
     CK(h, cudaSetDevice(h->cfg.device));
     k_iq_export<<<1, 32, 0, static_cast<cudaStream_t>(stream)>>>(h->sc, dst3_dev, nsamples);
     h->launches++;
@@ -828,6 +1040,7 @@ int sdrb_iq_export_device(sdrb_handle *h, double *dst3_dev, double nsamples, voi
 int sdrb_iq_prefix_device(sdrb_handle *h, const double *gains3_dev, int rank, void *stream)
 {
     if (!h || !gains3_dev || rank < 0) return fail(h, SDRB_ERR_ARG, "bad argument");
+    if (h->seamless) return fail(h, SDRB_ERR_STATE, "seamless handle: time-segment phases are not available");
     CK(h, cudaSetDevice(h->cfg.device));
     k_iq_prefix<<<1, 32, 0, static_cast<cudaStream_t>(stream)>>>(h->sc, gains3_dev, rank, h->pl.lam);
     h->launches++;

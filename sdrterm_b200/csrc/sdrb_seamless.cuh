@@ -1,0 +1,471 @@
+// sdrb_seamless.cuh -- the finish stage of the seamless streaming mode (DESIGN.md section 11).
+//
+// The default chain filters every chunk as if it were the whole signal.  The seamless mode filters
+// the whole stream: the front ends (k_tc / k_main) and the IQ kernels run unchanged, chunk-local;
+// everything chunk-local after them is replaced here.  A chunk's front-end outputs are the global
+// ones times one phasor phi_{c,r} = exp(-2 pi i ((f_r N c) mod fs) / fs), so the kernels below
+//
+//   k_seam_edges   decode the head / end-window samples of every new chunk (kept for later calls)
+//   k_seam_agg     chunk aggregates: the tile aggregates composed over a chunk (forward A, backward B)
+//   k_seam_head    the stream's real start: odd extension and zi, forward state at sample 0
+//   k_seam_fscan   forward modal state across chunks: affine scan with multiplier p^N per mode
+//   k_seam_tail    the stream's real end: anticausal state after the last chunk and zeta
+//   k_seam_carry   per emitted chunk: carry-ins in its own frame (forward state, anticausal window
+//                  over the next D chunks or the real end, zeta) and the fm halo y[k+1]
+//   k_seam_y       per emitted chunk: tile carries and the decimated outputs, global frame
+//   k_seam_demod   demodulation + output SOS from the chunk's zero state (segments, lane scan)
+//   k_seam_sscan   output SOS state across chunks: affine scan with the matrix A^M
+//   k_seam_frame   response to the carried SOS state, framing
+//
+// tests/seamless_ref.py (SeamlessTwin) is the numpy twin of this decomposition.
+#pragma once
+#include "sdrb_kernels.cuh"
+
+#define SEAM_NS 4           // output SOS state size in seamless mode (ellip(3): two sections)
+
+struct SeamDev {
+    int D;                     // lookahead in chunks
+    int nedge;                 // decoded samples kept per chunk: head (edge+1) + end window (nend)
+    long long fs;
+    const long long *step;     // [R] (f_r N) mod fs
+    const double2 *PN;         // [D+1][8] p_i^(N j)
+    double AM[SEAM_NS * SEAM_NS];   // A^M of the output cascade
+    const double *CAM;         // [M][ns] c A^i
+    // window buffers, slot = position in the window of unemitted chunks
+    double2 *edges;            // [W][nedge]
+    double2 *cagg;             // [W][R][16]   0..7 A (forward), 8..15 B (backward), global frame
+    double2 *G;                // [W][R][8]    forward state at the chunk start, global frame
+    double2 *cin;              // [W][R][24]   carry-ins in the chunk frame: Win0, Tn_end, zeta
+    double2 *ybuf;             // [W][R][M+1]  decimated outputs (global frame) + halo
+    double *echunk;            // [W][R][ns]   SOS end state of a chunk from a zero state
+    double *sst;               // [W][R][ns]   SOS state at the chunk start (after k_seam_sscan)
+    double2 *fwd;              // [R][8]       forward state at the next new chunk
+    double *sos;               // [R][ns]      SOS state at the next chunk to emit
+    double2 *endv;             // [R][16]      real end: 0..7 anticausal state, 8..15 zeta (global frame)
+};
+
+__device__ __forceinline__ double2 seam_phasor(const SeamDev &sd, int r, long long g)
+{
+    const unsigned long long fs = (unsigned long long)sd.fs;
+    const unsigned long long idx = ((unsigned long long)sd.step[r] * ((unsigned long long)g % fs)) % fs;
+    double s, c;
+    sincospi(-2.0 * ((double)idx / (double)sd.fs), &s, &c);
+    return make_double2(c, s);
+}
+
+template <int ENC>
+__global__ void __launch_bounds__(64)
+k_seam_edges(const __grid_constant__ DevPlan pl, SeamDev sd, const uint8_t *__restrict__ raw, int slot0, int nch)
+{
+    const int c = blockIdx.x;
+    if (c >= nch) return;
+    const uint8_t *rawc = raw + (size_t)c * pl.N * pl.sb;
+    double2 *e = sd.edges + (size_t)(slot0 + c) * sd.nedge;
+    for (int j = threadIdx.x; j < sd.nedge; j += blockDim.x) {
+        const long n = j <= pl.edge ? j : (long)pl.ws + (j - pl.edge - 1);
+        e[j] = decode_sample<ENC>(pl, rawc, n);
+    }
+}
+
+// warp <-> (chunk, row); lanes 0..7 compose the forward tile aggregates, lanes 8..15 the backward ones;
+// stored rotated into the global frame (phi_c A_c, phi_c B_c)
+__global__ void __launch_bounds__(256)
+k_seam_agg(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int slot0, int nch, long long g0)
+{
+    const int lane = threadIdx.x & 31;
+    const long item = (long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (item >= (long)nch * pl.R || lane >= 16) return;
+    const int c = slot0 + (int)(item / pl.R), r = (int)(item % pl.R), nt = pl.ntiles, m = lane & 7;
+    const double2 *ag = sc.agg + ((size_t)c * pl.R + r) * nt * 16;
+    const double2 *T1 = pl.T1 + (size_t)r * nt;
+    double2 a = make_double2(0.0, 0.0);
+    if (lane < 8) {
+        for (int t = 0; t < nt; t++) {
+            const double2 Pc = pl.Ppow[(t == nt - 1 ? pl.cnt_last : SDRB_TB) * 8 + m];
+            a = cfma(Pc, a, cmul(T1[t], ag[(size_t)t * 16 + m]));
+        }
+    } else {
+        for (int t = nt - 1; t >= 0; t--) {
+            const double2 Pc = pl.Ppow[(t == nt - 1 ? pl.cnt_last : SDRB_TB) * 8 + m];
+            a = cfma(Pc, a, cmul(T1[t], ag[(size_t)t * 16 + 8 + m]));
+        }
+    }
+    sd.cagg[((size_t)c * pl.R + r) * 16 + lane] = cmul(seam_phasor(sd, r, g0 + (c - slot0)), a);
+}
+
+// thread <-> row: forward state at sample 0 of the stream (sosfiltfilt's odd extension and zi)
+__global__ void k_seam_head(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int slot)
+{
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= pl.R) return;
+    const int edge = pl.edge;
+    const double2 *z = sd.edges + (size_t)slot * sd.nedge;
+    const double2 off0 = pl.correct_iq ? sc.off_tile[(size_t)slot * (pl.ntiles + 1)] : make_double2(0.0, 0.0);
+    double2 xs[64];
+    double2 o = off0;
+    for (int n = 0; n <= edge; n++) {
+        const double2 x = csub(z[n], o);
+        o = make_double2(fma(pl.Liq, x.x, o.x), fma(pl.Liq, x.y, o.y));
+        xs[n] = cmul(x, pl.Ehead[(size_t)r * (edge + 1) + n]);
+    }
+    for (int m = 0; m < 8; m++) {
+        const double2 e0 = csub(cscale(2.0, xs[0]), xs[edge]);
+        double2 w = cmul(pl.zhat[m], e0);
+        for (int j = 0; j < edge; j++) w = cfma(pl.p[m], w, csub(cscale(2.0, xs[0]), xs[edge - j]));
+        w = cfma(pl.alpha[(size_t)r * 8 + m], off0, w);
+        sd.fwd[(size_t)r * 8 + m] = cmul(w, pl.binv[(size_t)r * 8 + m]);
+    }
+}
+
+// block <-> row, warp <-> mode, lane <-> contiguous run of chunks: G[c] = state before chunk c,
+// G[c+1] = p^N G[c] + phi_c A_c, from the handle's forward state; the new state back into it
+__global__ void __launch_bounds__(256)
+k_seam_fscan(const __grid_constant__ DevPlan pl, SeamDev sd, int slot0, int nch)
+{
+    const int r = blockIdx.x, m = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const double2 PN = sd.PN[8 + m];
+    const int per = (nch + 31) / 32;
+    const int c0 = min(nch, lane * per), c1 = min(nch, c0 + per);
+    double2 a = make_double2(0.0, 0.0), mul = make_double2(1.0, 0.0);
+    for (int c = c0; c < c1; c++) {
+        a = cfma(PN, a, sd.cagg[((size_t)(slot0 + c) * pl.R + r) * 16 + m]);
+        mul = cmul(mul, PN);
+    }
+#pragma unroll
+    for (int lv = 0; lv < 5; lv++) {
+        const double2 pa = shfl_up_c(a, 1 << lv), pm = shfl_up_c(mul, 1 << lv);
+        if (lane >= (1 << lv)) { a = cfma(mul, pa, a); mul = cmul(mul, pm); }
+    }
+    const double2 st0 = sd.fwd[(size_t)r * 8 + m];
+    double2 ea = shfl_up_c(a, 1), em = shfl_up_c(mul, 1);
+    if (lane == 0) { ea = make_double2(0.0, 0.0); em = make_double2(1.0, 0.0); }
+    double2 s = cfma(em, st0, ea);
+    for (int c = c0; c < c1; c++) {
+        sd.G[((size_t)(slot0 + c) * pl.R + r) * 8 + m] = s;
+        s = cfma(PN, s, sd.cagg[((size_t)(slot0 + c) * pl.R + r) * 16 + m]);
+    }
+    if (lane == 31) sd.fwd[(size_t)r * 8 + m] = cfma(mul, st0, a);
+}
+
+// thread <-> row: the stream's real end (the last chunk sits in window slot `slot`, global index g)
+__global__ void k_seam_tail(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int slot, long long g)
+{
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= pl.R) return;
+    const int edge = pl.edge, nend = pl.nend, nt = pl.ntiles;
+    const double2 *z = sd.edges + (size_t)slot * sd.nedge + edge + 1;
+    const double2 offE = pl.correct_iq ? sc.off_tile[(size_t)slot * (nt + 1) + nt] : make_double2(0.0, 0.0);
+    double2 xs[64];
+    double2 o = offE;
+    for (int n = pl.N - 1; n >= pl.ws; n--) {
+        const double2 zn = z[n - pl.ws];
+        o = make_double2((o.x - pl.Liq * zn.x) * pl.lam_inv, (o.y - pl.Liq * zn.y) * pl.lam_inv);
+        xs[n - pl.ws] = cmul(csub(zn, o), pl.Eend[(size_t)r * nend + (n - pl.ws)]);
+    }
+    const double2 ph = seam_phasor(sd, r, g);
+    const double2 sE = cmul(offE, pl.phE[r]);
+    double2 seq[64];
+    for (int j = 0; j < edge; j++) seq[j] = csub(cscale(2.0, xs[nend - 1]), xs[nend - 2 - j]);
+    double2 wL1[8], wL[8];
+    double2 yf = cscale(pl.d, seq[edge - 1]);
+    for (int m = 0; m < 8; m++) {
+        double2 w = csub(cmul(pl.beta[(size_t)r * 8 + m], cmul(cconj(ph), sd.fwd[(size_t)r * 8 + m])),
+                         cmul(pl.alpha[(size_t)r * 8 + m], sE));
+        for (int j = 0; j < edge - 1; j++) w = cfma(pl.p[m], w, seq[j]);
+        wL1[m] = w;
+        wL[m] = cfma(pl.p[m], w, seq[edge - 1]);
+        yf = cfma(pl.c[m], wL1[m], yf);
+    }
+    for (int m = 0; m < 8; m++) {
+        double2 zt = cmul(pl.zhat[m], yf);
+        for (int l = 0; l < 8; l++) zt = csub(zt, cmul(pl.xi[m * 8 + l], wL[l]));
+        double2 T = make_double2(0.0, 0.0);
+        for (int j = edge - 1; j >= 0; j--) T = cfma(pl.p[m], T, seq[j]);
+        T = cmul(cfma(pl.alphaT[(size_t)r * 8 + m], sE, T), pl.binvT[(size_t)r * 8 + m]);
+        sd.endv[(size_t)r * 16 + m] = cmul(ph, T);
+        sd.endv[(size_t)r * 16 + 8 + m] = cmul(ph, zt);
+    }
+}
+
+// warp <-> (emitted chunk i, row), lane <-> mode.  Window slots 0..nwin-1 hold global chunks g0..;
+// `end` = the real end of the stream is known (slot nwin-1 is the last chunk).
+__global__ void __launch_bounds__(256)
+k_seam_carry(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int ne, int nwin, long long g0, int end)
+{
+    const int lane = threadIdx.x & 31;
+    const long item = (long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (item >= (long)ne * pl.R) return;
+    const int i = (int)(item / pl.R), r = (int)(item % pl.R), m = lane & 7, R = pl.R, M = pl.M;
+    const int dist = nwin - 1 - i;                       // chunks after this one in the window
+    const bool known = end && dist <= sd.D, last = end && dist == 0;
+    const int J = known ? dist : sd.D;
+    const double2 PN1 = sd.PN[8 + m];
+    double2 Tg = known ? sd.endv[(size_t)r * 16 + m] : make_double2(0.0, 0.0);
+    for (int j = J; j >= 1; j--)
+        Tg = cfma(PN1, Tg, sd.cagg[((size_t)(i + j) * R + r) * 16 + 8 + m]);
+    double2 Zg = make_double2(0.0, 0.0);
+    if (known) Zg = cmul(sd.PN[(size_t)dist * 8 + m], sd.endv[(size_t)r * 16 + 8 + m]);
+    const double2 phc = cconj(seam_phasor(sd, r, g0 + i));
+    if (lane < 8) {
+        double2 *ci = sd.cin + ((size_t)i * R + r) * 24;
+        ci[m] = cmul(phc, sd.G[((size_t)i * R + r) * 8 + m]);
+        ci[8 + m] = cmul(phc, Tg);
+        ci[16 + m] = cmul(phc, Zg);
+    }
+    if (last) return;
+    // halo: block 0 of the next chunk, from this chunk's horizon
+    double2 v = make_double2(0.0, 0.0);
+    if (lane < 8) {
+        v = cmul(pl.rb[(size_t)r * 8 + m], sd.G[((size_t)(i + 1) * R + r) * 8 + m]);
+        v = cfma(pl.rbT[(size_t)r * 8 + m], Tg, v);
+        if (known) v = cfma(pl.bnd[m], cmul(sd.PN[(size_t)(dist - 1) * 8 + m], sd.endv[(size_t)r * 16 + 8 + m]), v);
+    }
+#pragma unroll
+    for (int o = 4; o >= 1; o >>= 1) v = cadd(v, shfl_xor_c(v, o));
+    if (lane == 0) {
+        const double2 z0 = sd.edges[(size_t)(i + 1) * sd.nedge];
+        const double2 off1 = pl.correct_iq ? sc.off_tile[(size_t)i * (pl.ntiles + 1) + pl.ntiles] : make_double2(0.0, 0.0);
+        const double2 loc = csub(cscale(pl.g0, z0), cmul(pl.gamma[r], off1));
+        v = cfma(seam_phasor(sd, r, g0 + i + 1), loc, v);
+        sd.ybuf[((size_t)i * R + r) * (M + 1) + M] = v;
+    }
+}
+
+// warp <-> (emitted chunk, row): tile carries (lanes 0..7 forward, 8..15 backward) into sc.carry,
+// then lane <-> block outputs, rotated into the global frame
+__global__ void __launch_bounds__(256)
+k_seam_y(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int ne, int nwin, long long g0, int end)
+{
+    const int lane = threadIdx.x & 31;
+    const long item = (long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (item >= (long)ne * pl.R) return;
+    const int i = (int)(item / pl.R), r = (int)(item % pl.R), nt = pl.ntiles, R = pl.R, M = pl.M;
+    const double2 *ci = sd.cin + ((size_t)i * R + r) * 24;
+    const double2 *ag = sc.agg + ((size_t)i * R + r) * nt * 16;
+    const double2 *T1 = pl.T1 + (size_t)r * nt;
+    double2 *carry = sc.carry + ((size_t)i * R + r) * (nt + 1) * 16;
+    if (lane < 8) {
+        const int m = lane;
+        const double2 b = pl.beta[(size_t)r * 8 + m];
+        double2 w = ci[m];
+        for (int t = 0; t < nt; t++) {
+            carry[(size_t)t * 16 + m] = cmul(b, w);
+            w = cfma(pl.Ppow[SDRB_TB * 8 + m], w, cmul(T1[t], ag[(size_t)t * 16 + m]));
+        }
+    } else if (lane < 16) {
+        const int m = lane - 8;
+        const double2 b = pl.betaT[(size_t)r * 8 + m];
+        double2 T = ci[8 + m];
+        carry[(size_t)nt * 16 + 8 + m] = cmul(b, T);
+        for (int t = nt - 1; t >= 0; t--) {
+            T = cfma(pl.Ppow[SDRB_TB * 8 + m], T, cmul(T1[t], ag[(size_t)t * 16 + 8 + m]));
+            carry[(size_t)t * 16 + 8 + m] = cmul(b, T);
+        }
+    }
+    __syncwarp();
+    const double2 ph = seam_phasor(sd, r, g0 + i);
+    const bool has_z = end && nwin - 1 - i <= sd.D;     // warp-uniform: zeta reaches this chunk
+    double2 zz[8];
+#pragma unroll
+    for (int m = 0; m < 8; m++) zz[m] = ci[16 + m];
+    const double2 *yp = sc.ypart + ((size_t)i * R + r) * pl.Mf;
+    const double2 *offt = sc.off_tile + (size_t)i * (nt + 1);
+    double2 *y = sd.ybuf + ((size_t)i * R + r) * (M + 1);
+    const int l = lane;
+    for (int t = 0; t < nt; t++) {
+        const int k = t * SDRB_TB + l;
+        const double2 s = pl.correct_iq ? cscale(-1.0, offt[t]) : make_double2(0.0, 0.0);
+        double2 v = cfma(s, pl.psiY[((size_t)(t == nt - 1 ? 1 : 0) * R + r) * SDRB_TB + l], yp[k]);
+        v = cmul(T1[t], v);
+#pragma unroll
+        for (int m = 0; m < 8; m++) {
+            v = cfma(pl.RW[l * 8 + m], carry[(size_t)t * 16 + m], v);
+            v = cfma(pl.RT[(SDRB_TB - l) * 8 + m], carry[(size_t)(t + 1) * 16 + 8 + m], v);
+        }
+        if (has_z)
+#pragma unroll
+            for (int m = 0; m < 8; m++) v = cfma(pl.bnd[(size_t)k * 8 + m], zz[m], v);
+        y[k] = cmul(ph, v);
+    }
+}
+
+__device__ __forceinline__ double seam_demod_at(const double2 *y, int k, int M, bool last, int demod)
+{
+    if (demod == SDRB_FM) {
+        if (last && k == M - 1) k = M - 2;
+        const double2 a = y[k], b = y[k + 1];
+        const double2 pr = make_double2(fma(a.x, b.x, a.y * b.y), fma(a.y, b.x, -a.x * b.y));
+        return atan2(pr.y, pr.x);
+    }
+    const double2 a = y[k];
+    if (demod == SDRB_AM) { const double re = fma(a.x, a.x, -a.y * a.y), im = 2.0 * a.x * a.y; return hypot(re, im); }
+    return demod == SDRB_RE ? a.x : a.y;
+}
+
+__device__ __forceinline__ void seam_sos_step(const double *sos, int nsec, double *st, double &xc)
+{
+    for (int s = 0; s < nsec; s++) {
+        const double b0 = sos[6 * s], b1 = sos[6 * s + 1], b2 = sos[6 * s + 2], a1 = sos[6 * s + 4], a2 = sos[6 * s + 5];
+        const double xn = fma(b0, xc, st[2 * s]);
+        st[2 * s] = fma(b1, xc, -a1 * xn) + st[2 * s + 1];
+        st[2 * s + 1] = fma(b2, xc, -a2 * xn);
+        xc = xn;
+    }
+}
+
+// warp <-> (emitted chunk, row), lane <-> segment of Lseg = M/32 outputs.  Without an output
+// filter the demodulated values are framed and stored; with it each lane runs the DF2T recurrence
+// over its segment from a zero state, a lane scan (A^Lseg powers) gives every segment its state
+// from the chunk start, the segment is re-run from that state, and the chunk's zero-state end
+// state goes to echunk.  The response to the state carried from earlier chunks is k_seam_frame's.
+__global__ void __launch_bounds__(256)
+k_seam_demod(const __grid_constant__ DevPlan pl, SeamDev sd, double *out, int ne, int nwin, int end)
+{
+    const int lane = threadIdx.x & 31;
+    const long item = (long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (item >= (long)ne * pl.R) return;
+    const int i = (int)(item / pl.R), r = (int)(item % pl.R), M = pl.M, Ls = pl.sos_Lseg;
+    const bool last = end && i == nwin - 1;
+    const double2 *y = sd.ybuf + ((size_t)i * pl.R + r) * (M + 1);
+    double *o = out + (size_t)r * ne * M + (size_t)i * M;
+    if (pl.nsec_out == 0) {
+        for (int k = lane; k < M; k += 32) {
+            const double v = seam_demod_at(y, k, M, last, pl.demod);
+            o[k] = pl.be_out ? bswap_double(v) : v;
+        }
+        return;
+    }
+    const int lo = lane * Ls;
+    double st[SEAM_NS] = {0.0, 0.0, 0.0, 0.0};
+    for (int k = lo; k < lo + Ls; k++) {
+        double x = seam_demod_at(y, k, M, last, pl.demod);
+        o[k] = x;
+        seam_sos_step(pl.out_sos, pl.nsec_out, st, x);
+    }
+    // inclusive lane scan of the segment end states: S_g = sum_{h<=g} AL^(g-h) e_h
+#pragma unroll
+    for (int lv = 0; lv < 5; lv++) {
+        double pv[SEAM_NS];
+#pragma unroll
+        for (int j = 0; j < SEAM_NS; j++) pv[j] = __shfl_up_sync(0xffffffffu, st[j], 1 << lv);
+        if (lane >= (1 << lv)) {
+            const double *Ap = pl.sos_AP + lv * 16;
+#pragma unroll
+            for (int a = 0; a < SEAM_NS; a++) {
+                double acc = st[a];
+#pragma unroll
+                for (int b = 0; b < SEAM_NS; b++) acc = fma(Ap[a * 4 + b], pv[b], acc);
+                st[a] = acc;
+            }
+        }
+    }
+    double sin_[SEAM_NS];
+#pragma unroll
+    for (int j = 0; j < SEAM_NS; j++) {
+        sin_[j] = __shfl_up_sync(0xffffffffu, st[j], 1);
+        if (lane == 0) sin_[j] = 0.0;
+    }
+    if (lane == 31)
+        for (int j = 0; j < SEAM_NS; j++) sd.echunk[((size_t)i * pl.R + r) * SEAM_NS + j] = st[j];
+    for (int k = lo; k < lo + Ls; k++) {
+        double x = o[k];
+        seam_sos_step(pl.out_sos, pl.nsec_out, sin_, x);
+        o[k] = x;
+    }
+}
+
+// one warp per row, lane <-> contiguous run of chunks: sst[c] = SOS state at the start of emitted
+// chunk c, s[c+1] = A^M s[c] + echunk[c], from the handle's state; the new state back into it
+__global__ void __launch_bounds__(32)
+k_seam_sscan(const __grid_constant__ DevPlan pl, SeamDev sd, int ne)
+{
+    const int r = blockIdx.x, lane = threadIdx.x;
+    const int per = (ne + 31) / 32;
+    const int c0 = min(ne, lane * per), c1 = min(ne, c0 + per);
+    double a[SEAM_NS] = {0.0, 0.0, 0.0, 0.0};
+    double mm[SEAM_NS * SEAM_NS];
+#pragma unroll
+    for (int j = 0; j < SEAM_NS * SEAM_NS; j++) mm[j] = (j % (SEAM_NS + 1)) == 0 ? 1.0 : 0.0;
+    auto matvec = [&](const double *A, const double *x, double *yv) {
+#pragma unroll
+        for (int p = 0; p < SEAM_NS; p++) {
+            double acc = 0.0;
+#pragma unroll
+            for (int q = 0; q < SEAM_NS; q++) acc = fma(A[p * SEAM_NS + q], x[q], acc);
+            yv[p] = acc;
+        }
+    };
+    auto matmul = [&](const double *A, const double *B, double *C) {     // C = A B
+#pragma unroll
+        for (int p = 0; p < SEAM_NS; p++)
+#pragma unroll
+            for (int q = 0; q < SEAM_NS; q++) {
+                double acc = 0.0;
+#pragma unroll
+                for (int k = 0; k < SEAM_NS; k++) acc = fma(A[p * SEAM_NS + k], B[k * SEAM_NS + q], acc);
+                C[p * SEAM_NS + q] = acc;
+            }
+    };
+    for (int c = c0; c < c1; c++) {
+        double t[SEAM_NS], t2[SEAM_NS * SEAM_NS];
+        matvec(sd.AM, a, t);
+        for (int j = 0; j < SEAM_NS; j++) a[j] = t[j] + sd.echunk[((size_t)c * pl.R + r) * SEAM_NS + j];
+        matmul(sd.AM, mm, t2);
+        for (int j = 0; j < SEAM_NS * SEAM_NS; j++) mm[j] = t2[j];
+    }
+#pragma unroll
+    for (int lv = 0; lv < 5; lv++) {
+        double pa[SEAM_NS], pm[SEAM_NS * SEAM_NS];
+#pragma unroll
+        for (int j = 0; j < SEAM_NS; j++) pa[j] = __shfl_up_sync(0xffffffffu, a[j], 1 << lv);
+#pragma unroll
+        for (int j = 0; j < SEAM_NS * SEAM_NS; j++) pm[j] = __shfl_up_sync(0xffffffffu, mm[j], 1 << lv);
+        if (lane >= (1 << lv)) {
+            double t[SEAM_NS], t2[SEAM_NS * SEAM_NS];
+            matvec(mm, pa, t);
+            for (int j = 0; j < SEAM_NS; j++) a[j] += t[j];
+            matmul(mm, pm, t2);
+            for (int j = 0; j < SEAM_NS * SEAM_NS; j++) mm[j] = t2[j];
+        }
+    }
+    double st0[SEAM_NS], ea[SEAM_NS], em[SEAM_NS * SEAM_NS];
+    for (int j = 0; j < SEAM_NS; j++) st0[j] = sd.sos[(size_t)r * SEAM_NS + j];
+#pragma unroll
+    for (int j = 0; j < SEAM_NS; j++) ea[j] = __shfl_up_sync(0xffffffffu, a[j], 1);
+#pragma unroll
+    for (int j = 0; j < SEAM_NS * SEAM_NS; j++) em[j] = __shfl_up_sync(0xffffffffu, mm[j], 1);
+    if (lane == 0) {
+        for (int j = 0; j < SEAM_NS; j++) ea[j] = 0.0;
+        for (int j = 0; j < SEAM_NS * SEAM_NS; j++) em[j] = (j % (SEAM_NS + 1)) == 0 ? 1.0 : 0.0;
+    }
+    double s[SEAM_NS];
+    matvec(em, st0, s);
+    for (int j = 0; j < SEAM_NS; j++) s[j] += ea[j];
+    for (int c = c0; c < c1; c++) {
+        double t[SEAM_NS];
+        for (int j = 0; j < SEAM_NS; j++) sd.sst[((size_t)c * pl.R + r) * SEAM_NS + j] = s[j];
+        matvec(sd.AM, s, t);
+        for (int j = 0; j < SEAM_NS; j++) s[j] = t[j] + sd.echunk[((size_t)c * pl.R + r) * SEAM_NS + j];
+    }
+    if (lane == 31) {
+        double t[SEAM_NS];
+        matvec(mm, st0, t);
+        for (int j = 0; j < SEAM_NS; j++) sd.sos[(size_t)r * SEAM_NS + j] = t[j] + a[j];
+    }
+}
+
+// thread <-> output: out += c A^k s[chunk], then framing
+__global__ void __launch_bounds__(256)
+k_seam_frame(const __grid_constant__ DevPlan pl, SeamDev sd, double *out, int ne)
+{
+    const size_t M = pl.M, total = (size_t)pl.R * ne * M;
+    for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (size_t)gridDim.x * blockDim.x) {
+        const size_t r = e / ((size_t)ne * M), rest = e % ((size_t)ne * M), i = rest / M, k = rest % M;
+        const double *s = sd.sst + (i * pl.R + r) * SEAM_NS;
+        const double *ca = sd.CAM + k * SEAM_NS;
+        double v = out[e];
+#pragma unroll
+        for (int j = 0; j < SEAM_NS; j++) v = fma(ca[j], s[j], v);
+        out[e] = pl.be_out ? bswap_double(v) : v;
+    }
+}

@@ -83,6 +83,12 @@ class DspProcessor(DataProcessor):
         self._correctIq = bool(kwargs.get('correctIq', False))
         self._normalize = bool(kwargs.get('normalize', False))
         self._device = int(kwargs.get('device', 0))
+        # seamless streaming (not a reference option, DESIGN.md section 11): the stream is filtered
+        # and demodulated as one signal instead of chunk by chunk
+        self._seamless = bool(kwargs.get('seamless', False))
+        if self._seamless and smooth:
+            raise ValueError('--smooth-output is per-chunk Savitzky-Golay by definition: not available with '
+                             '--seamless')
         self._engine = None
 
     # ---------------------------------------------------------------- properties (:78-103)
@@ -186,7 +192,8 @@ class DspProcessor(DataProcessor):
             chunk_bytes = 131072 if nb % 131072 == 0 else nb     # the reader may hand over several chunks at once
         plan, tc = cached_plan(self.__fs, enc, self._decimationFactor, self._rowsHz(), simo=self._simo(),
                                swap=swap, correct_iq=ciq, normalize=norm, demod=self._demodName(),
-                               omega_out=self.omegaOut, chunk_bytes=chunk_bytes)
+                               omega_out=self.omegaOut, chunk_bytes=chunk_bytes,
+                               **({'seamless': True} if self._seamless else {}))
         self._chunkBytes = chunk_bytes
         # --smooth-output (dsp_processor.py:159-160): standard mode only, the SIMO override of
         # _transformData never smooths (vfo_processor.py:80-84)
@@ -219,6 +226,8 @@ class DspProcessor(DataProcessor):
         into the other pinned buffer and frames / writes the output of batch i-1 (sdrb_wait).
         A batch is whatever the queue holds (at most MAX_BATCH chunks), so a live stream is not
         held back waiting for a full batch."""
+        if self._seamless:
+            return self._processSeamless(isDead, buffer, file)
         eof = False
         pending = None                                   # (slot, nchunks) in flight
         b = 0
@@ -292,6 +301,44 @@ class DspProcessor(DataProcessor):
             b += 1
         return pending, b
 
+    def _processSeamless(self, isDead, buffer, file) -> None:
+        """The consumer loop of the seamless mode, synchronous: every batch goes through
+        ``Engine.stream`` (which emits the chunks that have become final), and at end of stream or on
+        halt ``Engine.stream_end`` emits the chunks still held back, so no tail is lost."""
+        eof = False
+        pool = self._inputPool
+        while not (self._isDead or isDead.value or eof):
+            first = self._next(isDead, buffer)
+            if first is None:
+                break
+            batch = [first]
+            have = self._itemChunks(first)
+            while have < self.MAX_BATCH:
+                try:
+                    batch.append(buffer.get_nowait())
+                except _queue.Empty:
+                    break
+                have += self._itemChunks(batch[-1])
+            for c in batch:
+                if c is None or len(c) == 0:
+                    eof = True
+                    break
+                if self._engine is None:
+                    self._engine = self._makeEngine(c)
+                a = self._asBytes(c)
+                if a.size % self._chunkBytes:
+                    raise ValueError('queue items must be whole chunks of the size of the first one')
+                out = self._engine.stream(a)
+                home = pool.owner(a) if pool is not None else None
+                if home is not None:
+                    pool.release(home)                   # stream() has copied the bytes to the device
+                if out.shape[1]:
+                    self._emit(out, out.shape[1] // self._engine.M, file)
+        if self._engine is not None:
+            out = self._engine.stream_end()
+            if out.shape[1]:
+                self._emit(out, out.shape[1] // self._engine.M, file)
+
     def useInputPool(self, pool) -> None:
         """Queue items that are views of ``pool``'s buffers (misc.read_file.ChunkPool) are sent to
         the device from where they lie and handed back to the pool afterwards."""
@@ -358,6 +405,8 @@ class DspProcessor(DataProcessor):
             d['encoding'] = str(self.__fileInfo.get('bitsPerSample'))
         d['fs'] = self.__fs
         d['decimatedFs'] = self.__decimatedFs
+        if self._seamless:
+            d['seamless'] = True
         return dumps(d, indent=2, default=str)
 
     def __str__(self):

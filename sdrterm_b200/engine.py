@@ -42,6 +42,11 @@ class Engine:
         cfg.max_chunks = self.max_chunks
         cfg.iq_L = pl.Liq
         cfg.norm_xmin, cfg.norm_k = pl.norm if pl.norm is not None else (0.0, 0.0)
+        self.seamless = bool(getattr(pl, 'seamless', False))
+        cfg.seamless = int(self.seamless)
+        if self.seamless and smooth:
+            raise ValueError('--smooth-output is per-chunk Savitzky-Golay by definition: not available in '
+                             'seamless mode')
         tab = nat.Tables()
 
         def put(name, arr):
@@ -80,6 +85,15 @@ class Engine:
         tab.lam_tile[0], tab.lam_tile[1] = float(pl.lam_tile[0]), float(pl.lam_tile[1])
         if pl.fm_interp is not None:
             put('fm_interp', pl.fm_interp)
+        if self.seamless:
+            tab.lookahead, tab.fs = int(pl.lookahead), int(pl.fs)
+            step = np.ascontiguousarray(pl.chunk_step, dtype=np.int64)
+            self._keep.append(step)
+            tab.chunk_step = step.ctypes.data_as(C.POINTER(C.c_int64))
+            put('PN', pl.PN)
+            if pl.sos_AM is not None:
+                put('sos_AM', pl.sos_AM)
+                put('sos_CAM', pl.sos_CAM)
         # tc: prebuilt tensor-core tables (plan.cached_plan), or 'build'
         self.tc = (build_tc_or_none(pl) if isinstance(tc, str) else tc) if use_tc else None
         if self.tc is not None:
@@ -137,6 +151,8 @@ class Engine:
         buf = np.frombuffer(raw, dtype=np.uint8) if not isinstance(raw, np.ndarray) else raw
         buf = np.ascontiguousarray(buf).view(np.uint8).reshape(-1)
         n = self._nchunks(buf.size)
+        if self.seamless:
+            raise nat.SdrbError('seamless engine: use stream() / stream_end()')
         dt = np.dtype('>f8') if self.plan.big_endian_out else np.dtype('=f8')
         if out is None:
             out = np.empty((self.R, n * self.M), dtype=dt)
@@ -144,12 +160,70 @@ class Engine:
             nat.check(nat.lib().sdrb_process(self._h, buf.ctypes.data, n, out.ctypes.data), self._h)
         return out
 
+    # ------------------------------------------------------------------ seamless streaming
+    @property
+    def lookahead(self) -> int:
+        """D: in seamless mode a chunk's output is final once the D chunks after it exist."""
+        return int(nat.lib().sdrb_stream_lookahead(self._h)) if self.seamless else 0
+
+    def _out_array(self, nchunks: int) -> np.ndarray:
+        dt = np.dtype('>f8') if self.plan.big_endian_out else np.dtype('=f8')
+        return np.empty(self.R * nchunks * self.M, dtype=dt)
+
+    def _rows(self, flat: np.ndarray, k: int) -> np.ndarray:
+        return flat[:self.R * k * self.M].reshape(self.R, k * self.M)
+
+    def stream(self, raw) -> np.ndarray:
+        """Seamless mode: take whole chunks of the stream, return (R, k*M) for the k chunks that have
+        become final (the stream is filtered as one signal; see DESIGN.md section 11).  Batches
+        larger than ``max_chunks`` are fed in pieces."""
+        if not self.seamless:
+            raise nat.SdrbError('stream() needs a plan built with seamless=True')
+        buf = np.frombuffer(raw, dtype=np.uint8) if not isinstance(raw, np.ndarray) else raw
+        buf = np.ascontiguousarray(buf).view(np.uint8).reshape(-1)
+        n = self._nchunks(buf.size)
+        parts = []
+        for c0 in range(0, n, self.max_chunks):
+            k = min(self.max_chunks, n - c0)
+            out = self._out_array(k + self.lookahead)
+            got = C.c_size_t(0)
+            nat.check(nat.lib().sdrb_stream(self._h, buf[c0 * self.chunk_bytes:].ctypes.data, k, out.ctypes.data,
+                                            C.byref(got)), self._h)
+            parts.append(self._rows(out, got.value))
+        if not parts:
+            return self._rows(self._out_array(0), 0)
+        return np.concatenate(parts, axis=1) if len(parts) > 1 else parts[0]
+
+    def stream_end(self) -> np.ndarray:
+        """Seamless mode: end of stream.  Returns the chunks still held back, filtered with the stream's
+        real end as the boundary, and resets the stream (IQ corrector included)."""
+        if not self.seamless:
+            raise nat.SdrbError('stream_end() needs a plan built with seamless=True')
+        out = self._out_array(max(1, self.lookahead))
+        got = C.c_size_t(0)
+        nat.check(nat.lib().sdrb_stream_end(self._h, out.ctypes.data, C.byref(got)), self._h)
+        return self._rows(out, got.value)
+
+    def stream_device(self, raw_ptr: int, nchunks: int, out_ptr: int, stream: int = 0) -> int:
+        """Device pointers in/out, only enqueued on ``stream``; returns the number of chunks emitted."""
+        got = C.c_size_t(0)
+        nat.check(nat.lib().sdrb_stream_device(self._h, raw_ptr, nchunks, out_ptr, stream, C.byref(got)), self._h)
+        return got.value
+
+    def stream_end_device(self, out_ptr: int, stream: int = 0) -> int:
+        got = C.c_size_t(0)
+        nat.check(nat.lib().sdrb_stream_end_device(self._h, out_ptr, stream, C.byref(got)), self._h)
+        return got.value
+
     def set_smooth(self, window: int, polyorder: int = 3) -> None:
         """``--smooth-output``: ``scipy.signal.savgol_filter(z, window, 3)`` on every chunk's output
         row (reference dsp_processor.py:159-160), as one linear map per chunk: the interior FIR row
         and the two polynomial edge fits (mode='interp'), taken from SciPy itself applied to the
         identity so that the coefficients are the reference's."""
         from scipy.signal import savgol_filter
+        if self.seamless:
+            raise ValueError('--smooth-output is per-chunk Savitzky-Golay by definition: not available in '
+                             'seamless mode')
         w = int(window)
         if w > self.M:
             raise ValueError(f'smoothing window {w} longer than a chunk\'s {self.M} outputs')

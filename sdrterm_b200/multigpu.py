@@ -48,11 +48,18 @@ def bind_to_gpu_numa_node(device: int) -> bool:
         return False
 
 
+SEAMLESS_REFUSAL = ('seamless mode is single-GPU: time segments would need a halo of D chunks (the '
+                    'lookahead) and a hand-off of the forward filter state between ranks, which is not '
+                    'built yet')
+
+
 class TimeShardedChain:
     """One rank's share of a time-segment sharded stream.  ``step`` processes one device-resident
     segment of ``nchunks`` chunks; with world == 1 it is a plain ``process_device``."""
 
     def __init__(self, plan: Plan, max_chunks: int, device: int, dist=None, torch=None):
+        if getattr(plan, 'seamless', False):
+            raise ValueError(SEAMLESS_REFUSAL)
         self.plan, self.dist, self.torch = plan, dist, torch
         self.world = dist.get_world_size() if dist is not None else 1
         self.rank = dist.get_rank() if dist is not None else 0
@@ -186,6 +193,8 @@ class RowShardedBank:
 
     def __init__(self, fs: int, enc: str, dec: int, rows_hz, max_chunks: int, device: int, dist=None, torch=None,
                  min_rows: int | None = None, **plan_kw):
+        if plan_kw.get('seamless'):
+            raise ValueError(SEAMLESS_REFUSAL)
         self.dist, self.torch = dist, torch
         self.world = dist.get_world_size() if dist is not None else 1
         self.rank = dist.get_rank() if dist is not None else 0
@@ -289,14 +298,17 @@ class RowShardedBank:
 def run_file_sharded(path: str, out_path: str | None, *, fs: int, enc: str, dec: int, center: int = 0,
                      demod: str = 'fm', omega_out: int = 12500, correct_iq: bool = False, swap: bool = False,
                      data_offset: int = 0, batch_chunks: int = 2048, device: int | None = None, dist=None,
-                     torch=None) -> np.ndarray | None:
+                     torch=None, seamless: bool = False) -> np.ndarray | None:
     """BASELINE config 5: an offline IQ file, time-segment sharded over the ranks of ``dist``
     (``None`` = single process).  Every rank reads ITS segment of the file (whole 131072-byte
     chunks counted from ``data_offset``; the reference's stale-tail chunk, SURVEY 8-Q5, belongs to
     the last rank), runs an IQ-gain pre-pass over it when ``correct_iq`` (raw bytes only, no
     outputs), exchanges the gains, then demodulates its segment batch by batch through the
     double-buffered host path.  Rank r writes ``out_path + '.part%04d' % r`` (or returns the array
-    when ``out_path`` is None): the concatenation in rank order is the reference's output file."""
+    when ``out_path`` is None): the concatenation in rank order is the reference's output file.
+    ``seamless=True`` is refused (ValueError): see SEAMLESS_REFUSAL."""
+    if seamless:
+        raise ValueError(SEAMLESS_REFUSAL)
     if torch is None:
         import torch as _t
         torch = _t

@@ -218,6 +218,13 @@ class Plan:
     sos_AL: np.ndarray | None = None      # (ns, ns) A^Lseg of the output cascade (ns = 2*sections)
     sos_CA: np.ndarray | None = None      # (Lseg, ns) c A^i
     sos_AP: np.ndarray | None = None      # (5, ns, ns) (A^Lseg)^(2^lv)
+    # seamless streaming (DESIGN.md section 11): the whole stream is filtered, not each chunk
+    seamless: bool = False
+    lookahead: int = 0                    # D: chunk c is final once chunks c+1 .. c+D exist
+    chunk_step: np.ndarray | None = None  # (R,) int64: (f_r * N) mod fs, NCO phase step per chunk
+    PN: np.ndarray | None = None          # (D+1, 8) p_i^(N j): a modal state moved j whole chunks
+    sos_AM: np.ndarray | None = None      # (ns, ns) A^M of the output cascade: its state moved one chunk
+    sos_CAM: np.ndarray | None = None     # (M, ns) c A^i, i < M
 
     @property
     def chunk_bytes(self) -> int:
@@ -230,10 +237,28 @@ def reference_w(f_hz: int, fs: int) -> float:
     return float((-2j * np.pi * (f_hz / fs)).imag)
 
 
+LOOKAHEAD_TOL = 1e-13     # truncated anticausal tail of the seamless mode, relative to the input scale
+
+
+def lookahead_bound(p, rho_p, N: int, D: int) -> float:
+    """sum_i |rho_i/p_i| |p_i|^(D N) / (1 - |p_i|): what the anticausal modes of the samples after
+    chunk c+D can still add to an output of chunk c, per unit of input magnitude."""
+    a = np.abs(np.asarray(p))
+    return float(np.sum(np.abs(np.asarray(rho_p)) * a ** (D * N) / (1 - a)))
+
+
+def lookahead_chunks(p, rho_p, N: int, tol: float = LOOKAHEAD_TOL) -> int:
+    """Smallest D >= 1 whose truncation bound is <= tol."""
+    D = 1
+    while lookahead_bound(p, rho_p, N, D) > tol:
+        D += 1
+    return D
+
+
 def build_plan(fs: int, enc: str, dec: int, rows_hz, *, simo: bool = False, swap: bool = False,
                correct_iq: bool = False, normalize: bool = False, impedance: int = 50,
                demod: str = 'fm', omega_out: int = 12500, chunk_bytes: int = CHUNK_BYTES,
-               big_endian_out: bool | None = None) -> Plan:
+               big_endian_out: bool | None = None, seamless: bool = False) -> Plan:
     _heavy()
     if dec < 2:
         raise ValueError('Decimation must be at least 2.')
@@ -241,6 +266,9 @@ def build_plan(fs: int, enc: str, dec: int, rows_hz, *, simo: bool = False, swap
         raise ValueError(f'unknown encoding {enc!r}')
     q = int(dec)
     N = chunk_bytes // (2 * _ITEMSIZE[enc])
+    if seamless and N % q:
+        raise ValueError(f'seamless mode needs the decimation to divide the {N} samples of a chunk '
+                         f'(-d {q} leaves a ragged block); use a power of two')
     sos = np.ascontiguousarray(_sig.cheby1(8, 0.05, 0.8 / q, output='sos'), dtype=np.float64)
     zi = np.ascontiguousarray(_sig.sosfilt_zi(sos), dtype=np.float64)
     nsec = sos.shape[0]
@@ -382,6 +410,31 @@ def build_plan(fs: int, enc: str, dec: int, rows_hz, *, simo: bool = False, swap
         for lv in range(5):
             sos_AP[lv] = [[float(Apw[i, j]) for j in range(ns)] for i in range(ns)]
             Apw = Apw * Apw
+    sm = {}
+    if seamless:
+        D = lookahead_chunks(modes.p, modes.rho_p, N)
+        sm['lookahead'] = D
+        sm['chunk_step'] = np.array([(f * N) % fs if use_nco[r] else 0 for r, f in enumerate(rows_hz)],
+                                    dtype=np.int64)
+        sm['PN'] = np.array([[_c(pm[i] ** (N * j)) for i in range(n8)] for j in range(D + 1)])
+        if out_sos is not None:
+            mp.mp.dps = 40
+            A_, b_, c_, d_ = _cascade_state_space(out_sos)
+            ns = A_.rows
+            AM = A_ ** M
+            sm['sos_AM'] = np.array([[float(AM[i, j]) for j in range(ns)] for i in range(ns)])
+            # c A^i for i < M: the response of every output of a chunk to the state it starts from
+            Af = np.array([[float(A_[i, j]) for j in range(ns)] for i in range(ns)])
+            cam = np.zeros((M, ns))
+            cur = np.array([float(c_[0, j]) for j in range(ns)])
+            blk = sos_Lseg
+            for i in range(M):
+                if i % blk == 0:           # restart from the exact power every segment
+                    cm = c_ * (A_ ** i)
+                    cur = np.array([float(cm[0, j]) for j in range(ns)])
+                cam[i] = cur
+                cur = cur @ Af
+            sm['sos_CAM'] = cam
     fm_interp = None
     h = M >> 1
     if demod == 'fm' and not (M == 2 * h and h & (h - 1) == 0):
@@ -395,7 +448,8 @@ def build_plan(fs: int, enc: str, dec: int, rows_hz, *, simo: bool = False, swap
                 ws=ws, nend=nend, alpha=alpha, beta=beta, alphaT=alphaT, betaT=betaT, gamma=gamma, phE=phE, psiY=psiY,
                 lam_tile=lam_tile, demod=demod, out_sos=out_sos,
                 big_endian_out=bool(simo if big_endian_out is None else big_endian_out),
-                fm_interp=fm_interp, sos_Lseg=sos_Lseg, sos_AL=sos_AL, sos_CA=sos_CA, sos_AP=sos_AP)
+                fm_interp=fm_interp, sos_Lseg=sos_Lseg, sos_AL=sos_AL, sos_CA=sos_CA, sos_AP=sos_AP,
+                seamless=bool(seamless), **sm)
 
 
 # ------------------------------------------------------------------------------------------------

@@ -43,6 +43,11 @@ def buildParser() -> argparse.ArgumentParser:
     ap.add_argument('--smooth-output', dest='smooth_output', type=int, default=0)
     ap.add_argument('--vfo-host', dest='vfo_host', default='localhost')
     ap.add_argument('--swap-input-endianness', '-X', dest='swap', action='store_true')
+    ap.add_argument('--seamless', dest='seamless', action='store_true',
+                    help='not a reference option: filter and demodulate the whole stream as one signal '
+                         'instead of each 131072-byte chunk (no transient at chunk edges; output '
+                         'delayed by a few chunks; needs a power-of-two -d; no --smooth-output)')
+    ap.add_argument('--no-seamless', dest='seamless', action='store_false')
     ap.add_argument('--normalize-input', dest='normalize', action='store_true')
     ap.add_argument('--no-normalize-input', dest='normalize', action='store_false')
     return ap
@@ -56,6 +61,8 @@ def makeProcessor(a, fileInfo):
         raise ValueError('Decimation must be at least 2.')
     kw = dict(center=a.center, omegaOut=a.omegaOut, tuned=a.tuned, dec=a.dec, smooth=a.smooth_output,
               fileInfo=fileInfo, swapEndianness=a.swap, correctIq=a.correct_iq, normalize=a.normalize)
+    if a.seamless:
+        kw['seamless'] = True
     fs = fileInfo['sampRate']
     proc = VfoProcessor(fs, vfoHost=a.vfo_host, vfos=a.vfos, **kw) if a.simo else DspProcessor(fs, **kw)
     {'fm': proc.selectOutputFm, 'nfm': proc.selectOutputFm, 'am': proc.selectOutputAm,
