@@ -18,7 +18,7 @@
 extern "C" {
 #endif
 
-#define SDRB_ABI_VERSION 7
+#define SDRB_ABI_VERSION 8
 #define SDRB_TILE_BLOCKS 32
 #define SDRB_NPOLES 8
 #define SDRB_MAX_DECIMATION 256
@@ -31,7 +31,9 @@ enum sdrb_status {
     SDRB_ERR_STATE = -4
 };
 
-enum sdrb_demod { SDRB_FM = 0, SDRB_AM = 1, SDRB_RE = 2, SDRB_IM = 3 };
+/* SDRB_IQ is not a reference mode: the complex decimator output y itself, 2 doubles (Re, Im) per
+ * output, no output low-pass (n_out_sections 0), no --smooth-output. */
+enum sdrb_demod { SDRB_FM = 0, SDRB_AM = 1, SDRB_RE = 2, SDRB_IM = 3, SDRB_IQ = 4 };
 
 /* Geometry and switches of one processor.  Mirrors the keyword arguments that
  * src/misc/io_args.py:97-141 passes to DspProcessor/VfoProcessor and to readFile
@@ -55,7 +57,7 @@ typedef struct sdrb_config {
     int32_t N;               /* complex samples per chunk = 131072 / (2*itemsize) */
     int32_t edge;            /* sosfiltfilt pad length (27) */
     int32_t R;               /* rows: 1, or K+1 in --simo (vfo_processor.py:42-47) */
-    int32_t n_out_sections;  /* output low-pass SOS sections (0 for re/im) */
+    int32_t n_out_sections;  /* output low-pass SOS sections (0 for re/im/iq) */
     int32_t max_chunks;      /* largest number of chunks one sdrb_process* call will carry */
     double iq_L;             /* impedance / fs (read_file.py:65) */
     double norm_xmin;        /* read_file.py:177-196 */
@@ -140,16 +142,18 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
 int sdrb_destroy(sdrb_handle *h);
 const char *sdrb_last_error(const sdrb_handle *h);
 
-/* Geometry derived from the config: outputs per chunk-row M = ceil(N/q), bytes per chunk. */
+/* Geometry derived from the config: outputs per chunk-row M = ceil(N/q), bytes per chunk, and the
+ * doubles per chunk-row of the output buffers W (2M for SDRB_IQ: (Re, Im) interleaved, M otherwise). */
 int sdrb_outputs_per_chunk(const sdrb_handle *h);
 size_t sdrb_chunk_bytes(const sdrb_handle *h);
+int sdrb_row_doubles(const sdrb_handle *h);
 
 /* The hot path: feedBuffers' decode/normalise/IQ-correct (src/misc/read_file.py:100-103) +
  * DspProcessor._processChunk (src/dsp/dsp_processor.py:140-149) + framing (:162,
  * vfo_processor.py:84) over `nchunks` whole chunks.
  *   raw : nchunks * chunk_bytes bytes
- *   out : R * nchunks * M doubles, row-major [row][chunk][M] (each row is one output stream);
- *         byte-swapped to big-endian when cfg.big_endian_out
+ *   out : R * nchunks * W doubles, row-major [row][chunk][W] (each row is one output stream; W =
+ *         sdrb_row_doubles); byte-swapped to big-endian when cfg.big_endian_out
  * sdrb_process takes HOST buffers (pinned or pageable) and includes H2D/D2H; it returns after
  * the results are in `out`.  sdrb_process_device takes DEVICE buffers and only enqueues work on
  * `stream` (a cudaStream_t, may be NULL). */
@@ -181,7 +185,7 @@ int sdrb_iq_prefix_device(sdrb_handle *h, const double *gains3_dev, int rank, vo
  * M-ntail..M-1 = tail rows applied to the last `window` samples, every other output k = the FIR row
  * applied to samples k+lo .. k+lo+window-1.  `tab` is [nhead + 1 + ntail][window] doubles (head rows,
  * FIR row, tail rows); window 0 switches smoothing off.  Native-endian output only (the SIMO path of
- * the reference never smooths). */
+ * the reference never smooths).  SDRB_IQ output is never smoothed: SDRB_ERR_ARG. */
 int sdrb_set_smooth(sdrb_handle *h, int window, int nhead, int ntail, int lo, const double *tab);
 
 /* Pre-pass of time-segment sharding for segments longer than one batch: advance the IQ state over
@@ -196,7 +200,8 @@ int sdrb_set_profiling(sdrb_handle *h, int on);
 int sdrb_kernel_times(sdrb_handle *h, float ms[4]);
 
 /* Double-buffered streaming from pinned host memory: sdrb_submit enqueues H2D + kernels + D2H for
- * one batch on slot (0 or 1) and returns; sdrb_wait blocks until that slot's `out` is complete.
+ * one batch on slot (0 or 1) and returns; sdrb_wait blocks until that slot's `out` (R * nchunks * W
+ * doubles, laid out as for sdrb_process) is complete.
  * Batches must be submitted in stream order; the IQ-corrector state chains through them. */
 int sdrb_submit(sdrb_handle *h, int slot, const void *raw_host, size_t nchunks, double *out_host);
 int sdrb_wait(sdrb_handle *h, int slot);
@@ -234,11 +239,13 @@ long long sdrb_launch_count(const sdrb_handle *h);
  *   sdrb_fm_demod   fmDemod(data(R,M) c128, out(R,M) f64)        demodulation.py:25-38
  *   sdrb_am_demod   amDemod                                       demodulation.py:41-48
  *   sdrb_real_output / sdrb_imag_output                           demodulation.py:51-68
+ *   sdrb_iq_output  y(R,M) c128 -> out(R,2M) f64, (Re, Im) interleaved (not a reference operator)
  *   sdrb_shift_freq shiftFreq(y(N), shift(R,N), res(R,N))         demodulation.py:71-79 */
 int sdrb_fm_demod(int device, const double *y, int R, int M, double *out);
 int sdrb_am_demod(int device, const double *y, int R, int M, double *out);
 int sdrb_real_output(int device, const double *y, int R, int M, double *out);
 int sdrb_imag_output(int device, const double *y, int R, int M, double *out);
+int sdrb_iq_output(int device, const double *y, int R, int M, double *out);
 int sdrb_shift_freq(int device, const double *y, const double *shift, int R, int N, double *res);
 /* sdrb_fm_demod takes any even row length: 2*2^k rows run the FFT interpolation, other lengths a
  * dense scipy.signal.resample matrix built on the host in extended precision. */
@@ -278,10 +285,11 @@ int sdrb_read_x0(sdrb_handle *h, size_t nchunks, double *x0_host);
  * scipy.signal.decimate / sosfilt would treat the concatenated stream: the NCO phase runs on across
  * chunks, the decimator's zero-phase filter sees the stream's two real ends only, the fm
  * discriminator and the output low-pass carry their state.  The framing per chunk is unchanged
- * (M doubles per chunk and row, [row][chunk][M], big-endian when cfg.big_endian_out).
+ * (W doubles per chunk and row, [row][chunk][W], big-endian when cfg.big_endian_out).
  *   sdrb_stream         host `raw` of nchunks whole chunks in; emits every chunk that has become final
  *                       (a chunk is final once the lookahead D chunks after it exist), synchronously,
- *                       into host `out` (room for nchunks + D chunks); *nchunks_out = chunks emitted
+ *                       into host `out` (room for nchunks + D chunks of R * W doubles each);
+ *                       *nchunks_out = chunks emitted
  *   sdrb_stream_device  the same on device buffers, only enqueued on `stream` (`out_dev`: room for
  *                       nchunks chunks)
  *   sdrb_stream_end     end of stream: emits the chunks still held back, with the stream's real end

@@ -17,9 +17,9 @@ HEADER = os.path.join(ROOT, 'include', 'sdrterm_b200.h')
 SOURCES = [os.path.join(_HERE, 'csrc', f) for f in ('sdrb_api.cu', 'sdrb_kernels.cuh', 'sdrb_device.cuh', 'sdrb_tc.cuh', 'sdrb_finish.cuh',
                                                     'sdrb_spectrum.cuh', 'sdrb_seamless.cuh')]
 
-ABI_VERSION = 7
-FM, AM, RE, IM = 0, 1, 2, 3
-DEMOD_CODE = {'fm': FM, 'am': AM, 're': RE, 'im': IM}
+ABI_VERSION = 8
+FM, AM, RE, IM, IQ = 0, 1, 2, 3, 4
+DEMOD_CODE = {'fm': FM, 'am': AM, 're': RE, 'im': IM, 'iq': IQ}
 
 
 class SdrbError(RuntimeError):
@@ -65,7 +65,8 @@ EXPORTS = ['sdrb_create', 'sdrb_destroy', 'sdrb_last_error', 'sdrb_outputs_per_c
            'sdrb_shift_freq', 'sdrb_power_spectrum', 'sdrb_stft_db', 'sdrb_global_error', 'sdrb_process_device_phases',
            'sdrb_set_profiling', 'sdrb_kernel_times', 'sdrb_keep_decimated', 'sdrb_read_debug', 'sdrb_iq_export_device',
            'sdrb_iq_prefix_device', 'sdrb_decode_iq', 'sdrb_correct_iq', 'sdrb_keep_x0', 'sdrb_read_x0', 'sdrb_iq_gain', 'sdrb_set_smooth', 'sdrb_host_alloc', 'sdrb_host_free', 'sdrb_reserve_sms',
-           'sdrb_stream', 'sdrb_stream_device', 'sdrb_stream_end', 'sdrb_stream_end_device', 'sdrb_stream_lookahead']
+           'sdrb_stream', 'sdrb_stream_device', 'sdrb_stream_end', 'sdrb_stream_end_device', 'sdrb_stream_lookahead',
+           'sdrb_row_doubles', 'sdrb_iq_output']
 
 
 def nvcc_command(out: str = LIB_PATH) -> list[str]:
@@ -103,6 +104,7 @@ def lib():
         L.sdrb_last_error.restype = C.c_char_p
         L.sdrb_global_error.restype = C.c_char_p
         L.sdrb_outputs_per_chunk.argtypes = [vp]
+        L.sdrb_row_doubles.argtypes = [vp]
         L.sdrb_chunk_bytes.argtypes = [vp]
         L.sdrb_chunk_bytes.restype = sz
         L.sdrb_process.argtypes = [vp, vp, sz, vp]
@@ -121,7 +123,7 @@ def lib():
         L.sdrb_iq_prefix_device.argtypes = [vp, vp, C.c_int, vp]
         L.sdrb_launch_count.argtypes = [vp]
         L.sdrb_launch_count.restype = C.c_longlong
-        for name in ('sdrb_fm_demod', 'sdrb_am_demod', 'sdrb_real_output', 'sdrb_imag_output'):
+        for name in ('sdrb_fm_demod', 'sdrb_am_demod', 'sdrb_real_output', 'sdrb_imag_output', 'sdrb_iq_output'):
             getattr(L, name).argtypes = [C.c_int, vp, C.c_int, C.c_int, vp]
         L.sdrb_shift_freq.argtypes = [C.c_int, vp, vp, C.c_int, C.c_int, vp]
         L.sdrb_power_spectrum.argtypes = [C.c_int, vp, vp, C.c_int, C.c_int, vp]

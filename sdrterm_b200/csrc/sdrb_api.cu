@@ -328,8 +328,12 @@ int launch_chain_t(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, 
         const unsigned grid = (unsigned)std::min<size_t>((items + FIN_WARPS - 1) / FIN_WARPS, (size_t)(h->num_sms - h->reserved_sms) * 2);
         // behind the IQ kernels of the same call (or, without IQ correction, behind the front end)
         const bool pdl = h->pdl && ((phases & PH_MAIN) || ((phases & PH_IQSCAN) && IQ));
-        CK(h, launch_pdl(k_finish<ENC>, dim3(grid), dim3(32 * FIN_WARPS), h->finish_smem, st, pdl, pl, h->sc, raw, out,
-                         (int)nch, h->keep_y));
+        if (pl.demod == SDRB_IQ)
+            CK(h, launch_pdl(k_finish<ENC, true>, dim3(grid), dim3(32 * FIN_WARPS), h->finish_smem, st, pdl, pl, h->sc, raw,
+                             out, (int)nch, h->keep_y));
+        else
+            CK(h, launch_pdl(k_finish<ENC, false>, dim3(grid), dim3(32 * FIN_WARPS), h->finish_smem, st, pdl, pl, h->sc, raw,
+                             out, (int)nch, h->keep_y));
         h->launches++;
         mark(3);
         mark(4);
@@ -337,8 +341,12 @@ int launch_chain_t(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, 
         k_fixup<ENC><<<(unsigned)(nch * pl.R), 128, 0, st>>>(pl, h->sc, raw, (int)nch);
         h->launches++;
         mark(3);
-        k_demod<<<(unsigned)(nch * pl.R), 128, h->demod_smem, st>>>(pl, h->sc.y, out, h->sc.fftbuf, h->sc.zrow,
-                                                                    (int)nch, pl.demod, 1, pl.be_out);
+        if (pl.demod == SDRB_IQ)
+            k_demod<true><<<(unsigned)(nch * pl.R), 128, 0, st>>>(pl, h->sc.y, out, nullptr, nullptr, (int)nch, pl.demod, 0,
+                                                                  pl.be_out);
+        else
+            k_demod<false><<<(unsigned)(nch * pl.R), 128, h->demod_smem, st>>>(pl, h->sc.y, out, h->sc.fftbuf, h->sc.zrow,
+                                                                               (int)nch, pl.demod, 1, pl.be_out);
         h->launches++;
         mark(4);
     }
@@ -355,6 +363,8 @@ int launch_chain_t(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, 
 
 int launch_chain(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, cudaStream_t st, int phases = PH_ALL)
 {
+    if ((phases & PH_FINISH) && h->pl.demod == SDRB_IQ && ((uintptr_t)out & 15))
+        return fail(h, SDRB_ERR_ARG, "iq output is stored as 16-byte (Re, Im) pairs: `out` must be 16-byte aligned");
     switch (h->enc_code) {
     case ENC_b: return h->pl.correct_iq ? launch_chain_t<ENC_b, true>(h, raw, nch, out, st, phases) : launch_chain_t<ENC_b, false>(h, raw, nch, out, st, phases);
     case ENC_B: return h->pl.correct_iq ? launch_chain_t<ENC_B, true>(h, raw, nch, out, st, phases) : launch_chain_t<ENC_B, false>(h, raw, nch, out, st, phases);
@@ -374,7 +384,8 @@ int set_smem_attr_t(sdrb_handle *h)
 {
     CK(h, cudaFuncSetAttribute(k_main<ENC, IQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->main_smem));
     if (h->finish_on)
-        CK(h, cudaFuncSetAttribute(k_finish<ENC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->finish_smem));
+        CK(h, cudaFuncSetAttribute(h->pl.demod == SDRB_IQ ? k_finish<ENC, true> : k_finish<ENC, false>,
+                                   cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->finish_smem));
     return 0;
 }
 int set_smem_attr(sdrb_handle *h)
@@ -428,6 +439,9 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
         if (cfg->n_out_sections > 0 && !tab->out_sos) return fail(nullptr, SDRB_ERR_ARG, "out_sos is NULL");
     }
     if (cfg->N / cfg->q < 1) return fail(nullptr, SDRB_ERR_ARG, "chunk shorter than one block");
+    if (cfg->demod > SDRB_IQ) return fail(nullptr, SDRB_ERR_ARG, "unknown demodulation %d", (int)cfg->demod);
+    if (cfg->demod == SDRB_IQ && cfg->n_out_sections != 0)
+        return fail(nullptr, SDRB_ERR_ARG, "iq output has no output low-pass (n_out_sections must be 0)");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
         return fail(nullptr, SDRB_ERR_CUDA, "no CUDA device: libsdrterm_b200 has no CPU fallback");
@@ -447,6 +461,7 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
     pl.normalize = cfg->normalize; pl.demod = cfg->demod; pl.be_out = cfg->big_endian_out;
     pl.q = cfg->q; pl.N = cfg->N; pl.edge = cfg->edge; pl.L = cfg->N + 2 * cfg->edge;
     pl.Mf = cfg->N / cfg->q; pl.rem = cfg->N - pl.Mf * cfg->q; pl.M = pl.Mf + (pl.rem ? 1 : 0);
+    pl.W = cfg->demod == SDRB_IQ ? 2 * pl.M : pl.M;
     pl.ntiles = (pl.Mf + SDRB_TB - 1) / SDRB_TB; pl.cnt_last = pl.Mf - (pl.ntiles - 1) * SDRB_TB;
     pl.Hq = (cfg->q + 1) / 2; pl.KS = (pl.Hq + 3) / 4; pl.R = cfg->R;
     pl.RL = tab->RL;
@@ -593,7 +608,7 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
     pl.demod_in_smem = dsm <= 96 * 1024 ? 1 : 0;
     h->demod_smem = pl.demod_in_smem ? dsm : 0;
     if (h->demod_smem > 48 * 1024)
-        if (cudaFuncSetAttribute(k_demod, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->demod_smem) != cudaSuccess)
+        if (cudaFuncSetAttribute(k_demod<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->demod_smem) != cudaSuccess)
             return bail(fail(h, SDRB_ERR_CUDA, "cudaFuncSetAttribute(k_demod) failed"));
 
     // scratch for max_chunks (seamless: plus the D chunks held back between calls)
@@ -679,6 +694,7 @@ int sdrb_destroy(sdrb_handle *h)
 }
 
 int sdrb_outputs_per_chunk(const sdrb_handle *h) { return h ? h->pl.M : SDRB_ERR_ARG; }
+int sdrb_row_doubles(const sdrb_handle *h) { return h ? h->pl.W : SDRB_ERR_ARG; }
 size_t sdrb_chunk_bytes(const sdrb_handle *h) { return h ? (size_t)h->pl.N * 2 * h->pl.itemsize : 0; }
 long long sdrb_launch_count(const sdrb_handle *h) { return h ? h->launches : 0; }
 
@@ -698,7 +714,7 @@ static int ensure_slot(sdrb_handle *h, int s)
     Slot &sl = h->slot[s];
     if (!sl.raw) CK(h, cudaMalloc(&sl.raw, h->max_chunks * sdrb_chunk_bytes(h)));
     const size_t och = h->max_chunks + (h->seamless ? (size_t)h->sd.D : 0);
-    if (!sl.out) CK(h, cudaMalloc(&sl.out, och * (size_t)h->pl.R * h->pl.M * sizeof(double)));
+    if (!sl.out) CK(h, cudaMalloc(&sl.out, och * (size_t)h->pl.R * h->pl.W * sizeof(double)));
     return 0;
 }
 
@@ -720,7 +736,7 @@ int sdrb_submit(sdrb_handle *h, int s, const void *raw_host, size_t nchunks, dou
     rc = launch_chain(h, sl.raw, nchunks, sl.out, sl.stream);
     if (rc) return rc;
     CK(h, cudaEventRecord(h->iq_done, sl.stream));
-    CK(h, cudaMemcpyAsync(out_host, sl.out, nchunks * (size_t)h->pl.R * h->pl.M * sizeof(double),
+    CK(h, cudaMemcpyAsync(out_host, sl.out, nchunks * (size_t)h->pl.R * h->pl.W * sizeof(double),
                           cudaMemcpyDeviceToHost, sl.stream));
     CK(h, cudaEventRecord(sl.done, sl.stream));
     sl.host_out = out_host; sl.nchunks = nchunks;
@@ -739,24 +755,24 @@ int sdrb_process(sdrb_handle *h, const void *raw, size_t nchunks, double *out)
 {
     if (!h || (!raw && nchunks) || (!out && nchunks)) return fail(h, SDRB_ERR_ARG, "null argument");
     if (h->seamless) return fail(h, SDRB_ERR_STATE, "seamless handle: use sdrb_stream / sdrb_stream_end");
-    const size_t cb = sdrb_chunk_bytes(h), M = (size_t)h->pl.M, R = (size_t)h->pl.R;
+    const size_t cb = sdrb_chunk_bytes(h), W = (size_t)h->pl.W, R = (size_t)h->pl.R;
     if (nchunks <= h->max_chunks) {
         if (nchunks == 0) return SDRB_OK;
         int rc = sdrb_submit(h, 0, raw, nchunks, out);
         if (rc) return rc;
         return sdrb_wait(h, 0);
     }
-    // more chunks than one batch holds: rows of `out` are nchunks*M long, so each batch is staged
+    // more chunks than one batch holds: rows of `out` are nchunks*W long, so each batch is staged
     // through a per-slot buffer and scattered row by row; the two slots alternate, so the H2D of
     // batch i+1 overlaps the kernels of batch i
-    std::vector<double> tmp[2] = {std::vector<double>(h->max_chunks * R * M), std::vector<double>(h->max_chunks * R * M)};
+    std::vector<double> tmp[2] = {std::vector<double>(h->max_chunks * R * W), std::vector<double>(h->max_chunks * R * W)};
     size_t start[2] = {0, 0}, count[2] = {0, 0};
     auto drain = [&](int s) -> int {
         if (!count[s]) return 0;
         int rc = sdrb_wait(h, s);
         if (rc) return rc;
         for (size_t r = 0; r < R; r++)
-            memcpy(out + r * nchunks * M + start[s] * M, tmp[s].data() + r * count[s] * M, count[s] * M * sizeof(double));
+            memcpy(out + r * nchunks * W + start[s] * W, tmp[s].data() + r * count[s] * W, count[s] * W * sizeof(double));
         count[s] = 0;
         return 0;
     };
@@ -903,6 +919,8 @@ int sdrb_stream_device(sdrb_handle *h, const void *raw_dev, size_t nchunks, doub
     if (!h || (!raw_dev && nchunks) || !out_dev) return fail(h, SDRB_ERR_ARG, "null argument");
     if (!h->seamless) return fail(h, SDRB_ERR_STATE, "sdrb_stream needs a handle created with cfg.seamless");
     if (nchunks > h->max_chunks) return fail(h, SDRB_ERR_ARG, "nchunks %zu > max_chunks %zu", nchunks, h->max_chunks);
+    if (h->pl.demod == SDRB_IQ && ((uintptr_t)out_dev & 15))
+        return fail(h, SDRB_ERR_ARG, "iq output is stored as 16-byte (Re, Im) pairs: `out` must be 16-byte aligned");
     CK(h, cudaSetDevice(h->cfg.device));
     return seam_step(h, static_cast<const uint8_t *>(raw_dev), nchunks, out_dev, static_cast<cudaStream_t>(stream), false,
                      nchunks_out);
@@ -913,6 +931,8 @@ int sdrb_stream_end_device(sdrb_handle *h, double *out_dev, void *stream, size_t
     if (nchunks_out) *nchunks_out = 0;
     if (!h || !out_dev) return fail(h, SDRB_ERR_ARG, "null argument");
     if (!h->seamless) return fail(h, SDRB_ERR_STATE, "sdrb_stream_end needs a handle created with cfg.seamless");
+    if (h->pl.demod == SDRB_IQ && ((uintptr_t)out_dev & 15))
+        return fail(h, SDRB_ERR_ARG, "iq output is stored as 16-byte (Re, Im) pairs: `out` must be 16-byte aligned");
     CK(h, cudaSetDevice(h->cfg.device));
     return seam_step(h, nullptr, 0, out_dev, static_cast<cudaStream_t>(stream), true, nchunks_out);
 }
@@ -933,7 +953,7 @@ static int seam_host(sdrb_handle *h, const void *raw_host, size_t nchunks, doubl
     rc = seam_step(h, sl.raw, nchunks, sl.out, sl.stream, end, &ne);
     if (rc) return rc;
     if (ne)
-        CK(h, cudaMemcpyAsync(out_host, sl.out, ne * (size_t)h->pl.R * h->pl.M * sizeof(double), cudaMemcpyDeviceToHost,
+        CK(h, cudaMemcpyAsync(out_host, sl.out, ne * (size_t)h->pl.R * h->pl.W * sizeof(double), cudaMemcpyDeviceToHost,
                               sl.stream));
     CK(h, cudaStreamSynchronize(sl.stream));
     if (nchunks_out) *nchunks_out = ne;
@@ -962,6 +982,8 @@ int sdrb_set_smooth(sdrb_handle *h, int window, int nhead, int ntail, int lo, co
         return fail(h, SDRB_ERR_ARG, "bad argument");
     if (h->seamless && window > 0)
         return fail(h, SDRB_ERR_ARG, "--smooth-output is per-chunk Savitzky-Golay by definition: not available in seamless mode");
+    if (h->pl.demod == SDRB_IQ && window > 0)
+        return fail(h, SDRB_ERR_ARG, "--smooth-output is not available with iq output (complex baseband is not smoothed)");
     if (window > h->pl.M) return fail(h, SDRB_ERR_ARG, "smoothing window %d longer than a chunk's %d outputs", window, h->pl.M);
     CK(h, cudaSetDevice(h->cfg.device));
     CK(h, cudaDeviceSynchronize());
@@ -1214,6 +1236,7 @@ static int demod_op(int device, const double *y, int R, int M, double *out, int 
     if (rc) return rc;
     DevPlan pl{};
     pl.M = M; pl.R = R; pl.nsec_out = 0;
+    pl.W = demod == SDRB_IQ ? 2 * M : M;
     const int h2 = M >> 1;
     pl.fft_ok = (M == 2 * h2) && is_pow2(h2);
     pl.fft_n = pl.fft_ok ? M : 0;
@@ -1225,7 +1248,7 @@ static int demod_op(int device, const double *y, int R, int M, double *out, int 
     pl.demod_in_smem = dsm <= 48 * 1024;
     CK(nullptr, d_tw.alloc(tw.size() * sizeof(double2)));
     CK(nullptr, d_y.alloc((size_t)R * M * sizeof(double2)));
-    CK(nullptr, d_out.alloc((size_t)R * M * sizeof(double)));
+    CK(nullptr, d_out.alloc((size_t)R * pl.W * sizeof(double)));
     if (!pl.demod_in_smem) {
         CK(nullptr, d_fft.alloc((size_t)R * 2 * M * sizeof(double2)));
         CK(nullptr, d_z.alloc((size_t)R * M * sizeof(double)));
@@ -1241,11 +1264,14 @@ static int demod_op(int device, const double *y, int R, int M, double *out, int 
     CK(nullptr, cudaMemcpy(d_y.p, y, (size_t)R * M * sizeof(double2), cudaMemcpyHostToDevice));
     pl.tw = d_tw.as<double2>();
     // rows are laid out [R][M]: run as R "rows" of a single chunk
-    k_demod<<<R, 128, pl.demod_in_smem ? dsm : 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), d_fft.as<double2>(),
-                                                    d_z.as<double>(), 1, demod, 0, 0);
+    if (demod == SDRB_IQ)
+        k_demod<true><<<R, 128, 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), nullptr, nullptr, 1, demod, 0, 0);
+    else
+        k_demod<false><<<R, 128, pl.demod_in_smem ? dsm : 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), d_fft.as<double2>(),
+                                                               d_z.as<double>(), 1, demod, 0, 0);
     CK(nullptr, cudaGetLastError());
     CK(nullptr, cudaDeviceSynchronize());
-    CK(nullptr, cudaMemcpy(out, d_out.p, (size_t)R * M * sizeof(double), cudaMemcpyDeviceToHost));
+    CK(nullptr, cudaMemcpy(out, d_out.p, (size_t)R * pl.W * sizeof(double), cudaMemcpyDeviceToHost));
     return SDRB_OK;
 }
 
@@ -1253,6 +1279,7 @@ int sdrb_fm_demod(int device, const double *y, int R, int M, double *out) { retu
 int sdrb_am_demod(int device, const double *y, int R, int M, double *out) { return demod_op(device, y, R, M, out, SDRB_AM); }
 int sdrb_real_output(int device, const double *y, int R, int M, double *out) { return demod_op(device, y, R, M, out, SDRB_RE); }
 int sdrb_imag_output(int device, const double *y, int R, int M, double *out) { return demod_op(device, y, R, M, out, SDRB_IM); }
+int sdrb_iq_output(int device, const double *y, int R, int M, double *out) { return demod_op(device, y, R, M, out, SDRB_IQ); }
 
 int sdrb_shift_freq(int device, const double *y, const double *shift, int R, int N, double *res)
 {

@@ -64,6 +64,7 @@ struct DevPlan {
     const double *fm_interp;  // [M][M/2] or null
     const double *sos_CA;     // [sos_Lseg][ns]  c A^i
     const unsigned char *use_nco;  // [R]
+    int W;                 // doubles per chunk-row of the output: 2M for iq ((Re, Im) pairs), M otherwise
 };
 
 // ---------------------------------------------------------------- programmatic dependent launch

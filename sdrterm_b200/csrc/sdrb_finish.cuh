@@ -5,7 +5,8 @@
 //   2. carries of the 8 forward / 8 anticausal modal states across the tiles of the chunk
 //   3. decimated outputs y[k] = partial output of the front end + carry-in response (+ boundary)
 //   4. demodulation: fm (pair phase, 2x trigonometric interpolation by a real-input FFT of half
-//      the length and its inverse) | am | re | im
+//      the length and its inverse) | am | re | im; the iq instance (IQO) stores y straight from
+//      registers instead, (Re, Im) per output, and skips 3b-5
 //   5. output low-pass (zero initial state per chunk) in 32 lane segments, chained by a
 //      Kogge-Stone scan of the segment maps; framing (native or big-endian doubles)
 //
@@ -128,7 +129,7 @@ __device__ __forceinline__ double fin_demod_scalar(double2 a, int demod)
     return demod == 2 ? a.x : a.y;
 }
 
-template <int ENC>
+template <int ENC, bool IQO>
 __global__ void __launch_bounds__(32 * FIN_WARPS, 2)
 k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc, const uint8_t *__restrict__ raw,
          double *__restrict__ out, int nchunks, int keep_y)
@@ -420,7 +421,16 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
                     if (keep_y) yg[k] = v;
                     yv[u] = v;
                 }
-                if (pl.demod == 0) {
+                if constexpr (IQO) {
+                    // 16 contiguous bytes per lane, 512 per warp and tile: no trip through zrow
+                    double2 *o2 = reinterpret_cast<double2 *>(out + ((size_t)r * nchunks + chunk) * pl.W);
+#pragma unroll
+                    for (int u = 0; u < 2; u++) {
+                        double2 v = yv[u];
+                        if (pl.be_out) v = make_double2(bswap_double(v.x), bswap_double(v.y));
+                        o2[(t0 + u) * SDRB_TB + lane] = v;
+                    }
+                } else if (pl.demod == 0) {
                     const bool odd = lane & 1;
                     const double2 snd = odd ? yv[0] : yv[1];
                     const double2 rcv = shfl_xor_c(snd, 1);
@@ -442,7 +452,7 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
         __syncwarp();
         FIN_DBG(7);
         // ---------------------------------------------------------------- 3b. fm: 2x interpolation
-        if (pl.demod == 0) {
+        if (!IQO && pl.demod == 0) {
             // even outputs of scipy.signal.resample(ph, 2h) are the phases themselves (already in
             // zrow), the odd ones come from the half-sample-shifted spectrum.  Forward FFT of
             // z[m] = ph[2m] + i ph[2m+1], n2 = h/2 points
@@ -486,7 +496,7 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
         }
         FIN_DBG(8);
         // ---------------------------------------------------------------- 4. output low-pass
-        if (pl.nsec_out > 0) {
+        if (!IQO && pl.nsec_out > 0) {
             double *zs = zrow + (size_t)lane * (Ls + 1);
             const double *c0 = pl.out_sos, *c1 = pl.out_sos + 6;
             double s0 = 0, s1 = 0, s2 = 0, s3 = 0;
@@ -526,12 +536,14 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
         }
         FIN_DBG(9);
         // ---------------------------------------------------------------- 5. framing
-        double *o = out + ((size_t)r * nchunks + chunk) * M;
-        for (int k = lane; k < M; k += 32) {
-            const double v = zrow[k + (k >> lsh)];
-            o[k] = pl.be_out ? bswap_double(v) : v;
+        if constexpr (!IQO) {
+            double *o = out + ((size_t)r * nchunks + chunk) * M;
+            for (int k = lane; k < M; k += 32) {
+                const double v = zrow[k + (k >> lsh)];
+                o[k] = pl.be_out ? bswap_double(v) : v;
+            }
+            __syncwarp();
         }
-        __syncwarp();
         FIN_DBG(10);
     }
 }

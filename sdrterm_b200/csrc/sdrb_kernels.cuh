@@ -6,7 +6,8 @@
 //   k_iqgain / k_iqscan / k_iqtiles   IQ-corrector offset at every tile start, carried across
 //              chunks and calls
 //   k_fixup    head / end segments, cross-tile carries, boundary term -> decimated complex y
-//   k_demod    fm (pair phase + 2x FFT interpolation) | am | re | im, segmented output SOS, framing
+//   k_demod    fm (pair phase + 2x FFT interpolation) | am | re | im, segmented output SOS, framing;
+//              iq: y itself framed as (Re, Im) pairs
 //
 // Reference behaviour being reproduced: src/misc/read_file.py:100-103 (decode, normalise, IQ
 // correction), src/dsp/demodulation.py:71-79 (NCO), src/dsp/dsp_processor.py:147 (scipy
@@ -807,7 +808,9 @@ __device__ __forceinline__ double bswap_double(double v)
 }
 
 // One CTA per (chunk, row): y[M] complex -> out[row][chunk*M .. +M) doubles.
-// Generic entry used both by the chain (y from sc.y) and by the module-level operators.
+// Generic entry used both by the chain (y from sc.y) and by the module-level operators.  The iq
+// instance (IQO) frames y itself as out[row][chunk*2M .. +2M): (Re, Im) pairs, no output low-pass.
+template <bool IQO>
 __global__ void __launch_bounds__(256)
 k_demod(const __grid_constant__ DevPlan pl, const double2 *__restrict__ yall, double *__restrict__ out,
         double2 *fftglob, double *zglob, int nchunks, int demod, int apply_sos, int be_out)
@@ -817,6 +820,15 @@ k_demod(const __grid_constant__ DevPlan pl, const double2 *__restrict__ yall, do
     if (chunk >= nchunks) return;
     const int M = pl.M, h = M >> 1;
     const double2 *y = yall + ((size_t)chunk * pl.R + r) * M;
+    if constexpr (IQO) {
+        double2 *o2 = reinterpret_cast<double2 *>(out + ((size_t)r * nchunks + chunk) * 2 * M);
+        for (int k = threadIdx.x; k < M; k += blockDim.x) {
+            double2 v = y[k];
+            if (be_out) v = make_double2(bswap_double(v.x), bswap_double(v.y));
+            o2[k] = v;
+        }
+        return;
+    }
     double2 *bufA, *bufB;
     double *z;
     if (pl.demod_in_smem) {

@@ -13,7 +13,8 @@
 //   k_seam_carry   per emitted chunk: carry-ins in its own frame (forward state, anticausal window
 //                  over the next D chunks or the real end, zeta) and the fm halo y[k+1]
 //   k_seam_y       per emitted chunk: tile carries and the decimated outputs, global frame
-//   k_seam_demod   demodulation + output SOS from the chunk's zero state (segments, lane scan)
+//   k_seam_demod   demodulation + output SOS from the chunk's zero state (segments, lane scan);
+//                  iq: y itself, (Re, Im) pairs
 //   k_seam_sscan   output SOS state across chunks: affine scan with the matrix A^M
 //   k_seam_frame   response to the carried SOS state, framing
 //
@@ -327,6 +328,15 @@ k_seam_demod(const __grid_constant__ DevPlan pl, SeamDev sd, double *out, int ne
     const int i = (int)(item / pl.R), r = (int)(item % pl.R), M = pl.M, Ls = pl.sos_Lseg;
     const bool last = end && i == nwin - 1;
     const double2 *y = sd.ybuf + ((size_t)i * pl.R + r) * (M + 1);
+    if (pl.demod == SDRB_IQ) {     // rows of ne * 2M doubles, no output low-pass
+        double2 *o2 = reinterpret_cast<double2 *>(out + ((size_t)r * ne + i) * pl.W);
+        for (int k = lane; k < M; k += 32) {
+            double2 v = y[k];
+            if (pl.be_out) v = make_double2(bswap_double(v.x), bswap_double(v.y));
+            o2[k] = v;
+        }
+        return;
+    }
     double *o = out + (size_t)r * ne * M + (size_t)i * M;
     if (pl.nsec_out == 0) {
         for (int k = lane; k < M; k += 32) {

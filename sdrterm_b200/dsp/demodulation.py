@@ -8,7 +8,7 @@ import numpy as np
 
 from .. import _native as nat
 
-__all__ = ['fmDemod', 'amDemod', 'realOutput', 'imagOutput', 'shiftFreq']
+__all__ = ['fmDemod', 'amDemod', 'realOutput', 'imagOutput', 'iqOutput', 'shiftFreq']
 
 
 def _rows(data, out):
@@ -47,6 +47,20 @@ def realOutput(data, res) -> None:
 def imagOutput(data, res) -> None:
     """``res = imag(data)`` (demodulation.py:61-68)."""
     _run('sdrb_imag_output', data, res)
+
+
+def iqOutput(data, res) -> None:
+    """``res[r, 2k] = real(data[r, k])``, ``res[r, 2k+1] = imag(data[r, k])``: the complex rows as
+    interleaved doubles, ``res`` shaped (R, 2M).  Not a reference operator (``-m iq``)."""
+    d = np.ascontiguousarray(np.atleast_2d(data), dtype=np.complex128)
+    if not isinstance(res, np.ndarray):
+        raise TypeError('output must be a numpy array')
+    o2 = np.atleast_2d(res)
+    if o2.shape != (d.shape[0], 2 * d.shape[1]):
+        raise ValueError(f'output shape {o2.shape} does not match (R, 2M) = {(d.shape[0], 2 * d.shape[1])}')
+    out = np.empty(o2.shape, dtype=np.float64)
+    nat.check(nat.lib().sdrb_iq_output(0, d.ctypes.data, d.shape[0], d.shape[1], out.ctypes.data))
+    o2[...] = out
 
 
 def shiftFreq(y, shift, res) -> None:

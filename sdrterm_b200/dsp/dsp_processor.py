@@ -23,9 +23,9 @@ from typing import Any, Callable
 import numpy as np
 
 from .data_processor import DataProcessor
-from .demodulation import amDemod, fmDemod, imagOutput, realOutput
+from .demodulation import amDemod, fmDemod, imagOutput, iqOutput, realOutput
 
-_DEMOD_NAME = {fmDemod: 'fm', amDemod: 'am', realOutput: 're', imagOutput: 'im'}
+_DEMOD_NAME = {fmDemod: 'fm', amDemod: 'am', realOutput: 're', imagOutput: 'im', iqOutput: 'iq'}
 
 
 def generateEllipFilter(fs: int, deg: int, Wn, btype: str):
@@ -147,6 +147,11 @@ class DspProcessor(DataProcessor):
         self.bandwidth = self.decimatedFs
         self._setDemod(imagOutput)
 
+    def selectOutputIq(self):
+        """Not a reference mode: the complex baseband itself, (Re, Im) doubles per output."""
+        self.bandwidth = self.decimatedFs
+        self._setDemod(iqOutput)
+
     # ---------------------------------------------------------------- NCO table (:185-187)
     def _generateShift(self, c: int) -> None:
         """Kept for API parity (tests read ``_shift``); the device path builds its own phasor
@@ -164,7 +169,7 @@ class DspProcessor(DataProcessor):
     def _demodName(self) -> str:
         name = _DEMOD_NAME.get(getattr(self, 'demod', None))
         if name is None:
-            raise ValueError('no demodulation selected (call selectOutputFm/Am/Real/Imag first)')
+            raise ValueError('no demodulation selected (call selectOutputFm/Am/Real/Imag/Iq first)')
         return name
 
     def _makeEngine(self, first):
@@ -200,6 +205,10 @@ class DspProcessor(DataProcessor):
         smooth = int(self.smooth) if (self.smooth and not self._simo()) else 0
         return Engine(plan, max_chunks=self.MAX_BATCH, device=self._device, smooth=smooth, tc=tc)
 
+    def _rowDoubles(self) -> int:
+        """Doubles per chunk and row of the engine's output: 2M for iq ((Re, Im) pairs), M otherwise."""
+        return 2 * self._engine.M if self.demod is iqOutput else self._engine.M
+
     @staticmethod
     def _asBytes(chunk) -> np.ndarray:
         if isinstance(chunk, np.ndarray):
@@ -218,7 +227,7 @@ class DspProcessor(DataProcessor):
         eng = self._engine
         n = self.MAX_BATCH
         self._hin = [PinnedBuffer(n * self._chunkBytes) for _ in range(2)]
-        self._hout = [PinnedBuffer(eng.R * n * eng.M * 8) for _ in range(2)]
+        self._hout = [PinnedBuffer(eng.R * n * self._rowDoubles() * 8) for _ in range(2)]
 
     def _processData(self, isDead, buffer, file=None) -> None:
         """The consumer loop (dsp_processor.py:164-183), double-buffered: while the device works on
@@ -333,11 +342,11 @@ class DspProcessor(DataProcessor):
                 if home is not None:
                     pool.release(home)                   # stream() has copied the bytes to the device
                 if out.shape[1]:
-                    self._emit(out, out.shape[1] // self._engine.M, file)
+                    self._emit(out, out.shape[1] // self._rowDoubles(), file)
         if self._engine is not None:
             out = self._engine.stream_end()
             if out.shape[1]:
-                self._emit(out, out.shape[1] // self._engine.M, file)
+                self._emit(out, out.shape[1] // self._rowDoubles(), file)
 
     def useInputPool(self, pool) -> None:
         """Queue items that are views of ``pool``'s buffers (misc.read_file.ChunkPool) are sent to
@@ -368,7 +377,8 @@ class DspProcessor(DataProcessor):
         eng.wait(slot)
         if home is not None:
             self._inputPool.release(home)                 # the device has the bytes: the reader may refill it
-        out = self._hout[slot].view(np.float64)[:eng.R * n * eng.M].reshape(eng.R, n * eng.M)
+        W = self._rowDoubles()
+        out = self._hout[slot].view(np.float64)[:eng.R * n * W].reshape(eng.R, n * W)
         if eng.plan.big_endian_out:
             out = out.view('>f8')
         self._emit(out, n, file)

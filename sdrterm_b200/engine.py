@@ -2,7 +2,8 @@
 
 This is the thin host layer between the reference-shaped processors (dsp/*.py) and the C ABI.
 Inputs are whole 131072-byte chunks of raw IQ bytes; outputs are float64 rows
-``[row][chunk][M]`` framed as the reference frames them (native doubles, or big-endian in SIMO).
+``[row][chunk][W]`` framed as the reference frames them (native doubles, or big-endian in SIMO).
+W is M, except for iq output: 2M doubles, (Re, Im) of each decimator output interleaved.
 """
 from __future__ import annotations
 
@@ -44,6 +45,8 @@ class Engine:
         cfg.norm_xmin, cfg.norm_k = pl.norm if pl.norm is not None else (0.0, 0.0)
         self.seamless = bool(getattr(pl, 'seamless', False))
         cfg.seamless = int(self.seamless)
+        if pl.demod == 'iq' and smooth:
+            raise ValueError('--smooth-output is not available with iq output')
         if self.seamless and smooth:
             raise ValueError('--smooth-output is per-chunk Savitzky-Golay by definition: not available in '
                              'seamless mode')
@@ -110,6 +113,7 @@ class Engine:
                 tab.tc_xor[i] = int(tc.xor_mask[i])
         nat.check(L.sdrb_create(C.byref(cfg), C.byref(tab), C.byref(self._h)))
         self.M = int(L.sdrb_outputs_per_chunk(self._h))
+        self.W = int(L.sdrb_row_doubles(self._h))       # doubles per chunk and row of the output
         if keep_decimated:
             nat.check(L.sdrb_keep_decimated(self._h, 1), self._h)
         if keep_x0:
@@ -146,7 +150,7 @@ class Engine:
         return n
 
     def process(self, raw, out: np.ndarray | None = None) -> np.ndarray:
-        """Host bytes in, (R, nchunks*M) float64 out (H2D + kernels + D2H, synchronous).  With
+        """Host bytes in, (R, nchunks*W) float64 out (H2D + kernels + D2H, synchronous).  With
         big-endian framing the returned array holds the byte-swapped doubles (dtype '>f8')."""
         buf = np.frombuffer(raw, dtype=np.uint8) if not isinstance(raw, np.ndarray) else raw
         buf = np.ascontiguousarray(buf).view(np.uint8).reshape(-1)
@@ -155,7 +159,7 @@ class Engine:
             raise nat.SdrbError('seamless engine: use stream() / stream_end()')
         dt = np.dtype('>f8') if self.plan.big_endian_out else np.dtype('=f8')
         if out is None:
-            out = np.empty((self.R, n * self.M), dtype=dt)
+            out = np.empty((self.R, n * self.W), dtype=dt)
         if n:
             nat.check(nat.lib().sdrb_process(self._h, buf.ctypes.data, n, out.ctypes.data), self._h)
         return out
@@ -168,13 +172,13 @@ class Engine:
 
     def _out_array(self, nchunks: int) -> np.ndarray:
         dt = np.dtype('>f8') if self.plan.big_endian_out else np.dtype('=f8')
-        return np.empty(self.R * nchunks * self.M, dtype=dt)
+        return np.empty(self.R * nchunks * self.W, dtype=dt)
 
     def _rows(self, flat: np.ndarray, k: int) -> np.ndarray:
-        return flat[:self.R * k * self.M].reshape(self.R, k * self.M)
+        return flat[:self.R * k * self.W].reshape(self.R, k * self.W)
 
     def stream(self, raw) -> np.ndarray:
-        """Seamless mode: take whole chunks of the stream, return (R, k*M) for the k chunks that have
+        """Seamless mode: take whole chunks of the stream, return (R, k*W) for the k chunks that have
         become final (the stream is filtered as one signal; see DESIGN.md section 11).  Batches
         larger than ``max_chunks`` are fed in pieces."""
         if not self.seamless:
@@ -224,6 +228,8 @@ class Engine:
         if self.seamless:
             raise ValueError('--smooth-output is per-chunk Savitzky-Golay by definition: not available in '
                              'seamless mode')
+        if self.plan.demod == 'iq':
+            raise ValueError('--smooth-output is not available with iq output')
         w = int(window)
         if w > self.M:
             raise ValueError(f'smoothing window {w} longer than a chunk\'s {self.M} outputs')

@@ -18,6 +18,7 @@ class DemodulationChoices(str, Enum):
     AM = 'am'
     REAL = 're'
     IMAG = 'im'
+    IQ = 'iq'
 
     def __str__(self):
         return self.value
@@ -26,7 +27,7 @@ class DemodulationChoices(str, Enum):
 def selectDemodulation(demodType, processor) -> Callable:
     tprint(f'{demodType} requested')
     table = {'fm': 'selectOutputFm', 'nfm': 'selectOutputFm', 'am': 'selectOutputAm',
-             're': 'selectOutputReal', 'im': 'selectOutputImag'}
+             're': 'selectOutputReal', 'im': 'selectOutputImag', 'iq': 'selectOutputIq'}
     name = table.get(str(demodType.value if isinstance(demodType, Enum) else demodType))
     if name is None:
         raise ValueError(f'Invalid demod type {demodType}')

@@ -255,6 +255,11 @@ class RowShardedBank:
     def M(self) -> int:
         return self.plan.M
 
+    @property
+    def W(self) -> int:
+        """Doubles per chunk and row of the output (2M for iq)."""
+        return self.plan.W
+
     def _post(self, i: int, src, nbytes: int):
         """Start batch i on its way to the ranks of the time group."""
         if self.row_groups == 1:
@@ -268,7 +273,7 @@ class RowShardedBank:
 
     def run(self, batches, nchunks: int, outs, stream: int = 0) -> None:
         """``batches``: list of uint8 device tensors (on the leader; elsewhere only the count
-        matters); ``outs``: list of (rows, nchunks*M) float64 device tensors of this rank.  The
+        matters); ``outs``: list of (rows, nchunks*W) float64 device tensors of this rank.  The
         kernels go to ``stream``, which must be the current torch stream."""
         n = len(batches)
         if nchunks > self.max_chunks or len(outs) < n:
@@ -354,10 +359,10 @@ def run_file_sharded(path: str, out_path: str | None, *, fs: int, enc: str, dec:
         start = sharding.exchange_iq_gain(dist, torch, gain, count * plan.N, plan.lam,
                                           device=torch.device('cuda', device) if dist.get_backend() == 'nccl' else None)
         eng.iq_state = start
-    out = np.empty((1, count * plan.M), dtype=np.float64)
+    out = np.empty((1, count * plan.W), dtype=np.float64)
     for b0 in range(0, count, batch_chunks):
         n = min(batch_chunks, count - b0)
-        out[:, b0 * plan.M:(b0 + n) * plan.M] = eng.process(raw[b0 * CHUNK_BYTES:(b0 + n) * CHUNK_BYTES])
+        out[:, b0 * plan.W:(b0 + n) * plan.W] = eng.process(raw[b0 * CHUNK_BYTES:(b0 + n) * CHUNK_BYTES])
     eng.close()
     if out_path is None:
         return out

@@ -230,6 +230,11 @@ class Plan:
     def chunk_bytes(self) -> int:
         return self.N * 2 * _ITEMSIZE[self.enc]
 
+    @property
+    def W(self) -> int:
+        """Doubles per chunk and row of the output: 2M for iq ((Re, Im) interleaved), M otherwise."""
+        return 2 * self.M if self.demod == 'iq' else self.M
+
 
 def reference_w(f_hz: int, fs: int) -> float:
     """Phase increment per sample exactly as the reference forms it:
@@ -390,7 +395,7 @@ def build_plan(fs: int, enc: str, dec: int, rows_hz, *, simo: bool = False, swap
         out_sos = np.ascontiguousarray(
             _sig.ellip(3, 1, 30, omega_out, btype='lowpass', analog=False, output='sos',
                        fs=fs // q), dtype=np.float64)
-    elif demod not in ('re', 'im'):
+    elif demod not in ('re', 'im', 'iq'):          # iq: the complex decimator output, no output low-pass
         raise ValueError(f'Invalid demod type {demod}')
     sos_Lseg, sos_AL, sos_CA, sos_AP = 0, None, None, None
     if out_sos is not None:
