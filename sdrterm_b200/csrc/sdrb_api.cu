@@ -8,6 +8,7 @@
 #include <cstring>
 #include <string>
 #include <mutex>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/sdrterm_b200.h"
@@ -58,7 +59,6 @@ struct sdrb_handle {
     CUtensorMap map_b{};
     size_t tc_smem = 0;
     int num_sms = 148;
-    bool pdl = false;               // programmatic dependent launch inside a step (SDRB_PDL=1)
     int reserved_sms = 0;           // SMs the persistent kernels leave free (for a collective running beside them)
     double2 *x0_buf = nullptr;      // sdrb_keep_x0
     int smooth_w = 0, smooth_nhead = 0, smooth_ntail = 0, smooth_lo = 0;   // --smooth-output (window 0 = off)
@@ -106,6 +106,25 @@ int itemsize_of(int code)
     return sz[code];
 }
 
+// The one place a runtime encoding code becomes a kernel template argument: calls
+// f(std::integral_constant<int, ENC_x>{}) and returns its result.
+template <class F>
+int with_enc(sdrb_handle *h, int code, F &&f)
+{
+    switch (code) {
+    case ENC_b: return f(std::integral_constant<int, ENC_b>{});
+    case ENC_B: return f(std::integral_constant<int, ENC_B>{});
+    case ENC_h: return f(std::integral_constant<int, ENC_h>{});
+    case ENC_H: return f(std::integral_constant<int, ENC_H>{});
+    case ENC_i: return f(std::integral_constant<int, ENC_i>{});
+    case ENC_I: return f(std::integral_constant<int, ENC_I>{});
+    case ENC_f: return f(std::integral_constant<int, ENC_f>{});
+    case ENC_d: return f(std::integral_constant<int, ENC_d>{});
+    case ENC_Z: return f(std::integral_constant<int, ENC_Z>{});
+    }
+    return fail(h, SDRB_ERR_ARG, "bad encoding code %d", code);
+}
+
 template <typename T>
 int upload(sdrb_handle *h, const T *src, size_t count, const T **dst)
 {
@@ -149,20 +168,6 @@ int env_int(const char *name, int dflt);
 int launch_tc(sdrb_handle *h, const uint8_t *raw, size_t nch, cudaStream_t st, bool iq);
 
 enum { PH_MAIN = 1, PH_IQSCAN = 2, PH_FINISH = 4, PH_ALL = 7 };
-
-// Launch with the programmatic stream-serialisation attribute (see pdl_wait in sdrb_device.cuh);
-// SDRB_PDL=1 switches it on (ordinary launches otherwise).
-template <typename... KArgs, typename... Args>
-cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, bool pdl, Args... args)
-{
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
-}
 
 // ------------------------------------------------------------------ tensor-core front end
 typedef CUresult (*encode_tiled_fn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
@@ -228,7 +233,7 @@ int tc_attr(sdrb_handle *h)
 
 int setup_tc(sdrb_handle *h, const sdrb_tables *tab)
 {
-    if (!tab->tc_enable || env_int("SDRB_NO_TC", 0)) return 0;
+    if (!tab->tc_enable) return 0;
     const int R = h->pl.R;
     if ((tab->tc_K != 256 && tab->tc_K != 512) || tab->tc_nout != TC_NOUT || tab->tc_ncol != TC_NCOL ||
         tab->tc_isz < 1 || tab->tc_isz > 2 || tab->tc_npad != TC_NPAD || tab->tc_nrowc != TC_NROWC ||
@@ -274,9 +279,6 @@ int setup_tc(sdrb_handle *h, const sdrb_tables *tab)
     nstage = std::min(nstage, TC_MAX_ASTAGES);
     if (nstage < 2) return fail(h, SDRB_ERR_ARG, "k_tc: no room for the A ring (%zu bytes fixed)", fixed);
     tc.nstage = nstage;
-    tc.prefetch_tiles = env_int("SDRB_TC_PREFETCH", 0);
-    tc.abl = env_int("SDRB_TC_ABL", 0);                        // timing experiments only: wrong results
-    if (tc.abl & 1) tc.xor_word = 0;
     h->tc_smem = tc_smem_bytes(tc.nregion, nstage);
     if ((rc = tc_attr<true>(h)) || (rc = tc_attr<false>(h))) return rc;
     h->tc_on = true;
@@ -305,35 +307,27 @@ int launch_chain_t(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, 
     }
     mark(1);
     if ((phases & PH_IQSCAN) && IQ) {
-        int nth = 1024;
-        while (nth > 32 && (size_t)nth / 2 >= nch) nth /= 2;
-        if (h->finish_on && pl.ntiles <= 32 && !h->seamless) {
-            // whole-tile chunks: warp-parallel gains, the chunk scan; k_finish derives the offsets
-            // at the tile starts itself
-            const bool pdl = h->pdl && (phases & PH_MAIN);        // only right behind the front end of the same call
-            CK(h, launch_pdl(k_iqgain_w, dim3((unsigned)((nch + 7) / 8)), dim3(256), 0, st, pdl, pl, h->sc, (int)nch));
-            CK(h, launch_pdl(k_iqscan_c, dim3(1), dim3(1024), 0, st, h->pdl, pl, h->sc, (int)nch));
-            h->launches += 2;
-        } else {
-            const unsigned gb = (unsigned)((nch + 127) / 128);
+        // chunk gains -> the chunk scan (offset at every chunk start) -> the offsets at the tile
+        // starts; with whole-tile chunks the gains are warp-parallel and k_finish derives the
+        // tile-start offsets itself
+        const bool whole_tiles = h->finish_on && pl.ntiles <= 32 && !h->seamless;
+        const unsigned gb = (unsigned)((nch + 127) / 128);
+        if (whole_tiles)
+            k_iqgain_w<<<(unsigned)((nch + 7) / 8), 256, 0, st>>>(pl, h->sc, (int)nch);
+        else
             k_iqgain<ENC><<<gb, 128, 0, st>>>(pl, h->sc, raw, (int)nch);
-            k_iqscan<<<1, nth, 0, st>>>(pl, h->sc, (int)nch);
-            k_iqtiles<<<gb, 128, 0, st>>>(pl, h->sc, (int)nch);
-            h->launches += 3;
-        }
+        k_iqscan_c<<<1, 1024, 0, st>>>(pl, h->sc, (int)nch);
+        if (!whole_tiles) k_iqtiles<<<gb, 128, 0, st>>>(pl, h->sc, (int)nch);
+        h->launches += whole_tiles ? 2 : 3;
     }
     mark(2);
     if ((phases & PH_FINISH) && h->finish_on) {
         const size_t items = nch * (size_t)pl.R;
         const unsigned grid = (unsigned)std::min<size_t>((items + FIN_WARPS - 1) / FIN_WARPS, (size_t)(h->num_sms - h->reserved_sms) * 2);
-        // behind the IQ kernels of the same call (or, without IQ correction, behind the front end)
-        const bool pdl = h->pdl && ((phases & PH_MAIN) || ((phases & PH_IQSCAN) && IQ));
         if (pl.demod == SDRB_IQ)
-            CK(h, launch_pdl(k_finish<ENC, true>, dim3(grid), dim3(32 * FIN_WARPS), h->finish_smem, st, pdl, pl, h->sc, raw,
-                             out, (int)nch, h->keep_y));
+            k_finish<ENC, true><<<grid, 32 * FIN_WARPS, h->finish_smem, st>>>(pl, h->sc, raw, out, (int)nch, h->keep_y);
         else
-            CK(h, launch_pdl(k_finish<ENC, false>, dim3(grid), dim3(32 * FIN_WARPS), h->finish_smem, st, pdl, pl, h->sc, raw,
-                             out, (int)nch, h->keep_y));
+            k_finish<ENC, false><<<grid, 32 * FIN_WARPS, h->finish_smem, st>>>(pl, h->sc, raw, out, (int)nch, h->keep_y);
         h->launches++;
         mark(3);
         mark(4);
@@ -365,18 +359,11 @@ int launch_chain(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, cu
 {
     if ((phases & PH_FINISH) && h->pl.demod == SDRB_IQ && ((uintptr_t)out & 15))
         return fail(h, SDRB_ERR_ARG, "iq output is stored as 16-byte (Re, Im) pairs: `out` must be 16-byte aligned");
-    switch (h->enc_code) {
-    case ENC_b: return h->pl.correct_iq ? launch_chain_t<ENC_b, true>(h, raw, nch, out, st, phases) : launch_chain_t<ENC_b, false>(h, raw, nch, out, st, phases);
-    case ENC_B: return h->pl.correct_iq ? launch_chain_t<ENC_B, true>(h, raw, nch, out, st, phases) : launch_chain_t<ENC_B, false>(h, raw, nch, out, st, phases);
-    case ENC_h: return h->pl.correct_iq ? launch_chain_t<ENC_h, true>(h, raw, nch, out, st, phases) : launch_chain_t<ENC_h, false>(h, raw, nch, out, st, phases);
-    case ENC_H: return h->pl.correct_iq ? launch_chain_t<ENC_H, true>(h, raw, nch, out, st, phases) : launch_chain_t<ENC_H, false>(h, raw, nch, out, st, phases);
-    case ENC_i: return h->pl.correct_iq ? launch_chain_t<ENC_i, true>(h, raw, nch, out, st, phases) : launch_chain_t<ENC_i, false>(h, raw, nch, out, st, phases);
-    case ENC_I: return h->pl.correct_iq ? launch_chain_t<ENC_I, true>(h, raw, nch, out, st, phases) : launch_chain_t<ENC_I, false>(h, raw, nch, out, st, phases);
-    case ENC_f: return h->pl.correct_iq ? launch_chain_t<ENC_f, true>(h, raw, nch, out, st, phases) : launch_chain_t<ENC_f, false>(h, raw, nch, out, st, phases);
-    case ENC_d: return h->pl.correct_iq ? launch_chain_t<ENC_d, true>(h, raw, nch, out, st, phases) : launch_chain_t<ENC_d, false>(h, raw, nch, out, st, phases);
-    case ENC_Z: return h->pl.correct_iq ? launch_chain_t<ENC_Z, true>(h, raw, nch, out, st, phases) : launch_chain_t<ENC_Z, false>(h, raw, nch, out, st, phases);
-    }
-    return fail(h, SDRB_ERR_ARG, "bad encoding code %d", h->enc_code);
+    return with_enc(h, h->enc_code, [&](auto enc) {
+        constexpr int E = decltype(enc)::value;
+        return h->pl.correct_iq ? launch_chain_t<E, true>(h, raw, nch, out, st, phases)
+                                : launch_chain_t<E, false>(h, raw, nch, out, st, phases);
+    });
 }
 
 template <int ENC, bool IQ>
@@ -390,14 +377,10 @@ int set_smem_attr_t(sdrb_handle *h)
 }
 int set_smem_attr(sdrb_handle *h)
 {
-    switch (h->enc_code) {
-    case ENC_b: return h->pl.correct_iq ? set_smem_attr_t<ENC_b, true>(h) : set_smem_attr_t<ENC_b, false>(h); case ENC_B: return h->pl.correct_iq ? set_smem_attr_t<ENC_B, true>(h) : set_smem_attr_t<ENC_B, false>(h);
-    case ENC_h: return h->pl.correct_iq ? set_smem_attr_t<ENC_h, true>(h) : set_smem_attr_t<ENC_h, false>(h); case ENC_H: return h->pl.correct_iq ? set_smem_attr_t<ENC_H, true>(h) : set_smem_attr_t<ENC_H, false>(h);
-    case ENC_i: return h->pl.correct_iq ? set_smem_attr_t<ENC_i, true>(h) : set_smem_attr_t<ENC_i, false>(h); case ENC_I: return h->pl.correct_iq ? set_smem_attr_t<ENC_I, true>(h) : set_smem_attr_t<ENC_I, false>(h);
-    case ENC_f: return h->pl.correct_iq ? set_smem_attr_t<ENC_f, true>(h) : set_smem_attr_t<ENC_f, false>(h); case ENC_d: return h->pl.correct_iq ? set_smem_attr_t<ENC_d, true>(h) : set_smem_attr_t<ENC_d, false>(h);
-    case ENC_Z: return h->pl.correct_iq ? set_smem_attr_t<ENC_Z, true>(h) : set_smem_attr_t<ENC_Z, false>(h);
-    }
-    return SDRB_ERR_ARG;
+    return with_enc(h, h->enc_code, [&](auto enc) {
+        constexpr int E = decltype(enc)::value;
+        return h->pl.correct_iq ? set_smem_attr_t<E, true>(h) : set_smem_attr_t<E, false>(h);
+    });
 }
 
 int env_int(const char *name, int dflt)
@@ -451,7 +434,6 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
     h->cfg = *cfg;
     h->enc_code = code;
     h->max_chunks = (size_t)cfg->max_chunks;
-    h->pdl = env_int("SDRB_PDL", 0) != 0;       // measured neutral on B200 (DESIGN.md 3.7): off unless asked for
     int rc = 0;
     auto bail = [&](int c) { std::string e = h->error; sdrb_destroy(h); g_error = e; return c; };
     if (cudaSetDevice(cfg->device) != cudaSuccess) return bail(fail(h, SDRB_ERR_CUDA, "cudaSetDevice failed"));
@@ -796,19 +778,7 @@ int sdrb_process(sdrb_handle *h, const void *raw, size_t nchunks, double *out)
 
 }  // extern "C"
 namespace {
-template <int ENC>
-void launch_iqchunk(sdrb_handle *h, const uint8_t *raw, size_t nch, cudaStream_t st)
-{
-    k_iqchunk<ENC><<<(unsigned)((nch + 7) / 8), 256, 0, st>>>(h->pl, h->sc, raw, (int)nch);
-}
-
 // ------------------------------------------------------------------ seamless streaming
-template <int ENC>
-void launch_seam_edges(sdrb_handle *h, const uint8_t *raw, int slot0, size_t nch, cudaStream_t st)
-{
-    k_seam_edges<ENC><<<(unsigned)nch, 64, 0, st>>>(h->pl, h->sd, raw, slot0, (int)nch);
-}
-
 // Copy window slots [from, from + n) to [0, n) of a [slot][per] buffer (from > 0; a slot is never
 // read after it has been written when the ranges overlap).
 template <typename T>
@@ -847,17 +817,11 @@ int seam_step(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, cudaS
         rc = launch_chain(h, raw, nch, nullptr, st, PH_MAIN | PH_IQSCAN);
         h->sc = base;
         if (rc) return rc;
-        switch (h->enc_code) {
-        case ENC_b: launch_seam_edges<ENC_b>(h, raw, s0, nch, st); break;
-        case ENC_B: launch_seam_edges<ENC_B>(h, raw, s0, nch, st); break;
-        case ENC_h: launch_seam_edges<ENC_h>(h, raw, s0, nch, st); break;
-        case ENC_H: launch_seam_edges<ENC_H>(h, raw, s0, nch, st); break;
-        case ENC_i: launch_seam_edges<ENC_i>(h, raw, s0, nch, st); break;
-        case ENC_I: launch_seam_edges<ENC_I>(h, raw, s0, nch, st); break;
-        case ENC_f: launch_seam_edges<ENC_f>(h, raw, s0, nch, st); break;
-        case ENC_d: launch_seam_edges<ENC_d>(h, raw, s0, nch, st); break;
-        default:    launch_seam_edges<ENC_Z>(h, raw, s0, nch, st); break;
-        }
+        rc = with_enc(h, h->enc_code, [&](auto enc) {
+            k_seam_edges<decltype(enc)::value><<<(unsigned)nch, 64, 0, st>>>(pl, sd, raw, s0, (int)nch);
+            return 0;
+        });
+        if (rc) return rc;
         const size_t items = nch * (size_t)R;
         k_seam_agg<<<(unsigned)((items + 7) / 8), 256, 0, st>>>(pl, h->sc, sd, s0, (int)nch, h->seen);
         if (h->seen == 0) k_seam_head<<<(unsigned)((R + 63) / 64), 64, 0, st>>>(pl, h->sc, sd, s0);
@@ -1016,17 +980,11 @@ int sdrb_iq_gain(sdrb_handle *h, const void *raw_host, size_t nchunks)
     Slot &sl = h->slot[0];
     CK(h, cudaMemcpyAsync(sl.raw, raw_host, nchunks * sdrb_chunk_bytes(h), cudaMemcpyHostToDevice, sl.stream));
     CK(h, cudaStreamWaitEvent(sl.stream, h->iq_done, 0));
-    switch (h->enc_code) {
-    case ENC_b: launch_iqchunk<ENC_b>(h, sl.raw, nchunks, sl.stream); break;
-    case ENC_B: launch_iqchunk<ENC_B>(h, sl.raw, nchunks, sl.stream); break;
-    case ENC_h: launch_iqchunk<ENC_h>(h, sl.raw, nchunks, sl.stream); break;
-    case ENC_H: launch_iqchunk<ENC_H>(h, sl.raw, nchunks, sl.stream); break;
-    case ENC_i: launch_iqchunk<ENC_i>(h, sl.raw, nchunks, sl.stream); break;
-    case ENC_I: launch_iqchunk<ENC_I>(h, sl.raw, nchunks, sl.stream); break;
-    case ENC_f: launch_iqchunk<ENC_f>(h, sl.raw, nchunks, sl.stream); break;
-    case ENC_d: launch_iqchunk<ENC_d>(h, sl.raw, nchunks, sl.stream); break;
-    default:    launch_iqchunk<ENC_Z>(h, sl.raw, nchunks, sl.stream); break;
-    }
+    rc = with_enc(h, h->enc_code, [&](auto enc) {
+        k_iqchunk<decltype(enc)::value><<<(unsigned)((nchunks + 7) / 8), 256, 0, sl.stream>>>(h->pl, h->sc, sl.raw, (int)nchunks);
+        return 0;
+    });
+    if (rc) return rc;
     k_iqscan_c<<<1, 1024, 0, sl.stream>>>(h->pl, h->sc, (int)nchunks);
     h->launches += 2;
     CK(h, cudaGetLastError());
@@ -1404,16 +1362,12 @@ int sdrb_decode_iq(int device, const void *raw, size_t nsamples, char enc, int s
     const unsigned grid = (unsigned)std::min<size_t>((nsamples + 255) / 256, 148 * 8);
     const uint8_t *r8 = d_raw.as<uint8_t>();
     double2 *z = d_z.as<double2>();
-    switch (code) {
-    case ENC_b: k_decode<ENC_b><<<grid, 256>>>(r8, z, nsamples, swap); break;
-    case ENC_B: k_decode<ENC_B><<<grid, 256>>>(r8, z, nsamples, swap); break;
-    case ENC_h: k_decode<ENC_h><<<grid, 256>>>(r8, z, nsamples, swap); break;
-    case ENC_H: k_decode<ENC_H><<<grid, 256>>>(r8, z, nsamples, swap); break;
-    case ENC_i: k_decode<ENC_i><<<grid, 256>>>(r8, z, nsamples, swap); break;
-    case ENC_I: k_decode<ENC_I><<<grid, 256>>>(r8, z, nsamples, swap); break;
-    case ENC_f: k_decode<ENC_f><<<grid, 256>>>(r8, z, nsamples, swap); break;
-    default:    k_decode<ENC_d><<<grid, 256>>>(r8, z, nsamples, swap); break;
-    }
+    rc = with_enc(nullptr, code, [&](auto enc) {
+        constexpr int E = decltype(enc)::value;
+        if constexpr (E != ENC_Z) k_decode<E><<<grid, 256>>>(r8, z, nsamples, swap);   // ENC_Z is refused above
+        return 0;
+    });
+    if (rc) return rc;
     CK(nullptr, cudaGetLastError());
     CK(nullptr, cudaDeviceSynchronize());
     CK(nullptr, cudaMemcpy(z_out, d_z.p, nsamples * sizeof(double2), cudaMemcpyDeviceToHost));

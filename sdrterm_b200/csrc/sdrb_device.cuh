@@ -67,15 +67,6 @@ struct DevPlan {
     int W;                 // doubles per chunk-row of the output: 2M for iq ((Re, Im) pairs), M otherwise
 };
 
-// ---------------------------------------------------------------- programmatic dependent launch
-// The kernels of one step form a chain on one stream.  A kernel launched with the programmatic
-// stream-serialisation attribute may become resident while its predecessor still runs: it does its
-// own set-up (tables into shared memory), then pdl_wait() blocks until the predecessor has
-// completed and its writes are visible.  pdl_trigger() in the predecessor allows that early
-// scheduling.  Both are no-ops for a kernel launched the ordinary way.
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-
 // ---------------------------------------------------------------- complex helpers (double2)
 __device__ __forceinline__ double2 cmul(double2 a, double2 b)
 {

@@ -168,9 +168,6 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
     double2 *seqA = fa + (size_t)nt * 16, *seqB = seqA + 32;             // dead before zrow is written
     double *zrow = reinterpret_cast<double *>(fa + n2);
     __syncthreads();
-    // everything above reads only the plan's tables: with a programmatic dependent launch it runs
-    // while the IQ-offset kernels (and the tail of the front end) are still busy
-    pdl_wait();
 
     // lane-invariant tables: this lane's block position l = lane inside every tile
     // (the filter is real: poles 4..7 are the conjugates of 0..3 and so are their weights, hence

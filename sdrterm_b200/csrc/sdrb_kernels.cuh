@@ -3,7 +3,7 @@
 //   k_main     raw tile -> shared memory; run-wise IQ correction, NCO and the even/odd block sums
 //              on the FP64 tensor pipe (DMMA.8x8x4), all from registers; tile-local modal scans
 //              -> partial outputs + tile aggregates
-//   k_iqgain / k_iqscan / k_iqtiles   IQ-corrector offset at every tile start, carried across
+//   k_iqgain / k_iqscan_c / k_iqtiles   IQ-corrector offset at every tile start, carried across
 //              chunks and calls
 //   k_fixup    head / end segments, cross-tile carries, boundary term -> decimated complex y
 //   k_demod    fm (pair phase + 2x FFT interpolation) | am | re | im, segmented output SOS, framing;
@@ -22,8 +22,8 @@ struct Scratch {
     double2 *agg;       // [nch][R][ntiles][16]   0..7 Wout, 8..15 Tin
     double2 *tile_agg;  // [nch][ntiles]
     double2 *off_tile;  // [nch][ntiles+1]
-    double2 *gain;      // [nch] offset gained over a chunk from zero (whole-tile fast path)
-    double2 *start;     // [nch] offset at the chunk start            "
+    double2 *gain;      // [nch] offset gained over a chunk from zero
+    double2 *start;     // [nch] offset at the chunk start
     double2 *carry;     // [nch][R][ntiles+1][16] 0..7 Win[t], 8..15 Tn[t]
     double2 *y;         // [nch][R][M]
     double2 *iq_state;  // [1] offset before the batch (in) / after it (out)
@@ -353,7 +353,7 @@ k_main(const __grid_constant__ DevPlan pl, Scratch sc, const uint8_t *__restrict
 }
 
 // -------------------------------------------------------------------------------- IQ kernels
-// k_iqgain: thread <-> chunk, offset gained over the chunk from a zero state -> off_tile[c][nt].
+// k_iqgain: thread <-> chunk, offset gained over the chunk from a zero state -> gain[c].
 template <int ENC>
 __global__ void __launch_bounds__(128)
 k_iqgain(const __grid_constant__ DevPlan pl, Scratch sc, const uint8_t *__restrict__ raw, int nchunks)
@@ -389,7 +389,7 @@ k_iqgain(const __grid_constant__ DevPlan pl, Scratch sc, const uint8_t *__restri
         const double lr = pl.lam_j[pl.rem];
         o.x = fma(lr, o.x, pl.Liq * acc.x); o.y = fma(lr, o.y, pl.Liq * acc.y);
     }
-    sc.off_tile[(size_t)c * (nt + 1) + nt] = o;
+    sc.gain[blockIdx.x * blockDim.x + threadIdx.x] = o;   // = c, recomputed: 40 instead of 42 registers for ENC_d
 }
 
 // k_iqgain_w: warp <-> chunk, lane <-> tile (whole-tile chunks, ntiles <= 32): the same gain as
@@ -397,8 +397,6 @@ k_iqgain(const __grid_constant__ DevPlan pl, Scratch sc, const uint8_t *__restri
 __global__ void __launch_bounds__(256)
 k_iqgain_w(const __grid_constant__ DevPlan pl, Scratch sc, int nchunks)
 {
-    pdl_trigger();
-    pdl_wait();                                   // tile_agg comes from the block front end
     const int lane = threadIdx.x & 31;
     const int c = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (c >= nchunks) return;
@@ -457,8 +455,6 @@ k_iqscan_c(const __grid_constant__ DevPlan pl, Scratch sc, int nchunks)
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const double2 *__restrict__ gain = sc.gain;
     double2 *__restrict__ start = sc.start;
-    pdl_trigger();
-    pdl_wait();                                   // gain[] comes from k_iqgain_w / k_iqchunk
     if (tid == 0) s_state = sc.iq_state[0];
     __syncthreads();
     for (int base = 0; base < nchunks; base += 1024 * 8) {
@@ -516,58 +512,7 @@ k_iqscan_c(const __grid_constant__ DevPlan pl, Scratch sc, int nchunks)
     if (tid == 0) sc.iq_state[0] = s_state;
 }
 
-// k_iqscan: one CTA; exclusive scan of the per-chunk affine maps o -> lam_N*o + gain, starting from
-// the handle's IQ state; writes the offset at every chunk start to off_tile[c][0] and the new state.
-__global__ void __launch_bounds__(1024)
-k_iqscan(const __grid_constant__ DevPlan pl, Scratch sc, int nchunks)
-{
-    __shared__ double2 s_a[1024];
-    __shared__ double s_m[1024];
-    const int tid = threadIdx.x, nth = blockDim.x, nt = pl.ntiles;
-    const int per = (nchunks + nth - 1) / nth;
-    const int c0 = min(nchunks, tid * per), c1 = min(nchunks, c0 + per);
-    double2 a = make_double2(0.0, 0.0);
-    double mlt = 1.0;
-    for (int c = c0; c < c1; c++) {
-        const double2 g = sc.off_tile[(size_t)c * (nt + 1) + nt];
-        a.x = fma(pl.lam_N, a.x, g.x); a.y = fma(pl.lam_N, a.y, g.y);
-        mlt *= pl.lam_N;
-    }
-    s_a[tid] = a; s_m[tid] = mlt;
-    __syncthreads();
-    // Hillis-Steele inclusive scan of affine maps (m, a): later o earlier = (m2*m1, m2*a1 + a2)
-    for (int d = 1; d < nth; d <<= 1) {
-        double2 pa = make_double2(0.0, 0.0);
-        double pm = 1.0;
-        const bool has = tid >= d;
-        if (has) { pa = s_a[tid - d]; pm = s_m[tid - d]; }
-        __syncthreads();
-        if (has) {
-            const double mm = s_m[tid];
-            s_a[tid] = make_double2(fma(mm, pa.x, s_a[tid].x), fma(mm, pa.y, s_a[tid].y));
-            s_m[tid] = mm * pm;
-        }
-        __syncthreads();
-    }
-    const double2 st0 = sc.iq_state[0];
-    double2 o = st0;
-    if (tid > 0) {
-        const double2 pa = s_a[tid - 1]; const double pm = s_m[tid - 1];
-        o = make_double2(fma(pm, st0.x, pa.x), fma(pm, st0.y, pa.y));
-    }
-    for (int c = c0; c < c1; c++) {
-        sc.off_tile[(size_t)c * (nt + 1)] = o;
-        const double2 g = sc.off_tile[(size_t)c * (nt + 1) + nt];
-        o.x = fma(pl.lam_N, o.x, g.x); o.y = fma(pl.lam_N, o.y, g.y);
-    }
-    __syncthreads();
-    if (tid == nth - 1) {
-        const double2 pa = s_a[tid]; const double pm = s_m[tid];
-        sc.iq_state[0] = make_double2(fma(pm, st0.x, pa.x), fma(pm, st0.y, pa.y));
-    }
-}
-
-// k_iqtiles: thread <-> chunk, offsets at the tile starts from the chunk-start offset.
+// k_iqtiles: thread <-> chunk, offsets at the tile starts from the chunk-start offset start[c].
 __global__ void __launch_bounds__(128)
 k_iqtiles(const __grid_constant__ DevPlan pl, Scratch sc, int nchunks)
 {
@@ -576,7 +521,7 @@ k_iqtiles(const __grid_constant__ DevPlan pl, Scratch sc, int nchunks)
     const int nt = pl.ntiles;
     const double2 *ta = sc.tile_agg + (size_t)c * nt;
     double2 *ot = sc.off_tile + (size_t)c * (nt + 1);
-    double2 o = ot[0];
+    double2 o = sc.start[c];
     int t = 0;
     for (; t + 8 <= nt; t += 8) {
         double2 g[8];

@@ -6,7 +6,8 @@ algorithm and every table against the oracle without a GPU.  Structure mirrors t
                             UNcorrected samples, IQ-EMA block aggregates, tile-local scans, partial
                             outputs + tile aggregates; the IQ corrector enters only through the
                             decoupled terms of DESIGN.md 3.3)
-  emu_iq_scan <-> k_iqscan (offset at every tile start, carried across chunks and calls)
+  emu_iq_scan <-> k_iqgain / k_iqscan_c / k_iqtiles (offset at every tile start, carried across
+                            chunks and calls)
   emu_fixup   <-> k_fixup  (head / end segments, cross-tile carries, boundary term -> decimated y)
   emu_demod   <-> k_demod  (fm pair-phase + 2x FFT interpolation | am | re | im, output SOS)
 """

@@ -80,9 +80,14 @@ def test_general_finish_kernels_match_fused(name, monkeypatch):
 
 
 def test_batch_split_and_state_carry():
-    """Feeding chunk by chunk (max_chunks=1) equals one batch: the IQ state chains."""
+    """Feeding chunk by chunk (max_chunks=1) equals one batch: the IQ state chains.  The same on
+    the general IQ path (k_iqgain -> k_iqscan_c -> k_iqtiles) with 9000 small ragged chunks in one
+    batch, more than the 8192 that k_iqscan_c scans per round: against the oracle, offset included,
+    and against batches of 1000."""
+    import signals
     from gpu_util import chunked, plan_for
     from sdrterm_b200.engine import Engine
+    from sdrterm_b200.plan import build_plan
     raw, body, kw = case_stream('c1_fm_wav_int16')
     pl = plan_for(kw)
     chunks = chunked(body)
@@ -93,6 +98,23 @@ def test_batch_split_and_state_carry():
     with Engine(pl, max_chunks=2) as e3:
         c = e3.process(chunks)            # internal batching path
     assert rel_err(b, a) < 1e-13 and rel_err(c, a) < 1e-13
+
+    nch, cb = 9000, 1024                  # 256 samples per chunk at -d 50: 5 blocks + 6 samples
+    body = signals.c1_bytes(nch * cb // 4, seed=13, header=False)
+    kw = dict(fs=1_024_000, enc='h', center=15000, dec=50, demod='am', omega_out=5000, correct_iq=True,
+              vfos=None, simo=False, normalize=False, swap=False, big_endian=None, chunk_bytes=cb)
+    ch = orc.Chain(**kw)
+    pl = build_plan(kw['fs'], 'h', 50, ch.rows, correct_iq=True, demod='am', omega_out=5000, chunk_bytes=cb)
+    assert pl.rem != 0
+    with Engine(pl, max_chunks=nch) as e4:
+        whole = e4.process(body)
+        off = e4.iq_state
+    with Engine(pl, max_chunks=1000) as e5:
+        split = e5.process(body)
+    ref = ch.run(body)
+    assert whole.shape == ref.shape and rel_err(whole, ref) < TOL
+    assert abs(off - ch._off[0]) <= 1e-9 * max(1.0, abs(ch._off[0]))
+    assert rel_err(split, whole) < 1e-13
 
 
 def test_tc_long_stream_matches_oracle_and_fp64_path():
