@@ -18,7 +18,7 @@
 extern "C" {
 #endif
 
-#define SDRB_ABI_VERSION 8
+#define SDRB_ABI_VERSION 9
 #define SDRB_TILE_BLOCKS 32
 #define SDRB_NPOLES 8
 #define SDRB_MAX_DECIMATION 256
@@ -33,7 +33,12 @@ enum sdrb_status {
 
 /* SDRB_IQ is not a reference mode: the complex decimator output y itself, 2 doubles (Re, Im) per
  * output, no output low-pass (n_out_sections 0), no --smooth-output. */
-enum sdrb_demod { SDRB_FM = 0, SDRB_AM = 1, SDRB_RE = 2, SDRB_IM = 3, SDRB_IQ = 4 };
+/* SDRB_USB / SDRB_LSB are not reference modes either: single-sideband audio.  With B = omegaOut
+ * (0 < B < fs_d / 2, fs_d = fs / q) and the prototype h = ellip(3, 1, 30, B/2) at fs_d (out_sos,
+ * n_out_sections 2), each row is s[k] = Re(sum_m h[m] e^{j Omega m} y[k-m]), Omega = +pi B / fs_d
+ * (usb, the band [0, B] Hz) or -pi B / fs_d (lsb, [-B, 0] Hz): M doubles per chunk and row, from
+ * a zero filter state per chunk (or once per stream in seamless mode). */
+enum sdrb_demod { SDRB_FM = 0, SDRB_AM = 1, SDRB_RE = 2, SDRB_IM = 3, SDRB_IQ = 4, SDRB_USB = 5, SDRB_LSB = 6 };
 
 /* Geometry and switches of one processor.  Mirrors the keyword arguments that
  * src/misc/io_args.py:97-141 passes to DspProcessor/VfoProcessor and to readFile
@@ -57,7 +62,7 @@ typedef struct sdrb_config {
     int32_t N;               /* complex samples per chunk = 131072 / (2*itemsize) */
     int32_t edge;            /* sosfiltfilt pad length (27) */
     int32_t R;               /* rows: 1, or K+1 in --simo (vfo_processor.py:42-47) */
-    int32_t n_out_sections;  /* output low-pass SOS sections (0 for re/im/iq) */
+    int32_t n_out_sections;  /* output low-pass SOS sections (0 for re/im/iq; usb/lsb: the prototype's) */
     int32_t max_chunks;      /* largest number of chunks one sdrb_process* call will carry */
     double iq_L;             /* impedance / fs (read_file.py:65) */
     double norm_xmin;        /* read_file.py:177-196 */
@@ -132,6 +137,13 @@ typedef struct sdrb_tables {
     const double *PN;        /* [lookahead+1][8] complex: p_i^(N j) */
     const double *sos_AM;    /* [ns][ns]: A^M of the output cascade */
     const double *sos_CAM;   /* [M][ns]: c A^i, i < M */
+    /* single sideband (SDRB_USB / SDRB_LSB).  The band-pass is the rotated prototype
+     * (e^{j Omega} A, e^{j Omega} b, c, d); its segment and chunk maps are the real tables above times
+     * powers of e^{j Omega}: A'^L = e^{j Omega L} A^L, c'A'^k = e^{j Omega k} c A^k.  The kernels hold
+     * the 4 complex states in the frame of the chunk's first output (Weaver: y e^{-j Omega k} through
+     * the real cascade), so they need only the rotations. */
+    double ssb_omega;        /* Omega = +-pi B / fs_d */
+    const double *ssb_rot;   /* [M+1] complex: e^{j Omega k}, k = 0..M (k = M: the seamless chunk map) */
 } sdrb_tables;
 
 typedef struct sdrb_handle sdrb_handle;
@@ -240,12 +252,16 @@ long long sdrb_launch_count(const sdrb_handle *h);
  *   sdrb_am_demod   amDemod                                       demodulation.py:41-48
  *   sdrb_real_output / sdrb_imag_output                           demodulation.py:51-68
  *   sdrb_iq_output  y(R,M) c128 -> out(R,2M) f64, (Re, Im) interleaved (not a reference operator)
+ *   sdrb_ssb_demod  y(R,M) c128 -> out(R,M) f64: s = Re(e^{j omega k} sosfilt(sos, y e^{-j omega k})),
+ *                   the single-sideband band-pass of the prototype sos ([nsec][6], nsec 1..4) rotated
+ *                   by omega (0 < |omega| < pi/2), zero state per row, any M (not a reference operator)
  *   sdrb_shift_freq shiftFreq(y(N), shift(R,N), res(R,N))         demodulation.py:71-79 */
 int sdrb_fm_demod(int device, const double *y, int R, int M, double *out);
 int sdrb_am_demod(int device, const double *y, int R, int M, double *out);
 int sdrb_real_output(int device, const double *y, int R, int M, double *out);
 int sdrb_imag_output(int device, const double *y, int R, int M, double *out);
 int sdrb_iq_output(int device, const double *y, int R, int M, double *out);
+int sdrb_ssb_demod(int device, const double *y, int R, int M, const double *sos, int nsec, double omega, double *out);
 int sdrb_shift_freq(int device, const double *y, const double *shift, int R, int N, double *res);
 /* sdrb_fm_demod takes any even row length: 2*2^k rows run the FFT interpolation, other lengths a
  * dense scipy.signal.resample matrix built on the host in extended precision. */

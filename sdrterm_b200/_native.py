@@ -17,9 +17,9 @@ HEADER = os.path.join(ROOT, 'include', 'sdrterm_b200.h')
 SOURCES = [os.path.join(_HERE, 'csrc', f) for f in ('sdrb_api.cu', 'sdrb_kernels.cuh', 'sdrb_device.cuh', 'sdrb_tc.cuh', 'sdrb_finish.cuh',
                                                     'sdrb_spectrum.cuh', 'sdrb_seamless.cuh')]
 
-ABI_VERSION = 8
-FM, AM, RE, IM, IQ = 0, 1, 2, 3, 4
-DEMOD_CODE = {'fm': FM, 'am': AM, 're': RE, 'im': IM, 'iq': IQ}
+ABI_VERSION = 9
+FM, AM, RE, IM, IQ, USB, LSB = 0, 1, 2, 3, 4, 5, 6
+DEMOD_CODE = {'fm': FM, 'am': AM, 're': RE, 'im': IM, 'iq': IQ, 'usb': USB, 'lsb': LSB}
 
 
 class SdrbError(RuntimeError):
@@ -55,7 +55,8 @@ class Tables(C.Structure):
                 ('tc_Bq', C.POINTER(C.c_int8)), ('tc_cst', _DP), ('tc_rowc', _DP),
                 ('tc_xor', C.c_uint8 * 16),
                 ('lookahead', C.c_int32), ('fs', C.c_int64), ('chunk_step', C.POINTER(C.c_int64)),
-                ('PN', _DP), ('sos_AM', _DP), ('sos_CAM', _DP)]
+                ('PN', _DP), ('sos_AM', _DP), ('sos_CAM', _DP),
+                ('ssb_omega', C.c_double), ('ssb_rot', _DP)]
 
 
 EXPORTS = ['sdrb_create', 'sdrb_destroy', 'sdrb_last_error', 'sdrb_outputs_per_chunk',
@@ -66,7 +67,7 @@ EXPORTS = ['sdrb_create', 'sdrb_destroy', 'sdrb_last_error', 'sdrb_outputs_per_c
            'sdrb_set_profiling', 'sdrb_kernel_times', 'sdrb_keep_decimated', 'sdrb_read_debug', 'sdrb_iq_export_device',
            'sdrb_iq_prefix_device', 'sdrb_decode_iq', 'sdrb_correct_iq', 'sdrb_keep_x0', 'sdrb_read_x0', 'sdrb_iq_gain', 'sdrb_set_smooth', 'sdrb_host_alloc', 'sdrb_host_free', 'sdrb_reserve_sms',
            'sdrb_stream', 'sdrb_stream_device', 'sdrb_stream_end', 'sdrb_stream_end_device', 'sdrb_stream_lookahead',
-           'sdrb_row_doubles', 'sdrb_iq_output']
+           'sdrb_row_doubles', 'sdrb_iq_output', 'sdrb_ssb_demod']
 
 
 def nvcc_command(out: str = LIB_PATH) -> list[str]:
@@ -125,6 +126,7 @@ def lib():
         L.sdrb_launch_count.restype = C.c_longlong
         for name in ('sdrb_fm_demod', 'sdrb_am_demod', 'sdrb_real_output', 'sdrb_imag_output', 'sdrb_iq_output'):
             getattr(L, name).argtypes = [C.c_int, vp, C.c_int, C.c_int, vp]
+        L.sdrb_ssb_demod.argtypes = [C.c_int, vp, C.c_int, C.c_int, vp, C.c_int, C.c_double, vp]
         L.sdrb_shift_freq.argtypes = [C.c_int, vp, vp, C.c_int, C.c_int, vp]
         L.sdrb_power_spectrum.argtypes = [C.c_int, vp, vp, C.c_int, C.c_int, vp]
         L.sdrb_stft_db.argtypes = [C.c_int, vp, vp, C.c_int, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp]

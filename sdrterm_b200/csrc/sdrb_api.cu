@@ -152,6 +152,9 @@ inline double2 c2(const double *a, size_t i) { return make_double2(a[2 * i], a[2
 inline double2 hmul(double2 a, double2 b) { return make_double2(a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x); }
 
 bool is_pow2(int v) { return v > 0 && (v & (v - 1)) == 0; }
+bool is_ssb(int demod) { return demod == SDRB_USB || demod == SDRB_LSB; }
+// the finish-kernel instance of a demodulation (OUT_REAL / OUT_IQ / OUT_SSB)
+int out_kind(int demod) { return demod == SDRB_IQ ? OUT_IQ : (is_ssb(demod) ? OUT_SSB : OUT_REAL); }
 
 std::vector<double2> make_twiddles(int n)
 {
@@ -325,9 +328,11 @@ int launch_chain_t(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, 
         const size_t items = nch * (size_t)pl.R;
         const unsigned grid = (unsigned)std::min<size_t>((items + FIN_WARPS - 1) / FIN_WARPS, (size_t)(h->num_sms - h->reserved_sms) * 2);
         if (pl.demod == SDRB_IQ)
-            k_finish<ENC, true><<<grid, 32 * FIN_WARPS, h->finish_smem, st>>>(pl, h->sc, raw, out, (int)nch, h->keep_y);
+            k_finish<ENC, OUT_IQ><<<grid, 32 * FIN_WARPS, h->finish_smem, st>>>(pl, h->sc, raw, out, (int)nch, h->keep_y);
+        else if (is_ssb(pl.demod))
+            k_finish<ENC, OUT_SSB><<<grid, 32 * FIN_WARPS, h->finish_smem, st>>>(pl, h->sc, raw, out, (int)nch, h->keep_y);
         else
-            k_finish<ENC, false><<<grid, 32 * FIN_WARPS, h->finish_smem, st>>>(pl, h->sc, raw, out, (int)nch, h->keep_y);
+            k_finish<ENC, OUT_REAL><<<grid, 32 * FIN_WARPS, h->finish_smem, st>>>(pl, h->sc, raw, out, (int)nch, h->keep_y);
         h->launches++;
         mark(3);
         mark(4);
@@ -336,11 +341,14 @@ int launch_chain_t(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, 
         h->launches++;
         mark(3);
         if (pl.demod == SDRB_IQ)
-            k_demod<true><<<(unsigned)(nch * pl.R), 128, 0, st>>>(pl, h->sc.y, out, nullptr, nullptr, (int)nch, pl.demod, 0,
-                                                                  pl.be_out);
+            k_demod<OUT_IQ><<<(unsigned)(nch * pl.R), 128, 0, st>>>(pl, h->sc.y, out, nullptr, nullptr, (int)nch, pl.demod, 0,
+                                                                    pl.be_out);
+        else if (is_ssb(pl.demod))
+            k_demod<OUT_SSB><<<(unsigned)(nch * pl.R), 128, h->demod_smem, st>>>(pl, h->sc.y, out, h->sc.fftbuf, h->sc.zrow,
+                                                                                 (int)nch, pl.demod, 1, pl.be_out);
         else
-            k_demod<false><<<(unsigned)(nch * pl.R), 128, h->demod_smem, st>>>(pl, h->sc.y, out, h->sc.fftbuf, h->sc.zrow,
-                                                                               (int)nch, pl.demod, 1, pl.be_out);
+            k_demod<OUT_REAL><<<(unsigned)(nch * pl.R), 128, h->demod_smem, st>>>(pl, h->sc.y, out, h->sc.fftbuf, h->sc.zrow,
+                                                                                  (int)nch, pl.demod, 1, pl.be_out);
         h->launches++;
         mark(4);
     }
@@ -370,9 +378,11 @@ template <int ENC, bool IQ>
 int set_smem_attr_t(sdrb_handle *h)
 {
     CK(h, cudaFuncSetAttribute(k_main<ENC, IQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->main_smem));
-    if (h->finish_on)
-        CK(h, cudaFuncSetAttribute(h->pl.demod == SDRB_IQ ? k_finish<ENC, true> : k_finish<ENC, false>,
+    if (h->finish_on) {
+        const int ok = out_kind(h->pl.demod);
+        CK(h, cudaFuncSetAttribute(ok == OUT_IQ ? k_finish<ENC, OUT_IQ> : (ok == OUT_SSB ? k_finish<ENC, OUT_SSB> : k_finish<ENC, OUT_REAL>),
                                    cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->finish_smem));
+    }
     return 0;
 }
 int set_smem_attr(sdrb_handle *h)
@@ -422,9 +432,20 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
         if (cfg->n_out_sections > 0 && !tab->out_sos) return fail(nullptr, SDRB_ERR_ARG, "out_sos is NULL");
     }
     if (cfg->N / cfg->q < 1) return fail(nullptr, SDRB_ERR_ARG, "chunk shorter than one block");
-    if (cfg->demod > SDRB_IQ) return fail(nullptr, SDRB_ERR_ARG, "unknown demodulation %d", (int)cfg->demod);
+    if (cfg->demod > SDRB_LSB) return fail(nullptr, SDRB_ERR_ARG, "unknown demodulation %d", (int)cfg->demod);
     if (cfg->demod == SDRB_IQ && cfg->n_out_sections != 0)
         return fail(nullptr, SDRB_ERR_ARG, "iq output has no output low-pass (n_out_sections must be 0)");
+    if (is_ssb(cfg->demod)) {
+        // the band-pass is the rotated prototype: sections, a rotation inside (0, pi/2) of the
+        // sideband's sign, and the table of its powers that matches it
+        const double om = tab->ssb_omega, sgn = cfg->demod == SDRB_USB ? 1.0 : -1.0;
+        if (cfg->n_out_sections < 1 || !tab->out_sos || !tab->ssb_rot || !(sgn * om > 0.0) || !(sgn * om < M_PI / 2))
+            return fail(nullptr, SDRB_ERR_ARG, "usb/lsb needs the prototype sections and a rotation 0 < %s < pi/2 (got %g)",
+                        cfg->demod == SDRB_USB ? "Omega" : "-Omega", om);
+        if (std::fabs(tab->ssb_rot[0] - 1.0) > 1e-12 || std::fabs(tab->ssb_rot[1]) > 1e-12 ||
+            std::fabs(tab->ssb_rot[2] - std::cos(om)) > 1e-12 || std::fabs(tab->ssb_rot[3] - std::sin(om)) > 1e-12)
+            return fail(nullptr, SDRB_ERR_ARG, "ssb_rot does not start 1, e^{j Omega}");
+    }
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
         return fail(nullptr, SDRB_ERR_CUDA, "no CUDA device: libsdrterm_b200 has no CPU fallback");
@@ -444,6 +465,7 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
     pl.q = cfg->q; pl.N = cfg->N; pl.edge = cfg->edge; pl.L = cfg->N + 2 * cfg->edge;
     pl.Mf = cfg->N / cfg->q; pl.rem = cfg->N - pl.Mf * cfg->q; pl.M = pl.Mf + (pl.rem ? 1 : 0);
     pl.W = cfg->demod == SDRB_IQ ? 2 * pl.M : pl.M;
+    pl.ssb_omega = is_ssb(cfg->demod) ? tab->ssb_omega : 0.0;
     pl.ntiles = (pl.Mf + SDRB_TB - 1) / SDRB_TB; pl.cnt_last = pl.Mf - (pl.ntiles - 1) * SDRB_TB;
     pl.Hq = (cfg->q + 1) / 2; pl.KS = (pl.Hq + 3) / 4; pl.R = cfg->R;
     pl.RL = tab->RL;
@@ -553,6 +575,8 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
     if (cfg->n_out_sections > 0) UP(upload(h, tab->sos_CA, (size_t)pl.sos_Lseg * pl.sos_ns, &pl.sos_CA));
     pl.fm_interp = nullptr;
     if (cfg->demod == SDRB_FM && !pl.fft_ok) UP(upload(h, tab->fm_interp, (size_t)M * h2, &pl.fm_interp));
+    pl.ssb_rot = nullptr;
+    if (is_ssb(cfg->demod)) UP(upload(h, reinterpret_cast<const double2 *>(tab->ssb_rot), (size_t)M + 1, &pl.ssb_rot));
 
     // launch geometry
     auto smem_for = [&](int tpc, int w) {
@@ -590,7 +614,8 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
     pl.demod_in_smem = dsm <= 96 * 1024 ? 1 : 0;
     h->demod_smem = pl.demod_in_smem ? dsm : 0;
     if (h->demod_smem > 48 * 1024)
-        if (cudaFuncSetAttribute(k_demod<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->demod_smem) != cudaSuccess)
+        if (cudaFuncSetAttribute(is_ssb(cfg->demod) ? k_demod<OUT_SSB> : k_demod<OUT_REAL>,
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->demod_smem) != cudaSuccess)
             return bail(fail(h, SDRB_ERR_CUDA, "cudaFuncSetAttribute(k_demod) failed"));
 
     // scratch for max_chunks (seamless: plus the D chunks held back between calls)
@@ -637,12 +662,13 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
         UP(dalloc(h, nch * R * 8, &sd.G));
         UP(dalloc(h, nch * R * 24, &sd.cin));
         UP(dalloc(h, nch * R * (M + 1), &sd.ybuf));
-        UP(dalloc(h, nch * R * SEAM_NS, &sd.echunk));
-        UP(dalloc(h, nch * R * SEAM_NS, &sd.sst));
+        const size_t sn = (size_t)SEAM_NS * (is_ssb(cfg->demod) ? 2 : 1);   // doubles per SOS state (usb / lsb: complex)
+        UP(dalloc(h, nch * R * sn, &sd.echunk));
+        UP(dalloc(h, nch * R * sn, &sd.sst));
         UP(dalloc(h, (size_t)R * 8, &sd.fwd));
-        UP(dalloc(h, (size_t)R * SEAM_NS, &sd.sos));
+        UP(dalloc(h, (size_t)R * sn, &sd.sos));
         UP(dalloc(h, (size_t)R * 16, &sd.endv));
-        if (cudaMemset(sd.sos, 0, (size_t)R * SEAM_NS * sizeof(double)) != cudaSuccess)
+        if (cudaMemset(sd.sos, 0, (size_t)R * sn * sizeof(double)) != cudaSuccess)
             return bail(fail(h, SDRB_ERR_CUDA, "memset failed"));
     }
 #undef UP
@@ -842,12 +868,20 @@ int seam_step(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, cudaS
         const unsigned wg = (unsigned)((items + 7) / 8);
         k_seam_carry<<<wg, 256, 0, st>>>(pl, h->sc, sd, ne, h->nwin, g0, end ? 1 : 0);
         k_seam_y<<<wg, 256, 0, st>>>(pl, h->sc, sd, ne, h->nwin, g0, end ? 1 : 0);
-        k_seam_demod<<<wg, 256, 0, st>>>(pl, sd, out, ne, h->nwin, end ? 1 : 0);
+        const bool ssb = is_ssb(pl.demod);
+        if (ssb) k_seam_demod<true><<<wg, 256, 0, st>>>(pl, sd, out, ne, h->nwin, end ? 1 : 0);
+        else k_seam_demod<false><<<wg, 256, 0, st>>>(pl, sd, out, ne, h->nwin, end ? 1 : 0);
         h->launches += 3;
         if (pl.nsec_out) {
-            k_seam_sscan<<<(unsigned)R, 32, 0, st>>>(pl, sd, ne);
             const size_t total = items * M;
-            k_seam_frame<<<(unsigned)std::min<size_t>((total + 255) / 256, (size_t)h->num_sms * 16), 256, 0, st>>>(pl, sd, out, ne);
+            const unsigned fg = (unsigned)std::min<size_t>((total + 255) / 256, (size_t)h->num_sms * 16);
+            if (ssb) {
+                k_seam_sscan<double2><<<(unsigned)R, 32, 0, st>>>(pl, sd, ne);
+                k_seam_frame<true><<<fg, 256, 0, st>>>(pl, sd, out, ne);
+            } else {
+                k_seam_sscan<double><<<(unsigned)R, 32, 0, st>>>(pl, sd, ne);
+                k_seam_frame<false><<<fg, 256, 0, st>>>(pl, sd, out, ne);
+            }
             h->launches += 2;
         }
         CK(h, cudaGetLastError());
@@ -868,7 +902,7 @@ int seam_step(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, cudaS
     if (end) {   // a new stream starts from scratch: counters, output filter and IQ corrector
         h->seen = h->emitted = 0;
         h->nwin = 0;
-        CK(h, cudaMemsetAsync(sd.sos, 0, (size_t)R * SEAM_NS * sizeof(double), st));
+        CK(h, cudaMemsetAsync(sd.sos, 0, (size_t)R * SEAM_NS * (is_ssb(pl.demod) ? 2 : 1) * sizeof(double), st));
         CK(h, cudaMemsetAsync(h->sc.iq_state, 0, sizeof(double2), st));
     }
     return 0;
@@ -1223,10 +1257,10 @@ static int demod_op(int device, const double *y, int R, int M, double *out, int 
     pl.tw = d_tw.as<double2>();
     // rows are laid out [R][M]: run as R "rows" of a single chunk
     if (demod == SDRB_IQ)
-        k_demod<true><<<R, 128, 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), nullptr, nullptr, 1, demod, 0, 0);
+        k_demod<OUT_IQ><<<R, 128, 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), nullptr, nullptr, 1, demod, 0, 0);
     else
-        k_demod<false><<<R, 128, pl.demod_in_smem ? dsm : 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), d_fft.as<double2>(),
-                                                               d_z.as<double>(), 1, demod, 0, 0);
+        k_demod<OUT_REAL><<<R, 128, pl.demod_in_smem ? dsm : 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), d_fft.as<double2>(),
+                                                                  d_z.as<double>(), 1, demod, 0, 0);
     CK(nullptr, cudaGetLastError());
     CK(nullptr, cudaDeviceSynchronize());
     CK(nullptr, cudaMemcpy(out, d_out.p, (size_t)R * pl.W * sizeof(double), cudaMemcpyDeviceToHost));
@@ -1238,6 +1272,83 @@ int sdrb_am_demod(int device, const double *y, int R, int M, double *out) { retu
 int sdrb_real_output(int device, const double *y, int R, int M, double *out) { return demod_op(device, y, R, M, out, SDRB_RE); }
 int sdrb_imag_output(int device, const double *y, int R, int M, double *out) { return demod_op(device, y, R, M, out, SDRB_IM); }
 int sdrb_iq_output(int device, const double *y, int R, int M, double *out) { return demod_op(device, y, R, M, out, SDRB_IQ); }
+
+int sdrb_ssb_demod(int device, const double *y, int R, int M, const double *sos, int nsec, double omega, double *out)
+{
+    if (!y || !out || !sos || R < 1 || M < 1 || nsec < 1 || nsec > 4) return fail(nullptr, SDRB_ERR_ARG, "bad argument");
+    if (!(std::fabs(omega) > 0.0) || !(std::fabs(omega) < M_PI / 2))
+        return fail(nullptr, SDRB_ERR_ARG, "ssb rotation %g outside 0 < |omega| < pi/2", omega);
+    for (int s = 0; s < nsec; s++)
+        if (sos[6 * s + 3] != 1.0) return fail(nullptr, SDRB_ERR_ARG, "sos section %d is not normalised (a0 != 1)", s);
+    int rc = need_device(device);
+    if (rc) return rc;
+    DevPlan pl{};
+    pl.M = pl.W = M; pl.R = R; pl.nsec_out = nsec; pl.sos_ns = 2 * nsec; pl.sos_Lseg = (M + 31) / 32;
+    pl.ssb_omega = omega;
+    for (int i = 0; i < 6 * nsec; i++) pl.out_sos[i] = sos[i];
+    // the prototype's state space (A, c) in extended precision -- the same DF2T state variables as
+    // plan.py's _cascade_state_space -- then A^Lseg, c A^i (i < Lseg) and e^{j omega k} (k <= M)
+    const int ns = pl.sos_ns, Ls = pl.sos_Lseg;
+    std::vector<long double> A((size_t)ns * ns, 0.0L), cvec(ns, 0.0L);
+    {
+        std::vector<long double> u(ns + 1, 0.0L);
+        u[ns] = 1.0L;
+        for (int k = 0; k < nsec; k++) {
+            const long double b0 = sos[6 * k], b1 = sos[6 * k + 1], b2 = sos[6 * k + 2], a1 = sos[6 * k + 4], a2 = sos[6 * k + 5];
+            std::vector<long double> yv(ns + 1), z0(ns + 1), z1(ns + 1);
+            for (int j = 0; j <= ns; j++) yv[j] = b0 * u[j];
+            yv[2 * k] += 1.0L;
+            for (int j = 0; j <= ns; j++) { z0[j] = b1 * u[j] - a1 * yv[j]; z1[j] = b2 * u[j] - a2 * yv[j]; }
+            z0[2 * k + 1] += 1.0L;
+            for (int j = 0; j < ns; j++) { A[(size_t)(2 * k) * ns + j] = z0[j]; A[(size_t)(2 * k + 1) * ns + j] = z1[j]; }
+            u = yv;
+        }
+        for (int j = 0; j < ns; j++) cvec[j] = u[j];
+    }
+    std::vector<double> ca((size_t)Ls * ns);
+    std::vector<long double> P((size_t)ns * ns, 0.0L), cur = cvec;
+    for (int i = 0; i < ns; i++) P[(size_t)i * ns + i] = 1.0L;
+    for (int i = 0; i < Ls; i++) {
+        for (int j = 0; j < ns; j++) ca[(size_t)i * ns + j] = (double)cur[j];
+        std::vector<long double> nx(ns, 0.0L), NP((size_t)ns * ns, 0.0L);
+        for (int j = 0; j < ns; j++)
+            for (int b = 0; b < ns; b++) nx[j] += cur[b] * A[(size_t)b * ns + j];
+        for (int a = 0; a < ns; a++)
+            for (int b = 0; b < ns; b++)
+                for (int k = 0; k < ns; k++) NP[(size_t)a * ns + b] += A[(size_t)a * ns + k] * P[(size_t)k * ns + b];
+        cur = nx;
+        P = NP;
+    }
+    for (int i = 0; i < ns * ns; i++) pl.sos_AL[i] = (double)P[i];       // A^Lseg
+    std::vector<double2> rot((size_t)M + 1);
+    for (int k = 0; k <= M; k++) {
+        const long double a = (long double)omega * (long double)k;
+        rot[k] = make_double2((double)cosl(a), (double)sinl(a));
+    }
+    DevBuf d_y, d_out, d_fft, d_z, d_ca, d_rot;
+    const size_t dsm = (size_t)M * (2 * sizeof(double2) + sizeof(double));
+    pl.demod_in_smem = dsm <= 48 * 1024;
+    CK(nullptr, d_y.alloc((size_t)R * M * sizeof(double2)));
+    CK(nullptr, d_out.alloc((size_t)R * M * sizeof(double)));
+    CK(nullptr, d_ca.alloc(ca.size() * sizeof(double)));
+    CK(nullptr, d_rot.alloc(rot.size() * sizeof(double2)));
+    if (!pl.demod_in_smem) {
+        CK(nullptr, d_fft.alloc((size_t)R * 2 * M * sizeof(double2)));
+        CK(nullptr, d_z.alloc((size_t)R * M * sizeof(double)));
+    }
+    CK(nullptr, cudaMemcpy(d_y.p, y, (size_t)R * M * sizeof(double2), cudaMemcpyHostToDevice));
+    CK(nullptr, cudaMemcpy(d_ca.p, ca.data(), ca.size() * sizeof(double), cudaMemcpyHostToDevice));
+    CK(nullptr, cudaMemcpy(d_rot.p, rot.data(), rot.size() * sizeof(double2), cudaMemcpyHostToDevice));
+    pl.sos_CA = d_ca.as<double>();
+    pl.ssb_rot = d_rot.as<double2>();
+    // rows are laid out [R][M]: run as R "rows" of a single chunk
+    k_demod<OUT_SSB><<<R, 128, pl.demod_in_smem ? dsm : 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), d_fft.as<double2>(),
+                                                             d_z.as<double>(), 1, SDRB_USB, 1, 0);
+    CK(nullptr, cudaGetLastError());
+    CK(nullptr, cudaDeviceSynchronize());
+    CK(nullptr, cudaMemcpy(out, d_out.p, (size_t)R * M * sizeof(double), cudaMemcpyDeviceToHost));
+    return SDRB_OK;
+}
 
 int sdrb_shift_freq(int device, const double *y, const double *shift, int R, int N, double *res)
 {

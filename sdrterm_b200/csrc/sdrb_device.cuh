@@ -65,7 +65,15 @@ struct DevPlan {
     const double *sos_CA;     // [sos_Lseg][ns]  c A^i
     const unsigned char *use_nco;  // [R]
     int W;                 // doubles per chunk-row of the output: 2M for iq ((Re, Im) pairs), M otherwise
+    // usb / lsb: the band-pass h[m] e^{j Omega m} runs in the Weaver frame, u[k] = y[k] e^{-j Omega k}
+    // through the real prototype out_sos (Re and Im alike), s[k] = Re(e^{j Omega k} v[k])
+    double ssb_omega;      // +pi B / fs_d (usb), -pi B / fs_d (lsb); 0 otherwise
+    const double2 *ssb_rot;   // [M+1] e^{j Omega k}, k = 0..M
 };
+
+// What a finish kernel instance writes: a real row from a demodulator (fm / am / re / im, output
+// low-pass), the complex decimator output itself (iq), or the single-sideband audio (usb / lsb).
+enum { OUT_REAL = 0, OUT_IQ = 1, OUT_SSB = 2 };
 
 // ---------------------------------------------------------------- complex helpers (double2)
 __device__ __forceinline__ double2 cmul(double2 a, double2 b)

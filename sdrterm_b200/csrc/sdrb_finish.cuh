@@ -5,10 +5,14 @@
 //   2. carries of the 8 forward / 8 anticausal modal states across the tiles of the chunk
 //   3. decimated outputs y[k] = partial output of the front end + carry-in response (+ boundary)
 //   4. demodulation: fm (pair phase, 2x trigonometric interpolation by a real-input FFT of half
-//      the length and its inverse) | am | re | im; the iq instance (IQO) stores y straight from
+//      the length and its inverse) | am | re | im; the iq instance (OUT_IQ) stores y straight from
 //      registers instead, (Re, Im) per output, and skips 3b-5
 //   5. output low-pass (zero initial state per chunk) in 32 lane segments, chained by a
 //      Kogge-Stone scan of the segment maps; framing (native or big-endian doubles)
+//   The usb / lsb instance (OUT_SSB) skips 3b and 4: it stages y in the warp's shared memory (Re in
+//   zrow, Im in the carry rows as they fall dead) and runs the complex band-pass as 32 lane
+//   segments in the Weaver frame (zero-state pass, 5-level scan of the complex 4-state segment maps,
+//   the response to the composed states), then frames the real part.
 //
 // It replaces k_fixup + k_demod for the common shapes (whole tiles, M a power of two <= 1024, at
 // most 2 output sections); those two kernels remain the general path.  Nothing leaves the SM
@@ -123,13 +127,22 @@ __device__ __forceinline__ double2 *fin_fft(double2 *src, double2 *dst, int n, i
     return src;
 }
 
+// usb / lsb staging layout: output k of lane segment g = k >> lsh sits at g*Ls + ((k + g) mod Ls), a
+// rotation inside its own aligned segment -- conflict-free both for the lane <-> block writes of
+// phase 3 and for the lane <-> segment passes, and it never leaves the 32-output tile of k (Ls <= 32)
+__device__ __forceinline__ int fin_ssb_at(int k, int lsh, int Ls)
+{
+    const int g = k >> lsh;
+    return (g << lsh) | ((k + g) & (Ls - 1));
+}
+
 __device__ __forceinline__ double fin_demod_scalar(double2 a, int demod)
 {
     if (demod == 1) return hypot(fma(a.x, a.x, -a.y * a.y), 2.0 * a.x * a.y);   // abs(square(z))
     return demod == 2 ? a.x : a.y;
 }
 
-template <int ENC, bool IQO>
+template <int ENC, int OUT>
 __global__ void __launch_bounds__(32 * FIN_WARPS, 2)
 k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc, const uint8_t *__restrict__ raw,
          double *__restrict__ out, int nchunks, int keep_y)
@@ -418,7 +431,7 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
                     if (keep_y) yg[k] = v;
                     yv[u] = v;
                 }
-                if constexpr (IQO) {
+                if constexpr (OUT == OUT_IQ) {
                     // 16 contiguous bytes per lane, 512 per warp and tile: no trip through zrow
                     double2 *o2 = reinterpret_cast<double2 *>(out + ((size_t)r * nchunks + chunk) * pl.W);
 #pragma unroll
@@ -426,6 +439,16 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
                         double2 v = yv[u];
                         if (pl.be_out) v = make_double2(bswap_double(v.x), bswap_double(v.y));
                         o2[(t0 + u) * SDRB_TB + lane] = v;
+                    }
+                } else if constexpr (OUT == OUT_SSB) {
+                    // Re y -> zrow; Im y -> the carry rows t0, t0+1, dead once every lane has read them
+                    __syncwarp();
+                    double *zim = reinterpret_cast<double *>(carry);
+#pragma unroll
+                    for (int u = 0; u < 2; u++) {
+                        const int a = fin_ssb_at((t0 + u) * SDRB_TB + lane, lsh, Ls);
+                        zrow[a] = yv[u].x;
+                        zim[a] = yv[u].y;
                     }
                 } else if (pl.demod == 0) {
                     const bool odd = lane & 1;
@@ -449,7 +472,7 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
         __syncwarp();
         FIN_DBG(7);
         // ---------------------------------------------------------------- 3b. fm: 2x interpolation
-        if (!IQO && pl.demod == 0) {
+        if (OUT == OUT_REAL && pl.demod == 0) {
             // even outputs of scipy.signal.resample(ph, 2h) are the phases themselves (already in
             // zrow), the odd ones come from the half-sample-shifted spectrum.  Forward FFT of
             // z[m] = ph[2m] + i ph[2m+1], n2 = h/2 points
@@ -493,7 +516,7 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
         }
         FIN_DBG(8);
         // ---------------------------------------------------------------- 4. output low-pass
-        if (!IQO && pl.nsec_out > 0) {
+        if (OUT == OUT_REAL && pl.nsec_out > 0) {
             double *zs = zrow + (size_t)lane * (Ls + 1);
             const double *c0 = pl.out_sos, *c1 = pl.out_sos + 6;
             double s0 = 0, s1 = 0, s2 = 0, s3 = 0;
@@ -531,12 +554,51 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
             }
             __syncwarp();
         }
+        // ---------------------------------------------------------------- 4'. usb / lsb band-pass
+        // u[k] = y[k] e^{-j Omega k} through the real prototype in lane segments of Ls outputs
+        // (e^{j Omega k} by recurrence from the segment start), the segment maps composed by the
+        // lane scan, every output then gets c A^j s_in of its segment; s[k] = Re(e^{j Omega k} v[k])
+        if constexpr (OUT == OUT_SSB) {
+            double *zim = reinterpret_cast<double *>(carry);
+            const int lo = lane * Ls;
+            const double2 e1 = pl.ssb_rot[1], r0 = pl.ssb_rot[lo];
+            double2 st[4], ph = r0;
+#pragma unroll
+            for (int a = 0; a < 4; a++) st[a] = make_double2(0.0, 0.0);
+#pragma unroll 2
+            for (int j = 0; j < Ls; j++) {
+                const int a = lo + ((j + lane) & (Ls - 1));
+                const double2 v = ssb_step<2>(pl.out_sos, 2, st, cmul(make_double2(zrow[a], zim[a]), cconj(ph)));
+                zrow[a] = v.x;
+                zim[a] = v.y;
+                ph = cmul(ph, e1);
+            }
+            ssb_lane_scan(pl.sos_AP, st, lane);
+            double2 si[4];
+#pragma unroll
+            for (int a = 0; a < 4; a++) {
+                si[a] = shfl_up_c(st[a], 1);
+                if (lane == 0) si[a] = make_double2(0.0, 0.0);
+            }
+            ph = r0;
+#pragma unroll 2
+            for (int j = 0; j < Ls; j++) {
+                const int a = lo + ((j + lane) & (Ls - 1));
+                const double *ca = pl.sos_CA + (size_t)j * 4;
+                double vx = zrow[a], vy = zim[a];
+#pragma unroll
+                for (int b = 0; b < 4; b++) { vx = fma(ca[b], si[b].x, vx); vy = fma(ca[b], si[b].y, vy); }
+                zrow[a] = fma(ph.x, vx, -ph.y * vy);
+                ph = cmul(ph, e1);
+            }
+            __syncwarp();
+        }
         FIN_DBG(9);
         // ---------------------------------------------------------------- 5. framing
-        if constexpr (!IQO) {
+        if constexpr (OUT != OUT_IQ) {
             double *o = out + ((size_t)r * nchunks + chunk) * M;
             for (int k = lane; k < M; k += 32) {
-                const double v = zrow[k + (k >> lsh)];
+                const double v = zrow[OUT == OUT_SSB ? fin_ssb_at(k, lsh, Ls) : k + (k >> lsh)];
                 o[k] = pl.be_out ? bswap_double(v) : v;
             }
             __syncwarp();

@@ -14,15 +14,19 @@
 //                  over the next D chunks or the real end, zeta) and the fm halo y[k+1]
 //   k_seam_y       per emitted chunk: tile carries and the decimated outputs, global frame
 //   k_seam_demod   demodulation + output SOS from the chunk's zero state (segments, lane scan);
-//                  iq: y itself, (Re, Im) pairs
-//   k_seam_sscan   output SOS state across chunks: affine scan with the matrix A^M
-//   k_seam_frame   response to the carried SOS state, framing
+//                  iq: y itself, (Re, Im) pairs; usb / lsb (SSB instance): the complex band-pass
+//                  from the chunk's zero state, its real part and the complex end state
+//   k_seam_sscan   output SOS state across chunks: affine scan with the matrix A^M (real states), or
+//                  e^{j Omega M} A^M (usb / lsb: complex states in the frame of each chunk's start)
+//   k_seam_frame   response to the carried SOS state (usb / lsb: Re(e^{j Omega k} c A^k s_c)), framing
 //
 // tests/seamless_ref.py (SeamlessTwin) is the numpy twin of this decomposition.
 #pragma once
+#include <type_traits>
 #include "sdrb_kernels.cuh"
 
-#define SEAM_NS 4           // output SOS state size in seamless mode (ellip(3): two sections)
+#define SEAM_NS 4           // output SOS state size in seamless mode (ellip(3): two sections); usb / lsb
+                            // carry SEAM_NS complex states (echunk, sst and sos hold double2 then)
 
 struct SeamDev {
     int D;                     // lookahead in chunks
@@ -38,12 +42,25 @@ struct SeamDev {
     double2 *G;                // [W][R][8]    forward state at the chunk start, global frame
     double2 *cin;              // [W][R][24]   carry-ins in the chunk frame: Win0, Tn_end, zeta
     double2 *ybuf;             // [W][R][M+1]  decimated outputs (global frame) + halo
-    double *echunk;            // [W][R][ns]   SOS end state of a chunk from a zero state
+    double *echunk;            // [W][R][ns]   SOS end state of a chunk from a zero state (usb / lsb: ns complex)
     double *sst;               // [W][R][ns]   SOS state at the chunk start (after k_seam_sscan)
     double2 *fwd;              // [R][8]       forward state at the next new chunk
-    double *sos;               // [R][ns]      SOS state at the next chunk to emit
+    double *sos;               // [R][ns]      SOS state at the next chunk to emit (usb / lsb: ns complex)
     double2 *endv;             // [R][16]      real end: 0..7 anticausal state, 8..15 zeta (global frame)
 };
+
+// the output SOS state of k_seam_sscan: real (fm / am) or complex (usb / lsb)
+template <typename T> __device__ __forceinline__ T seam_zero();
+template <> __device__ __forceinline__ double seam_zero<double>() { return 0.0; }
+template <> __device__ __forceinline__ double2 seam_zero<double2>() { return make_double2(0.0, 0.0); }
+__device__ __forceinline__ double seam_fma(double a, double x, double acc) { return fma(a, x, acc); }
+__device__ __forceinline__ double2 seam_fma(double a, double2 x, double2 acc) { return make_double2(fma(a, x.x, acc.x), fma(a, x.y, acc.y)); }
+__device__ __forceinline__ double seam_add(double a, double b) { return a + b; }
+__device__ __forceinline__ double2 seam_add(double2 a, double2 b) { return cadd(a, b); }
+__device__ __forceinline__ double seam_rot(double2, double x) { return x; }            // real states: no phasor
+__device__ __forceinline__ double2 seam_rot(double2 ph, double2 x) { return cmul(ph, x); }
+__device__ __forceinline__ double seam_shfl_up(double v, int d) { return __shfl_up_sync(0xffffffffu, v, d); }
+__device__ __forceinline__ double2 seam_shfl_up(double2 v, int d) { return shfl_up_c(v, d); }
 
 __device__ __forceinline__ double2 seam_phasor(const SeamDev &sd, int r, long long g)
 {
@@ -314,11 +331,45 @@ __device__ __forceinline__ void seam_sos_step(const double *sos, int nsec, doubl
     }
 }
 
+// usb / lsb of one (chunk, row), lane <-> segment: the Weaver-frame row u[k] = y[k] e^{-j Omega k}
+// (k from the chunk start) through the real prototype from a zero state, the lane scan, the segment
+// re-run from its composed state; out = Re(e^{j Omega k} v[k]), the complex end state -> echunk
+__device__ __forceinline__ void seam_ssb_demod(const DevPlan &pl, const SeamDev &sd, const double2 *y, double *o,
+                                               size_t ei, int lane)
+{
+    const int Ls = pl.sos_Lseg, lo = lane * Ls;
+    const double2 e1 = pl.ssb_rot[1], r0 = pl.ssb_rot[lo];
+    double2 st[SEAM_NS], ph = r0;
+#pragma unroll
+    for (int j = 0; j < SEAM_NS; j++) st[j] = make_double2(0.0, 0.0);
+    for (int k = lo; k < lo + Ls; k++) {
+        ssb_step<2>(pl.out_sos, 2, st, cmul(y[k], cconj(ph)));
+        ph = cmul(ph, e1);
+    }
+    ssb_lane_scan(pl.sos_AP, st, lane);
+    double2 si[SEAM_NS];
+#pragma unroll
+    for (int j = 0; j < SEAM_NS; j++) {
+        si[j] = shfl_up_c(st[j], 1);
+        if (lane == 0) si[j] = make_double2(0.0, 0.0);
+    }
+    if (lane == 31)
+        for (int j = 0; j < SEAM_NS; j++) reinterpret_cast<double2 *>(sd.echunk)[ei * SEAM_NS + j] = st[j];
+    ph = r0;
+    for (int k = lo; k < lo + Ls; k++) {
+        const double2 v = ssb_step<2>(pl.out_sos, 2, si, cmul(y[k], cconj(ph)));
+        o[k] = fma(ph.x, v.x, -ph.y * v.y);
+        ph = cmul(ph, e1);
+    }
+}
+
 // warp <-> (emitted chunk, row), lane <-> segment of Lseg = M/32 outputs.  Without an output
 // filter the demodulated values are framed and stored; with it each lane runs the DF2T recurrence
 // over its segment from a zero state, a lane scan (A^Lseg powers) gives every segment its state
 // from the chunk start, the segment is re-run from that state, and the chunk's zero-state end
 // state goes to echunk.  The response to the state carried from earlier chunks is k_seam_frame's.
+// The SSB instance does the same with the complex band-pass (seam_ssb_demod).
+template <bool SSB>
 __global__ void __launch_bounds__(256)
 k_seam_demod(const __grid_constant__ DevPlan pl, SeamDev sd, double *out, int ne, int nwin, int end)
 {
@@ -328,6 +379,10 @@ k_seam_demod(const __grid_constant__ DevPlan pl, SeamDev sd, double *out, int ne
     const int i = (int)(item / pl.R), r = (int)(item % pl.R), M = pl.M, Ls = pl.sos_Lseg;
     const bool last = end && i == nwin - 1;
     const double2 *y = sd.ybuf + ((size_t)i * pl.R + r) * (M + 1);
+    if constexpr (SSB) {
+        seam_ssb_demod(pl, sd, y, out + (size_t)r * ne * M + (size_t)i * M, (size_t)i * pl.R + r, lane);
+        return;
+    }
     if (pl.demod == SDRB_IQ) {     // rows of ne * 2M doubles, no output low-pass
         double2 *o2 = reinterpret_cast<double2 *>(out + ((size_t)r * ne + i) * pl.W);
         for (int k = lane; k < M; k += 32) {
@@ -385,23 +440,33 @@ k_seam_demod(const __grid_constant__ DevPlan pl, SeamDev sd, double *out, int ne
 }
 
 // one warp per row, lane <-> contiguous run of chunks: sst[c] = SOS state at the start of emitted
-// chunk c, s[c+1] = A^M s[c] + echunk[c], from the handle's state; the new state back into it
+// chunk c, s[c+1] = A^M s[c] + echunk[c], from the handle's state; the new state back into it.
+// T = double2 (usb / lsb): complex states in the frame of each chunk's first output, so the chunk
+// map is e^{j Omega M} (A^M s[c] + echunk[c]); a composed map is a real matrix times a phasor.
+template <typename T>
 __global__ void __launch_bounds__(32)
 k_seam_sscan(const __grid_constant__ DevPlan pl, SeamDev sd, int ne)
 {
+    constexpr bool CPX = std::is_same<T, double2>::value;
     const int r = blockIdx.x, lane = threadIdx.x;
     const int per = (ne + 31) / 32;
     const int c0 = min(ne, lane * per), c1 = min(ne, c0 + per);
-    double a[SEAM_NS] = {0.0, 0.0, 0.0, 0.0};
+    const T *ech = reinterpret_cast<const T *>(sd.echunk);
+    T *sst = reinterpret_cast<T *>(sd.sst), *sos = reinterpret_cast<T *>(sd.sos);
+    T a[SEAM_NS];
+#pragma unroll
+    for (int j = 0; j < SEAM_NS; j++) a[j] = seam_zero<T>();
     double mm[SEAM_NS * SEAM_NS];
 #pragma unroll
     for (int j = 0; j < SEAM_NS * SEAM_NS; j++) mm[j] = (j % (SEAM_NS + 1)) == 0 ? 1.0 : 0.0;
-    auto matvec = [&](const double *A, const double *x, double *yv) {
+    double2 EM = make_double2(1.0, 0.0), ph = EM;   // chunk phasor e^{j Omega M}; phasor of the composed map
+    if constexpr (CPX) EM = pl.ssb_rot[pl.M];
+    auto matvec = [&](const double *A, const T *x, T *yv) {
 #pragma unroll
         for (int p = 0; p < SEAM_NS; p++) {
-            double acc = 0.0;
+            T acc = seam_zero<T>();
 #pragma unroll
-            for (int q = 0; q < SEAM_NS; q++) acc = fma(A[p * SEAM_NS + q], x[q], acc);
+            for (int q = 0; q < SEAM_NS; q++) acc = seam_fma(A[p * SEAM_NS + q], x[q], acc);
             yv[p] = acc;
         }
     };
@@ -417,65 +482,86 @@ k_seam_sscan(const __grid_constant__ DevPlan pl, SeamDev sd, int ne)
             }
     };
     for (int c = c0; c < c1; c++) {
-        double t[SEAM_NS], t2[SEAM_NS * SEAM_NS];
+        T t[SEAM_NS];
+        double t2[SEAM_NS * SEAM_NS];
         matvec(sd.AM, a, t);
-        for (int j = 0; j < SEAM_NS; j++) a[j] = t[j] + sd.echunk[((size_t)c * pl.R + r) * SEAM_NS + j];
+        for (int j = 0; j < SEAM_NS; j++) a[j] = seam_rot(EM, seam_add(t[j], ech[((size_t)c * pl.R + r) * SEAM_NS + j]));
         matmul(sd.AM, mm, t2);
         for (int j = 0; j < SEAM_NS * SEAM_NS; j++) mm[j] = t2[j];
+        if constexpr (CPX) ph = cmul(ph, EM);
     }
 #pragma unroll
     for (int lv = 0; lv < 5; lv++) {
-        double pa[SEAM_NS], pm[SEAM_NS * SEAM_NS];
+        T pa[SEAM_NS];
+        double pm[SEAM_NS * SEAM_NS];
 #pragma unroll
-        for (int j = 0; j < SEAM_NS; j++) pa[j] = __shfl_up_sync(0xffffffffu, a[j], 1 << lv);
+        for (int j = 0; j < SEAM_NS; j++) pa[j] = seam_shfl_up(a[j], 1 << lv);
 #pragma unroll
         for (int j = 0; j < SEAM_NS * SEAM_NS; j++) pm[j] = __shfl_up_sync(0xffffffffu, mm[j], 1 << lv);
+        double2 pph = ph;
+        if constexpr (CPX) pph = shfl_up_c(ph, 1 << lv);
         if (lane >= (1 << lv)) {
-            double t[SEAM_NS], t2[SEAM_NS * SEAM_NS];
+            T t[SEAM_NS];
+            double t2[SEAM_NS * SEAM_NS];
             matvec(mm, pa, t);
-            for (int j = 0; j < SEAM_NS; j++) a[j] += t[j];
+            for (int j = 0; j < SEAM_NS; j++) a[j] = seam_add(a[j], seam_rot(ph, t[j]));
             matmul(mm, pm, t2);
             for (int j = 0; j < SEAM_NS * SEAM_NS; j++) mm[j] = t2[j];
+            if constexpr (CPX) ph = cmul(ph, pph);
         }
     }
-    double st0[SEAM_NS], ea[SEAM_NS], em[SEAM_NS * SEAM_NS];
-    for (int j = 0; j < SEAM_NS; j++) st0[j] = sd.sos[(size_t)r * SEAM_NS + j];
+    T st0[SEAM_NS], ea[SEAM_NS];
+    double em[SEAM_NS * SEAM_NS];
+    for (int j = 0; j < SEAM_NS; j++) st0[j] = sos[(size_t)r * SEAM_NS + j];
 #pragma unroll
-    for (int j = 0; j < SEAM_NS; j++) ea[j] = __shfl_up_sync(0xffffffffu, a[j], 1);
+    for (int j = 0; j < SEAM_NS; j++) ea[j] = seam_shfl_up(a[j], 1);
 #pragma unroll
     for (int j = 0; j < SEAM_NS * SEAM_NS; j++) em[j] = __shfl_up_sync(0xffffffffu, mm[j], 1);
+    double2 eph = ph;
+    if constexpr (CPX) eph = shfl_up_c(ph, 1);
     if (lane == 0) {
-        for (int j = 0; j < SEAM_NS; j++) ea[j] = 0.0;
+        for (int j = 0; j < SEAM_NS; j++) ea[j] = seam_zero<T>();
         for (int j = 0; j < SEAM_NS * SEAM_NS; j++) em[j] = (j % (SEAM_NS + 1)) == 0 ? 1.0 : 0.0;
+        eph = make_double2(1.0, 0.0);
     }
-    double s[SEAM_NS];
+    T s[SEAM_NS];
     matvec(em, st0, s);
-    for (int j = 0; j < SEAM_NS; j++) s[j] += ea[j];
+    for (int j = 0; j < SEAM_NS; j++) s[j] = seam_add(seam_rot(eph, s[j]), ea[j]);
     for (int c = c0; c < c1; c++) {
-        double t[SEAM_NS];
-        for (int j = 0; j < SEAM_NS; j++) sd.sst[((size_t)c * pl.R + r) * SEAM_NS + j] = s[j];
+        T t[SEAM_NS];
+        for (int j = 0; j < SEAM_NS; j++) sst[((size_t)c * pl.R + r) * SEAM_NS + j] = s[j];
         matvec(sd.AM, s, t);
-        for (int j = 0; j < SEAM_NS; j++) s[j] = t[j] + sd.echunk[((size_t)c * pl.R + r) * SEAM_NS + j];
+        for (int j = 0; j < SEAM_NS; j++) s[j] = seam_rot(EM, seam_add(t[j], ech[((size_t)c * pl.R + r) * SEAM_NS + j]));
     }
     if (lane == 31) {
-        double t[SEAM_NS];
+        T t[SEAM_NS];
         matvec(mm, st0, t);
-        for (int j = 0; j < SEAM_NS; j++) sd.sos[(size_t)r * SEAM_NS + j] = t[j] + a[j];
+        for (int j = 0; j < SEAM_NS; j++) sos[(size_t)r * SEAM_NS + j] = seam_add(seam_rot(ph, t[j]), a[j]);
     }
 }
 
-// thread <-> output: out += c A^k s[chunk], then framing
+// thread <-> output: out += c A^k s[chunk], then framing; SSB: out += Re(e^{j Omega k} c A^k s[chunk])
+template <bool SSB>
 __global__ void __launch_bounds__(256)
 k_seam_frame(const __grid_constant__ DevPlan pl, SeamDev sd, double *out, int ne)
 {
     const size_t M = pl.M, total = (size_t)pl.R * ne * M;
     for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (size_t)gridDim.x * blockDim.x) {
         const size_t r = e / ((size_t)ne * M), rest = e % ((size_t)ne * M), i = rest / M, k = rest % M;
-        const double *s = sd.sst + (i * pl.R + r) * SEAM_NS;
         const double *ca = sd.CAM + k * SEAM_NS;
         double v = out[e];
+        if constexpr (SSB) {
+            const double2 *s = reinterpret_cast<const double2 *>(sd.sst) + (i * pl.R + r) * SEAM_NS;
+            double2 w = make_double2(0.0, 0.0);
 #pragma unroll
-        for (int j = 0; j < SEAM_NS; j++) v = fma(ca[j], s[j], v);
+            for (int j = 0; j < SEAM_NS; j++) { w.x = fma(ca[j], s[j].x, w.x); w.y = fma(ca[j], s[j].y, w.y); }
+            const double2 ph = pl.ssb_rot[k];
+            v = fma(ph.x, w.x, fma(-ph.y, w.y, v));
+        } else {
+            const double *s = sd.sst + (i * pl.R + r) * SEAM_NS;
+#pragma unroll
+            for (int j = 0; j < SEAM_NS; j++) v = fma(ca[j], s[j], v);
+        }
         out[e] = pl.be_out ? bswap_double(v) : v;
     }
 }

@@ -8,7 +8,8 @@ import numpy as np
 
 from .. import _native as nat
 
-__all__ = ['fmDemod', 'amDemod', 'realOutput', 'imagOutput', 'iqOutput', 'shiftFreq']
+__all__ = ['fmDemod', 'amDemod', 'realOutput', 'imagOutput', 'iqOutput', 'ssbDemod', 'usbDemod', 'lsbDemod',
+           'shiftFreq']
 
 
 def _rows(data, out):
@@ -61,6 +62,34 @@ def iqOutput(data, res) -> None:
     out = np.empty(o2.shape, dtype=np.float64)
     nat.check(nat.lib().sdrb_iq_output(0, d.ctypes.data, d.shape[0], d.shape[1], out.ctypes.data))
     o2[...] = out
+
+
+def ssbDemod(data, res, sos, omega: float) -> None:
+    """Single-sideband demodulation, ``res`` shaped like ``data``: per row, from a zero filter state,
+    ``res[k] = real(exp(1j*omega*k) * sosfilt(sos, data * exp(-1j*omega*k))[k])`` -- the prototype
+    low-pass ``sos`` (1..4 sections) moved to a complex band-pass around ``omega`` (rad/sample,
+    0 < |omega| < pi/2; > 0 keeps the upper sideband, < 0 the lower).  Not a reference operator
+    (``-m usb`` / ``-m lsb``)."""
+    d, o2 = _rows(data, res)
+    s = np.ascontiguousarray(sos, dtype=np.float64).reshape(-1, 6)
+    out = np.empty(d.shape, dtype=np.float64)
+    nat.check(nat.lib().sdrb_ssb_demod(0, d.ctypes.data, d.shape[0], d.shape[1], s.ctypes.data, s.shape[0],
+                                       float(omega), out.ctypes.data))
+    o2[...] = out
+
+
+def usbDemod(data, res, sos, omega: float) -> None:
+    """``ssbDemod`` for the upper sideband (``omega > 0``): the operator ``-m usb`` selects."""
+    if not omega > 0:
+        raise ValueError('the upper sideband needs omega > 0')
+    ssbDemod(data, res, sos, omega)
+
+
+def lsbDemod(data, res, sos, omega: float) -> None:
+    """``ssbDemod`` for the lower sideband (``omega < 0``): the operator ``-m lsb`` selects."""
+    if not omega < 0:
+        raise ValueError('the lower sideband needs omega < 0')
+    ssbDemod(data, res, sos, omega)
 
 
 def shiftFreq(y, shift, res) -> None:

@@ -23,9 +23,10 @@ from typing import Any, Callable
 import numpy as np
 
 from .data_processor import DataProcessor
-from .demodulation import amDemod, fmDemod, imagOutput, iqOutput, realOutput
+from .demodulation import amDemod, fmDemod, imagOutput, iqOutput, lsbDemod, realOutput, usbDemod
 
-_DEMOD_NAME = {fmDemod: 'fm', amDemod: 'am', realOutput: 're', imagOutput: 'im', iqOutput: 'iq'}
+_DEMOD_NAME = {fmDemod: 'fm', amDemod: 'am', realOutput: 're', imagOutput: 'im', iqOutput: 'iq',
+               usbDemod: 'usb', lsbDemod: 'lsb'}
 
 
 def generateEllipFilter(fs: int, deg: int, Wn, btype: str):
@@ -152,6 +153,26 @@ class DspProcessor(DataProcessor):
         self.bandwidth = self.decimatedFs
         self._setDemod(iqOutput)
 
+    def _checkSideband(self) -> None:
+        if not 0 < self.omegaOut < self.__decimatedFs / 2:
+            raise ValueError(f'usb/lsb: the sideband width -w {self.omegaOut} Hz must lie strictly between 0 and '
+                             f'half the decimated rate ({self.__decimatedFs} / 2 Hz)')
+
+    def selectOutputUsb(self):
+        """Not a reference mode: the upper sideband [0, omegaOut] Hz from the tuned frequency as real
+        audio (the band-pass ellip(3, 1, 30, omegaOut/2) moved up by omegaOut/2)."""
+        self._checkSideband()
+        self.bandwidth = self.omegaOut
+        self._setDemod(usbDemod, generateEllipFilter(self.__decimatedFs, self._FILTER_DEGREE,
+                                                     self.omegaOut / 2, 'lowpass'))
+
+    def selectOutputLsb(self):
+        """Not a reference mode: the lower sideband [-omegaOut, 0] Hz, as selectOutputUsb."""
+        self._checkSideband()
+        self.bandwidth = self.omegaOut
+        self._setDemod(lsbDemod, generateEllipFilter(self.__decimatedFs, self._FILTER_DEGREE,
+                                                     self.omegaOut / 2, 'lowpass'))
+
     # ---------------------------------------------------------------- NCO table (:185-187)
     def _generateShift(self, c: int) -> None:
         """Kept for API parity (tests read ``_shift``); the device path builds its own phasor
@@ -169,7 +190,7 @@ class DspProcessor(DataProcessor):
     def _demodName(self) -> str:
         name = _DEMOD_NAME.get(getattr(self, 'demod', None))
         if name is None:
-            raise ValueError('no demodulation selected (call selectOutputFm/Am/Real/Imag/Iq first)')
+            raise ValueError('no demodulation selected (call selectOutputFm/Am/Real/Imag/Iq/Usb/Lsb first)')
         return name
 
     def _makeEngine(self, first):
@@ -417,6 +438,9 @@ class DspProcessor(DataProcessor):
         d['decimatedFs'] = self.__decimatedFs
         if self._seamless:
             d['seamless'] = True
+        name = _DEMOD_NAME.get(getattr(self, 'demod', None))
+        if name in ('usb', 'lsb'):
+            d['demodulation'] = name
         return dumps(d, indent=2, default=str)
 
     def __str__(self):

@@ -3,7 +3,8 @@
 This is the thin host layer between the reference-shaped processors (dsp/*.py) and the C ABI.
 Inputs are whole 131072-byte chunks of raw IQ bytes; outputs are float64 rows
 ``[row][chunk][W]`` framed as the reference frames them (native doubles, or big-endian in SIMO).
-W is M, except for iq output: 2M doubles, (Re, Im) of each decimator output interleaved.
+W is M, except for iq output: 2M doubles, (Re, Im) of each decimator output interleaved
+(usb / lsb: M real doubles of single-sideband audio).
 """
 from __future__ import annotations
 
@@ -88,6 +89,9 @@ class Engine:
         tab.lam_tile[0], tab.lam_tile[1] = float(pl.lam_tile[0]), float(pl.lam_tile[1])
         if pl.fm_interp is not None:
             put('fm_interp', pl.fm_interp)
+        if getattr(pl, 'ssb_rot', None) is not None:
+            tab.ssb_omega = float(pl.ssb_omega)
+            put('ssb_rot', pl.ssb_rot)
         if self.seamless:
             tab.lookahead, tab.fs = int(pl.lookahead), int(pl.fs)
             step = np.ascontiguousarray(pl.chunk_step, dtype=np.int64)

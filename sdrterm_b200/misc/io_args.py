@@ -19,6 +19,8 @@ class DemodulationChoices(str, Enum):
     REAL = 're'
     IMAG = 'im'
     IQ = 'iq'
+    USB = 'usb'
+    LSB = 'lsb'
 
     def __str__(self):
         return self.value
@@ -27,7 +29,8 @@ class DemodulationChoices(str, Enum):
 def selectDemodulation(demodType, processor) -> Callable:
     tprint(f'{demodType} requested')
     table = {'fm': 'selectOutputFm', 'nfm': 'selectOutputFm', 'am': 'selectOutputAm',
-             're': 'selectOutputReal', 'im': 'selectOutputImag', 'iq': 'selectOutputIq'}
+             're': 'selectOutputReal', 'im': 'selectOutputImag', 'iq': 'selectOutputIq',
+             'usb': 'selectOutputUsb', 'lsb': 'selectOutputLsb'}
     name = table.get(str(demodType.value if isinstance(demodType, Enum) else demodType))
     if name is None:
         raise ValueError(f'Invalid demod type {demodType}')

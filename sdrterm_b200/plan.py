@@ -225,6 +225,10 @@ class Plan:
     PN: np.ndarray | None = None          # (D+1, 8) p_i^(N j): a modal state moved j whole chunks
     sos_AM: np.ndarray | None = None      # (ns, ns) A^M of the output cascade: its state moved one chunk
     sos_CAM: np.ndarray | None = None     # (M, ns) c A^i, i < M
+    # single sideband (usb / lsb; DESIGN.md section 12): out_sos is the prototype, the band-pass is
+    # h[m] e^{j Omega m}; the kernels run it in the Weaver frame and need only e^{j Omega k}
+    ssb_omega: float = 0.0                # Omega = +pi B / fs_d (usb), -pi B / fs_d (lsb)
+    ssb_rot: np.ndarray | None = None     # (M+1,) e^{j Omega k}, k = 0..M
 
     @property
     def chunk_bytes(self) -> int:
@@ -240,6 +244,12 @@ def reference_w(f_hz: int, fs: int) -> float:
     """Phase increment per sample exactly as the reference forms it:
     ``-2j * pi * (f / fs)`` (dsp_processor.py:187, vfo_processor.py:48)."""
     return float((-2j * np.pi * (f_hz / fs)).imag)
+
+
+def ssb_omega(demod: str, omega_out: int, fs_d: int) -> float:
+    """The single-sideband rotation Omega = +pi B / fs_d (usb) or -pi B / fs_d (lsb), B = omegaOut."""
+    om = np.pi * omega_out / fs_d
+    return float(om if demod == 'usb' else -om)
 
 
 LOOKAHEAD_TOL = 1e-13     # truncated anticausal tail of the seamless mode, relative to the input scale
@@ -395,8 +405,24 @@ def build_plan(fs: int, enc: str, dec: int, rows_hz, *, simo: bool = False, swap
         out_sos = np.ascontiguousarray(
             _sig.ellip(3, 1, 30, omega_out, btype='lowpass', analog=False, output='sos',
                        fs=fs // q), dtype=np.float64)
+    elif demod in ('usb', 'lsb'):
+        # the sideband [0, B] (usb) or [-B, 0] (lsb) Hz: the fm/am output filter's design call at
+        # half the width, rotated by +-B/2
+        fs_d = fs // q
+        if not 0 < omega_out < fs_d / 2:
+            raise ValueError(f'{demod}: the sideband width -w {omega_out} Hz must lie strictly between 0 and '
+                             f'half the decimated rate ({fs_d} / 2 Hz)')
+        out_sos = np.ascontiguousarray(
+            _sig.ellip(3, 1, 30, omega_out / 2, btype='lowpass', analog=False, output='sos',
+                       fs=fs_d), dtype=np.float64)
     elif demod not in ('re', 'im', 'iq'):          # iq: the complex decimator output, no output low-pass
         raise ValueError(f'Invalid demod type {demod}')
+    ssb = {}
+    if demod in ('usb', 'lsb'):
+        om = ssb_omega(demod, omega_out, fs // q)
+        mp.mp.dps = 40
+        ssb['ssb_omega'] = om
+        ssb['ssb_rot'] = np.array([_c(mp.expj(mp.mpf(om) * k)) for k in range(M + 1)])
     sos_Lseg, sos_AL, sos_CA, sos_AP = 0, None, None, None
     if out_sos is not None:
         sos_Lseg = -(-M // 32)
@@ -454,7 +480,7 @@ def build_plan(fs: int, enc: str, dec: int, rows_hz, *, simo: bool = False, swap
                 lam_tile=lam_tile, demod=demod, out_sos=out_sos,
                 big_endian_out=bool(simo if big_endian_out is None else big_endian_out),
                 fm_interp=fm_interp, sos_Lseg=sos_Lseg, sos_AL=sos_AL, sos_CA=sos_CA, sos_AP=sos_AP,
-                seamless=bool(seamless), **sm)
+                seamless=bool(seamless), **sm, **ssb)
 
 
 # ------------------------------------------------------------------------------------------------

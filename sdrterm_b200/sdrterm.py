@@ -29,7 +29,7 @@ def buildParser() -> argparse.ArgumentParser:
     ap.add_argument('--output', '-o', dest='outFile', default=None, help='file or stdout')
     ap.add_argument('--plot', default=None, help='accepted and ignored (plots are out of scope)')
     ap.add_argument('--demodulation', '-m', dest='demod', type=str.lower, default='fm',
-                    choices=['fm', 'nfm', 'am', 're', 'im', 'iq'])
+                    choices=['fm', 'nfm', 'am', 're', 'im', 'iq', 'usb', 'lsb'])
     ap.add_argument('--tuned-frequency', '-t', dest='tuned', type=parseIntString, default=0)
     ap.add_argument('--vfos', default=None, help='CSV of integer offsets from the tuned frequency')
     ap.add_argument('--decimation', '-d', dest='dec', type=int, default=2)
@@ -66,7 +66,8 @@ def makeProcessor(a, fileInfo):
     fs = fileInfo['sampRate']
     proc = VfoProcessor(fs, vfoHost=a.vfo_host, vfos=a.vfos, **kw) if a.simo else DspProcessor(fs, **kw)
     {'fm': proc.selectOutputFm, 'nfm': proc.selectOutputFm, 'am': proc.selectOutputAm,
-     're': proc.selectOutputReal, 'im': proc.selectOutputImag, 'iq': proc.selectOutputIq}[a.demod]()
+     're': proc.selectOutputReal, 'im': proc.selectOutputImag, 'iq': proc.selectOutputIq,
+     'usb': proc.selectOutputUsb, 'lsb': proc.selectOutputLsb}[a.demod]()
     return proc
 
 
