@@ -18,7 +18,7 @@
 extern "C" {
 #endif
 
-#define SDRB_ABI_VERSION 9
+#define SDRB_ABI_VERSION 10
 #define SDRB_TILE_BLOCKS 32
 #define SDRB_NPOLES 8
 #define SDRB_MAX_DECIMATION 256
@@ -110,9 +110,8 @@ typedef struct sdrb_tables {
     const double *out_sos;   /* [n_out_sections][6] */
     const double *fm_interp; /* optional dense [M][M/2] matrix for non-power-of-two FM resample */
     int32_t sos_Lseg;        /* output SOS evaluated in 32 segments of this many samples */
-    const double *sos_AL;    /* [ns][ns], ns = 2*n_out_sections: A^Lseg of the output cascade */
-    const double *sos_CA;    /* [sos_Lseg][ns]: c A^i */
-    const double *sos_AP;    /* [5][ns][ns]: (A^Lseg)^(2^lv), lv = 0..4 */
+    const double *sos_CA;    /* [sos_Lseg][ns], ns = 2*n_out_sections: c A^i */
+    const double *sos_AP;    /* [5][ns][ns]: (A^Lseg)^(2^lv), lv = 0..4; required with an output SOS */
     /* tensor-core block front end (plan.py: build_tc); tc_enable == 0 selects the FP64 block
      * kernel.  The raw stream is the int8 A operand of an exact GEMM whose rows are super-blocks
      * of two blocks, against one tc_Bq slice per row of the bank. */

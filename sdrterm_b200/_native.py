@@ -15,9 +15,9 @@ ROOT = os.path.dirname(_HERE)
 LIB_PATH = os.environ.get('SDRB_LIB') or os.path.join(_HERE, 'libsdrterm_b200.so')   # SDRB_LIB: experiment builds
 HEADER = os.path.join(ROOT, 'include', 'sdrterm_b200.h')
 SOURCES = [os.path.join(_HERE, 'csrc', f) for f in ('sdrb_api.cu', 'sdrb_kernels.cuh', 'sdrb_device.cuh', 'sdrb_tc.cuh', 'sdrb_finish.cuh',
-                                                    'sdrb_spectrum.cuh', 'sdrb_seamless.cuh')]
+                                                    'sdrb_spectrum.cuh', 'sdrb_seamless.cuh', 'sdrb_outstage.cuh')]
 
-ABI_VERSION = 9
+ABI_VERSION = 10
 FM, AM, RE, IM, IQ, USB, LSB = 0, 1, 2, 3, 4, 5, 6
 DEMOD_CODE = {'fm': FM, 'am': AM, 're': RE, 'im': IM, 'iq': IQ, 'usb': USB, 'lsb': LSB}
 
@@ -48,7 +48,7 @@ class Tables(C.Structure):
                 ('run_len', C.c_int32 * 8), ('lam_run', C.c_double * 8), ('T2', _DP), ('T3', _DP), ('T1', _DP),
                 ('Ehead', _DP), ('Eend', _DP), ('alpha', _DP), ('alphaT', _DP), ('beta', _DP),
                 ('betaT', _DP), ('gamma', _DP), ('phE', _DP), ('psiY', _DP), ('use_nco', C.POINTER(C.c_uint8)), ('out_sos', _DP),
-                ('fm_interp', _DP), ('sos_Lseg', C.c_int32), ('sos_AL', _DP), ('sos_CA', _DP), ('sos_AP', _DP),
+                ('fm_interp', _DP), ('sos_Lseg', C.c_int32), ('sos_CA', _DP), ('sos_AP', _DP),
                 ('tc_enable', C.c_int32), ('tc_K', C.c_int32), ('tc_isz', C.c_int32),
                 ('tc_ncol', C.c_int32), ('tc_nout', C.c_int32), ('tc_npad', C.c_int32),
                 ('tc_S', C.c_int32), ('tc_S_yl', C.c_int32), ('tc_nrowc', C.c_int32), ('tc_a_signed', C.c_int32),

@@ -475,11 +475,9 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
     pl.lam_inv = tab->lam_inv;
     pl.sos_ns = 2 * cfg->n_out_sections; pl.sos_Lseg = tab->sos_Lseg;
     if (cfg->n_out_sections > 0) {
-        if (!tab->sos_AL || !tab->sos_CA || tab->sos_Lseg * 32 < pl.M)
+        if (!tab->sos_CA || !tab->sos_AP || tab->sos_Lseg * 32 < pl.M)
             return bail(fail(h, SDRB_ERR_ARG, "output SOS segment tables missing or too short"));
-        for (int i = 0; i < pl.sos_ns * pl.sos_ns; i++) pl.sos_AL[i] = tab->sos_AL[i];
-        if (pl.sos_ns == 4 && tab->sos_AP)
-            for (int i = 0; i < 80; i++) pl.sos_AP[i] = tab->sos_AP[i];
+        for (int i = 0; i < 5 * pl.sos_ns * pl.sos_ns; i++) pl.sos_AP[i] = tab->sos_AP[i];
     }
     pl.ws = std::min(pl.q * pl.Mf, pl.N - 1 - pl.edge); pl.nend = pl.N - pl.ws;
     pl.k_bnd = tab->k_bnd; pl.nsec_out = cfg->n_out_sections;
@@ -605,7 +603,7 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
         const bool pow2 = is_pow2(M);
         h->finish_on = !env_int("SDRB_NO_FINISH", 0) && pl.rem == 0 && pl.cnt_last == SDRB_TB && q >= pl.edge + 1 &&
                        pow2 && M >= 64 && M <= 1024 && pl.edge + 1 <= 32 && pl.ntiles <= 32 &&
-                       (cfg->n_out_sections == 0 || (cfg->n_out_sections == 2 && tab->sos_AP));
+                       (cfg->n_out_sections == 0 || cfg->n_out_sections == 2);
         h->finish_smem = h->finish_on ? finish_smem_bytes(M, pl.edge) : 0;
         if (h->finish_smem > 227 * 1024) h->finish_on = false;
     }
@@ -646,7 +644,7 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
         SeamDev &sd = h->sd;
         if (pl.rem != 0 || pl.cnt_last != SDRB_TB || tab->lookahead < 1 || !tab->PN || !tab->chunk_step ||
             tab->fs <= 0 || tab->fs >= (1LL << 31) || (cfg->n_out_sections != 0 && cfg->n_out_sections != 2) ||
-            (cfg->n_out_sections && (!tab->sos_AM || !tab->sos_CAM || !tab->sos_AP || pl.sos_Lseg * 32 != M)) ||
+            (cfg->n_out_sections && (!tab->sos_AM || !tab->sos_CAM || pl.sos_Lseg * 32 != M)) ||
             pl.edge + 1 > 64 || pl.nend > 64)
             return bail(fail(h, SDRB_ERR_ARG, "seamless mode needs the decimation to divide the chunk (q | N), "
                                               "a lookahead >= 1 and its tables"));
@@ -1287,7 +1285,8 @@ int sdrb_ssb_demod(int device, const double *y, int R, int M, const double *sos,
     pl.ssb_omega = omega;
     for (int i = 0; i < 6 * nsec; i++) pl.out_sos[i] = sos[i];
     // the prototype's state space (A, c) in extended precision -- the same DF2T state variables as
-    // plan.py's _cascade_state_space -- then A^Lseg, c A^i (i < Lseg) and e^{j omega k} (k <= M)
+    // plan.py's _cascade_state_space -- then A^Lseg and its squarings, c A^i (i < Lseg) and
+    // e^{j omega k} (k <= M)
     const int ns = pl.sos_ns, Ls = pl.sos_Lseg;
     std::vector<long double> A((size_t)ns * ns, 0.0L), cvec(ns, 0.0L);
     {
@@ -1319,7 +1318,14 @@ int sdrb_ssb_demod(int device, const double *y, int R, int M, const double *sos,
         cur = nx;
         P = NP;
     }
-    for (int i = 0; i < ns * ns; i++) pl.sos_AL[i] = (double)P[i];       // A^Lseg
+    for (int lv = 0; lv < 5; lv++) {                                      // (A^Lseg)^(2^lv)
+        for (int i = 0; i < ns * ns; i++) pl.sos_AP[lv * ns * ns + i] = (double)P[i];
+        std::vector<long double> PP((size_t)ns * ns, 0.0L);
+        for (int a = 0; a < ns; a++)
+            for (int b = 0; b < ns; b++)
+                for (int k = 0; k < ns; k++) PP[(size_t)a * ns + b] += P[(size_t)a * ns + k] * P[(size_t)k * ns + b];
+        P = PP;
+    }
     std::vector<double2> rot((size_t)M + 1);
     for (int k = 0; k <= M; k++) {
         const long double a = (long double)omega * (long double)k;

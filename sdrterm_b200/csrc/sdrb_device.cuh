@@ -22,8 +22,7 @@ struct DevPlan {
     int demod_in_smem;     // FFT / row buffers fit shared memory
     double Liq, lam, lam_q, lam_N, lam_inv, g0, d, norm_xmin, norm_k;
     double lam_run[8];     // lam^run_len
-    double sos_AL[64];     // [ns][ns] A^Lseg of the output cascade
-    double sos_AP[80];     // [5][4][4] (A^Lseg)^(2^lv), two-section cascades (k_finish's lane scan)
+    double sos_AP[320];    // [5][ns][ns] (A^Lseg)^(2^lv), ns = sos_ns (packed): the lane scan's segment maps
     double lamq_pow[5];    // lam_q^(1,2,4,8,16)
     double lam_pw[33];     // lam^k, k = 0..32 (k_finish's IQ scans)
     double mu_pw[33];      // lam^-k

@@ -7,12 +7,11 @@
 //   4. demodulation: fm (pair phase, 2x trigonometric interpolation by a real-input FFT of half
 //      the length and its inverse) | am | re | im; the iq instance (OUT_IQ) stores y straight from
 //      registers instead, (Re, Im) per output, and skips 3b-5
-//   5. output low-pass (zero initial state per chunk) in 32 lane segments, chained by a
-//      Kogge-Stone scan of the segment maps; framing (native or big-endian doubles)
+//   5. output low-pass (zero initial state per chunk): sdrb_outstage.cuh's output stage, 32 lane
+//      segments composed by a Kogge-Stone scan of the segment maps; framing (native or big-endian)
 //   The usb / lsb instance (OUT_SSB) skips 3b and 4: it stages y in the warp's shared memory (Re in
-//   zrow, Im in the carry rows as they fall dead) and runs the complex band-pass as 32 lane
-//   segments in the Weaver frame (zero-state pass, 5-level scan of the complex 4-state segment maps,
-//   the response to the composed states), then frames the real part.
+//   zrow, Im in the carry rows as they fall dead) and runs the same output stage on complex states
+//   (the band-pass in the Weaver frame), then frames the real part.
 //
 // It replaces k_fixup + k_demod for the common shapes (whole tiles, M a power of two <= 1024, at
 // most 2 output sections); those two kernels remain the general path.  Nothing leaves the SM
@@ -24,6 +23,7 @@
 // emu_demod, emu_fm_interp_real) is the numpy twin.
 #pragma once
 #include "sdrb_kernels.cuh"
+#include "sdrb_outstage.cuh"
 
 #define FIN_WARPS 8      // two CTAs of eight warps per SM: the per-CTA table set-up is paid twice per SM, not four times
 #define FIN_DBG(ev) do { if (sc.dbg && blockIdx.x == 0 && warp == 0 && lane == 0 && nit < 16) sc.dbg[512 + nit * 16 + (ev)] = clock64(); } while (0)
@@ -134,12 +134,6 @@ __device__ __forceinline__ int fin_ssb_at(int k, int lsh, int Ls)
 {
     const int g = k >> lsh;
     return (g << lsh) | ((k + g) & (Ls - 1));
-}
-
-__device__ __forceinline__ double fin_demod_scalar(double2 a, int demod)
-{
-    if (demod == 1) return hypot(fma(a.x, a.x, -a.y * a.y), 2.0 * a.x * a.y);   // abs(square(z))
-    return demod == 2 ? a.x : a.y;
 }
 
 template <int ENC, int OUT>
@@ -435,11 +429,7 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
                     // 16 contiguous bytes per lane, 512 per warp and tile: no trip through zrow
                     double2 *o2 = reinterpret_cast<double2 *>(out + ((size_t)r * nchunks + chunk) * pl.W);
 #pragma unroll
-                    for (int u = 0; u < 2; u++) {
-                        double2 v = yv[u];
-                        if (pl.be_out) v = make_double2(bswap_double(v.x), bswap_double(v.y));
-                        o2[(t0 + u) * SDRB_TB + lane] = v;
-                    }
+                    for (int u = 0; u < 2; u++) frame_store(o2 + (t0 + u) * SDRB_TB + lane, yv[u], pl.be_out);
                 } else if constexpr (OUT == OUT_SSB) {
                     // Re y -> zrow; Im y -> the carry rows t0, t0+1, dead once every lane has read them
                     __syncwarp();
@@ -454,9 +444,7 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
                     const bool odd = lane & 1;
                     const double2 snd = odd ? yv[0] : yv[1];
                     const double2 rcv = shfl_xor_c(snd, 1);
-                    const double2 a = odd ? rcv : yv[0], b = odd ? yv[1] : rcv;
-                    const double re = fma(a.x, b.x, a.y * b.y), im = fma(a.y, b.x, -a.x * b.y);   // a conj(b)
-                    const double v = atan2(im, re);
+                    const double v = pair_phase(odd ? rcv : yv[0], odd ? yv[1] : rcv);
                     const int i = 16 * (t0 + (odd ? 1 : 0)) + (lane >> 1);
                     ph[i] = v;
                     zrow[2 * i + ((2 * i) >> lsh)] = v;
@@ -464,7 +452,7 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
 #pragma unroll
                     for (int u = 0; u < 2; u++) {
                         const int k = (t0 + u) * SDRB_TB + lane;
-                        zrow[k + (k >> lsh)] = fin_demod_scalar(yv[u], pl.demod);
+                        zrow[k + (k >> lsh)] = demod_scalar(yv[u], pl.demod);
                     }
                 }
             }
@@ -515,92 +503,31 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
             __syncwarp();
         }
         FIN_DBG(8);
-        // ---------------------------------------------------------------- 4. output low-pass
-        if (OUT == OUT_REAL && pl.nsec_out > 0) {
-            double *zs = zrow + (size_t)lane * (Ls + 1);
-            const double *c0 = pl.out_sos, *c1 = pl.out_sos + 6;
-            double s0 = 0, s1 = 0, s2 = 0, s3 = 0;
-#pragma unroll 4
-            for (int k = 0; k < Ls; k++) {
-                const double xc = zs[k];
-                const double xn = __dadd_rn(__dmul_rn(c0[0], xc), s0);
-                s0 = __dadd_rn(__dadd_rn(__dmul_rn(c0[1], xc), -__dmul_rn(c0[4], xn)), s1);
-                s1 = __dadd_rn(__dmul_rn(c0[2], xc), -__dmul_rn(c0[5], xn));
-                const double xm = __dadd_rn(__dmul_rn(c1[0], xn), s2);
-                s2 = __dadd_rn(__dadd_rn(__dmul_rn(c1[1], xn), -__dmul_rn(c1[4], xm)), s3);
-                s3 = __dadd_rn(__dmul_rn(c1[2], xn), -__dmul_rn(c1[5], xm));
-                zs[k] = xm;
+        // ---------------------------------------------------------------- 4. output filter
+        // fm / am: the low-pass over the padded row (segment g at g (Ls + 1)); usb / lsb: the band-pass
+        // over y staged at fin_ssb_at, Re in zrow and Im in the carry rows; the kept output -> zrow
+        if constexpr (OUT != OUT_IQ) {
+            if (OUT == OUT_SSB || pl.nsec_out > 0) {
+                const double *zim = reinterpret_cast<const double *>(carry);
+                double *zs = zrow + (OUT == OUT_SSB ? 0 : (size_t)lane * (Ls + 1));
+                auto at = [&](int j) { return OUT == OUT_SSB ? lane * Ls + ((j + lane) & (Ls - 1)) : j; };
+                std::conditional_t<OUT == OUT_SSB, double2, double> st[4];
+                sos_segments(
+                    pl, 2, lane * Ls, Ls, lane,
+                    [&](int j) {
+                        if constexpr (OUT == OUT_SSB) return make_double2(zs[at(j)], zim[at(j)]);
+                        else return zs[at(j)];
+                    },
+                    [&](int j) -> double & { return zs[at(j)]; }, st);
+                __syncwarp();
             }
-            // inclusive Kogge-Stone scan of the segment maps s -> A^Ls s + b_lane
-#pragma unroll
-            for (int lv = 0; lv < 5; lv++) {
-                const double o0 = __shfl_up_sync(0xffffffffu, s0, 1 << lv), o1 = __shfl_up_sync(0xffffffffu, s1, 1 << lv);
-                const double o2 = __shfl_up_sync(0xffffffffu, s2, 1 << lv), o3 = __shfl_up_sync(0xffffffffu, s3, 1 << lv);
-                if (lane >= (1 << lv)) {
-                    const double *A = pl.sos_AP + lv * 16;
-                    s0 = fma(A[0], o0, fma(A[1], o1, fma(A[2], o2, fma(A[3], o3, s0))));
-                    s1 = fma(A[4], o0, fma(A[5], o1, fma(A[6], o2, fma(A[7], o3, s1))));
-                    s2 = fma(A[8], o0, fma(A[9], o1, fma(A[10], o2, fma(A[11], o3, s2))));
-                    s3 = fma(A[12], o0, fma(A[13], o1, fma(A[14], o2, fma(A[15], o3, s3))));
-                }
-            }
-            double i0 = __shfl_up_sync(0xffffffffu, s0, 1), i1 = __shfl_up_sync(0xffffffffu, s1, 1);
-            double i2 = __shfl_up_sync(0xffffffffu, s2, 1), i3 = __shfl_up_sync(0xffffffffu, s3, 1);
-            if (lane == 0) { i0 = 0; i1 = 0; i2 = 0; i3 = 0; }
-#pragma unroll 4
-            for (int k = 0; k < Ls; k++) {
-                const double *ca = pl.sos_CA + (size_t)k * 4;
-                zs[k] = fma(ca[0], i0, fma(ca[1], i1, fma(ca[2], i2, fma(ca[3], i3, zs[k]))));
-            }
-            __syncwarp();
-        }
-        // ---------------------------------------------------------------- 4'. usb / lsb band-pass
-        // u[k] = y[k] e^{-j Omega k} through the real prototype in lane segments of Ls outputs
-        // (e^{j Omega k} by recurrence from the segment start), the segment maps composed by the
-        // lane scan, every output then gets c A^j s_in of its segment; s[k] = Re(e^{j Omega k} v[k])
-        if constexpr (OUT == OUT_SSB) {
-            double *zim = reinterpret_cast<double *>(carry);
-            const int lo = lane * Ls;
-            const double2 e1 = pl.ssb_rot[1], r0 = pl.ssb_rot[lo];
-            double2 st[4], ph = r0;
-#pragma unroll
-            for (int a = 0; a < 4; a++) st[a] = make_double2(0.0, 0.0);
-#pragma unroll 2
-            for (int j = 0; j < Ls; j++) {
-                const int a = lo + ((j + lane) & (Ls - 1));
-                const double2 v = ssb_step<2>(pl.out_sos, 2, st, cmul(make_double2(zrow[a], zim[a]), cconj(ph)));
-                zrow[a] = v.x;
-                zim[a] = v.y;
-                ph = cmul(ph, e1);
-            }
-            ssb_lane_scan(pl.sos_AP, st, lane);
-            double2 si[4];
-#pragma unroll
-            for (int a = 0; a < 4; a++) {
-                si[a] = shfl_up_c(st[a], 1);
-                if (lane == 0) si[a] = make_double2(0.0, 0.0);
-            }
-            ph = r0;
-#pragma unroll 2
-            for (int j = 0; j < Ls; j++) {
-                const int a = lo + ((j + lane) & (Ls - 1));
-                const double *ca = pl.sos_CA + (size_t)j * 4;
-                double vx = zrow[a], vy = zim[a];
-#pragma unroll
-                for (int b = 0; b < 4; b++) { vx = fma(ca[b], si[b].x, vx); vy = fma(ca[b], si[b].y, vy); }
-                zrow[a] = fma(ph.x, vx, -ph.y * vy);
-                ph = cmul(ph, e1);
-            }
-            __syncwarp();
         }
         FIN_DBG(9);
         // ---------------------------------------------------------------- 5. framing
         if constexpr (OUT != OUT_IQ) {
             double *o = out + ((size_t)r * nchunks + chunk) * M;
-            for (int k = lane; k < M; k += 32) {
-                const double v = zrow[OUT == OUT_SSB ? fin_ssb_at(k, lsh, Ls) : k + (k >> lsh)];
-                o[k] = pl.be_out ? bswap_double(v) : v;
-            }
+            for (int k = lane; k < M; k += 32)
+                frame_store(o + k, zrow[OUT == OUT_SSB ? fin_ssb_at(k, lsh, Ls) : k + (k >> lsh)], pl.be_out);
             __syncwarp();
         }
         FIN_DBG(10);

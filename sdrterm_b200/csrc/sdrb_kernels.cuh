@@ -6,9 +6,10 @@
 //   k_iqgain / k_iqscan_c / k_iqtiles   IQ-corrector offset at every tile start, carried across
 //              chunks and calls
 //   k_fixup    head / end segments, cross-tile carries, boundary term -> decimated complex y
-//   k_demod    fm (pair phase + 2x FFT interpolation) | am | re | im, segmented output SOS, framing;
-//              iq: y itself framed as (Re, Im) pairs; usb / lsb: the complex band-pass in 32
-//              lane segments (Weaver frame), its real part framed
+//   k_demod    fm (pair phase + 2x FFT interpolation) | am | re | im, output SOS, framing; iq: y
+//              itself framed as (Re, Im) pairs; usb / lsb: the complex band-pass on y, its real part
+//              framed.  The demodulator scalars and the output SOS (32 lane segments, lane scan,
+//              per-output correction) are sdrb_outstage.cuh's, shared with k_finish and seamless mode
 //
 // Reference behaviour being reproduced: src/misc/read_file.py:100-103 (decode, normalise, IQ
 // correction), src/dsp/demodulation.py:71-79 (NCO), src/dsp/dsp_processor.py:147 (scipy
@@ -16,6 +17,7 @@
 // tests/emulator.py is the numpy twin of these kernels (same tables, same decomposition).
 #pragma once
 #include "sdrb_device.cuh"
+#include "sdrb_outstage.cuh"
 
 // Scratch written by k_main / read by k_fixup, per batch of chunks.
 struct Scratch {
@@ -745,63 +747,11 @@ __device__ __forceinline__ void fft_pass(const double2 *in, double2 *out, int n,
     }
 }
 
-__device__ __forceinline__ double bswap_double(double v)
-{
-    unsigned long long u = (unsigned long long)__double_as_longlong(v);
-    uint32_t lo = (uint32_t)u, hi = (uint32_t)(u >> 32);
-    u = ((unsigned long long)__byte_perm(lo, 0, 0x0123) << 32) | __byte_perm(hi, 0, 0x0123);
-    return __longlong_as_double((long long)u);
-}
-
-// ---------------------------------------------------------------- single sideband (usb / lsb)
-// One output of the SSB band-pass in the Weaver frame: the real prototype's DF2T cascade (out_sos,
-// nsec <= NS sections) on a complex input, Re and Im alike; st = 2 states per section.
-template <int NS>
-__device__ __forceinline__ double2 ssb_step(const double *sos, int nsec, double2 *st, double2 x)
-{
-#pragma unroll
-    for (int s = 0; s < NS; s++) {
-        if (s < nsec) {
-            const double *cf = sos + 6 * s;
-            const double2 xn = make_double2(fma(cf[0], x.x, st[2 * s].x), fma(cf[0], x.y, st[2 * s].y));
-            st[2 * s] = make_double2(fma(cf[1], x.x, fma(-cf[4], xn.x, st[2 * s + 1].x)),
-                                     fma(cf[1], x.y, fma(-cf[4], xn.y, st[2 * s + 1].y)));
-            st[2 * s + 1] = make_double2(fma(cf[2], x.x, -cf[5] * xn.x), fma(cf[2], x.y, -cf[5] * xn.y));
-            x = xn;
-        }
-    }
-    return x;
-}
-
-// Inclusive Kogge-Stone scan of the 32 lane-segment maps s -> A^Ls s + e_lane of a two-section
-// cascade on complex states (AP = (A^Ls)^(2^lv), real: it acts on Re and Im alike); afterwards
-// lane l holds the state after segment l, from a zero state at the start of segment 0.
-__device__ __forceinline__ void ssb_lane_scan(const double *AP, double2 *st, int lane)
-{
-#pragma unroll
-    for (int lv = 0; lv < 5; lv++) {
-        double2 o[4];
-#pragma unroll
-        for (int j = 0; j < 4; j++) o[j] = shfl_up_c(st[j], 1 << lv);
-        if (lane >= (1 << lv)) {
-            const double *A = AP + lv * 16;
-#pragma unroll
-            for (int a = 0; a < 4; a++) {
-                double2 acc = st[a];
-#pragma unroll
-                for (int b = 0; b < 4; b++) { acc.x = fma(A[a * 4 + b], o[b].x, acc.x); acc.y = fma(A[a * 4 + b], o[b].y, acc.y); }
-                st[a] = acc;
-            }
-        }
-    }
-}
-
 // One CTA per (chunk, row): y[M] complex -> out[row][chunk*M .. +M) doubles.
 // Generic entry used both by the chain (y from sc.y) and by the module-level operators.  The iq
 // instance (OUT_IQ) frames y itself as out[row][chunk*2M .. +2M): (Re, Im) pairs, no output
-// low-pass.  The usb / lsb instance (OUT_SSB) runs the complex band-pass: warp 0, lane <-> segment
-// of the Weaver-frame row u[k] = y[k] e^{-j Omega k} through the real prototype (up to 4 sections),
-// segments chained with A^Lseg, s[k] = Re(e^{j Omega k} v[k]).
+// low-pass.  The output filter (up to 4 sections) runs on warp 0, lane <-> segment of Lseg outputs
+// (sdrb_outstage.cuh); the usb / lsb instance (OUT_SSB) runs it as the complex band-pass on y itself.
 template <int OUT>
 __global__ void __launch_bounds__(256)
 k_demod(const __grid_constant__ DevPlan pl, const double2 *__restrict__ yall, double *__restrict__ out,
@@ -814,11 +764,7 @@ k_demod(const __grid_constant__ DevPlan pl, const double2 *__restrict__ yall, do
     const double2 *y = yall + ((size_t)chunk * pl.R + r) * M;
     if constexpr (OUT == OUT_IQ) {
         double2 *o2 = reinterpret_cast<double2 *>(out + ((size_t)r * nchunks + chunk) * 2 * M);
-        for (int k = threadIdx.x; k < M; k += blockDim.x) {
-            double2 v = y[k];
-            if (be_out) v = make_double2(bswap_double(v.x), bswap_double(v.y));
-            o2[k] = v;
-        }
+        for (int k = threadIdx.x; k < M; k += blockDim.x) frame_store(o2 + k, y[k], be_out);
         return;
     }
     double2 *bufA, *bufB;
@@ -832,58 +778,8 @@ k_demod(const __grid_constant__ DevPlan pl, const double2 *__restrict__ yall, do
         bufB = bufA + M;
         z = zglob + (size_t)blockIdx.x * M;
     }
-    if constexpr (OUT == OUT_SSB) {
-        if (threadIdx.x < 32) {
-            const int lane = threadIdx.x, Ls = pl.sos_Lseg, ns = pl.sos_ns, nsec = pl.nsec_out;
-            const int lo = min(M, lane * Ls), hi = min(M, lo + Ls);
-            double2 *v = bufA;                                   // Weaver-frame filter output
-            double2 st[8];
-#pragma unroll
-            for (int a = 0; a < 8; a++) st[a] = make_double2(0.0, 0.0);
-            for (int k = lo; k < hi; k++) v[k] = ssb_step<4>(pl.out_sos, nsec, st, cmul(y[k], cconj(pl.ssb_rot[k])));
-            // chain: s_in(seg+1) = A^Ls s_in(seg) + s_loc(seg), walked by every lane
-            double2 sin_mine[8], cur[8];
-#pragma unroll
-            for (int a = 0; a < 8; a++) { sin_mine[a] = make_double2(0.0, 0.0); cur[a] = sin_mine[a]; }
-            for (int seg = 0; seg < 32; seg++) {
-                if (seg == lane) {
-#pragma unroll
-                    for (int a = 0; a < 8; a++) sin_mine[a] = cur[a];
-                }
-                double2 nxt[8];
-#pragma unroll
-                for (int a = 0; a < 8; a++) {
-                    double2 w = (a < ns) ? shfl_c(st[a], seg) : make_double2(0.0, 0.0);
-                    if (a < ns)
-                        for (int b = 0; b < ns; b++) {
-                            w.x = fma(pl.sos_AL[a * ns + b], cur[b].x, w.x);
-                            w.y = fma(pl.sos_AL[a * ns + b], cur[b].y, w.y);
-                        }
-                    nxt[a] = w;
-                }
-#pragma unroll
-                for (int a = 0; a < 8; a++) cur[a] = nxt[a];
-            }
-            for (int k = lo; k < hi; k++) {
-                const double *ca = pl.sos_CA + (size_t)(k - lo) * ns;
-                double2 w = v[k];
-                for (int a = 0; a < ns; a++) { w.x = fma(ca[a], sin_mine[a].x, w.x); w.y = fma(ca[a], sin_mine[a].y, w.y); }
-                const double2 ph = pl.ssb_rot[k];
-                z[k] = fma(ph.x, w.x, -ph.y * w.y);
-            }
-        }
-        __syncthreads();
-        double *o = out + ((size_t)r * nchunks + chunk) * M;
-        for (int k = threadIdx.x; k < M; k += blockDim.x) o[k] = be_out ? bswap_double(z[k]) : z[k];
-        return;
-    }
-    if (demod == 0) {          // fm: demodulation.py:25-38
-        for (int i = threadIdx.x; i < h; i += blockDim.x) {
-            const double2 a = y[2 * i], b = y[2 * i + 1];
-            // a * conj(b)
-            const double re = fma(a.x, b.x, a.y * b.y), im = fma(a.y, b.x, -a.x * b.y);
-            bufA[i] = make_double2(atan2(im, re), 0.0);
-        }
+    if (OUT == OUT_REAL && demod == 0) {   // fm: demodulation.py:25-38
+        for (int i = threadIdx.x; i < h; i += blockDim.x) bufA[i] = make_double2(pair_phase(y[2 * i], y[2 * i + 1]), 0.0);
         __syncthreads();
         if (pl.fft_ok) {
             double2 *src = bufA, *dst = bufB;
@@ -920,67 +816,24 @@ k_demod(const __grid_constant__ DevPlan pl, const double2 *__restrict__ yall, do
                 z[k] = acc;
             }
         }
-    } else if (demod == 1) {   // am: abs(square(z)) (demodulation.py:41-48)
-        for (int k = threadIdx.x; k < M; k += blockDim.x) {
-            const double2 a = y[k];
-            z[k] = hypot(fma(a.x, a.x, -a.y * a.y), 2.0 * a.x * a.y);
-        }
-    } else if (demod == 2) {
-        for (int k = threadIdx.x; k < M; k += blockDim.x) z[k] = y[k].x;
-    } else {
-        for (int k = threadIdx.x; k < M; k += blockDim.x) z[k] = y[k].y;
+    } else if (OUT == OUT_REAL) {          // am | re | im
+        for (int k = threadIdx.x; k < M; k += blockDim.x) z[k] = demod_scalar(y[k], demod);
     }
     __syncthreads();
-    // output low-pass (scipy.signal.sosfilt, zero initial state) in 32 segments: each lane of
-    // warp 0 runs SciPy's DF2T recurrence over its segment from a zero state, the segment-end
-    // states are chained with A^Lseg, and every sample then gets c A^i s_in of its segment.
-    if (apply_sos && pl.nsec_out > 0 && threadIdx.x < 32) {
-        const int lane = threadIdx.x, Ls = pl.sos_Lseg, ns = pl.sos_ns, nsec = pl.nsec_out;
-        const int lo = min(M, lane * Ls), hi = min(M, lo + Ls);
-        double st[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-        for (int k = lo; k < hi; k++) {
-            double xc = z[k];
-#pragma unroll
-            for (int s = 0; s < 4; s++) {
-                if (s < nsec) {
-                    const double *cf = pl.out_sos + 6 * s;
-                    const double xn = __dadd_rn(__dmul_rn(cf[0], xc), st[2 * s]);
-                    st[2 * s] = __dadd_rn(__dadd_rn(__dmul_rn(cf[1], xc), -__dmul_rn(cf[4], xn)), st[2 * s + 1]);
-                    st[2 * s + 1] = __dadd_rn(__dmul_rn(cf[2], xc), -__dmul_rn(cf[5], xn));
-                    xc = xn;
-                }
-            }
-            z[k] = xc;
-        }
-        // chain: s_in(seg+1) = A^Ls s_in(seg) + s_loc(seg); every lane walks the chain and keeps
-        // the value that belongs to its own segment
-        double sin_mine[8] = {0, 0, 0, 0, 0, 0, 0, 0}, cur[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-        for (int seg = 0; seg < 32; seg++) {
-            if (seg == lane) {
-#pragma unroll
-                for (int a = 0; a < 8; a++) sin_mine[a] = cur[a];
-            }
-            double nxt[8];
-#pragma unroll
-            for (int a = 0; a < 8; a++) {
-                double v = (a < ns) ? __shfl_sync(0xffffffffu, st[a], seg) : 0.0;
-                if (a < ns)
-                    for (int b = 0; b < ns; b++) v = fma(pl.sos_AL[a * ns + b], cur[b], v);
-                nxt[a] = v;
-            }
-#pragma unroll
-            for (int a = 0; a < 8; a++) cur[a] = nxt[a];
-        }
-        for (int k = lo; k < hi; k++) {
-            const double *ca = pl.sos_CA + (size_t)(k - lo) * ns;
-            double v = z[k];
-            for (int a = 0; a < ns; a++) v = fma(ca[a], sin_mine[a], v);
-            z[k] = v;
-        }
+    if ((OUT == OUT_SSB || (apply_sos && pl.nsec_out > 0)) && threadIdx.x < 32) {
+        const int lane = threadIdx.x, Ls = pl.sos_Lseg, lo = min(M, lane * Ls);
+        std::conditional_t<OUT == OUT_SSB, double2, double> st[8];
+        sos_segments(
+            pl, pl.nsec_out, lo, min(M, lo + Ls) - lo, lane,
+            [&](int j) {
+                if constexpr (OUT == OUT_SSB) return y[lo + j];
+                else return z[lo + j];
+            },
+            [&](int j) -> double & { return z[lo + j]; }, st);
     }
     __syncthreads();
     double *o = out + ((size_t)r * nchunks + chunk) * M;
-    for (int k = threadIdx.x; k < M; k += blockDim.x) o[k] = be_out ? bswap_double(z[k]) : z[k];
+    for (int k = threadIdx.x; k < M; k += blockDim.x) frame_store(o + k, z[k], be_out);
 }
 
 // demodulation.py:71-79  res[m,n] = y[n] * shift[m,n]

@@ -13,9 +13,9 @@
 //   k_seam_carry   per emitted chunk: carry-ins in its own frame (forward state, anticausal window
 //                  over the next D chunks or the real end, zeta) and the fm halo y[k+1]
 //   k_seam_y       per emitted chunk: tile carries and the decimated outputs, global frame
-//   k_seam_demod   demodulation + output SOS from the chunk's zero state (segments, lane scan);
-//                  iq: y itself, (Re, Im) pairs; usb / lsb (SSB instance): the complex band-pass
-//                  from the chunk's zero state, its real part and the complex end state
+//   k_seam_demod   demodulation + output SOS from the chunk's zero state (the shared output stage of
+//                  sdrb_outstage.cuh) and the chunk's end state; iq: y itself, (Re, Im) pairs;
+//                  usb / lsb (SSB instance): the complex band-pass, its real part, a complex end state
 //   k_seam_sscan   output SOS state across chunks: affine scan with the matrix A^M (real states), or
 //                  e^{j Omega M} A^M (usb / lsb: complex states in the frame of each chunk's start)
 //   k_seam_frame   response to the carried SOS state (usb / lsb: Re(e^{j Omega k} c A^k s_c)), framing
@@ -24,6 +24,7 @@
 #pragma once
 #include <type_traits>
 #include "sdrb_kernels.cuh"
+#include "sdrb_outstage.cuh"
 
 #define SEAM_NS 4           // output SOS state size in seamless mode (ellip(3): two sections); usb / lsb
                             // carry SEAM_NS complex states (echunk, sst and sos hold double2 then)
@@ -50,17 +51,10 @@ struct SeamDev {
 };
 
 // the output SOS state of k_seam_sscan: real (fm / am) or complex (usb / lsb)
-template <typename T> __device__ __forceinline__ T seam_zero();
-template <> __device__ __forceinline__ double seam_zero<double>() { return 0.0; }
-template <> __device__ __forceinline__ double2 seam_zero<double2>() { return make_double2(0.0, 0.0); }
-__device__ __forceinline__ double seam_fma(double a, double x, double acc) { return fma(a, x, acc); }
-__device__ __forceinline__ double2 seam_fma(double a, double2 x, double2 acc) { return make_double2(fma(a, x.x, acc.x), fma(a, x.y, acc.y)); }
 __device__ __forceinline__ double seam_add(double a, double b) { return a + b; }
 __device__ __forceinline__ double2 seam_add(double2 a, double2 b) { return cadd(a, b); }
 __device__ __forceinline__ double seam_rot(double2, double x) { return x; }            // real states: no phasor
 __device__ __forceinline__ double2 seam_rot(double2 ph, double2 x) { return cmul(ph, x); }
-__device__ __forceinline__ double seam_shfl_up(double v, int d) { return __shfl_up_sync(0xffffffffu, v, d); }
-__device__ __forceinline__ double2 seam_shfl_up(double2 v, int d) { return shfl_up_c(v, d); }
 
 __device__ __forceinline__ double2 seam_phasor(const SeamDev &sd, int r, long long g)
 {
@@ -309,134 +303,47 @@ k_seam_y(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int ne, int
 
 __device__ __forceinline__ double seam_demod_at(const double2 *y, int k, int M, bool last, int demod)
 {
-    if (demod == SDRB_FM) {
-        if (last && k == M - 1) k = M - 2;
-        const double2 a = y[k], b = y[k + 1];
-        const double2 pr = make_double2(fma(a.x, b.x, a.y * b.y), fma(a.y, b.x, -a.x * b.y));
-        return atan2(pr.y, pr.x);
-    }
-    const double2 a = y[k];
-    if (demod == SDRB_AM) { const double re = fma(a.x, a.x, -a.y * a.y), im = 2.0 * a.x * a.y; return hypot(re, im); }
-    return demod == SDRB_RE ? a.x : a.y;
-}
-
-__device__ __forceinline__ void seam_sos_step(const double *sos, int nsec, double *st, double &xc)
-{
-    for (int s = 0; s < nsec; s++) {
-        const double b0 = sos[6 * s], b1 = sos[6 * s + 1], b2 = sos[6 * s + 2], a1 = sos[6 * s + 4], a2 = sos[6 * s + 5];
-        const double xn = fma(b0, xc, st[2 * s]);
-        st[2 * s] = fma(b1, xc, -a1 * xn) + st[2 * s + 1];
-        st[2 * s + 1] = fma(b2, xc, -a2 * xn);
-        xc = xn;
-    }
-}
-
-// usb / lsb of one (chunk, row), lane <-> segment: the Weaver-frame row u[k] = y[k] e^{-j Omega k}
-// (k from the chunk start) through the real prototype from a zero state, the lane scan, the segment
-// re-run from its composed state; out = Re(e^{j Omega k} v[k]), the complex end state -> echunk
-__device__ __forceinline__ void seam_ssb_demod(const DevPlan &pl, const SeamDev &sd, const double2 *y, double *o,
-                                               size_t ei, int lane)
-{
-    const int Ls = pl.sos_Lseg, lo = lane * Ls;
-    const double2 e1 = pl.ssb_rot[1], r0 = pl.ssb_rot[lo];
-    double2 st[SEAM_NS], ph = r0;
-#pragma unroll
-    for (int j = 0; j < SEAM_NS; j++) st[j] = make_double2(0.0, 0.0);
-    for (int k = lo; k < lo + Ls; k++) {
-        ssb_step<2>(pl.out_sos, 2, st, cmul(y[k], cconj(ph)));
-        ph = cmul(ph, e1);
-    }
-    ssb_lane_scan(pl.sos_AP, st, lane);
-    double2 si[SEAM_NS];
-#pragma unroll
-    for (int j = 0; j < SEAM_NS; j++) {
-        si[j] = shfl_up_c(st[j], 1);
-        if (lane == 0) si[j] = make_double2(0.0, 0.0);
-    }
-    if (lane == 31)
-        for (int j = 0; j < SEAM_NS; j++) reinterpret_cast<double2 *>(sd.echunk)[ei * SEAM_NS + j] = st[j];
-    ph = r0;
-    for (int k = lo; k < lo + Ls; k++) {
-        const double2 v = ssb_step<2>(pl.out_sos, 2, si, cmul(y[k], cconj(ph)));
-        o[k] = fma(ph.x, v.x, -ph.y * v.y);
-        ph = cmul(ph, e1);
-    }
+    if (demod != SDRB_FM) return demod_scalar(y[k], demod);
+    if (last && k == M - 1) k = M - 2;
+    return pair_phase(y[k], y[k + 1]);
 }
 
 // warp <-> (emitted chunk, row), lane <-> segment of Lseg = M/32 outputs.  Without an output
-// filter the demodulated values are framed and stored; with it each lane runs the DF2T recurrence
-// over its segment from a zero state, a lane scan (A^Lseg powers) gives every segment its state
-// from the chunk start, the segment is re-run from that state, and the chunk's zero-state end
-// state goes to echunk.  The response to the state carried from earlier chunks is k_seam_frame's.
-// The SSB instance does the same with the complex band-pass (seam_ssb_demod).
+// filter the demodulated values are framed and stored; with it the output stage runs the cascade
+// from the chunk's zero state (sdrb_outstage.cuh) and the chunk's zero-state end state goes to
+// echunk.  The response to the state carried from earlier chunks is k_seam_frame's.  The SSB
+// instance runs the complex band-pass on y, its end state complex.
 template <bool SSB>
 __global__ void __launch_bounds__(256)
 k_seam_demod(const __grid_constant__ DevPlan pl, SeamDev sd, double *out, int ne, int nwin, int end)
 {
+    using T = std::conditional_t<SSB, double2, double>;
     const int lane = threadIdx.x & 31;
     const long item = (long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (item >= (long)ne * pl.R) return;
-    const int i = (int)(item / pl.R), r = (int)(item % pl.R), M = pl.M, Ls = pl.sos_Lseg;
+    const int i = (int)(item / pl.R), r = (int)(item % pl.R), M = pl.M, lo = lane * pl.sos_Lseg;
     const bool last = end && i == nwin - 1;
     const double2 *y = sd.ybuf + ((size_t)i * pl.R + r) * (M + 1);
-    if constexpr (SSB) {
-        seam_ssb_demod(pl, sd, y, out + (size_t)r * ne * M + (size_t)i * M, (size_t)i * pl.R + r, lane);
-        return;
-    }
-    if (pl.demod == SDRB_IQ) {     // rows of ne * 2M doubles, no output low-pass
-        double2 *o2 = reinterpret_cast<double2 *>(out + ((size_t)r * ne + i) * pl.W);
-        for (int k = lane; k < M; k += 32) {
-            double2 v = y[k];
-            if (pl.be_out) v = make_double2(bswap_double(v.x), bswap_double(v.y));
-            o2[k] = v;
-        }
-        return;
-    }
     double *o = out + (size_t)r * ne * M + (size_t)i * M;
-    if (pl.nsec_out == 0) {
-        for (int k = lane; k < M; k += 32) {
-            const double v = seam_demod_at(y, k, M, last, pl.demod);
-            o[k] = pl.be_out ? bswap_double(v) : v;
-        }
+    if (!SSB && pl.demod == SDRB_IQ) {     // rows of ne * 2M doubles, no output low-pass
+        double2 *o2 = reinterpret_cast<double2 *>(out + ((size_t)r * ne + i) * pl.W);
+        for (int k = lane; k < M; k += 32) frame_store(o2 + k, y[k], pl.be_out);
         return;
     }
-    const int lo = lane * Ls;
-    double st[SEAM_NS] = {0.0, 0.0, 0.0, 0.0};
-    for (int k = lo; k < lo + Ls; k++) {
-        double x = seam_demod_at(y, k, M, last, pl.demod);
-        o[k] = x;
-        seam_sos_step(pl.out_sos, pl.nsec_out, st, x);
+    if (!SSB && pl.nsec_out == 0) {
+        for (int k = lane; k < M; k += 32) frame_store(o + k, seam_demod_at(y, k, M, last, pl.demod), pl.be_out);
+        return;
     }
-    // inclusive lane scan of the segment end states: S_g = sum_{h<=g} AL^(g-h) e_h
-#pragma unroll
-    for (int lv = 0; lv < 5; lv++) {
-        double pv[SEAM_NS];
-#pragma unroll
-        for (int j = 0; j < SEAM_NS; j++) pv[j] = __shfl_up_sync(0xffffffffu, st[j], 1 << lv);
-        if (lane >= (1 << lv)) {
-            const double *Ap = pl.sos_AP + lv * 16;
-#pragma unroll
-            for (int a = 0; a < SEAM_NS; a++) {
-                double acc = st[a];
-#pragma unroll
-                for (int b = 0; b < SEAM_NS; b++) acc = fma(Ap[a * 4 + b], pv[b], acc);
-                st[a] = acc;
-            }
-        }
-    }
-    double sin_[SEAM_NS];
-#pragma unroll
-    for (int j = 0; j < SEAM_NS; j++) {
-        sin_[j] = __shfl_up_sync(0xffffffffu, st[j], 1);
-        if (lane == 0) sin_[j] = 0.0;
-    }
+    T st[SEAM_NS];
+    sos_segments(
+        pl, SEAM_NS / 2, lo, pl.sos_Lseg, lane,
+        [&](int j) {
+            if constexpr (SSB) return y[lo + j];
+            else return seam_demod_at(y, lo + j, M, last, pl.demod);
+        },
+        [&](int j) -> double & { return o[lo + j]; }, st);
     if (lane == 31)
-        for (int j = 0; j < SEAM_NS; j++) sd.echunk[((size_t)i * pl.R + r) * SEAM_NS + j] = st[j];
-    for (int k = lo; k < lo + Ls; k++) {
-        double x = o[k];
-        seam_sos_step(pl.out_sos, pl.nsec_out, sin_, x);
-        o[k] = x;
-    }
+        for (int j = 0; j < SEAM_NS; j++) reinterpret_cast<T *>(sd.echunk)[((size_t)i * pl.R + r) * SEAM_NS + j] = st[j];
 }
 
 // one warp per row, lane <-> contiguous run of chunks: sst[c] = SOS state at the start of emitted
@@ -455,7 +362,7 @@ k_seam_sscan(const __grid_constant__ DevPlan pl, SeamDev sd, int ne)
     T *sst = reinterpret_cast<T *>(sd.sst), *sos = reinterpret_cast<T *>(sd.sos);
     T a[SEAM_NS];
 #pragma unroll
-    for (int j = 0; j < SEAM_NS; j++) a[j] = seam_zero<T>();
+    for (int j = 0; j < SEAM_NS; j++) a[j] = zero_of<T>();
     double mm[SEAM_NS * SEAM_NS];
 #pragma unroll
     for (int j = 0; j < SEAM_NS * SEAM_NS; j++) mm[j] = (j % (SEAM_NS + 1)) == 0 ? 1.0 : 0.0;
@@ -464,9 +371,9 @@ k_seam_sscan(const __grid_constant__ DevPlan pl, SeamDev sd, int ne)
     auto matvec = [&](const double *A, const T *x, T *yv) {
 #pragma unroll
         for (int p = 0; p < SEAM_NS; p++) {
-            T acc = seam_zero<T>();
+            T acc = zero_of<T>();
 #pragma unroll
-            for (int q = 0; q < SEAM_NS; q++) acc = seam_fma(A[p * SEAM_NS + q], x[q], acc);
+            for (int q = 0; q < SEAM_NS; q++) acc = rfma(A[p * SEAM_NS + q], x[q], acc);
             yv[p] = acc;
         }
     };
@@ -495,7 +402,7 @@ k_seam_sscan(const __grid_constant__ DevPlan pl, SeamDev sd, int ne)
         T pa[SEAM_NS];
         double pm[SEAM_NS * SEAM_NS];
 #pragma unroll
-        for (int j = 0; j < SEAM_NS; j++) pa[j] = seam_shfl_up(a[j], 1 << lv);
+        for (int j = 0; j < SEAM_NS; j++) pa[j] = shfl_up_t(a[j], 1 << lv);
 #pragma unroll
         for (int j = 0; j < SEAM_NS * SEAM_NS; j++) pm[j] = __shfl_up_sync(0xffffffffu, mm[j], 1 << lv);
         double2 pph = ph;
@@ -514,13 +421,13 @@ k_seam_sscan(const __grid_constant__ DevPlan pl, SeamDev sd, int ne)
     double em[SEAM_NS * SEAM_NS];
     for (int j = 0; j < SEAM_NS; j++) st0[j] = sos[(size_t)r * SEAM_NS + j];
 #pragma unroll
-    for (int j = 0; j < SEAM_NS; j++) ea[j] = seam_shfl_up(a[j], 1);
+    for (int j = 0; j < SEAM_NS; j++) ea[j] = shfl_up_t(a[j], 1);
 #pragma unroll
     for (int j = 0; j < SEAM_NS * SEAM_NS; j++) em[j] = __shfl_up_sync(0xffffffffu, mm[j], 1);
     double2 eph = ph;
     if constexpr (CPX) eph = shfl_up_c(ph, 1);
     if (lane == 0) {
-        for (int j = 0; j < SEAM_NS; j++) ea[j] = seam_zero<T>();
+        for (int j = 0; j < SEAM_NS; j++) ea[j] = zero_of<T>();
         for (int j = 0; j < SEAM_NS * SEAM_NS; j++) em[j] = (j % (SEAM_NS + 1)) == 0 ? 1.0 : 0.0;
         eph = make_double2(1.0, 0.0);
     }
@@ -545,23 +452,12 @@ template <bool SSB>
 __global__ void __launch_bounds__(256)
 k_seam_frame(const __grid_constant__ DevPlan pl, SeamDev sd, double *out, int ne)
 {
+    using T = std::conditional_t<SSB, double2, double>;
     const size_t M = pl.M, total = (size_t)pl.R * ne * M;
     for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (size_t)gridDim.x * blockDim.x) {
         const size_t r = e / ((size_t)ne * M), rest = e % ((size_t)ne * M), i = rest / M, k = rest % M;
-        const double *ca = sd.CAM + k * SEAM_NS;
-        double v = out[e];
-        if constexpr (SSB) {
-            const double2 *s = reinterpret_cast<const double2 *>(sd.sst) + (i * pl.R + r) * SEAM_NS;
-            double2 w = make_double2(0.0, 0.0);
-#pragma unroll
-            for (int j = 0; j < SEAM_NS; j++) { w.x = fma(ca[j], s[j].x, w.x); w.y = fma(ca[j], s[j].y, w.y); }
-            const double2 ph = pl.ssb_rot[k];
-            v = fma(ph.x, w.x, fma(-ph.y, w.y, v));
-        } else {
-            const double *s = sd.sst + (i * pl.R + r) * SEAM_NS;
-#pragma unroll
-            for (int j = 0; j < SEAM_NS; j++) v = fma(ca[j], s[j], v);
-        }
-        out[e] = pl.be_out ? bswap_double(v) : v;
+        const T *s = reinterpret_cast<const T *>(sd.sst) + (i * pl.R + r) * SEAM_NS;
+        const double2 ph = SSB ? pl.ssb_rot[k] : make_double2(1.0, 0.0);
+        frame_store(out + e, add_response<SEAM_NS>(out[e], sd.CAM + k * SEAM_NS, SEAM_NS, s, ph), pl.be_out);
     }
 }

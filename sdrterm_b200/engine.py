@@ -81,8 +81,7 @@ class Engine:
         self._keep.append(nco)
         tab.use_nco = nco.ctypes.data_as(C.POINTER(C.c_uint8))
         tab.sos_Lseg = int(pl.sos_Lseg)
-        if pl.sos_AL is not None:
-            put('sos_AL', pl.sos_AL)
+        if pl.sos_CA is not None:
             put('sos_CA', pl.sos_CA)
             put('sos_AP', pl.sos_AP)
         tab.lam_N = float(pl.lam_N)

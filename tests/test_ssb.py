@@ -166,7 +166,7 @@ def test_header_constants_match_python():
     m = re.search(r'enum sdrb_demod \{([^}]*)\}', src)
     consts = dict((k, int(v)) for k, v in re.findall(r'(SDRB_\w+) = (\d+)', m.group(1)))
     assert consts['SDRB_USB'] == nat.USB and consts['SDRB_LSB'] == nat.LSB
-    assert int(re.search(r'#define SDRB_ABI_VERSION (\d+)', src).group(1)) == nat.ABI_VERSION == 9
+    assert int(re.search(r'#define SDRB_ABI_VERSION (\d+)', src).group(1)) == nat.ABI_VERSION == 10
     assert 'sdrb_ssb_demod' in nat.EXPORTS and 'int sdrb_ssb_demod(' in src
     assert [f[0] for f in nat.Tables._fields_][-2:] == ['ssb_omega', 'ssb_rot']
 
