@@ -417,9 +417,9 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
     if (cfg->R < 1 || cfg->edge < 1 || cfg->N <= cfg->edge + 1 || cfg->max_chunks < 1 || cfg->n_out_sections < 0 ||
         cfg->n_out_sections > 4)
         return fail(nullptr, SDRB_ERR_ARG, "bad geometry");
-    {   // k_fixup stages (edge+1) head samples and nend = max(rem, edge+1) window samples in s_x[320]
+    {   // k_fixup stages (edge+1) head samples and nend = max(rem, edge+1) window samples in shared memory
         const int rem = cfg->N % cfg->q;
-        if (cfg->edge + 1 + std::max(rem, cfg->edge + 1) > 320)
+        if (cfg->edge + 1 + std::max(rem, cfg->edge + 1) > SDRB_NEDGE)
             return fail(nullptr, SDRB_ERR_ARG, "filter pad %d too long for the fix-up kernel", cfg->edge);
     }
     {
@@ -644,8 +644,7 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
         SeamDev &sd = h->sd;
         if (pl.rem != 0 || pl.cnt_last != SDRB_TB || tab->lookahead < 1 || !tab->PN || !tab->chunk_step ||
             tab->fs <= 0 || tab->fs >= (1LL << 31) || (cfg->n_out_sections != 0 && cfg->n_out_sections != 2) ||
-            (cfg->n_out_sections && (!tab->sos_AM || !tab->sos_CAM || pl.sos_Lseg * 32 != M)) ||
-            pl.edge + 1 > 64 || pl.nend > 64)
+            (cfg->n_out_sections && (!tab->sos_AM || !tab->sos_CAM || pl.sos_Lseg * 32 != M)))
             return bail(fail(h, SDRB_ERR_ARG, "seamless mode needs the decimation to divide the chunk (q | N), "
                                               "a lookahead >= 1 and its tables"));
         sd.D = tab->lookahead; sd.fs = tab->fs; sd.nedge = pl.edge + 1 + pl.nend;
@@ -848,7 +847,7 @@ int seam_step(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, cudaS
         if (rc) return rc;
         const size_t items = nch * (size_t)R;
         k_seam_agg<<<(unsigned)((items + 7) / 8), 256, 0, st>>>(pl, h->sc, sd, s0, (int)nch, h->seen);
-        if (h->seen == 0) k_seam_head<<<(unsigned)((R + 63) / 64), 64, 0, st>>>(pl, h->sc, sd, s0);
+        if (h->seen == 0) k_seam_head<<<(unsigned)R, 32, 0, st>>>(pl, h->sc, sd, s0);
         k_seam_fscan<<<(unsigned)R, 256, 0, st>>>(pl, sd, s0, (int)nch);
         h->launches += 3 + (h->seen == 0);
         h->seen += (long long)nch;
@@ -859,7 +858,7 @@ int seam_step(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, cudaS
     const long long g0 = h->emitted;
     if (ne > 0) {
         if (end) {
-            k_seam_tail<<<(unsigned)((R + 63) / 64), 64, 0, st>>>(pl, h->sc, sd, h->nwin - 1, h->seen - 1);
+            k_seam_tail<<<(unsigned)R, 32, 0, st>>>(pl, h->sc, sd, h->nwin - 1, h->seen - 1);
             h->launches++;
         }
         const size_t items = (size_t)ne * R;

@@ -7,6 +7,7 @@
 #define SDRB_TB 32          // blocks per tile == warp width (lane <-> block)
 #define SDRB_NP 8           // poles of the cheby1 order-8 decimation low-pass
 #define SDRB_XSTRIDE 33     // exchange buffer row stride in doubles
+#define SDRB_NEDGE 320      // edge samples a chunk-boundary kernel stages: head (edge+1) + end window (nend)
 
 enum { ENC_b = 0, ENC_B, ENC_h, ENC_H, ENC_i, ENC_I, ENC_f, ENC_d, ENC_Z };
 

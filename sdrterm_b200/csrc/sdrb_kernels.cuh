@@ -568,19 +568,165 @@ __global__ void k_iq_prefix(Scratch sc, const double *gains3, int rank, double l
     }
 }
 
+// ------------------------------------------------------------------------- chunk boundary
+// sosfiltfilt's boundary at a chunk's edges and the modal carries across its tiles, shared by k_fixup
+// and the seamless kernels: one warp stages the edge samples in shared memory, lane <-> mode i runs
+// the modal pieces.  The front ends sum the UNcorrected rotated samples, so their frame has
+// W~ = (w + alpha s) / beta and T~ = (T + alphaT s) / betaT, s = off[n] e^{jwn} (DESIGN.md 3.3).
+
+// Edge samples s[0..n), raw -> IQ-corrected (read_file.py:72-77) from o, the offset at sample nb:
+// s[0..nb) BACKWARD (off[n] = (off[n+1] - L z[n]) / lam), s[nb..n) forward; then times the NCO
+// phases E[0..n).
+__device__ __forceinline__ void stage_edge(const DevPlan &pl, double2 *s, int n, int nb, double2 o,
+                                           const double2 *E, int lane)
+{
+    if (pl.correct_iq) {
+        if (lane == 0) {
+            for (int j = nb - 1; j >= 0; j--) {
+                const double2 z = s[j];
+                o.x = fma(-pl.Liq, z.x, o.x) * pl.lam_inv; o.y = fma(-pl.Liq, z.y, o.y) * pl.lam_inv;
+                s[j] = csub(z, o);
+            }
+        } else if (lane == 1) {
+            for (int j = nb; j < n; j++) {
+                const double2 x = csub(s[j], o);
+                o.x = fma(x.x, pl.Liq, o.x); o.y = fma(x.y, pl.Liq, o.y);
+                s[j] = x;
+            }
+        }
+    }
+    __syncwarp();
+    for (int j = lane; j < n; j += 32) s[j] = cmul(s[j], E[j]);
+    __syncwarp();
+}
+__device__ __forceinline__ void stage_head(const DevPlan &pl, int r, double2 *s_h, double2 off0, int lane)
+{
+    stage_edge(pl, s_h, pl.edge + 1, 0, off0, pl.Ehead + (size_t)r * (pl.edge + 1), lane);
+}
+__device__ __forceinline__ void stage_end(const DevPlan &pl, int r, double2 *s_e, double2 offE, int lane)
+{
+    stage_edge(pl, s_e, pl.nend, pl.nend - pl.rem, offE, pl.Eend + (size_t)r * pl.nend, lane);
+}
+
+// Mode i: the forward state at n = edge from the staged head (odd extension 2 x0 - x[edge-j], zi),
+// as W~ with s = o, the offset at sample 0.
+__device__ __forceinline__ double2 head_state(const DevPlan &pl, int r, const double2 *s_h, double2 o, int i)
+{
+    const int edge = pl.edge;
+    const double2 p = pl.p[i], x0 = s_h[0];
+    double2 w = cmul(pl.zhat[i], csub(cscale(2.0, x0), s_h[edge]));
+    for (int j = 0; j < edge; j++) {
+        const double2 ext = csub(cscale(2.0, x0), s_h[edge - j]);
+        w = cfma(p, w, ext);
+    }
+    if (pl.correct_iq) w = cmul(cfma(pl.alpha[(size_t)r * 8 + i], o, w), pl.binv[(size_t)r * 8 + i]);
+    return w;
+}
+
+struct EndState {
+    double2 w, T, Tt, zeta;     // at q*Mf: the true forward and anticausal states, T~; zeta
+};
+
+// Mode i from W~, the forward state at q*Mf, and the staged end window: the partial block then the
+// tail extension 2 x[N-1] - x[N-2-j] run forward (w at the last two samples) and anticausally back to
+// q*Mf (T); zeta from y_f at the last sample.  o is the offset at q*Mf.  All 32 lanes must call it
+// (the cross-mode sums shuffle within groups of 8 lanes); the modes' results are those of lanes 0..7.
+__device__ __forceinline__ EndState end_state(const DevPlan &pl, int r, const double2 *s_e, double2 o, double2 Wt, int i)
+{
+    const bool iq = pl.correct_iq != 0;
+    const int nend = pl.nend, rem = pl.rem, nseq = rem + pl.edge;
+    const double2 p = pl.p[i];
+    const double2 sE = iq ? cmul(o, pl.phE[r]) : make_double2(0.0, 0.0);   // rotated offset at q*Mf
+    EndState e;
+    double2 w = iq ? csub(cmul(pl.beta[(size_t)r * 8 + i], Wt), cmul(pl.alpha[(size_t)r * 8 + i], sE)) : Wt;
+    e.w = w;
+    const double2 xN1 = s_e[nend - 1];
+    auto seq = [&](int k) {
+        return k < rem ? s_e[nend - rem + k] : csub(cscale(2.0, xN1), s_e[nend - 2 - (k - rem)]);
+    };
+    double2 wL1 = w, last = make_double2(0.0, 0.0);
+    for (int k = 0; k < nseq; k++) {
+        const double2 v = seq(k);
+        if (k == nseq - 1) { wL1 = w; last = v; }
+        w = cfma(p, w, v);
+    }
+    double2 T = make_double2(0.0, 0.0);
+    for (int k = nseq - 1; k >= 0; k--) T = cfma(p, T, seq(k));
+    e.T = T;
+    e.Tt = iq ? cmul(cfma(pl.alphaT[(size_t)r * 8 + i], sE, T), pl.binvT[(size_t)r * 8 + i]) : T;
+    // y_f[L-1] = sum_l c_l w_l[L-1] + d ext[L-1]   (reduce over the 8 mode lanes)
+    double2 part = cmul(pl.c[i], wL1);
+    for (int sft = 1; sft < 8; sft <<= 1) part = cadd(part, shfl_xor_c(part, sft));
+    const double2 yfL1 = make_double2(fma(pl.d, last.x, part.x), fma(pl.d, last.y, part.y));
+    e.zeta = cmul(pl.zhat[i], yfL1);
+    for (int l = 0; l < 8; l++) e.zeta = csub(e.zeta, cmul(pl.xi[i * 8 + l], shfl_c(w, l)));
+    return e;
+}
+
+// Mode i's carries across a chunk's tiles from the state w at one end: forward from tile 0 (the
+// carry-in of tile t goes to slot t, column i) or backward from q*Mf (slot t+1, column 8+i; the state
+// at tile 0 to slot 0).  store(slot * 16 + column, be w) keeps them, pre-scaled by beta / betaT for
+// the outputs; returns the state at the other end.
+template <class Store>
+__device__ __forceinline__ double2 tile_carries(const DevPlan &pl, const double2 *T1, const double2 *agg, int i,
+                                                bool fwd, double2 be, double2 w, Store store)
+{
+    const int nt = pl.ntiles, o = fwd ? i : 8 + i;
+    for (int s = 0; s < nt; s++) {
+        const int t = fwd ? s : nt - 1 - s;
+        store((size_t)(fwd ? t : t + 1) * 16 + o, cmul(be, w));
+        const int cnt = (t == nt - 1) ? pl.cnt_last : SDRB_TB;
+        w = cfma(pl.Ppow[(size_t)cnt * 8 + i], w, cmul(T1[t], agg[(size_t)t * 16 + o]));
+    }
+    if (!fwd) store((size_t)o, cmul(be, w));
+    return w;
+}
+
+// Outputs at the full-block starts k = first, first + stride, .. < Mf (tile t, block l):
+// T1 (ypart - off psiY) + sum RW Win + RT Tn, plus bnd zeta from k = k_bnd on; each goes to store(k, v).
+template <class Store>
+__device__ __forceinline__ void block_outputs(const DevPlan &pl, int r, const double2 *ypart, const double2 *offt,
+                                              const double2 *T1, const double2 *carry, const double2 *zeta,
+                                              int k_bnd, int first, int stride, Store store)
+{
+    const int nt = pl.ntiles;
+    for (int k = first; k < pl.Mf; k += stride) {
+        const int t = k / SDRB_TB, l = k % SDRB_TB;
+        const int kind = (t == nt - 1) ? 1 : 0;
+        const int cnt = kind ? pl.cnt_last : SDRB_TB;
+        double2 v = ypart[k];
+        if (pl.correct_iq) {
+            const double2 s = make_double2(-offt[t].x, -offt[t].y);
+            v = cfma(s, pl.psiY[((size_t)kind * pl.R + r) * SDRB_TB + l], v);
+        }
+        v = cmul(T1[t], v);
+        const double2 *Win = carry + (size_t)t * 16, *Tn = carry + (size_t)(t + 1) * 16 + 8;
+#pragma unroll
+        for (int i = 0; i < 8; i++) {
+            v = cfma(pl.RW[(size_t)l * 8 + i], Win[i], v);
+            v = cfma(pl.RT[(size_t)(cnt - l) * 8 + i], Tn[i], v);
+        }
+        if (k >= k_bnd) {
+#pragma unroll
+            for (int i = 0; i < 8; i++) v = cfma(pl.bnd[(size_t)k * 8 + i], zeta[i], v);
+        }
+        store(k, v);
+    }
+}
+
 // ----------------------------------------------------------------------------------- k_fixup
-// One CTA per (chunk, row).  Warp 0: raw head / end-window samples are fetched by all lanes at
-// once, then lanes 0..7 <-> poles run the head, the cross-tile carries, the end segment and the
-// boundary vector zeta; then all threads emit y[k].
+// One CTA per (chunk, row).  Warp 0 stages the head and end-window samples; lanes 0..7 <-> modes run
+// the head, the forward carries, the end segment and zeta, the partial block's output and the
+// backward carries; then all threads emit the outputs at the full-block starts.
 template <int ENC>
 __global__ void __launch_bounds__(128)
 k_fixup(const __grid_constant__ DevPlan pl, Scratch sc, const uint8_t *__restrict__ raw, int nchunks)
 {
-    __shared__ double2 s_x[320];       // head samples (edge+1) then end-window samples (nend)
+    __shared__ double2 s_x[SDRB_NEDGE];    // head samples (edge+1) then end-window samples (nend)
     __shared__ double2 s_zeta[SDRB_NP];
     const int chunk = blockIdx.x / pl.R, r = blockIdx.x % pl.R;
     if (chunk >= nchunks) return;
-    const int nt = pl.ntiles, edge = pl.edge, q = pl.q;
+    const int nt = pl.ntiles, edge = pl.edge;
     const uint8_t *rawc = raw + (size_t)chunk * pl.N * pl.sb;
     const double2 *offt = sc.off_tile + (size_t)chunk * (nt + 1);
     const double2 *aggr = sc.agg + ((size_t)chunk * pl.R + r) * nt * 16;
@@ -588,145 +734,34 @@ k_fixup(const __grid_constant__ DevPlan pl, Scratch sc, const uint8_t *__restric
     double2 *yrow = sc.y + ((size_t)chunk * pl.R + r) * pl.M;
     const double2 *T1r = pl.T1 + (size_t)r * nt;
     double2 *s_h = s_x, *s_e = s_x + (edge + 1);
-    const bool iq = pl.correct_iq != 0;
 
     if (threadIdx.x < 32) {
-        const int lane = threadIdx.x;
+        const int lane = threadIdx.x, i = lane & 7;
         // fetch: raw head samples and the raw end window; every load is independent
         for (int n = lane; n <= edge; n += 32) s_h[n] = decode_sample<ENC>(pl, rawc, n);
-        for (int i = lane; i < pl.nend; i += 32) s_e[i] = decode_sample<ENC>(pl, rawc, (long)pl.ws + i);
+        for (int j = lane; j < pl.nend; j += 32) s_e[j] = decode_sample<ENC>(pl, rawc, (long)pl.ws + j);
         __syncwarp();
-        // serial IQ recurrences over these few samples (read_file.py:72-77): the head runs forward
-        // from the chunk-start offset, the partial block forward from the offset at q*Mf, and the
-        // window samples inside full blocks BACKWARD from the offset at q*Mf
-        // (off[n] = (off[n+1] - L z[n]) / lam), then the NCO phases
-        if (iq) {
-            if (lane == 0) {
-                double2 o = offt[0];
-                for (int n = 0; n <= edge; n++) {
-                    const double2 x = csub(s_h[n], o);
-                    o.x = fma(x.x, pl.Liq, o.x); o.y = fma(x.y, pl.Liq, o.y);
-                    s_h[n] = x;
-                }
-            } else if (lane == 1 && pl.rem) {
-                double2 o = offt[nt];
-                for (int i = pl.nend - pl.rem; i < pl.nend; i++) {
-                    const double2 x = csub(s_e[i], o);
-                    o.x = fma(x.x, pl.Liq, o.x); o.y = fma(x.y, pl.Liq, o.y);
-                    s_e[i] = x;
-                }
-            } else if (lane == 2) {
-                double2 o = offt[nt];
-                for (int i = pl.nend - pl.rem - 1; i >= 0; i--) {
-                    const double2 z = s_e[i];
-                    o.x = fma(-pl.Liq, z.x, o.x) * pl.lam_inv; o.y = fma(-pl.Liq, z.y, o.y) * pl.lam_inv;
-                    s_e[i] = csub(z, o);
-                }
-            }
-            __syncwarp();
-        }
-        for (int n = lane; n <= edge; n += 32) s_h[n] = cmul(s_h[n], pl.Ehead[(size_t)r * (edge + 1) + n]);
-        for (int i = lane; i < pl.nend; i += 32) s_e[i] = cmul(s_e[i], pl.Eend[(size_t)r * pl.nend + i]);
-        __syncwarp();
-
-        const int i = lane & 7;                       // pole handled by this lane (lanes >= 8 mirror)
-        const double2 p = pl.p[i];
-        // head: odd extension, zi, edge samples -> state at n = edge
-        const double2 x0 = s_h[0];
-        double2 w = cmul(pl.zhat[i], csub(cscale(2.0, x0), s_h[edge]));
-        for (int j = 0; j < edge; j++) {
-            const double2 ext = csub(cscale(2.0, x0), s_h[edge - j]);
-            w = cfma(p, w, ext);
-        }
-        // forward carries across tiles, in the frame of the UNcorrected samples the front ends
-        // summed: W~ = (w + alpha s) / beta with s = off e^{jwn} (n = 0: the chunk-start offset);
-        // the carries are stored pre-scaled by beta for the output stage
-        const double2 al = pl.alpha[(size_t)r * 8 + i], be = pl.beta[(size_t)r * 8 + i];
-        const double2 alT = pl.alphaT[(size_t)r * 8 + i], beT = pl.betaT[(size_t)r * 8 + i];
-        const double2 sE = iq ? cmul(offt[nt], pl.phE[r]) : make_double2(0.0, 0.0);   // rotated offset at q*Mf
-        if (iq) w = cmul(cfma(al, offt[0], w), pl.binv[(size_t)r * 8 + i]);
-        for (int t = 0; t < nt; t++) {
-            if (lane < 8) carry[(size_t)t * 16 + i] = iq ? cmul(be, w) : w;
-            const int kind = (t == nt - 1) ? 1 : 0;
-            const int cnt = kind ? pl.cnt_last : SDRB_TB;
-            w = cfma(pl.Ppow[(size_t)cnt * 8 + i], w, cmul(T1r[t], aggr[(size_t)t * 16 + i]));
-        }
-        if (iq) w = csub(cmul(be, w), cmul(al, sE));              // back to the true state at q*Mf
-        if (lane < 8) carry[(size_t)nt * 16 + i] = iq ? cfma(al, sE, w) : w;   // = beta W~
-        const double2 wEnd = w;
-        // end segment: partial block then tail extension
-        const int nseq = pl.rem + edge;
-        const double2 xN1 = s_e[pl.nend - 1];
-        double2 wL1 = w, last = make_double2(0.0, 0.0);
-        for (int k = 0; k < nseq; k++) {
-            const double2 v = (k < pl.rem) ? s_e[pl.nend - pl.rem + k]
-                                           : csub(cscale(2.0, xN1), s_e[pl.nend - 2 - (k - pl.rem)]);
-            if (k == nseq - 1) { wL1 = w; last = v; }
-            w = cfma(p, w, v);
-        }
-        const double2 wL = w;
-        double2 T = make_double2(0.0, 0.0);
-        for (int k = nseq - 1; k >= 0; k--) {
-            const double2 v = (k < pl.rem) ? s_e[pl.nend - pl.rem + k]
-                                           : csub(cscale(2.0, xN1), s_e[pl.nend - 2 - (k - pl.rem)]);
-            T = cfma(p, T, v);
-        }
-        const double2 Tend = T;
-        // y_f[L-1] = sum_l c_l w_l[L-1] + d ext[L-1]   (reduce over the 8 pole lanes)
-        double2 part = cmul(pl.c[i], wL1);
-        for (int sft = 1; sft < 8; sft <<= 1) part = cadd(part, shfl_xor_c(part, sft));
-        const double2 yfL1 = make_double2(fma(pl.d, last.x, part.x), fma(pl.d, last.y, part.y));
-        double2 zeta = cmul(pl.zhat[i], yfL1);
-        for (int l = 0; l < 8; l++) {
-            const double2 wl = shfl_c(wL, l);
-            zeta = csub(zeta, cmul(pl.xi[i * 8 + l], wl));
-        }
-        if (lane < 8) s_zeta[i] = zeta;
-        if (pl.rem) {
-            double2 v = cfma(pl.rho[i], wEnd, cmul(pl.rho_p[i], Tend));
-            v = cfma(pl.bnd[(size_t)pl.Mf * 8 + i], zeta, v);
+        stage_head(pl, r, s_h, offt[0], lane);
+        stage_end(pl, r, s_e, offt[nt], lane);
+        double2 w = head_state(pl, r, s_h, offt[0], i);
+        auto keep = [&](size_t j, double2 v) { carry[j] = v; };
+        if (lane < 8) w = tile_carries(pl, T1r, aggr, i, true, pl.beta[(size_t)r * 8 + i], w, keep);
+        const EndState e = end_state(pl, r, s_e, offt[nt], w, i);
+        if (lane < 8) s_zeta[i] = e.zeta;
+        if (pl.rem) {       // the output at the partial block
+            double2 v = cfma(pl.rho[i], e.w, cmul(pl.rho_p[i], e.T));
+            v = cfma(pl.bnd[(size_t)pl.Mf * 8 + i], e.zeta, v);
             for (int sft = 1; sft < 8; sft <<= 1) v = cadd(v, shfl_xor_c(v, sft));
             if (lane == 0) {
                 const double2 xp = s_e[pl.nend - pl.rem];
                 yrow[pl.Mf] = make_double2(fma(pl.g0, xp.x, v.x), fma(pl.g0, xp.y, v.y));
             }
         }
-        // backward carries: T~ = (T + alphaT s) / betaT at q*Mf, stored pre-scaled by betaT
-        T = Tend;
-        if (iq) T = cmul(cfma(alT, sE, T), pl.binvT[(size_t)r * 8 + i]);
-        if (lane < 8) carry[(size_t)nt * 16 + 8 + i] = iq ? cmul(beT, T) : T;
-        for (int t = nt - 1; t >= 0; t--) {
-            const int kind = (t == nt - 1) ? 1 : 0;
-            const int cnt = kind ? pl.cnt_last : SDRB_TB;
-            T = cfma(pl.Ppow[(size_t)cnt * 8 + i], T, cmul(T1r[t], aggr[(size_t)t * 16 + 8 + i]));
-            if (lane < 8) carry[(size_t)t * 16 + 8 + i] = iq ? cmul(beT, T) : T;
-        }
+        if (lane < 8) tile_carries(pl, T1r, aggr, i, false, pl.betaT[(size_t)r * 8 + i], e.Tt, keep);
     }
     __syncthreads();
-    // outputs at the full-block starts
-    const double2 *ypr = sc.ypart + ((size_t)chunk * pl.R + r) * pl.Mf;
-    for (int k = threadIdx.x; k < pl.Mf; k += blockDim.x) {
-        const int t = k / SDRB_TB, l = k % SDRB_TB;
-        const int kind = (t == nt - 1) ? 1 : 0;
-        const int cnt = kind ? pl.cnt_last : SDRB_TB;
-        double2 v = ypr[k];
-        if (iq) {
-            const double2 s = make_double2(-offt[t].x, -offt[t].y);
-            v = cfma(s, pl.psiY[((size_t)kind * pl.R + r) * SDRB_TB + l], v);
-        }
-        v = cmul(T1r[t], v);
-        const double2 *Win = carry + (size_t)t * 16, *Tn = carry + (size_t)(t + 1) * 16 + 8;
-#pragma unroll
-        for (int i = 0; i < 8; i++) {
-            v = cfma(pl.RW[(size_t)l * 8 + i], Win[i], v);
-            v = cfma(pl.RT[(size_t)(cnt - l) * 8 + i], Tn[i], v);
-        }
-        if (k >= pl.k_bnd) {
-#pragma unroll
-            for (int i = 0; i < 8; i++) v = cfma(pl.bnd[(size_t)k * 8 + i], s_zeta[i], v);
-        }
-        yrow[k] = v;
-    }
+    block_outputs(pl, r, sc.ypart + ((size_t)chunk * pl.R + r) * pl.Mf, offt, T1r, carry, s_zeta, pl.k_bnd,
+                  threadIdx.x, blockDim.x, [&](int k, double2 v) { yrow[k] = v; });
 }
 
 // ----------------------------------------------------------------------------------- k_demod

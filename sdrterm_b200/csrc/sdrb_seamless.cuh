@@ -10,6 +10,7 @@
 //   k_seam_head    the stream's real start: odd extension and zi, forward state at sample 0
 //   k_seam_fscan   forward modal state across chunks: affine scan with multiplier p^N per mode
 //   k_seam_tail    the stream's real end: anticausal state after the last chunk and zeta
+//                  (k_seam_agg / head / tail / y run k_fixup's chunk-boundary functions, sdrb_kernels.cuh)
 //   k_seam_carry   per emitted chunk: carry-ins in its own frame (forward state, anticausal window
 //                  over the next D chunks or the real end, zeta) and the fm halo y[k+1]
 //   k_seam_y       per emitted chunk: tile carries and the decimated outputs, global frame
@@ -87,46 +88,25 @@ k_seam_agg(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int slot0
     const int lane = threadIdx.x & 31;
     const long item = (long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (item >= (long)nch * pl.R || lane >= 16) return;
-    const int c = slot0 + (int)(item / pl.R), r = (int)(item % pl.R), nt = pl.ntiles, m = lane & 7;
-    const double2 *ag = sc.agg + ((size_t)c * pl.R + r) * nt * 16;
-    const double2 *T1 = pl.T1 + (size_t)r * nt;
-    double2 a = make_double2(0.0, 0.0);
-    if (lane < 8) {
-        for (int t = 0; t < nt; t++) {
-            const double2 Pc = pl.Ppow[(t == nt - 1 ? pl.cnt_last : SDRB_TB) * 8 + m];
-            a = cfma(Pc, a, cmul(T1[t], ag[(size_t)t * 16 + m]));
-        }
-    } else {
-        for (int t = nt - 1; t >= 0; t--) {
-            const double2 Pc = pl.Ppow[(t == nt - 1 ? pl.cnt_last : SDRB_TB) * 8 + m];
-            a = cfma(Pc, a, cmul(T1[t], ag[(size_t)t * 16 + 8 + m]));
-        }
-    }
+    const int c = slot0 + (int)(item / pl.R), r = (int)(item % pl.R), nt = pl.ntiles;
+    const double2 a = tile_carries(pl, pl.T1 + (size_t)r * nt, sc.agg + ((size_t)c * pl.R + r) * nt * 16, lane & 7,
+                                   lane < 8, make_double2(1.0, 0.0), make_double2(0.0, 0.0), [](size_t, double2) {});
     sd.cagg[((size_t)c * pl.R + r) * 16 + lane] = cmul(seam_phasor(sd, r, g0 + (c - slot0)), a);
 }
 
-// thread <-> row: forward state at sample 0 of the stream (sosfiltfilt's odd extension and zi)
-__global__ void k_seam_head(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int slot)
+// warp <-> row: forward state at sample 0 of the stream (sosfiltfilt's odd extension and zi)
+__global__ void __launch_bounds__(32)
+k_seam_head(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int slot)
 {
-    const int r = blockIdx.x * blockDim.x + threadIdx.x;
-    if (r >= pl.R) return;
-    const int edge = pl.edge;
+    __shared__ double2 s_h[SDRB_NEDGE];
+    const int r = blockIdx.x, lane = threadIdx.x;
     const double2 *z = sd.edges + (size_t)slot * sd.nedge;
-    const double2 off0 = pl.correct_iq ? sc.off_tile[(size_t)slot * (pl.ntiles + 1)] : make_double2(0.0, 0.0);
-    double2 xs[64];
-    double2 o = off0;
-    for (int n = 0; n <= edge; n++) {
-        const double2 x = csub(z[n], o);
-        o = make_double2(fma(pl.Liq, x.x, o.x), fma(pl.Liq, x.y, o.y));
-        xs[n] = cmul(x, pl.Ehead[(size_t)r * (edge + 1) + n]);
-    }
-    for (int m = 0; m < 8; m++) {
-        const double2 e0 = csub(cscale(2.0, xs[0]), xs[edge]);
-        double2 w = cmul(pl.zhat[m], e0);
-        for (int j = 0; j < edge; j++) w = cfma(pl.p[m], w, csub(cscale(2.0, xs[0]), xs[edge - j]));
-        w = cfma(pl.alpha[(size_t)r * 8 + m], off0, w);
-        sd.fwd[(size_t)r * 8 + m] = cmul(w, pl.binv[(size_t)r * 8 + m]);
-    }
+    const double2 off0 = sc.off_tile[(size_t)slot * (pl.ntiles + 1)];
+    for (int n = lane; n <= pl.edge; n += 32) s_h[n] = z[n];
+    __syncwarp();
+    stage_head(pl, r, s_h, off0, lane);
+    const double2 w = head_state(pl, r, s_h, off0, lane & 7);
+    if (lane < 8) sd.fwd[(size_t)r * 8 + lane] = w;
 }
 
 // block <-> row, warp <-> mode, lane <-> contiguous run of chunks: G[c] = state before chunk c,
@@ -159,43 +139,22 @@ k_seam_fscan(const __grid_constant__ DevPlan pl, SeamDev sd, int slot0, int nch)
     if (lane == 31) sd.fwd[(size_t)r * 8 + m] = cfma(mul, st0, a);
 }
 
-// thread <-> row: the stream's real end (the last chunk sits in window slot `slot`, global index g)
-__global__ void k_seam_tail(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int slot, long long g)
+// warp <-> row: the stream's real end (the last chunk sits in window slot `slot`, global index g)
+__global__ void __launch_bounds__(32)
+k_seam_tail(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int slot, long long g)
 {
-    const int r = blockIdx.x * blockDim.x + threadIdx.x;
-    if (r >= pl.R) return;
-    const int edge = pl.edge, nend = pl.nend, nt = pl.ntiles;
-    const double2 *z = sd.edges + (size_t)slot * sd.nedge + edge + 1;
-    const double2 offE = pl.correct_iq ? sc.off_tile[(size_t)slot * (nt + 1) + nt] : make_double2(0.0, 0.0);
-    double2 xs[64];
-    double2 o = offE;
-    for (int n = pl.N - 1; n >= pl.ws; n--) {
-        const double2 zn = z[n - pl.ws];
-        o = make_double2((o.x - pl.Liq * zn.x) * pl.lam_inv, (o.y - pl.Liq * zn.y) * pl.lam_inv);
-        xs[n - pl.ws] = cmul(csub(zn, o), pl.Eend[(size_t)r * nend + (n - pl.ws)]);
-    }
+    __shared__ double2 s_e[SDRB_NEDGE];
+    const int r = blockIdx.x, lane = threadIdx.x, m = lane & 7;
+    const double2 *z = sd.edges + (size_t)slot * sd.nedge + pl.edge + 1;
+    const double2 offE = sc.off_tile[(size_t)slot * (pl.ntiles + 1) + pl.ntiles];
+    for (int j = lane; j < pl.nend; j += 32) s_e[j] = z[j];
+    __syncwarp();
+    stage_end(pl, r, s_e, offE, lane);
     const double2 ph = seam_phasor(sd, r, g);
-    const double2 sE = cmul(offE, pl.phE[r]);
-    double2 seq[64];
-    for (int j = 0; j < edge; j++) seq[j] = csub(cscale(2.0, xs[nend - 1]), xs[nend - 2 - j]);
-    double2 wL1[8], wL[8];
-    double2 yf = cscale(pl.d, seq[edge - 1]);
-    for (int m = 0; m < 8; m++) {
-        double2 w = csub(cmul(pl.beta[(size_t)r * 8 + m], cmul(cconj(ph), sd.fwd[(size_t)r * 8 + m])),
-                         cmul(pl.alpha[(size_t)r * 8 + m], sE));
-        for (int j = 0; j < edge - 1; j++) w = cfma(pl.p[m], w, seq[j]);
-        wL1[m] = w;
-        wL[m] = cfma(pl.p[m], w, seq[edge - 1]);
-        yf = cfma(pl.c[m], wL1[m], yf);
-    }
-    for (int m = 0; m < 8; m++) {
-        double2 zt = cmul(pl.zhat[m], yf);
-        for (int l = 0; l < 8; l++) zt = csub(zt, cmul(pl.xi[m * 8 + l], wL[l]));
-        double2 T = make_double2(0.0, 0.0);
-        for (int j = edge - 1; j >= 0; j--) T = cfma(pl.p[m], T, seq[j]);
-        T = cmul(cfma(pl.alphaT[(size_t)r * 8 + m], sE, T), pl.binvT[(size_t)r * 8 + m]);
-        sd.endv[(size_t)r * 16 + m] = cmul(ph, T);
-        sd.endv[(size_t)r * 16 + 8 + m] = cmul(ph, zt);
+    const EndState e = end_state(pl, r, s_e, offE, cmul(cconj(ph), sd.fwd[(size_t)r * 8 + m]), m);
+    if (lane < 8) {
+        sd.endv[(size_t)r * 16 + m] = cmul(ph, e.Tt);
+        sd.endv[(size_t)r * 16 + 8 + m] = cmul(ph, e.zeta);
     }
 }
 
@@ -251,54 +210,20 @@ k_seam_y(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int ne, int
     const int lane = threadIdx.x & 31;
     const long item = (long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (item >= (long)ne * pl.R) return;
-    const int i = (int)(item / pl.R), r = (int)(item % pl.R), nt = pl.ntiles, R = pl.R, M = pl.M;
+    const int i = (int)(item / pl.R), r = (int)(item % pl.R), nt = pl.ntiles, R = pl.R, M = pl.M, m = lane & 7;
     const double2 *ci = sd.cin + ((size_t)i * R + r) * 24;
-    const double2 *ag = sc.agg + ((size_t)i * R + r) * nt * 16;
     const double2 *T1 = pl.T1 + (size_t)r * nt;
     double2 *carry = sc.carry + ((size_t)i * R + r) * (nt + 1) * 16;
-    if (lane < 8) {
-        const int m = lane;
-        const double2 b = pl.beta[(size_t)r * 8 + m];
-        double2 w = ci[m];
-        for (int t = 0; t < nt; t++) {
-            carry[(size_t)t * 16 + m] = cmul(b, w);
-            w = cfma(pl.Ppow[SDRB_TB * 8 + m], w, cmul(T1[t], ag[(size_t)t * 16 + m]));
-        }
-    } else if (lane < 16) {
-        const int m = lane - 8;
-        const double2 b = pl.betaT[(size_t)r * 8 + m];
-        double2 T = ci[8 + m];
-        carry[(size_t)nt * 16 + 8 + m] = cmul(b, T);
-        for (int t = nt - 1; t >= 0; t--) {
-            T = cfma(pl.Ppow[SDRB_TB * 8 + m], T, cmul(T1[t], ag[(size_t)t * 16 + 8 + m]));
-            carry[(size_t)t * 16 + 8 + m] = cmul(b, T);
-        }
-    }
+    auto keep = [&](size_t j, double2 v) { carry[j] = v; };
+    if (lane < 16)
+        tile_carries(pl, T1, sc.agg + ((size_t)i * R + r) * nt * 16, m, lane < 8,
+                     (lane < 8 ? pl.beta : pl.betaT)[(size_t)r * 8 + m], ci[lane], keep);
     __syncwarp();
     const double2 ph = seam_phasor(sd, r, g0 + i);
-    const bool has_z = end && nwin - 1 - i <= sd.D;     // warp-uniform: zeta reaches this chunk
-    double2 zz[8];
-#pragma unroll
-    for (int m = 0; m < 8; m++) zz[m] = ci[16 + m];
-    const double2 *yp = sc.ypart + ((size_t)i * R + r) * pl.Mf;
-    const double2 *offt = sc.off_tile + (size_t)i * (nt + 1);
+    const bool has_z = end && nwin - 1 - i <= sd.D;     // zeta reaches this chunk
     double2 *y = sd.ybuf + ((size_t)i * R + r) * (M + 1);
-    const int l = lane;
-    for (int t = 0; t < nt; t++) {
-        const int k = t * SDRB_TB + l;
-        const double2 s = pl.correct_iq ? cscale(-1.0, offt[t]) : make_double2(0.0, 0.0);
-        double2 v = cfma(s, pl.psiY[((size_t)(t == nt - 1 ? 1 : 0) * R + r) * SDRB_TB + l], yp[k]);
-        v = cmul(T1[t], v);
-#pragma unroll
-        for (int m = 0; m < 8; m++) {
-            v = cfma(pl.RW[l * 8 + m], carry[(size_t)t * 16 + m], v);
-            v = cfma(pl.RT[(SDRB_TB - l) * 8 + m], carry[(size_t)(t + 1) * 16 + 8 + m], v);
-        }
-        if (has_z)
-#pragma unroll
-            for (int m = 0; m < 8; m++) v = cfma(pl.bnd[(size_t)k * 8 + m], zz[m], v);
-        y[k] = cmul(ph, v);
-    }
+    block_outputs(pl, r, sc.ypart + ((size_t)i * R + r) * pl.Mf, sc.off_tile + (size_t)i * (nt + 1), T1, carry,
+                  ci + 16, has_z ? 0 : M, lane, 32, [&](int k, double2 v) { y[k] = cmul(ph, v); });
 }
 
 __device__ __forceinline__ double seam_demod_at(const double2 *y, int k, int M, bool last, int demod)
