@@ -6,7 +6,7 @@ so = os.path.join(ROOT, 'sdrterm_b200', 'libsdrterm_b200.so')
 out = subprocess.run(['cuobjdump', '-sass', so], capture_output=True, text=True).stdout
 WANT = ['UTCIMMA', 'UTCBAR', 'LDTM', 'UTMALDG', 'UTMAPF', 'SYNCS', 'DMMA', 'DFMA', 'DADD', 'DMUL', 'F2F', 'IMAD', 'LDS', 'STS',
         'SHFL', 'LDG', 'STG', 'LDGSTS', 'MUFU']
-KEEP = ('k_tc', 'k_main', 'k_finish', 'k_fixup', 'k_demod', 'k_iqgain_w', 'k_iqscan_c', 'k_iqchunk', 'k_savgol', 'k_gfft4',
+KEEP = ('k_tc', 'k_main', 'k_finish', 'k_fixup', 'k_demod', 'k_iqgain', 'k_iqtiles', 'k_iqscan_c', 'k_iqchunk', 'k_savgol', 'k_gfft4',
         'k_gfft2', 'k_spectrum_db', 'k_stft_db', 'k_decode', 'k_correct_iq')
 print('# cuobjdump -sass sdrterm_b200/libsdrterm_b200.so (microbench/sass_excerpt.py): Blackwell-native instructions per kernel')
 print('# UTCIMMA = tcgen05.mma.kind::i8, LDTM = tcgen05.ld, UTMALDG = TMA tensor load, UTMAPF = TMA L2 prefetch,')

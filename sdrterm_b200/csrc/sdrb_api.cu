@@ -311,17 +311,13 @@ int launch_chain_t(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, 
     mark(1);
     if ((phases & PH_IQSCAN) && IQ) {
         // chunk gains -> the chunk scan (offset at every chunk start) -> the offsets at the tile
-        // starts; with whole-tile chunks the gains are warp-parallel and k_finish derives the
-        // tile-start offsets itself
-        const bool whole_tiles = h->finish_on && pl.ntiles <= 32 && !h->seamless;
-        const unsigned gb = (unsigned)((nch + 127) / 128);
-        if (whole_tiles)
-            k_iqgain_w<<<(unsigned)((nch + 7) / 8), 256, 0, st>>>(pl, h->sc, (int)nch);
-        else
-            k_iqgain<ENC><<<gb, 128, 0, st>>>(pl, h->sc, raw, (int)nch);
+        // starts, which k_finish derives itself
+        const bool finish_tiles = h->finish_on && pl.ntiles <= 32 && !h->seamless;
+        const unsigned gw = (unsigned)((nch + 7) / 8);    // warp <-> chunk, 8 warps per CTA
+        k_iqgain<ENC><<<gw, 256, 0, st>>>(pl, h->sc, raw, (int)nch);
         k_iqscan_c<<<1, 1024, 0, st>>>(pl, h->sc, (int)nch);
-        if (!whole_tiles) k_iqtiles<<<gb, 128, 0, st>>>(pl, h->sc, (int)nch);
-        h->launches += whole_tiles ? 2 : 3;
+        if (!finish_tiles) k_iqtiles<<<gw, 256, 0, st>>>(pl, h->sc, (int)nch);
+        h->launches += finish_tiles ? 2 : 3;
     }
     mark(2);
     if ((phases & PH_FINISH) && h->finish_on) {

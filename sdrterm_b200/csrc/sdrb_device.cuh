@@ -102,6 +102,58 @@ __device__ __forceinline__ double2 shfl_xor_c(double2 v, int m)
     return make_double2(__shfl_xor_sync(0xffffffffu, v.x, m), __shfl_xor_sync(0xffffffffu, v.y, m));
 }
 
+// ---------------------------------------------------------------- affine scans o -> m o + a
+// Inclusive composition of the lanes' maps across the warp, in place: lane l ends with the map of
+// lanes 0..l, the later lane's map applied last.  The complex overload (multiplier mul) keeps the
+// operand order of cmul, which does not round symmetrically.
+__device__ __forceinline__ void warp_affine_scan(double &m, double2 &a, int lane)
+{
+#pragma unroll
+    for (int lv = 0; lv < 5; lv++) {
+        const double pm = __shfl_up_sync(0xffffffffu, m, 1 << lv);
+        const double2 pa = shfl_up_c(a, 1 << lv);
+        if (lane >= (1 << lv)) { a.x = fma(m, pa.x, a.x); a.y = fma(m, pa.y, a.y); m *= pm; }
+    }
+}
+__device__ __forceinline__ void warp_affine_scan(double2 &mul, double2 &a, int lane)
+{
+#pragma unroll
+    for (int lv = 0; lv < 5; lv++) {
+        const double2 pa = shfl_up_c(a, 1 << lv), pm = shfl_up_c(mul, 1 << lv);
+        if (lane >= (1 << lv)) { a = cfma(mul, pa, a); mul = cmul(mul, pm); }
+    }
+}
+
+// The same across a CTA of up to 1024 threads: each thread's map (m, a) -> its exclusive map
+// (em, ea), identity on thread 0, and the block total (tm, ta).  The warps' totals hop through
+// s_m / s_a[32]; the caller syncs the block before it reuses them.
+__device__ __forceinline__ void block_affine_scan(double m, double2 a, double *s_m, double2 *s_a,
+                                                  double &em, double2 &ea, double &tm, double2 &ta)
+{
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    warp_affine_scan(m, a, lane);
+    if (lane == 31) { s_a[warp] = a; s_m[warp] = m; }
+    __syncthreads();
+    if (warp == 0) {
+        double wm = 1.0;
+        double2 wa = make_double2(0.0, 0.0);
+        if (lane < nw) { wm = s_m[lane]; wa = s_a[lane]; }
+        warp_affine_scan(wm, wa, lane);
+        s_a[lane] = wa; s_m[lane] = wm;
+    }
+    __syncthreads();
+    // (warps before) then (lanes before in this warp)
+    em = __shfl_up_sync(0xffffffffu, m, 1);
+    ea = shfl_up_c(a, 1);
+    if (lane == 0) { em = 1.0; ea = make_double2(0.0, 0.0); }
+    if (warp > 0) {
+        const double wm = s_m[warp - 1];
+        const double2 wa = s_a[warp - 1];
+        ea.x = fma(em, wa.x, ea.x); ea.y = fma(em, wa.y, ea.y); em *= wm;
+    }
+    tm = s_m[nw - 1]; ta = s_a[nw - 1];
+}
+
 // ---------------------------------------------------------------- decode (read_file.py:100-101)
 // One complex sample n of a chunk: raw bytes -> (re, im) doubles, bit-exact for every integer
 // encoding; float32 widens exactly.  `swap` = stored order differs from the GPU's little-endian.

@@ -210,24 +210,13 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
             xe = decode_sample<ENC>(pl, rawc, (long)pl.ws + lane);
         }
         // offsets at the tile starts from the chunk-start offset and the tile aggregates of the
-        // front end: lane t scans the maps o -> lam_tile o + agg[t] and keeps the offset entering
-        // tile t (shuffled out where needed); oE = the offset at the end of the chunk
+        // front end: lane t keeps the offset entering tile t (shuffled out where needed); oE = the
+        // offset at the end of the chunk
         double2 offr = make_double2(0.0, 0.0), oE = offr;
         if (iq) {
-            double m = 1.0;
-            double2 a = make_double2(0.0, 0.0);
-            if (lane < nt) { m = pl.lam_tile[lane == nt - 1 ? 1 : 0]; a = sc.tile_agg[(size_t)chunk * nt + lane]; }
-            const double2 o0 = sc.start[chunk];
-#pragma unroll
-            for (int lv = 0; lv < 5; lv++) {
-                const double pm = __shfl_up_sync(0xffffffffu, m, 1 << lv);
-                const double2 pa = shfl_up_c(a, 1 << lv);
-                if (lane >= (1 << lv)) { a.x = fma(m, pa.x, a.x); a.y = fma(m, pa.y, a.y); m *= pm; }
-            }
-            const double2 incl = make_double2(fma(m, o0.x, a.x), fma(m, o0.y, a.y));   // offset leaving tile `lane`
-            offr = shfl_up_c(incl, 1);
-            if (lane == 0) offr = o0;
-            oE = shfl_c(incl, nt - 1);
+            const TileOffsets to = tile_offsets(pl, sc.tile_agg + (size_t)chunk * nt, sc.start[chunk], lane);
+            offr = to.in;
+            oE = to.end;
         }
         {   // the next item's inputs start their way into L2 now
             const int nitem = item + nw;

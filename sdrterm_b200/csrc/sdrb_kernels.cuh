@@ -4,7 +4,10 @@
 //              on the FP64 tensor pipe (DMMA.8x8x4), all from registers; tile-local modal scans
 //              -> partial outputs + tile aggregates
 //   k_iqgain / k_iqscan_c / k_iqtiles   IQ-corrector offset at every tile start, carried across
-//              chunks and calls
+//              chunks and calls: chunk gains (warp <-> chunk), the chunk scan (one CTA), the tile
+//              offsets (warp <-> chunk; k_finish derives them itself); tile_offsets is the one
+//              tile-offset routine of all three and k_finish
+//   k_iqchunk  chunk gains straight from the raw bytes (time-segment sharding)
 //   k_fixup    head / end segments, cross-tile carries, boundary term -> decimated complex y
 //   k_demod    fm (pair phase + 2x FFT interpolation) | am | re | im, output SOS, framing; iq: y
 //              itself framed as (Re, Im) pairs; usb / lsb: the complex band-pass on y, its real part
@@ -356,32 +359,53 @@ k_main(const __grid_constant__ DevPlan pl, Scratch sc, const uint8_t *__restrict
 }
 
 // -------------------------------------------------------------------------------- IQ kernels
-// k_iqgain: thread <-> chunk, offset gained over the chunk from a zero state -> gain[c].
-template <int ENC>
-__global__ void __launch_bounds__(128)
-k_iqgain(const __grid_constant__ DevPlan pl, Scratch sc, const uint8_t *__restrict__ raw, int nchunks)
+// The offsets over one chunk's tiles, warp <-> chunk: lane <-> run [t0, t1) of per = ceil(nt/32)
+// consecutive tiles (per = 1 whenever nt <= 32), whose maps o -> lam_tile o + agg[t] the lane folds
+// serially before the warp composes the runs.  From o0, the offset at the chunk start: `in` = the
+// offset entering tile t0, `end` = the offset at q*Mf; `gain` = the composed offset term of the whole
+// chunk (the offset it gains from a zero start).
+struct TileOffsets {
+    double2 in, end, gain;
+    int t0, t1;
+};
+__device__ __forceinline__ TileOffsets tile_offsets(const DevPlan &pl, const double2 *ta, double2 o0, int lane)
 {
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= nchunks) return;
-    const int nt = pl.ntiles;
-    const double2 *ta = sc.tile_agg + (size_t)c * nt;
-    double2 o = make_double2(0.0, 0.0);
-    int t = 0;
-    for (; t + 8 <= nt; t += 8) {
-        double2 g[8];
-#pragma unroll
-        for (int i = 0; i < 8; i++) g[i] = ta[t + i];
-#pragma unroll
-        for (int i = 0; i < 8; i++) {
-            const double lt = pl.lam_tile[(t + i) == nt - 1 ? 1 : 0];
-            o.x = fma(lt, o.x, g[i].x); o.y = fma(lt, o.y, g[i].y);
-        }
-    }
-    for (; t < nt; t++) {
+    const int nt = pl.ntiles, per = (nt + 31) >> 5;
+    TileOffsets r;
+    r.t0 = min(nt, lane * per);
+    r.t1 = min(nt, r.t0 + per);
+    double m = 1.0;
+    double2 a = make_double2(0.0, 0.0);
+    if (r.t0 < r.t1) { m = pl.lam_tile[r.t0 == nt - 1 ? 1 : 0]; a = ta[r.t0]; }
+#pragma unroll 4         // (a deeper unroll costs k_iqgain its 32-register budget)
+    for (int t = r.t0 + 1; t < r.t1; t++) {
         const double lt = pl.lam_tile[t == nt - 1 ? 1 : 0];
         const double2 g = ta[t];
-        o.x = fma(lt, o.x, g.x); o.y = fma(lt, o.y, g.y);
+        a.x = fma(lt, a.x, g.x); a.y = fma(lt, a.y, g.y);
+        m *= lt;
     }
+    warp_affine_scan(m, a, lane);
+    const int last = 31 - __clz(__ballot_sync(0xffffffffu, r.t0 < r.t1));   // the lane with tile nt-1
+    const double2 incl = make_double2(fma(m, o0.x, a.x), fma(m, o0.y, a.y));   // offset leaving tile t1-1
+    r.in = shfl_up_c(incl, 1);
+    if (lane == 0) r.in = o0;
+    r.end = shfl_c(incl, last);
+    r.gain = shfl_c(a, last);
+    return r;
+}
+
+// k_iqgain: warp <-> chunk, the offset gained over the chunk from a zero state -> gain[c]: the tile
+// maps, then the samples of the partial block (one lane, serially).  At most 32 registers: 8 CTAs
+// per SM, so that a batch of 8192 chunks runs in one wave.
+template <int ENC>
+__global__ void __launch_bounds__(256, 8)
+k_iqgain(const __grid_constant__ DevPlan pl, Scratch sc, const uint8_t *__restrict__ raw, int nchunks)
+{
+    const int lane = threadIdx.x & 31;
+    const int c = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (c >= nchunks) return;
+    double2 o = tile_offsets(pl, sc.tile_agg + (size_t)c * pl.ntiles, make_double2(0.0, 0.0), lane).gain;
+    if (lane != 0) return;
     if (pl.rem) {
         const uint8_t *rawc = raw + (size_t)c * pl.N * pl.sb;
         double2 acc = make_double2(0.0, 0.0);
@@ -392,28 +416,7 @@ k_iqgain(const __grid_constant__ DevPlan pl, Scratch sc, const uint8_t *__restri
         const double lr = pl.lam_j[pl.rem];
         o.x = fma(lr, o.x, pl.Liq * acc.x); o.y = fma(lr, o.y, pl.Liq * acc.y);
     }
-    sc.gain[blockIdx.x * blockDim.x + threadIdx.x] = o;   // = c, recomputed: 40 instead of 42 registers for ENC_d
-}
-
-// k_iqgain_w: warp <-> chunk, lane <-> tile (whole-tile chunks, ntiles <= 32): the same gain as
-// k_iqgain by a warp scan of the tile maps o -> lam_tile o + agg[t]; coalesced, no serial loop.
-__global__ void __launch_bounds__(256)
-k_iqgain_w(const __grid_constant__ DevPlan pl, Scratch sc, int nchunks)
-{
-    const int lane = threadIdx.x & 31;
-    const int c = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (c >= nchunks) return;
-    const int nt = pl.ntiles;
-    double m = 1.0;
-    double2 a = make_double2(0.0, 0.0);
-    if (lane < nt) { m = pl.lam_tile[lane == nt - 1 ? 1 : 0]; a = sc.tile_agg[(size_t)c * nt + lane]; }
-#pragma unroll
-    for (int lv = 0; lv < 5; lv++) {
-        const double pm = __shfl_up_sync(0xffffffffu, m, 1 << lv);
-        const double2 pa = shfl_up_c(a, 1 << lv);
-        if (lane >= (1 << lv)) { a.x = fma(m, pa.x, a.x); a.y = fma(m, pa.y, a.y); m *= pm; }
-    }
-    if (lane == nt - 1) sc.gain[c] = a;
+    sc.gain[c] = o;
 }
 
 // k_iqchunk: warp <-> chunk: the offset a whole chunk gains from a zero state, straight from the raw
@@ -437,25 +440,20 @@ k_iqchunk(const __grid_constant__ DevPlan pl, Scratch sc, const uint8_t *__restr
         a.x = fma(pl.lam, a.x, z.x); a.y = fma(pl.lam, a.y, z.y);
         m *= pl.lam;
     }
-#pragma unroll
-    for (int lv = 0; lv < 5; lv++) {
-        const double pm = __shfl_up_sync(0xffffffffu, m, 1 << lv);
-        const double2 pa = shfl_up_c(a, 1 << lv);
-        if (lane >= (1 << lv)) { a.x = fma(m, pa.x, a.x); a.y = fma(m, pa.y, a.y); m *= pm; }
-    }
+    warp_affine_scan(m, a, lane);
     if (lane == 31) sc.gain[c] = make_double2(pl.Liq * a.x, pl.Liq * a.y);
 }
 
 // k_iqscan_c: one CTA of 1024 threads; exclusive scan of the per-chunk maps o -> lam_N o + gain[c]
 // from the handle's IQ state -> start[c] and the new state.  8 chunks per thread and round (their
-// gains are loaded together), warp-shuffle scans, one shared-memory hop across the 32 warps.
+// gains are loaded together).
 __global__ void __launch_bounds__(1024)
 k_iqscan_c(const __grid_constant__ DevPlan pl, Scratch sc, int nchunks)
 {
     __shared__ double2 s_a[32];
     __shared__ double s_m[32];
     __shared__ double2 s_state;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int tid = threadIdx.x;
     const double2 *__restrict__ gain = sc.gain;
     double2 *__restrict__ start = sc.start;
     if (tid == 0) s_state = sc.iq_state[0];
@@ -470,36 +468,9 @@ k_iqscan_c(const __grid_constant__ DevPlan pl, Scratch sc, int nchunks)
 #pragma unroll
         for (int i = 0; i < 8; i++)
             if (c0 + i < nchunks) { a.x = fma(pl.lam_N, a.x, g[i].x); a.y = fma(pl.lam_N, a.y, g[i].y); m *= pl.lam_N; }
-        // inclusive scan of the thread maps inside the warp
-#pragma unroll
-        for (int lv = 0; lv < 5; lv++) {
-            const double pm = __shfl_up_sync(0xffffffffu, m, 1 << lv);
-            const double2 pa = shfl_up_c(a, 1 << lv);
-            if (lane >= (1 << lv)) { a.x = fma(m, pa.x, a.x); a.y = fma(m, pa.y, a.y); m *= pm; }
-        }
-        if (lane == 31) { s_a[warp] = a; s_m[warp] = m; }
-        __syncthreads();
-        if (warp == 0) {
-            double wm = s_m[lane];
-            double2 wa = s_a[lane];
-#pragma unroll
-            for (int lv = 0; lv < 5; lv++) {
-                const double pm = __shfl_up_sync(0xffffffffu, wm, 1 << lv);
-                const double2 pa = shfl_up_c(wa, 1 << lv);
-                if (lane >= (1 << lv)) { wa.x = fma(wm, pa.x, wa.x); wa.y = fma(wm, pa.y, wa.y); wm *= pm; }
-            }
-            s_a[lane] = wa; s_m[lane] = wm;
-        }
-        __syncthreads();
-        // exclusive map of this thread = (warps before) then (lanes before in this warp)
-        double em = __shfl_up_sync(0xffffffffu, m, 1);
-        double2 ea = shfl_up_c(a, 1);
-        if (lane == 0) { em = 1.0; ea = make_double2(0.0, 0.0); }
-        if (warp > 0) {
-            const double wm = s_m[warp - 1];
-            const double2 wa = s_a[warp - 1];
-            ea.x = fma(em, wa.x, ea.x); ea.y = fma(em, wa.y, ea.y); em *= wm;
-        }
+        double em, tm;
+        double2 ea, ta;
+        block_affine_scan(m, a, s_m, s_a, em, ea, tm, ta);
         const double2 st0 = s_state;
         double2 o = make_double2(fma(em, st0.x, ea.x), fma(em, st0.y, ea.y));
 #pragma unroll
@@ -509,41 +480,31 @@ k_iqscan_c(const __grid_constant__ DevPlan pl, Scratch sc, int nchunks)
                 o.x = fma(pl.lam_N, o.x, g[i].x); o.y = fma(pl.lam_N, o.y, g[i].y);
             }
         __syncthreads();
-        if (tid == 1023) s_state = make_double2(fma(s_m[31], st0.x, s_a[31].x), fma(s_m[31], st0.y, s_a[31].y));
+        if (tid == 1023) s_state = make_double2(fma(tm, st0.x, ta.x), fma(tm, st0.y, ta.y));
         __syncthreads();
     }
     if (tid == 0) sc.iq_state[0] = s_state;
 }
 
-// k_iqtiles: thread <-> chunk, offsets at the tile starts from the chunk-start offset start[c].
-__global__ void __launch_bounds__(128)
+// k_iqtiles: warp <-> chunk, offsets at the tile starts from the chunk-start offset start[c].
+__global__ void __launch_bounds__(256)
 k_iqtiles(const __grid_constant__ DevPlan pl, Scratch sc, int nchunks)
 {
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    const int lane = threadIdx.x & 31;
+    const int c = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (c >= nchunks) return;
     const int nt = pl.ntiles;
     const double2 *ta = sc.tile_agg + (size_t)c * nt;
     double2 *ot = sc.off_tile + (size_t)c * (nt + 1);
-    double2 o = sc.start[c];
-    int t = 0;
-    for (; t + 8 <= nt; t += 8) {
-        double2 g[8];
-#pragma unroll
-        for (int i = 0; i < 8; i++) g[i] = ta[t + i];
-#pragma unroll
-        for (int i = 0; i < 8; i++) {
-            ot[t + i] = o;
-            const double lt = pl.lam_tile[(t + i) == nt - 1 ? 1 : 0];
-            o.x = fma(lt, o.x, g[i].x); o.y = fma(lt, o.y, g[i].y);
-        }
-    }
-    for (; t < nt; t++) {
+    const TileOffsets to = tile_offsets(pl, ta, sc.start[c], lane);
+    double2 o = to.in;
+    for (int t = to.t0; t < to.t1; t++) {
         ot[t] = o;
         const double lt = pl.lam_tile[t == nt - 1 ? 1 : 0];
         const double2 g = ta[t];
         o.x = fma(lt, o.x, g.x); o.y = fma(lt, o.y, g.y);
     }
-    ot[nt] = o;      // offset at sample q*Mf
+    if (to.t0 < to.t1 && to.t1 == nt) ot[nt] = to.end;      // offset at sample q*Mf
 }
 
 // Time-segment sharding (SURVEY 8e): the IQ offset a segment gained from a zero start, and the
@@ -900,7 +861,7 @@ k_correct_iq(double2 *__restrict__ z, size_t n, double2 *__restrict__ off_io, do
 {
     __shared__ double2 s_a[32];
     __shared__ double s_m[32];
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int tid = threadIdx.x;
     const double lam = 1.0 - L;
     const size_t per = (n + blockDim.x - 1) / blockDim.x;
     const size_t i0 = min(n, (size_t)tid * per), i1 = min(n, i0 + per);
@@ -911,34 +872,9 @@ k_correct_iq(double2 *__restrict__ z, size_t n, double2 *__restrict__ off_io, do
         a.x = fma(lam, a.x, L * v.x); a.y = fma(lam, a.y, L * v.y);
         m *= lam;
     }
-#pragma unroll
-    for (int lv = 0; lv < 5; lv++) {
-        const double pm = __shfl_up_sync(0xffffffffu, m, 1 << lv);
-        const double2 pa = shfl_up_c(a, 1 << lv);
-        if (lane >= (1 << lv)) { a.x = fma(m, pa.x, a.x); a.y = fma(m, pa.y, a.y); m *= pm; }
-    }
-    if (lane == 31) { s_a[warp] = a; s_m[warp] = m; }
-    __syncthreads();
-    if (warp == 0) {
-        double wm = s_m[lane];
-        double2 wa = s_a[lane];
-#pragma unroll
-        for (int lv = 0; lv < 5; lv++) {
-            const double pm = __shfl_up_sync(0xffffffffu, wm, 1 << lv);
-            const double2 pa = shfl_up_c(wa, 1 << lv);
-            if (lane >= (1 << lv)) { wa.x = fma(wm, pa.x, wa.x); wa.y = fma(wm, pa.y, wa.y); wm *= pm; }
-        }
-        s_a[lane] = wa; s_m[lane] = wm;
-    }
-    __syncthreads();
-    double em = __shfl_up_sync(0xffffffffu, m, 1);
-    double2 ea = shfl_up_c(a, 1);
-    if (lane == 0) { em = 1.0; ea = make_double2(0.0, 0.0); }
-    if (warp > 0) {
-        const double wm = s_m[warp - 1];
-        const double2 wa = s_a[warp - 1];
-        ea.x = fma(em, wa.x, ea.x); ea.y = fma(em, wa.y, ea.y); em *= wm;
-    }
+    double em, tm;
+    double2 ea, ta;
+    block_affine_scan(m, a, s_m, s_a, em, ea, tm, ta);
     const double2 st0 = off_io[0];
     double2 o = make_double2(fma(em, st0.x, ea.x), fma(em, st0.y, ea.y));
     for (size_t i = i0; i < i1; i++) {

@@ -123,11 +123,7 @@ k_seam_fscan(const __grid_constant__ DevPlan pl, SeamDev sd, int slot0, int nch)
         a = cfma(PN, a, sd.cagg[((size_t)(slot0 + c) * pl.R + r) * 16 + m]);
         mul = cmul(mul, PN);
     }
-#pragma unroll
-    for (int lv = 0; lv < 5; lv++) {
-        const double2 pa = shfl_up_c(a, 1 << lv), pm = shfl_up_c(mul, 1 << lv);
-        if (lane >= (1 << lv)) { a = cfma(mul, pa, a); mul = cmul(mul, pm); }
-    }
+    warp_affine_scan(mul, a, lane);
     const double2 st0 = sd.fwd[(size_t)r * 8 + m];
     double2 ea = shfl_up_c(a, 1), em = shfl_up_c(mul, 1);
     if (lane == 0) { ea = make_double2(0.0, 0.0); em = make_double2(1.0, 0.0); }

@@ -6,8 +6,6 @@ algorithm and every table against the oracle without a GPU.  Structure mirrors t
                             UNcorrected samples, IQ-EMA block aggregates, tile-local scans, partial
                             outputs + tile aggregates; the IQ corrector enters only through the
                             decoupled terms of DESIGN.md 3.3)
-  emu_iq_scan <-> k_iqgain / k_iqscan_c / k_iqtiles (offset at every tile start, carried across
-                            chunks and calls)
   emu_fixup   <-> k_fixup  (head / end segments, cross-tile carries, boundary term -> decimated y)
   emu_demod   <-> k_demod  (fm pair-phase + 2x FFT interpolation | am | re | im, output SOS)
 """
@@ -139,15 +137,6 @@ def emu_main(pl: Plan, z: np.ndarray):
             Wout[r, t] = W[cnt]
             Tin[r, t] = T[0]
     return dict(ypart=ypart, Wout=Wout, Tin=Tin, tile_agg=tile_agg)
-
-
-def emu_iq_scan(pl: Plan, tile_aggs: np.ndarray, off0: complex):
-    """tile_aggs: (nchunks, ntiles).  Returns off at every tile start (nchunks, ntiles+1)
-    [last column = offset at sample q*Mf], off at every chunk start, and the state after the
-    batch.  The partial block + nothing else remains: its samples advance the state too."""
-    nch = tile_aggs.shape[0]
-    off_tile = np.zeros((nch, pl.ntiles + 1), dtype=np.complex128)
-    return off_tile
 
 
 def emu_fixup(pl: Plan, z: np.ndarray, mo: dict, off_chunk: complex):

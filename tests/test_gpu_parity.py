@@ -67,7 +67,8 @@ def test_stage_parity_vs_emulator(name):
 @pytest.mark.parametrize('name', ['c1_fm_wav_int16', 'c2_am_u8_d64', 'c3_simo16_int16be', 'enc_H_swap_im'])
 def test_general_finish_kernels_match_fused(name, monkeypatch):
     """k_fixup + k_demod (the general path, forced with SDRB_NO_FINISH=1) against the fused
-    k_finish on shapes both handle, and against the oracle."""
+    k_finish on shapes both handle, and against the oracle.  Both paths take the chunk gains and the
+    chunk scan from the same kernels, so the IQ state is bit-identical."""
     from gpu_util import run_case
     kw, pl, chunks, out_f, y_f, off_f = run_case(name)
     monkeypatch.setenv('SDRB_NO_FINISH', '1')
@@ -77,6 +78,7 @@ def test_general_finish_kernels_match_fused(name, monkeypatch):
     assert rel_err(y_g, y_f) < 1e-12
     assert rel_err(np.asarray(out_g, dtype=np.float64), np.asarray(out_f, dtype=np.float64)) < 1e-11
     assert rel_err(np.asarray(out_g, dtype=np.float64), oo) < TOL
+    assert off_g == off_f
 
 
 def test_batch_split_and_state_carry():
