@@ -62,7 +62,8 @@ struct sdrb_handle {
     int reserved_sms = 0;           // SMs the persistent kernels leave free (for a collective running beside them)
     double2 *x0_buf = nullptr;      // sdrb_keep_x0
     int smooth_w = 0, smooth_nhead = 0, smooth_ntail = 0, smooth_lo = 0;   // --smooth-output (window 0 = off)
-    double *smooth_S = nullptr, *smooth_tmp = nullptr;
+    const double *smooth_S = nullptr;
+    double *smooth_tmp = nullptr;
     // seamless streaming (cfg.seamless): window of unemitted chunks in slots 0..nwin-1 of the scratch
     bool seamless = false;
     SeamDev sd{};
@@ -125,18 +126,36 @@ int with_enc(sdrb_handle *h, int code, F &&f)
     return fail(h, SDRB_ERR_ARG, "bad encoding code %d", code);
 }
 
-template <typename T>
-int upload(sdrb_handle *h, const T *src, size_t count, const T **dst)
+bool is_ssb(int demod) { return demod == SDRB_USB || demod == SDRB_LSB; }
+
+// The one place a demodulation code becomes the output kind of the finish, demod and seamless
+// kernels: calls f(std::integral_constant<int, OUT_REAL | OUT_IQ | OUT_SSB>{}) and returns its result.
+template <class F>
+int with_out(int demod, F &&f)
 {
-    void *d = nullptr;
-    if (count == 0) count = 1;
-    CK(h, cudaMalloc(&d, count * sizeof(T)));
-    h->owned.push_back(d);
-    if (src) CK(h, cudaMemcpy(d, src, count * sizeof(T), cudaMemcpyHostToDevice));
-    else CK(h, cudaMemset(d, 0, count * sizeof(T)));
-    *dst = static_cast<const T *>(d);
+    if (demod == SDRB_IQ) return f(std::integral_constant<int, OUT_IQ>{});
+    if (is_ssb(demod)) return f(std::integral_constant<int, OUT_SSB>{});
+    return f(std::integral_constant<int, OUT_REAL>{});
+}
+
+// Every kernel launch on a handle: sdrb_launch_count counts each one here.
+template <typename... P, typename... A>
+void launch(sdrb_handle *h, void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, A &&...args)
+{
+    kernel<<<grid, block, smem, st>>>(std::forward<A>(args)...);
+    h->launches++;
+}
+
+int need_device(int device)
+{
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+        return fail(nullptr, SDRB_ERR_CUDA, "no CUDA device: libsdrterm_b200 has no CPU fallback");
+    if (device < 0 || device >= ndev) return fail(nullptr, SDRB_ERR_ARG, "bad device ordinal");
+    CK(nullptr, cudaSetDevice(device));
     return 0;
 }
+
 template <typename T>
 int dalloc(sdrb_handle *h, size_t count, T **dst)
 {
@@ -147,14 +166,21 @@ int dalloc(sdrb_handle *h, size_t count, T **dst)
     *dst = static_cast<T *>(d);
     return 0;
 }
+template <typename T>
+int upload(sdrb_handle *h, const T *src, size_t count, const T **dst)
+{
+    T *d = nullptr;
+    if (int rc = dalloc(h, count, &d)) return rc;
+    if (src) CK(h, cudaMemcpy(d, src, std::max<size_t>(count, 1) * sizeof(T), cudaMemcpyHostToDevice));
+    else CK(h, cudaMemset(d, 0, std::max<size_t>(count, 1) * sizeof(T)));
+    *dst = d;
+    return 0;
+}
 
 inline double2 c2(const double *a, size_t i) { return make_double2(a[2 * i], a[2 * i + 1]); }
 inline double2 hmul(double2 a, double2 b) { return make_double2(a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x); }
 
 bool is_pow2(int v) { return v > 0 && (v & (v - 1)) == 0; }
-bool is_ssb(int demod) { return demod == SDRB_USB || demod == SDRB_LSB; }
-// the finish-kernel instance of a demodulation (OUT_REAL / OUT_IQ / OUT_SSB)
-int out_kind(int demod) { return demod == SDRB_IQ ? OUT_IQ : (is_ssb(demod) ? OUT_SSB : OUT_REAL); }
 
 std::vector<double2> make_twiddles(int n)
 {
@@ -167,8 +193,11 @@ std::vector<double2> make_twiddles(int n)
     return tw;
 }
 
-int env_int(const char *name, int dflt);
-int launch_tc(sdrb_handle *h, const uint8_t *raw, size_t nch, cudaStream_t st, bool iq);
+int env_int(const char *name, int dflt)
+{
+    const char *v = getenv(name);
+    return (v && *v) ? atoi(v) : dflt;
+}
 
 enum { PH_MAIN = 1, PH_IQSCAN = 2, PH_FINISH = 4, PH_ALL = 7 };
 
@@ -206,16 +235,7 @@ int make_byte_map(sdrb_handle *h, CUtensorMap *map, const void *base, uint64_t r
 }
 
 template <bool IQ>
-int launch_tc_t(sdrb_handle *h, const CUtensorMap &map_a, int n_mtiles, int total_wtiles, cudaStream_t st)
-{
-    // one row of the bank per CTA: the grid is a whole number of row groups
-    const int R = h->pl.R;
-    const int slots = std::max(1, std::min((h->num_sms - h->reserved_sms) / R, n_mtiles));
-    k_tc<IQ><<<slots * R, TC_THREADS, h->tc_smem, st>>>(h->pl, h->tc, h->sc, map_a, h->map_b, n_mtiles, total_wtiles);
-    return 0;
-}
-
-int launch_tc(sdrb_handle *h, const uint8_t *raw, size_t nch, cudaStream_t st, bool iq)
+int launch_tc(sdrb_handle *h, const Scratch &sc, const uint8_t *raw, size_t nch, cudaStream_t st)
 {
     // GEMM rows are super-blocks of two blocks: [nch * Mf / 2][K] bytes, 128 rows per MMA tile
     const uint64_t rows = (uint64_t)nch * h->pl.Mf / 2;
@@ -224,72 +244,60 @@ int launch_tc(sdrb_handle *h, const uint8_t *raw, size_t nch, cudaStream_t st, b
     if (rc) return rc;
     const int n_mtiles = (int)((rows + 127) / 128);
     const int total_wtiles = (int)(rows / 32);
-    return iq ? launch_tc_t<true>(h, map_a, n_mtiles, total_wtiles, st) : launch_tc_t<false>(h, map_a, n_mtiles, total_wtiles, st);
-}
-
-template <bool IQ>
-int tc_attr(sdrb_handle *h)
-{
-    CK(h, cudaFuncSetAttribute(k_tc<IQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->tc_smem));
+    // one row of the bank per CTA: the grid is a whole number of row groups
+    const int R = h->pl.R;
+    const int slots = std::max(1, std::min((h->num_sms - h->reserved_sms) / R, n_mtiles));
+    launch(h, k_tc<IQ>, slots * R, TC_THREADS, h->tc_smem, st, h->pl, h->tc, sc, map_a, h->map_b, n_mtiles, total_wtiles);
     return 0;
 }
 
+// k_tc's A ring takes whatever shared memory the B slice leaves (227 KB per CTA on sm_100)
+int tc_stages(int K)
+{
+    const size_t cap = 227 * 1024, fixed = tc_fixed_bytes(K / 128);
+    const int nstage = fixed < cap ? (int)((cap - fixed) / TC_REGION_BYTES) : 0;
+    return std::min({nstage, env_int("SDRB_TC_ASTAGES", TC_MAX_ASTAGES), TC_MAX_ASTAGES});
+}
+
+// The tensor-core tables, which validate() has checked; wider banks take the FP64 block kernel.
 int setup_tc(sdrb_handle *h, const sdrb_tables *tab)
 {
-    if (!tab->tc_enable) return 0;
     const int R = h->pl.R;
-    if ((tab->tc_K != 256 && tab->tc_K != 512) || tab->tc_nout != TC_NOUT || tab->tc_ncol != TC_NCOL ||
-        tab->tc_isz < 1 || tab->tc_isz > 2 || tab->tc_npad != TC_NPAD || tab->tc_nrowc != TC_NROWC ||
-        tab->tc_K != 2 * h->pl.q * h->pl.sb || h->pl.rem != 0 || h->pl.cnt_last != SDRB_TB || (h->pl.Mf / 2) % 128 ||
-        h->pl.q < h->pl.edge + 1 || h->pl.normalize || !tab->tc_Bq || !tab->tc_cst || !tab->tc_rowc)
-        return fail(h, SDRB_ERR_ARG, "tensor-core tables do not match the configuration");
-    cudaDeviceProp prop;
-    CK(h, cudaGetDeviceProperties(&prop, h->cfg.device));
-    h->num_sms = prop.multiProcessorCount;
-    if (R > TC_MAX_R) return 0;              // wider banks take the FP64 block kernel
+    if (!tab->tc_enable || R > TC_MAX_R) return 0;
     TcDev &tc = h->tc;
     tc.K = tab->tc_K; tc.isz = tab->tc_isz;
     tc.nregion = tc.K / 128;
     memcpy(&tc.xor_word, tab->tc_xor, 4);
-    for (int i = 0; i < 16; i++)
-        if (tab->tc_xor[i] != tab->tc_xor[i & 3]) return fail(h, SDRB_ERR_ARG, "XOR pattern is not 4-periodic");
     // instruction descriptor: D = s32, A = s8 / u8 (tc_a_signed), B = s8, N, M
     tc.idesc = (2u << 4) | ((tab->tc_a_signed ? 1u : 0u) << 7) | (1u << 10) | ((uint32_t)(TC_NPAD >> 3) << 17) | ((128u >> 4) << 24);
     tc.scale = ldexp(1.0, -tab->tc_S);
     tc.scale16 = ldexp(1.0, 16 - tab->tc_S);
     tc.scale_yl = ldexp(1.0, -tab->tc_S_yl);
     tc.scale16_yl = ldexp(1.0, 16 - tab->tc_S_yl);
-    int rc = upload(h, reinterpret_cast<const double2 *>(tab->tc_rowc), (size_t)R * TC_NROWC, &tc.rowc);
-    if (rc) return rc;
     std::vector<double> cstb((size_t)R * (TC_NOUT + 4));
     for (int r = 0; r < R; r++)
         for (int o = 0; o < TC_NOUT + 4; o++) {
             const double sc = o < 36 ? tc.scale : (o < TC_NOUT ? tc.scale_yl : 1.0);
             cstb[(size_t)r * (TC_NOUT + 4) + o] = tab->tc_cst[(size_t)r * (TC_NOUT + 4) + o] - TC_BIAS32 * sc;
         }
-    rc = upload(h, cstb.data(), cstb.size(), &tc.cstb);
-    if (rc) return rc;
     const int8_t *d_bq = nullptr;
-    rc = upload(h, tab->tc_Bq, (size_t)R * TC_NPAD * tc.K, &d_bq);
-    if (rc) return rc;
-    rc = make_byte_map(h, &h->map_b, d_bq, (uint64_t)R * TC_NPAD, (uint32_t)tc.K, (uint32_t)TC_NPAD);
-    if (rc) return rc;
-    // the A ring takes whatever shared memory the B slice leaves (227 KB per CTA on sm_100)
-    const size_t cap = 227 * 1024;
-    const size_t fixed = tc_fixed_bytes(tc.nregion);
-    int nstage = fixed < cap ? (int)((cap - fixed) / TC_REGION_BYTES) : 0;
-    nstage = std::min(nstage, env_int("SDRB_TC_ASTAGES", TC_MAX_ASTAGES));
-    nstage = std::min(nstage, TC_MAX_ASTAGES);
-    if (nstage < 2) return fail(h, SDRB_ERR_ARG, "k_tc: no room for the A ring (%zu bytes fixed)", fixed);
-    tc.nstage = nstage;
-    h->tc_smem = tc_smem_bytes(tc.nregion, nstage);
-    if ((rc = tc_attr<true>(h)) || (rc = tc_attr<false>(h))) return rc;
+    int rc;
+    if ((rc = upload(h, reinterpret_cast<const double2 *>(tab->tc_rowc), (size_t)R * TC_NROWC, &tc.rowc)) ||
+        (rc = upload(h, cstb.data(), cstb.size(), &tc.cstb)) ||
+        (rc = upload(h, tab->tc_Bq, (size_t)R * TC_NPAD * tc.K, &d_bq)) ||
+        (rc = make_byte_map(h, &h->map_b, d_bq, (uint64_t)R * TC_NPAD, (uint32_t)tc.K, (uint32_t)TC_NPAD)))
+        return rc;
+    tc.nstage = tc_stages(tc.K);
+    h->tc_smem = tc_smem_bytes(tc.nregion, tc.nstage);
+    CK(h, cudaFuncSetAttribute(k_tc<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->tc_smem));
+    CK(h, cudaFuncSetAttribute(k_tc<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->tc_smem));
     h->tc_on = true;
     return 0;
 }
 
 template <int ENC, bool IQ>
-int launch_chain_t(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, cudaStream_t st, int phases)
+int launch_chain_t(sdrb_handle *h, const Scratch &sc, const uint8_t *raw, size_t nch, double *out, cudaStream_t st,
+                   int phases)
 {
     const DevPlan &pl = h->pl;
     const bool prof = h->profiling && phases == PH_ALL;
@@ -300,13 +308,12 @@ int launch_chain_t(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, 
     mark(0);
     if (phases & PH_MAIN) {
         if (h->tc_on && ((uintptr_t)raw & 15) == 0) {
-            int rc = launch_tc(h, raw, nch, st, IQ);
+            int rc = launch_tc<IQ>(h, sc, raw, nch, st);
             if (rc) return rc;
         } else {
             const int groups = (pl.ntiles + h->tpc - 1) / h->tpc;
-            k_main<ENC, IQ><<<(unsigned)(nch * groups), 32 * h->warps, h->main_smem, st>>>(pl, h->sc, raw, (int)nch, h->tpc);
+            launch(h, k_main<ENC, IQ>, (unsigned)(nch * groups), 32 * h->warps, h->main_smem, st, pl, sc, raw, (int)nch, h->tpc);
         }
-        h->launches++;
     }
     mark(1);
     if ((phases & PH_IQSCAN) && IQ) {
@@ -314,59 +321,53 @@ int launch_chain_t(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, 
         // starts, which k_finish derives itself
         const bool finish_tiles = h->finish_on && pl.ntiles <= 32 && !h->seamless;
         const unsigned gw = (unsigned)((nch + 7) / 8);    // warp <-> chunk, 8 warps per CTA
-        k_iqgain<ENC><<<gw, 256, 0, st>>>(pl, h->sc, raw, (int)nch);
-        k_iqscan_c<<<1, 1024, 0, st>>>(pl, h->sc, (int)nch);
-        if (!finish_tiles) k_iqtiles<<<gw, 256, 0, st>>>(pl, h->sc, (int)nch);
-        h->launches += finish_tiles ? 2 : 3;
+        launch(h, k_iqgain<ENC>, gw, 256, 0, st, pl, sc, raw, (int)nch);
+        launch(h, k_iqscan_c, 1, 1024, 0, st, pl, sc, (int)nch);
+        if (!finish_tiles) launch(h, k_iqtiles, gw, 256, 0, st, pl, sc, (int)nch);
     }
     mark(2);
+    const unsigned rows = (unsigned)(nch * pl.R);
     if ((phases & PH_FINISH) && h->finish_on) {
-        const size_t items = nch * (size_t)pl.R;
-        const unsigned grid = (unsigned)std::min<size_t>((items + FIN_WARPS - 1) / FIN_WARPS, (size_t)(h->num_sms - h->reserved_sms) * 2);
-        if (pl.demod == SDRB_IQ)
-            k_finish<ENC, OUT_IQ><<<grid, 32 * FIN_WARPS, h->finish_smem, st>>>(pl, h->sc, raw, out, (int)nch, h->keep_y);
-        else if (is_ssb(pl.demod))
-            k_finish<ENC, OUT_SSB><<<grid, 32 * FIN_WARPS, h->finish_smem, st>>>(pl, h->sc, raw, out, (int)nch, h->keep_y);
-        else
-            k_finish<ENC, OUT_REAL><<<grid, 32 * FIN_WARPS, h->finish_smem, st>>>(pl, h->sc, raw, out, (int)nch, h->keep_y);
-        h->launches++;
+        const unsigned grid = (unsigned)std::min<size_t>((rows + FIN_WARPS - 1) / FIN_WARPS, (size_t)(h->num_sms - h->reserved_sms) * 2);
+        with_out(pl.demod, [&](auto ok) {
+            launch(h, k_finish<ENC, decltype(ok)::value>, grid, 32 * FIN_WARPS, h->finish_smem, st, pl, sc, raw, out, (int)nch,
+                   h->keep_y);
+            return 0;
+        });
         mark(3);
         mark(4);
     } else if (phases & PH_FINISH) {
-        k_fixup<ENC><<<(unsigned)(nch * pl.R), 128, 0, st>>>(pl, h->sc, raw, (int)nch);
-        h->launches++;
+        launch(h, k_fixup<ENC>, rows, 128, 0, st, pl, sc, raw, (int)nch);
         mark(3);
-        if (pl.demod == SDRB_IQ)
-            k_demod<OUT_IQ><<<(unsigned)(nch * pl.R), 128, 0, st>>>(pl, h->sc.y, out, nullptr, nullptr, (int)nch, pl.demod, 0,
-                                                                    pl.be_out);
-        else if (is_ssb(pl.demod))
-            k_demod<OUT_SSB><<<(unsigned)(nch * pl.R), 128, h->demod_smem, st>>>(pl, h->sc.y, out, h->sc.fftbuf, h->sc.zrow,
-                                                                                 (int)nch, pl.demod, 1, pl.be_out);
-        else
-            k_demod<OUT_REAL><<<(unsigned)(nch * pl.R), 128, h->demod_smem, st>>>(pl, h->sc.y, out, h->sc.fftbuf, h->sc.zrow,
-                                                                                  (int)nch, pl.demod, 1, pl.be_out);
-        h->launches++;
+        with_out(pl.demod, [&](auto ok) {
+            constexpr int OK = decltype(ok)::value;
+            if constexpr (OK == OUT_IQ)
+                launch(h, k_demod<OK>, rows, 128, 0, st, pl, sc.y, out, nullptr, nullptr, (int)nch, pl.demod, 0, pl.be_out);
+            else
+                launch(h, k_demod<OK>, rows, 128, h->demod_smem, st, pl, sc.y, out, sc.fftbuf, sc.zrow, (int)nch, pl.demod, 1,
+                       pl.be_out);
+            return 0;
+        });
         mark(4);
     }
     if ((phases & PH_FINISH) && h->smooth_w > 0 && !pl.be_out) {
-        const size_t nseg = nch * (size_t)pl.R, bytes = nseg * pl.M * sizeof(double);
-        k_savgol<<<(unsigned)std::min<size_t>(nseg, (size_t)h->num_sms * 8), 256, 0, st>>>(out, h->smooth_tmp, h->smooth_S,
-                                                                                        h->smooth_w, h->smooth_nhead, h->smooth_ntail, h->smooth_lo, pl.M, nseg);
+        const size_t nseg = rows, bytes = nseg * pl.M * sizeof(double);
+        launch(h, k_savgol, (unsigned)std::min<size_t>(nseg, (size_t)h->num_sms * 8), 256, 0, st, out, h->smooth_tmp,
+               h->smooth_S, h->smooth_w, h->smooth_nhead, h->smooth_ntail, h->smooth_lo, pl.M, nseg);
         CK(h, cudaMemcpyAsync(out, h->smooth_tmp, bytes, cudaMemcpyDeviceToDevice, st));
-        h->launches++;
     }
     CK(h, cudaGetLastError());
     return 0;
 }
 
-int launch_chain(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, cudaStream_t st, int phases = PH_ALL)
+// The kernel chain over `nch` chunks on the scratch view `sc` (seamless mode: a window of h->sc).
+int launch_chain(sdrb_handle *h, const Scratch &sc, const uint8_t *raw, size_t nch, double *out, cudaStream_t st,
+                 int phases = PH_ALL)
 {
-    if ((phases & PH_FINISH) && h->pl.demod == SDRB_IQ && ((uintptr_t)out & 15))
-        return fail(h, SDRB_ERR_ARG, "iq output is stored as 16-byte (Re, Im) pairs: `out` must be 16-byte aligned");
     return with_enc(h, h->enc_code, [&](auto enc) {
         constexpr int E = decltype(enc)::value;
-        return h->pl.correct_iq ? launch_chain_t<E, true>(h, raw, nch, out, st, phases)
-                                : launch_chain_t<E, false>(h, raw, nch, out, st, phases);
+        return h->pl.correct_iq ? launch_chain_t<E, true>(h, sc, raw, nch, out, st, phases)
+                                : launch_chain_t<E, false>(h, sc, raw, nch, out, st, phases);
     });
 }
 
@@ -374,59 +375,105 @@ template <int ENC, bool IQ>
 int set_smem_attr_t(sdrb_handle *h)
 {
     CK(h, cudaFuncSetAttribute(k_main<ENC, IQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->main_smem));
-    if (h->finish_on) {
-        const int ok = out_kind(h->pl.demod);
-        CK(h, cudaFuncSetAttribute(ok == OUT_IQ ? k_finish<ENC, OUT_IQ> : (ok == OUT_SSB ? k_finish<ENC, OUT_SSB> : k_finish<ENC, OUT_REAL>),
-                                   cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->finish_smem));
-    }
-    return 0;
-}
-int set_smem_attr(sdrb_handle *h)
-{
-    return with_enc(h, h->enc_code, [&](auto enc) {
-        constexpr int E = decltype(enc)::value;
-        return h->pl.correct_iq ? set_smem_attr_t<E, true>(h) : set_smem_attr_t<E, false>(h);
+    return with_out(h->pl.demod, [&](auto ok) {
+        constexpr int OK = decltype(ok)::value;
+        if (h->finish_on)
+            CK(h, cudaFuncSetAttribute(k_finish<ENC, OK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->finish_smem));
+        if constexpr (OK != OUT_IQ)    // the iq k_demod only copies: no dynamic shared memory
+            if (h->demod_smem > 48 * 1024)
+                CK(h, cudaFuncSetAttribute(k_demod<OK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->demod_smem));
+        return 0;
     });
 }
 
-int env_int(const char *name, int dflt)
+// ------------------------------------------------------------------ sdrb_create, in stages
+// The plan's scalars and inline tables.  Reads only table pointers validate() requires first.
+DevPlan plan_of(const sdrb_config *cfg, const sdrb_tables *tab)
 {
-    const char *v = getenv(name);
-    return (v && *v) ? atoi(v) : dflt;
+    DevPlan pl{};
+    const int code = enc_code_of(cfg->enc);
+    pl.enc = code; pl.itemsize = itemsize_of(code); pl.swap = cfg->swap; pl.correct_iq = cfg->correct_iq;
+    pl.normalize = cfg->normalize; pl.demod = cfg->demod; pl.be_out = cfg->big_endian_out;
+    pl.q = cfg->q; pl.N = cfg->N; pl.edge = cfg->edge; pl.L = cfg->N + 2 * cfg->edge;
+    pl.Mf = cfg->N / cfg->q; pl.rem = cfg->N - pl.Mf * cfg->q; pl.M = pl.Mf + (pl.rem ? 1 : 0);
+    pl.W = cfg->demod == SDRB_IQ ? 2 * pl.M : pl.M;
+    pl.ssb_omega = is_ssb(cfg->demod) ? tab->ssb_omega : 0.0;
+    pl.ntiles = (pl.Mf + SDRB_TB - 1) / SDRB_TB; pl.cnt_last = pl.Mf - (pl.ntiles - 1) * SDRB_TB;
+    pl.Hq = (cfg->q + 1) / 2; pl.KS = (pl.Hq + 3) / 4; pl.R = cfg->R;
+    pl.RL = tab->RL;
+    pl.sb = 2 * pl.itemsize;
+    for (int i = 0; i < 8; i++) { pl.run_len[i] = tab->run_len[i]; pl.lam_run[i] = tab->lam_run[i]; }
+    pl.lam_inv = tab->lam_inv;
+    pl.sos_ns = 2 * cfg->n_out_sections; pl.sos_Lseg = tab->sos_Lseg;
+    pl.ws = std::min(pl.q * pl.Mf, pl.N - 1 - pl.edge); pl.nend = pl.N - pl.ws;
+    pl.k_bnd = tab->k_bnd; pl.nsec_out = cfg->n_out_sections;
+    pl.Liq = cfg->correct_iq ? cfg->iq_L : 0.0; pl.lam = tab->lam; pl.lam_q = tab->lam_q; pl.lam_N = tab->lam_N;
+    pl.g0 = tab->g0; pl.d = tab->d; pl.norm_xmin = cfg->norm_xmin; pl.norm_k = cfg->norm_k;
+    pl.lam_tile[0] = tab->lam_tile[0]; pl.lam_tile[1] = tab->lam_tile[1];
+    {
+        double v = tab->lam_q;
+        for (int i = 0; i < 5; i++) { pl.lamq_pow[i] = v; v *= v; }
+    }
+    for (int i = 0; i < SDRB_NP; i++) {
+        pl.p[i] = c2(tab->p, i); pl.P[i] = c2(tab->P, i); pl.rho[i] = c2(tab->rho, i);
+        pl.rho_p[i] = c2(tab->rho_p, i); pl.c[i] = c2(tab->c, i); pl.zhat[i] = c2(tab->zhat, i);
+        pl.bx[i] = c2(tab->bx, i);
+    }
+    for (int i = 0; i < SDRB_NP * SDRB_NP; i++) pl.xi[i] = c2(tab->xi, i);
+    for (int i = 0; i < 6 * cfg->n_out_sections; i++) pl.out_sos[i] = tab->out_sos[i];
+    for (int i = 0; i < 33; i++) { pl.lam_pw[i] = tab->lam_k[i]; pl.mu_pw[i] = tab->mu_k[i]; }
+    const int h2 = pl.M >> 1;
+    pl.fft_ok = (pl.M == 2 * h2) && is_pow2(h2) ? 1 : 0;
+    pl.fft_n = pl.fft_ok ? pl.M : 0;
+    return pl;
 }
 
-}  // namespace
-
-extern "C" {
-
-const char *sdrb_global_error(void) { return g_error.c_str(); }
-const char *sdrb_last_error(const sdrb_handle *h) { return h ? h->error.c_str() : g_error.c_str(); }
-
-int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **out)
+// k_main's tiles and warps per CTA (SDRB_TPC / SDRB_WARPS override them); returns its dynamic shared memory.
+size_t main_geometry(const DevPlan &pl, int &tpc, int &warps)
 {
-    if (!cfg || !tab || !out) return fail(nullptr, SDRB_ERR_ARG, "null argument");
+    const int R = pl.R;
+    auto smem_for = [&](int t, int w) {
+        return (size_t)t * main_tile_bytes(pl.RL, pl.sb) + (size_t)w * main_warp_bytes();
+    };
+    // k_main: a CTA's warps share TPC staged tiles and take (tile, row) items in rounds
+    // (more than one tile per CTA measured slower for banks: 33 rows, TPC 1/2/3 -> 205/191/153 G)
+    const int tpc_auto = R == 1 ? 2 : 1;
+    // warps per CTA for a bank: 8 (two CTAs of 126 registers per SM).  Measured, float32 q = 64,
+    // G VFO*samples/s at 257/65/33 rows: W=8 326/308/290, W=7 306/290/286, W=6 303/291/277,
+    // W=5 311/304/292 (microbench/bank_rows.py).
+    const int warps_auto = R == 1 ? 2 : (R >= 8 ? 8 : 4);
+    tpc = env_int("SDRB_TPC", tpc_auto);
+    if (tpc > pl.ntiles) tpc = pl.ntiles;
+    warps = env_int("SDRB_WARPS", R == 1 ? tpc : warps_auto);
+    if (tpc < 1) tpc = 1;
+    if (warps < 1) warps = 1;
+    if (warps > 8) warps = 8;
+    while (tpc > 1 && smem_for(tpc, warps) > 220 * 1024) tpc--;
+    while (warps > 1 && smem_for(tpc, warps) > 220 * 1024) warps--;
+    return smem_for(tpc, warps);
+}
+
+// Every configuration sdrb_create refuses: host code only, so a refusal touches no device.
+int validate(const sdrb_config *cfg, const sdrb_tables *tab)
+{
+    if (!cfg || !tab) return fail(nullptr, SDRB_ERR_ARG, "null argument");
     if (cfg->abi_version != SDRB_ABI_VERSION) return fail(nullptr, SDRB_ERR_ARG, "ABI version mismatch");
-    const int code = enc_code_of(cfg->enc);
-    if (code < 0) return fail(nullptr, SDRB_ERR_ARG, "unknown encoding '%c'", cfg->enc);
+    if (enc_code_of(cfg->enc) < 0) return fail(nullptr, SDRB_ERR_ARG, "unknown encoding '%c'", cfg->enc);
     if (cfg->q < 2 || cfg->q > SDRB_MAX_DECIMATION)
         return fail(nullptr, SDRB_ERR_ARG, "decimation %d outside 2..%d", cfg->q, SDRB_MAX_DECIMATION);
     if (cfg->R < 1 || cfg->edge < 1 || cfg->N <= cfg->edge + 1 || cfg->max_chunks < 1 || cfg->n_out_sections < 0 ||
         cfg->n_out_sections > 4)
         return fail(nullptr, SDRB_ERR_ARG, "bad geometry");
-    {   // k_fixup stages (edge+1) head samples and nend = max(rem, edge+1) window samples in shared memory
-        const int rem = cfg->N % cfg->q;
-        if (cfg->edge + 1 + std::max(rem, cfg->edge + 1) > SDRB_NEDGE)
-            return fail(nullptr, SDRB_ERR_ARG, "filter pad %d too long for the fix-up kernel", cfg->edge);
-    }
-    {
-        const void *need[] = {tab->p, tab->P, tab->rho, tab->rho_p, tab->c, tab->zhat, tab->xi, tab->Ec, tab->Oc,
-                              tab->Ppow, tab->pk, tab->Pt, tab->bx, tab->bnd, tab->lam_j, tab->lam_k, tab->mu_k,
-                              tab->T2, tab->T3, tab->T1, tab->Ehead, tab->Eend, tab->alpha, tab->alphaT, tab->beta,
-                              tab->betaT, tab->gamma, tab->phE, tab->psiY, tab->use_nco};
-        for (const void *ptr : need)
-            if (!ptr) return fail(nullptr, SDRB_ERR_ARG, "a required table pointer is NULL");
-        if (cfg->n_out_sections > 0 && !tab->out_sos) return fail(nullptr, SDRB_ERR_ARG, "out_sos is NULL");
-    }
+    // k_fixup stages (edge+1) head samples and nend = max(rem, edge+1) window samples in shared memory
+    if (cfg->edge + 1 + std::max(cfg->N % cfg->q, cfg->edge + 1) > SDRB_NEDGE)
+        return fail(nullptr, SDRB_ERR_ARG, "filter pad %d too long for the fix-up kernel", cfg->edge);
+    const void *need[] = {tab->p, tab->P, tab->rho, tab->rho_p, tab->c, tab->zhat, tab->xi, tab->Ec, tab->Oc,
+                          tab->Ppow, tab->pk, tab->Pt, tab->bx, tab->bnd, tab->lam_j, tab->lam_k, tab->mu_k,
+                          tab->T2, tab->T3, tab->T1, tab->Ehead, tab->Eend, tab->alpha, tab->alphaT, tab->beta,
+                          tab->betaT, tab->gamma, tab->phE, tab->psiY, tab->use_nco};
+    for (const void *ptr : need)
+        if (!ptr) return fail(nullptr, SDRB_ERR_ARG, "a required table pointer is NULL");
+    if (cfg->n_out_sections > 0 && !tab->out_sos) return fail(nullptr, SDRB_ERR_ARG, "out_sos is NULL");
     if (cfg->N / cfg->q < 1) return fail(nullptr, SDRB_ERR_ARG, "chunk shorter than one block");
     if (cfg->demod > SDRB_LSB) return fail(nullptr, SDRB_ERR_ARG, "unknown demodulation %d", (int)cfg->demod);
     if (cfg->demod == SDRB_IQ && cfg->n_out_sections != 0)
@@ -442,56 +489,44 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
             std::fabs(tab->ssb_rot[2] - std::cos(om)) > 1e-12 || std::fabs(tab->ssb_rot[3] - std::sin(om)) > 1e-12)
             return fail(nullptr, SDRB_ERR_ARG, "ssb_rot does not start 1, e^{j Omega}");
     }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        return fail(nullptr, SDRB_ERR_CUDA, "no CUDA device: libsdrterm_b200 has no CPU fallback");
-    if (cfg->device < 0 || cfg->device >= ndev) return fail(nullptr, SDRB_ERR_ARG, "bad device ordinal");
+    const DevPlan pl = plan_of(cfg, tab);
+    if (pl.RL != pl.KS) return fail(nullptr, SDRB_ERR_ARG, "RL %d does not match ceil(Hq/4) = %d", pl.RL, pl.KS);
+    if (pl.nsec_out > 0 && (!tab->sos_CA || !tab->sos_AP || tab->sos_Lseg * 32 < pl.M))
+        return fail(nullptr, SDRB_ERR_ARG, "output SOS segment tables missing or too short");
+    if (cfg->demod == SDRB_FM && !pl.fft_ok && !tab->fm_interp)
+        return fail(nullptr, SDRB_ERR_ARG, "FM with M=%d needs the dense interpolation table", pl.M);
+    int tpc, warps;
+    if (main_geometry(pl, tpc, warps) > 227 * 1024)
+        return fail(nullptr, SDRB_ERR_ARG, "decimation %d needs too much shared memory", pl.q);
+    if (cfg->seamless &&
+        (pl.rem != 0 || pl.cnt_last != SDRB_TB || tab->lookahead < 1 || !tab->PN || !tab->chunk_step || tab->fs <= 0 ||
+         tab->fs >= (1LL << 31) || (pl.nsec_out != 0 && pl.nsec_out != 2) ||
+         (pl.nsec_out && (!tab->sos_AM || !tab->sos_CAM || pl.sos_Lseg * 32 != pl.M))))
+        return fail(nullptr, SDRB_ERR_ARG, "seamless mode needs the decimation to divide the chunk (q | N), "
+                                           "a lookahead >= 1 and its tables");
+    if (tab->tc_enable) {
+        if ((tab->tc_K != 256 && tab->tc_K != 512) || tab->tc_nout != TC_NOUT || tab->tc_ncol != TC_NCOL ||
+            tab->tc_isz < 1 || tab->tc_isz > 2 || tab->tc_npad != TC_NPAD || tab->tc_nrowc != TC_NROWC ||
+            tab->tc_K != 2 * pl.q * pl.sb || pl.rem != 0 || pl.cnt_last != SDRB_TB || (pl.Mf / 2) % 128 ||
+            pl.q < pl.edge + 1 || pl.normalize || !tab->tc_Bq || !tab->tc_cst || !tab->tc_rowc)
+            return fail(nullptr, SDRB_ERR_ARG, "tensor-core tables do not match the configuration");
+        if (pl.R <= TC_MAX_R) {   // wider banks take the FP64 block kernel: these tables go unused
+            for (int i = 0; i < 16; i++)
+                if (tab->tc_xor[i] != tab->tc_xor[i & 3]) return fail(nullptr, SDRB_ERR_ARG, "XOR pattern is not 4-periodic");
+            if (tc_stages(tab->tc_K) < 2)
+                return fail(nullptr, SDRB_ERR_ARG, "k_tc: no room for the A ring (%zu bytes fixed)", tc_fixed_bytes(tab->tc_K / 128));
+        }
+    }
+    return 0;
+}
 
-    sdrb_handle *h = new sdrb_handle();
-    h->cfg = *cfg;
-    h->enc_code = code;
-    h->max_chunks = (size_t)cfg->max_chunks;
-    int rc = 0;
-    auto bail = [&](int c) { std::string e = h->error; sdrb_destroy(h); g_error = e; return c; };
-    if (cudaSetDevice(cfg->device) != cudaSuccess) return bail(fail(h, SDRB_ERR_CUDA, "cudaSetDevice failed"));
-
+// The plan's device tables: derived on the host, then uploaded.
+int plan_tables(sdrb_handle *h, const sdrb_tables *tab)
+{
     DevPlan &pl = h->pl;
-    pl.enc = code; pl.itemsize = itemsize_of(code); pl.swap = cfg->swap; pl.correct_iq = cfg->correct_iq;
-    pl.normalize = cfg->normalize; pl.demod = cfg->demod; pl.be_out = cfg->big_endian_out;
-    pl.q = cfg->q; pl.N = cfg->N; pl.edge = cfg->edge; pl.L = cfg->N + 2 * cfg->edge;
-    pl.Mf = cfg->N / cfg->q; pl.rem = cfg->N - pl.Mf * cfg->q; pl.M = pl.Mf + (pl.rem ? 1 : 0);
-    pl.W = cfg->demod == SDRB_IQ ? 2 * pl.M : pl.M;
-    pl.ssb_omega = is_ssb(cfg->demod) ? tab->ssb_omega : 0.0;
-    pl.ntiles = (pl.Mf + SDRB_TB - 1) / SDRB_TB; pl.cnt_last = pl.Mf - (pl.ntiles - 1) * SDRB_TB;
-    pl.Hq = (cfg->q + 1) / 2; pl.KS = (pl.Hq + 3) / 4; pl.R = cfg->R;
-    pl.RL = tab->RL;
-    if (pl.RL != pl.KS) return bail(fail(h, SDRB_ERR_ARG, "RL %d does not match ceil(Hq/4) = %d", pl.RL, pl.KS));
-    pl.sb = 2 * pl.itemsize;
-    for (int i = 0; i < 8; i++) { pl.run_len[i] = tab->run_len[i]; pl.lam_run[i] = tab->lam_run[i]; }
-    pl.lam_inv = tab->lam_inv;
-    pl.sos_ns = 2 * cfg->n_out_sections; pl.sos_Lseg = tab->sos_Lseg;
-    if (cfg->n_out_sections > 0) {
-        if (!tab->sos_CA || !tab->sos_AP || tab->sos_Lseg * 32 < pl.M)
-            return bail(fail(h, SDRB_ERR_ARG, "output SOS segment tables missing or too short"));
-        for (int i = 0; i < 5 * pl.sos_ns * pl.sos_ns; i++) pl.sos_AP[i] = tab->sos_AP[i];
-    }
-    pl.ws = std::min(pl.q * pl.Mf, pl.N - 1 - pl.edge); pl.nend = pl.N - pl.ws;
-    pl.k_bnd = tab->k_bnd; pl.nsec_out = cfg->n_out_sections;
-    pl.Liq = cfg->correct_iq ? cfg->iq_L : 0.0; pl.lam = tab->lam; pl.lam_q = tab->lam_q; pl.lam_N = tab->lam_N;
-    pl.g0 = tab->g0; pl.d = tab->d; pl.norm_xmin = cfg->norm_xmin; pl.norm_k = cfg->norm_k;
-    pl.lam_tile[0] = tab->lam_tile[0]; pl.lam_tile[1] = tab->lam_tile[1];
-    {
-        double v = tab->lam_q;
-        for (int i = 0; i < 5; i++) { pl.lamq_pow[i] = v; v *= v; }
-    }
-    for (int i = 0; i < SDRB_NP; i++) {
-        pl.p[i] = c2(tab->p, i); pl.P[i] = c2(tab->P, i); pl.rho[i] = c2(tab->rho, i);
-        pl.rho_p[i] = c2(tab->rho_p, i); pl.c[i] = c2(tab->c, i); pl.zhat[i] = c2(tab->zhat, i);
-    }
-    for (int i = 0; i < SDRB_NP * SDRB_NP; i++) pl.xi[i] = c2(tab->xi, i);
-    for (int i = 0; i < 6 * cfg->n_out_sections; i++) pl.out_sos[i] = tab->out_sos[i];
-
     const int q = pl.q, R = pl.R, Hq = pl.Hq, KS = pl.KS, nt = pl.ntiles, M = pl.M;
+    if (pl.nsec_out > 0)
+        for (int i = 0; i < 5 * pl.sos_ns * pl.sos_ns; i++) pl.sos_AP[i] = tab->sos_AP[i];
     // DMMA A fragments: lane -> (row o = lane>>2: mode o>>1, Re/Im o&1 ; col k = lane&3)
     std::vector<double> afrag((size_t)KS * 2 * 32, 0.0);
     for (int s = 0; s < KS; s++)
@@ -509,169 +544,196 @@ int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **ou
             rw[(size_t)l * 8 + i] = hmul(pl.rho[i], pp);
             rt[(size_t)l * 8 + i] = hmul(pl.rho_p[i], pp);
         }
-    std::vector<double2> prot((size_t)R * 16);
+    // per row: the rotating-frame block multipliers; the reciprocals of beta and the output weights
+    // derived from them (host doubles; |beta - 1| << 1)
+    std::vector<double2> prot((size_t)R * 16), binv((size_t)R * 8), binvT((size_t)R * 8), rb((size_t)R * 8), rbT((size_t)R * 8);
+    auto hinv = [](double2 a) { const double d = a.x * a.x + a.y * a.y; return make_double2(a.x / d, -a.y / d); };
     for (int r = 0; r < R; r++) {
         const double2 eps = c2(tab->T3, (size_t)r * (SDRB_TB + 1) + 1);
         for (int i = 0; i < 8; i++) {
             prot[(size_t)r * 16 + i] = hmul(make_double2(eps.x, -eps.y), pl.P[i]);
             prot[(size_t)r * 16 + 8 + i] = hmul(eps, pl.P[i]);
+            const double2 b = c2(tab->beta, (size_t)r * 8 + i), bT = c2(tab->betaT, (size_t)r * 8 + i);
+            binv[(size_t)r * 8 + i] = hinv(b); binvT[(size_t)r * 8 + i] = hinv(bT);
+            rb[(size_t)r * 8 + i] = hmul(pl.rho[i], b); rbT[(size_t)r * 8 + i] = hmul(pl.rho_p[i], bT);
         }
     }
-    const int h2 = M >> 1;
-    pl.fft_ok = (M == 2 * h2) && is_pow2(h2) ? 1 : 0;
-    pl.fft_n = pl.fft_ok ? M : 0;
-    if (cfg->demod == SDRB_FM && !pl.fft_ok && !tab->fm_interp)
-        return bail(fail(h, SDRB_ERR_ARG, "FM with M=%d needs the dense interpolation table", M));
-    std::vector<double2> tw = make_twiddles(pl.fft_n);
+    const std::vector<double2> tw = make_twiddles(pl.fft_n);
+    auto d2 = [](const double *a) { return reinterpret_cast<const double2 *>(a); };
+    int rc;
+    if ((rc = upload(h, afrag.data(), afrag.size(), &pl.Afrag)) ||
+        (rc = upload(h, tab->lam_j, (size_t)q + 1, &pl.lam_j)) ||
+        (rc = upload(h, d2(tab->Ppow), (size_t)(SDRB_TB + 1) * 8, &pl.Ppow)) ||
+        (rc = upload(h, d2(tab->pk), (size_t)(pl.edge + 1) * 8, &pl.pk)) ||
+        (rc = upload(h, d2(tab->Pt), (size_t)nt * 8, &pl.Pt)) ||
+        (rc = upload(h, rw.data(), rw.size(), &pl.RW)) ||
+        (rc = upload(h, rt.data(), rt.size(), &pl.RT)) ||
+        (rc = upload(h, d2(tab->bnd), (size_t)M * 8, &pl.bnd)) ||
+        (rc = upload(h, d2(tab->T2), (size_t)R * q, &pl.T2)) ||
+        (rc = upload(h, d2(tab->T3), (size_t)R * (SDRB_TB + 1), &pl.T3)) ||
+        (rc = upload(h, d2(tab->T1), (size_t)R * nt, &pl.T1)) ||
+        (rc = upload(h, d2(tab->Ehead), (size_t)R * (pl.edge + 1), &pl.Ehead)) ||
+        (rc = upload(h, d2(tab->Eend), (size_t)R * pl.nend, &pl.Eend)) ||
+        (rc = upload(h, d2(tab->alpha), (size_t)R * 8, &pl.alpha)) ||
+        (rc = upload(h, d2(tab->alphaT), (size_t)R * 8, &pl.alphaT)) ||
+        (rc = upload(h, d2(tab->beta), (size_t)R * 8, &pl.beta)) ||
+        (rc = upload(h, d2(tab->betaT), (size_t)R * 8, &pl.betaT)) ||
+        (rc = upload(h, d2(tab->gamma), (size_t)R, &pl.gamma)) ||
+        (rc = upload(h, d2(tab->phE), (size_t)R, &pl.phE)) ||
+        (rc = upload(h, binv.data(), binv.size(), &pl.binv)) ||
+        (rc = upload(h, binvT.data(), binvT.size(), &pl.binvT)) ||
+        (rc = upload(h, rb.data(), rb.size(), &pl.rb)) ||
+        (rc = upload(h, rbT.data(), rbT.size(), &pl.rbT)) ||
+        (rc = upload(h, d2(tab->psiY), (size_t)2 * R * SDRB_TB, &pl.psiY)) ||
+        (rc = upload(h, prot.data(), prot.size(), &pl.Prot)) ||
+        (rc = upload(h, tw.data(), tw.size(), &pl.tw)) ||
+        (rc = upload(h, tab->use_nco, (size_t)R, &pl.use_nco)) ||
+        (pl.nsec_out > 0 && (rc = upload(h, tab->sos_CA, (size_t)pl.sos_Lseg * pl.sos_ns, &pl.sos_CA))) ||
+        (pl.demod == SDRB_FM && !pl.fft_ok && (rc = upload(h, tab->fm_interp, (size_t)M * (M >> 1), &pl.fm_interp))) ||
+        (is_ssb(pl.demod) && (rc = upload(h, d2(tab->ssb_rot), (size_t)M + 1, &pl.ssb_rot))))
+        return rc;
+    return 0;
+}
 
-#define UP(expr) do { rc = (expr); if (rc) return bail(rc); } while (0)
-    UP(upload(h, afrag.data(), afrag.size(), &pl.Afrag));
-    UP(upload(h, tab->lam_j, (size_t)q + 1, &pl.lam_j));
-    UP(upload(h, reinterpret_cast<const double2 *>(tab->Ppow), (size_t)(SDRB_TB + 1) * 8, &pl.Ppow));
-    if (!tab->pk || !tab->lam_k || !tab->mu_k || !tab->Pt || !tab->bx) return bail(fail(h, SDRB_ERR_ARG, "pole / IQ power tables missing"));
-    UP(upload(h, reinterpret_cast<const double2 *>(tab->pk), (size_t)(pl.edge + 1) * 8, &pl.pk));
-    for (int i = 0; i < 33; i++) { pl.lam_pw[i] = tab->lam_k[i]; pl.mu_pw[i] = tab->mu_k[i]; }
-    UP(upload(h, reinterpret_cast<const double2 *>(tab->Pt), (size_t)nt * 8, &pl.Pt));
-    for (int i = 0; i < SDRB_NP; i++) pl.bx[i] = c2(tab->bx, i);
-    UP(upload(h, rw.data(), rw.size(), &pl.RW));
-    UP(upload(h, rt.data(), rt.size(), &pl.RT));
-    UP(upload(h, reinterpret_cast<const double2 *>(tab->bnd), (size_t)M * 8, &pl.bnd));
-    UP(upload(h, reinterpret_cast<const double2 *>(tab->T2), (size_t)R * q, &pl.T2));
-    UP(upload(h, reinterpret_cast<const double2 *>(tab->T3), (size_t)R * (SDRB_TB + 1), &pl.T3));
-    UP(upload(h, reinterpret_cast<const double2 *>(tab->T1), (size_t)R * nt, &pl.T1));
-    UP(upload(h, reinterpret_cast<const double2 *>(tab->Ehead), (size_t)R * (pl.edge + 1), &pl.Ehead));
-    UP(upload(h, reinterpret_cast<const double2 *>(tab->Eend), (size_t)R * pl.nend, &pl.Eend));
-    UP(upload(h, reinterpret_cast<const double2 *>(tab->alpha), (size_t)R * 8, &pl.alpha));
-    UP(upload(h, reinterpret_cast<const double2 *>(tab->alphaT), (size_t)R * 8, &pl.alphaT));
-    UP(upload(h, reinterpret_cast<const double2 *>(tab->beta), (size_t)R * 8, &pl.beta));
-    UP(upload(h, reinterpret_cast<const double2 *>(tab->betaT), (size_t)R * 8, &pl.betaT));
-    UP(upload(h, reinterpret_cast<const double2 *>(tab->gamma), (size_t)R, &pl.gamma));
-    UP(upload(h, reinterpret_cast<const double2 *>(tab->phE), (size_t)R, &pl.phE));
-    {   // reciprocals and output weights derived from them (host doubles; |beta - 1| << 1)
-        std::vector<double2> binv((size_t)R * 8), binvT((size_t)R * 8), rb((size_t)R * 8), rbT((size_t)R * 8);
-        auto hinv = [](double2 a) { const double d = a.x * a.x + a.y * a.y; return make_double2(a.x / d, -a.y / d); };
-        for (int r = 0; r < R; r++)
-            for (int i = 0; i < 8; i++) {
-                const double2 b = c2(tab->beta, (size_t)r * 8 + i), bT = c2(tab->betaT, (size_t)r * 8 + i);
-                binv[(size_t)r * 8 + i] = hinv(b); binvT[(size_t)r * 8 + i] = hinv(bT);
-                rb[(size_t)r * 8 + i] = hmul(pl.rho[i], b); rbT[(size_t)r * 8 + i] = hmul(pl.rho_p[i], bT);
-            }
-        UP(upload(h, binv.data(), binv.size(), &pl.binv));
-        UP(upload(h, binvT.data(), binvT.size(), &pl.binvT));
-        UP(upload(h, rb.data(), rb.size(), &pl.rb));
-        UP(upload(h, rbT.data(), rbT.size(), &pl.rbT));
-    }
-    UP(upload(h, reinterpret_cast<const double2 *>(tab->psiY), (size_t)2 * R * SDRB_TB, &pl.psiY));
-    UP(upload(h, prot.data(), prot.size(), &pl.Prot));
-    UP(upload(h, tw.data(), tw.size(), &pl.tw));
-    UP(upload(h, tab->use_nco, (size_t)R, &pl.use_nco));
-    pl.sos_CA = nullptr;
-    if (cfg->n_out_sections > 0) UP(upload(h, tab->sos_CA, (size_t)pl.sos_Lseg * pl.sos_ns, &pl.sos_CA));
-    pl.fm_interp = nullptr;
-    if (cfg->demod == SDRB_FM && !pl.fft_ok) UP(upload(h, tab->fm_interp, (size_t)M * h2, &pl.fm_interp));
-    pl.ssb_rot = nullptr;
-    if (is_ssb(cfg->demod)) UP(upload(h, reinterpret_cast<const double2 *>(tab->ssb_rot), (size_t)M + 1, &pl.ssb_rot));
-
-    // launch geometry
-    auto smem_for = [&](int tpc, int w) {
-        return (size_t)tpc * main_tile_bytes(pl.RL, pl.sb) + (size_t)w * main_warp_bytes();
-    };
-    // k_main: a CTA's warps share TPC staged tiles and take (tile, row) items in rounds
-    // (more than one tile per CTA measured slower for banks: 33 rows, TPC 1/2/3 -> 205/191/153 G)
-    const int tpc_auto = R == 1 ? 2 : 1;
-    // warps per CTA for a bank: 8 (two CTAs of 126 registers per SM).  Measured, float32 q = 64,
-    // G VFO*samples/s at 257/65/33 rows: W=8 326/308/290, W=7 306/290/286, W=6 303/291/277,
-    // W=5 311/304/292 (microbench/bank_rows.py).
-    const int warps_auto = R == 1 ? 2 : (R >= 8 ? 8 : 4);
-    h->tpc = env_int("SDRB_TPC", tpc_auto);
-    if (h->tpc > pl.ntiles) h->tpc = pl.ntiles;
-    h->warps = env_int("SDRB_WARPS", R == 1 ? h->tpc : warps_auto);
-    if (h->tpc < 1) h->tpc = 1;
-    if (h->warps < 1) h->warps = 1;
-    if (h->warps > 8) h->warps = 8;
-    while (h->tpc > 1 && smem_for(h->tpc, h->warps) > 220 * 1024) h->tpc--;
-    while (h->warps > 1 && smem_for(h->tpc, h->warps) > 220 * 1024) h->warps--;
-    h->main_smem = smem_for(h->tpc, h->warps);
-    if (h->main_smem > 227 * 1024) return bail(fail(h, SDRB_ERR_ARG, "decimation %d needs too much shared memory", q));
-    {
-        cudaDeviceProp prop;
-        if (cudaGetDeviceProperties(&prop, cfg->device) == cudaSuccess) h->num_sms = prop.multiProcessorCount;
-        const bool pow2 = is_pow2(M);
-        h->finish_on = !env_int("SDRB_NO_FINISH", 0) && pl.rem == 0 && pl.cnt_last == SDRB_TB && q >= pl.edge + 1 &&
-                       pow2 && M >= 64 && M <= 1024 && pl.edge + 1 <= 32 && pl.ntiles <= 32 &&
-                       (cfg->n_out_sections == 0 || cfg->n_out_sections == 2);
-        h->finish_smem = h->finish_on ? finish_smem_bytes(M, pl.edge) : 0;
-        if (h->finish_smem > 227 * 1024) h->finish_on = false;
-    }
-    UP(set_smem_attr(h));
+// Launch geometry: SM count, k_main's tiles and warps, the fused k_finish switch, k_demod's shared memory.
+int set_geometry(sdrb_handle *h)
+{
+    DevPlan &pl = h->pl;
+    cudaDeviceProp prop;
+    CK(h, cudaGetDeviceProperties(&prop, h->cfg.device));
+    h->num_sms = prop.multiProcessorCount;
+    h->main_smem = main_geometry(pl, h->tpc, h->warps);
+    const int M = pl.M;
+    h->finish_on = !env_int("SDRB_NO_FINISH", 0) && pl.rem == 0 && pl.cnt_last == SDRB_TB && pl.q >= pl.edge + 1 &&
+                   is_pow2(M) && M >= 64 && M <= 1024 && pl.edge + 1 <= 32 && pl.ntiles <= 32 &&
+                   (pl.nsec_out == 0 || pl.nsec_out == 2);
+    h->finish_smem = h->finish_on ? finish_smem_bytes(M, pl.edge) : 0;
+    if (h->finish_smem > 227 * 1024) h->finish_on = false;
     const size_t dsm = (size_t)M * (2 * sizeof(double2) + sizeof(double));
     pl.demod_in_smem = dsm <= 96 * 1024 ? 1 : 0;
     h->demod_smem = pl.demod_in_smem ? dsm : 0;
-    if (h->demod_smem > 48 * 1024)
-        if (cudaFuncSetAttribute(is_ssb(cfg->demod) ? k_demod<OUT_SSB> : k_demod<OUT_REAL>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->demod_smem) != cudaSuccess)
-            return bail(fail(h, SDRB_ERR_CUDA, "cudaFuncSetAttribute(k_demod) failed"));
+    return with_enc(h, h->enc_code, [&](auto enc) {
+        constexpr int E = decltype(enc)::value;
+        return h->pl.correct_iq ? set_smem_attr_t<E, true>(h) : set_smem_attr_t<E, false>(h);
+    });
+}
 
-    // scratch for max_chunks (seamless: plus the D chunks held back between calls)
-    const size_t nch = h->max_chunks + (cfg->seamless ? (size_t)std::max(tab->lookahead, 0) : 0);
+int alloc_scratch(sdrb_handle *h, size_t nch)
+{
+    const DevPlan &pl = h->pl;
+    const size_t R = pl.R, nt = pl.ntiles, M = pl.M;
     Scratch &sc = h->sc;
-    UP(dalloc(h, nch * R * pl.Mf, &sc.ypart));
-    UP(dalloc(h, nch * R * nt * 16, &sc.agg));
-    UP(dalloc(h, nch * nt, &sc.tile_agg));
-    UP(dalloc(h, nch * (nt + 1), &sc.off_tile));
-    UP(dalloc(h, nch, &sc.gain));
-    UP(dalloc(h, nch, &sc.start));
-    UP(dalloc(h, nch * R * (nt + 1) * 16, &sc.carry));
-    UP(dalloc(h, nch * R * M, &sc.y));
-    UP(dalloc(h, (size_t)1, &sc.iq_state));
-    if (cudaMemset(sc.iq_state, 0, sizeof(double2)) != cudaSuccess) return bail(fail(h, SDRB_ERR_CUDA, "memset failed"));
-    sc.fftbuf = nullptr; sc.zrow = nullptr; sc.dbg = nullptr; sc.x0 = nullptr;
-    if (env_int("SDRB_TC_DEBUG", 0)) {
-        UP(dalloc(h, (size_t)64 * 16, &sc.dbg));
-        cudaMemset(sc.dbg, 0, 64 * 16 * sizeof(unsigned long long));
+    int rc;
+    if ((rc = dalloc(h, nch * R * pl.Mf, &sc.ypart)) ||
+        (rc = dalloc(h, nch * R * nt * 16, &sc.agg)) ||
+        (rc = dalloc(h, nch * nt, &sc.tile_agg)) ||
+        (rc = dalloc(h, nch * (nt + 1), &sc.off_tile)) ||
+        (rc = dalloc(h, nch, &sc.gain)) ||
+        (rc = dalloc(h, nch, &sc.start)) ||
+        (rc = dalloc(h, nch * R * (nt + 1) * 16, &sc.carry)) ||
+        (rc = dalloc(h, nch * R * M, &sc.y)) ||
+        (rc = dalloc(h, (size_t)1, &sc.iq_state)) ||
+        (!pl.demod_in_smem && ((rc = dalloc(h, nch * R * 2 * M, &sc.fftbuf)) || (rc = dalloc(h, nch * R * M, &sc.zrow)))) ||
+        (env_int("SDRB_TC_DEBUG", 0) && (rc = dalloc(h, (size_t)64 * 16, &sc.dbg))))
+        return rc;
+    CK(h, cudaMemset(sc.iq_state, 0, sizeof(double2)));
+    if (sc.dbg) CK(h, cudaMemset(sc.dbg, 0, 64 * 16 * sizeof(unsigned long long)));
+    return 0;
+}
+
+int seam_setup(sdrb_handle *h, const sdrb_tables *tab, size_t nch)
+{
+    const DevPlan &pl = h->pl;
+    SeamDev &sd = h->sd;
+    const size_t R = pl.R, M = pl.M;
+    const size_t sn = (size_t)SEAM_NS * (is_ssb(pl.demod) ? 2 : 1);   // doubles per SOS state (usb / lsb: complex)
+    sd.D = tab->lookahead; sd.fs = tab->fs; sd.nedge = pl.edge + 1 + pl.nend;
+    if (pl.nsec_out)
+        for (int i = 0; i < SEAM_NS * SEAM_NS; i++) sd.AM[i] = tab->sos_AM[i];
+    int rc;
+    if ((rc = upload(h, reinterpret_cast<const long long *>(tab->chunk_step), R, &sd.step)) ||
+        (rc = upload(h, reinterpret_cast<const double2 *>(tab->PN), (size_t)(sd.D + 1) * 8, &sd.PN)) ||
+        (pl.nsec_out && (rc = upload(h, tab->sos_CAM, M * SEAM_NS, &sd.CAM))) ||
+        (rc = dalloc(h, nch * sd.nedge, &sd.edges)) ||
+        (rc = dalloc(h, nch * R * 16, &sd.cagg)) ||
+        (rc = dalloc(h, nch * R * 8, &sd.G)) ||
+        (rc = dalloc(h, nch * R * 24, &sd.cin)) ||
+        (rc = dalloc(h, nch * R * (M + 1), &sd.ybuf)) ||
+        (rc = dalloc(h, nch * R * sn, &sd.echunk)) ||
+        (rc = dalloc(h, nch * R * sn, &sd.sst)) ||
+        (rc = dalloc(h, R * 8, &sd.fwd)) ||
+        (rc = dalloc(h, R * sn, &sd.sos)) ||
+        (rc = dalloc(h, R * 16, &sd.endv)))
+        return rc;
+    CK(h, cudaMemset(sd.sos, 0, R * sn * sizeof(double)));
+    return 0;
+}
+
+int make_streams(sdrb_handle *h)
+{
+    for (Slot &sl : h->slot) {
+        CK(h, cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking));
+        CK(h, cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming));
     }
-    if (!pl.demod_in_smem) {
-        UP(dalloc(h, nch * R * 2 * M, &sc.fftbuf));
-        UP(dalloc(h, nch * R * M, &sc.zrow));
+    CK(h, cudaEventCreateWithFlags(&h->iq_done, cudaEventDisableTiming));
+    return 0;
+}
+
+// ------------------------------------------------------------------ handle entry points
+enum Kind { CHUNK_LOCAL, SEAMLESS, EITHER };
+// how a call takes its chunk count
+enum Count {
+    BATCH,    // up to max_chunks; 0 is a successful no-op (NOTHING_TO_DO)
+    SOME,     // 1..max_chunks
+    UPTO,     // 0..max_chunks, and 0 runs (the stream calls; calls that take no chunks pass 0)
+};
+constexpr int NOTHING_TO_DO = 1;
+
+// The check every handle call makes first: its own pointer and value arguments (`args`), the kind of
+// handle, the chunk count and, for iq, a 16-byte-aligned device output; then it sets the device.
+int entry(sdrb_handle *h, bool args, Kind kind, size_t nchunks = 0, Count count = UPTO, const void *iq_out = nullptr)
+{
+    if (!h || !args) return fail(h, SDRB_ERR_ARG, "null pointer or out-of-range argument");
+    if (kind != EITHER && h->seamless != (kind == SEAMLESS))
+        return fail(h, SDRB_ERR_STATE, h->seamless ? "seamless handle: use sdrb_stream / sdrb_stream_end (or their _device forms)"
+                                                   : "the sdrb_stream calls need a handle created with cfg.seamless");
+    if (nchunks == 0 && count == BATCH) return NOTHING_TO_DO;
+    if ((nchunks == 0 && count == SOME) || nchunks > h->max_chunks)
+        return fail(h, SDRB_ERR_ARG, "nchunks %zu outside %d..%zu", nchunks, count == SOME ? 1 : 0, h->max_chunks);
+    if (h->pl.demod == SDRB_IQ && ((uintptr_t)iq_out & 15))
+        return fail(h, SDRB_ERR_ARG, "iq output is stored as 16-byte (Re, Im) pairs: `out` must be 16-byte aligned");
+    CK(h, cudaSetDevice(h->cfg.device));
+    return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+const char *sdrb_global_error(void) { return g_error.c_str(); }
+const char *sdrb_last_error(const sdrb_handle *h) { return h ? h->error.c_str() : g_error.c_str(); }
+
+int sdrb_create(const sdrb_config *cfg, const sdrb_tables *tab, sdrb_handle **out)
+{
+    if (!out) return fail(nullptr, SDRB_ERR_ARG, "null argument");
+    int rc = validate(cfg, tab);
+    if (!rc) rc = need_device(cfg->device);
+    if (rc) return rc;
+    sdrb_handle *h = new sdrb_handle();
+    h->cfg = *cfg;
+    h->enc_code = enc_code_of(cfg->enc);
+    h->max_chunks = (size_t)cfg->max_chunks;
+    h->seamless = cfg->seamless;
+    h->pl = plan_of(cfg, tab);
+    // scratch for max_chunks (seamless: plus the D chunks held back between calls)
+    const size_t nch = h->max_chunks + (h->seamless ? (size_t)tab->lookahead : 0);
+    if ((rc = plan_tables(h, tab)) || (rc = setup_tc(h, tab)) || (rc = set_geometry(h)) || (rc = alloc_scratch(h, nch)) ||
+        (h->seamless && (rc = seam_setup(h, tab, nch))) || (rc = make_streams(h))) {
+        const std::string e = h->error;
+        sdrb_destroy(h);
+        g_error = e;
+        return rc;
     }
-    UP(setup_tc(h, tab));
-    if (cfg->seamless) {
-        h->seamless = true;
-        SeamDev &sd = h->sd;
-        if (pl.rem != 0 || pl.cnt_last != SDRB_TB || tab->lookahead < 1 || !tab->PN || !tab->chunk_step ||
-            tab->fs <= 0 || tab->fs >= (1LL << 31) || (cfg->n_out_sections != 0 && cfg->n_out_sections != 2) ||
-            (cfg->n_out_sections && (!tab->sos_AM || !tab->sos_CAM || pl.sos_Lseg * 32 != M)))
-            return bail(fail(h, SDRB_ERR_ARG, "seamless mode needs the decimation to divide the chunk (q | N), "
-                                              "a lookahead >= 1 and its tables"));
-        sd.D = tab->lookahead; sd.fs = tab->fs; sd.nedge = pl.edge + 1 + pl.nend;
-        UP(upload(h, reinterpret_cast<const long long *>(tab->chunk_step), (size_t)R, &sd.step));
-        UP(upload(h, reinterpret_cast<const double2 *>(tab->PN), (size_t)(sd.D + 1) * 8, &sd.PN));
-        if (cfg->n_out_sections) {
-            for (int i = 0; i < SEAM_NS * SEAM_NS; i++) sd.AM[i] = tab->sos_AM[i];
-            UP(upload(h, tab->sos_CAM, (size_t)M * SEAM_NS, &sd.CAM));
-        }
-        UP(dalloc(h, nch * sd.nedge, &sd.edges));
-        UP(dalloc(h, nch * R * 16, &sd.cagg));
-        UP(dalloc(h, nch * R * 8, &sd.G));
-        UP(dalloc(h, nch * R * 24, &sd.cin));
-        UP(dalloc(h, nch * R * (M + 1), &sd.ybuf));
-        const size_t sn = (size_t)SEAM_NS * (is_ssb(cfg->demod) ? 2 : 1);   // doubles per SOS state (usb / lsb: complex)
-        UP(dalloc(h, nch * R * sn, &sd.echunk));
-        UP(dalloc(h, nch * R * sn, &sd.sst));
-        UP(dalloc(h, (size_t)R * 8, &sd.fwd));
-        UP(dalloc(h, (size_t)R * sn, &sd.sos));
-        UP(dalloc(h, (size_t)R * 16, &sd.endv));
-        if (cudaMemset(sd.sos, 0, (size_t)R * sn * sizeof(double)) != cudaSuccess)
-            return bail(fail(h, SDRB_ERR_CUDA, "memset failed"));
-    }
-#undef UP
-    for (int s = 0; s < 2; s++) {
-        if (cudaStreamCreateWithFlags(&h->slot[s].stream, cudaStreamNonBlocking) != cudaSuccess ||
-            cudaEventCreateWithFlags(&h->slot[s].done, cudaEventDisableTiming) != cudaSuccess)
-            return bail(fail(h, SDRB_ERR_CUDA, "stream/event creation failed"));
-    }
-    if (cudaEventCreateWithFlags(&h->iq_done, cudaEventDisableTiming) != cudaSuccess)
-        return bail(fail(h, SDRB_ERR_CUDA, "event creation failed"));
     *out = h;
     return SDRB_OK;
 }
@@ -701,40 +763,34 @@ long long sdrb_launch_count(const sdrb_handle *h) { return h ? h->launches : 0; 
 
 int sdrb_process_device(sdrb_handle *h, const void *raw_dev, size_t nchunks, double *out_dev, void *stream)
 {
-    if (!h || !raw_dev || !out_dev) return fail(h, SDRB_ERR_ARG, "null argument");
-    if (h->seamless) return fail(h, SDRB_ERR_STATE, "seamless handle: use sdrb_stream_device / sdrb_stream_end_device");
-    if (nchunks == 0) return SDRB_OK;
-    if (nchunks > h->max_chunks) return fail(h, SDRB_ERR_ARG, "nchunks %zu > max_chunks %zu", nchunks, h->max_chunks);
-    CK(h, cudaSetDevice(h->cfg.device));
+    int rc = entry(h, raw_dev && out_dev, CHUNK_LOCAL, nchunks, BATCH, out_dev);
+    if (rc) return rc == NOTHING_TO_DO ? SDRB_OK : rc;
     h->last_nchunks = nchunks;
-    return launch_chain(h, static_cast<const uint8_t *>(raw_dev), nchunks, out_dev, static_cast<cudaStream_t>(stream));
+    return launch_chain(h, h->sc, static_cast<const uint8_t *>(raw_dev), nchunks, out_dev, static_cast<cudaStream_t>(stream));
 }
 
-static int ensure_slot(sdrb_handle *h, int s)
+// Host input of `nchunks` chunks into slot s's device staging (allocated on first use), on its stream.
+static int stage_in(sdrb_handle *h, int s, const void *raw_host, size_t nchunks)
 {
     Slot &sl = h->slot[s];
     if (!sl.raw) CK(h, cudaMalloc(&sl.raw, h->max_chunks * sdrb_chunk_bytes(h)));
     const size_t och = h->max_chunks + (h->seamless ? (size_t)h->sd.D : 0);
     if (!sl.out) CK(h, cudaMalloc(&sl.out, och * (size_t)h->pl.R * h->pl.W * sizeof(double)));
+    if (nchunks) CK(h, cudaMemcpyAsync(sl.raw, raw_host, nchunks * sdrb_chunk_bytes(h), cudaMemcpyHostToDevice, sl.stream));
     return 0;
 }
 
 int sdrb_submit(sdrb_handle *h, int s, const void *raw_host, size_t nchunks, double *out_host)
 {
-    if (!h || !raw_host || !out_host || s < 0 || s > 1) return fail(h, SDRB_ERR_ARG, "bad argument");
-    if (h->seamless) return fail(h, SDRB_ERR_STATE, "seamless handle: use sdrb_stream / sdrb_stream_end");
-    if (nchunks == 0 || nchunks > h->max_chunks) return fail(h, SDRB_ERR_ARG, "nchunks %zu outside 1..%zu", nchunks, h->max_chunks);
-    CK(h, cudaSetDevice(h->cfg.device));
-    int rc = ensure_slot(h, s);
+    int rc = entry(h, raw_host && out_host && (s == 0 || s == 1), CHUNK_LOCAL, nchunks, SOME);
+    if (!rc) rc = stage_in(h, s, raw_host, nchunks);
     if (rc) return rc;
     Slot &sl = h->slot[s];
-    const size_t cb = sdrb_chunk_bytes(h);
-    CK(h, cudaMemcpyAsync(sl.raw, raw_host, nchunks * cb, cudaMemcpyHostToDevice, sl.stream));
     // the scratch and the IQ state are shared between slots: kernels of consecutive batches
     // serialise on iq_done, while this batch's H2D overlaps the previous batch's kernels/D2H
     CK(h, cudaStreamWaitEvent(sl.stream, h->iq_done, 0));
     h->last_nchunks = nchunks;
-    rc = launch_chain(h, sl.raw, nchunks, sl.out, sl.stream);
+    rc = launch_chain(h, h->sc, sl.raw, nchunks, sl.out, sl.stream);
     if (rc) return rc;
     CK(h, cudaEventRecord(h->iq_done, sl.stream));
     CK(h, cudaMemcpyAsync(out_host, sl.out, nchunks * (size_t)h->pl.R * h->pl.W * sizeof(double),
@@ -746,20 +802,19 @@ int sdrb_submit(sdrb_handle *h, int s, const void *raw_host, size_t nchunks, dou
 
 int sdrb_wait(sdrb_handle *h, int s)
 {
-    if (!h || s < 0 || s > 1) return fail(h, SDRB_ERR_ARG, "bad argument");
-    CK(h, cudaSetDevice(h->cfg.device));
+    if (int rc = entry(h, s == 0 || s == 1, EITHER)) return rc;
     CK(h, cudaStreamSynchronize(h->slot[s].stream));
     return SDRB_OK;
 }
 
 int sdrb_process(sdrb_handle *h, const void *raw, size_t nchunks, double *out)
 {
-    if (!h || (!raw && nchunks) || (!out && nchunks)) return fail(h, SDRB_ERR_ARG, "null argument");
-    if (h->seamless) return fail(h, SDRB_ERR_STATE, "seamless handle: use sdrb_stream / sdrb_stream_end");
+    // any number of chunks: the batches below each take at most max_chunks
+    int rc = entry(h, (raw && out) || !nchunks, CHUNK_LOCAL, std::min<size_t>(nchunks, 1), BATCH);
+    if (rc) return rc == NOTHING_TO_DO ? SDRB_OK : rc;
     const size_t cb = sdrb_chunk_bytes(h), W = (size_t)h->pl.W, R = (size_t)h->pl.R;
     if (nchunks <= h->max_chunks) {
-        if (nchunks == 0) return SDRB_OK;
-        int rc = sdrb_submit(h, 0, raw, nchunks, out);
+        rc = sdrb_submit(h, 0, raw, nchunks, out);
         if (rc) return rc;
         return sdrb_wait(h, 0);
     }
@@ -781,7 +836,7 @@ int sdrb_process(sdrb_handle *h, const void *raw, size_t nchunks, double *out)
     int b = 0;
     while (done < nchunks) {
         const int s = b & 1;
-        int rc = drain(s);
+        rc = drain(s);
         if (rc) return rc;
         const size_t n = std::min(h->max_chunks, nchunks - done);
         rc = sdrb_submit(h, s, static_cast<const uint8_t *>(raw) + done * cb, n, tmp[s].data());
@@ -790,7 +845,7 @@ int sdrb_process(sdrb_handle *h, const void *raw, size_t nchunks, double *out)
         done += n;
         b++;
     }
-    int rc = drain(b & 1);
+    rc = drain(b & 1);
     if (rc) return rc;
     return drain((b + 1) & 1);
 }
@@ -825,27 +880,24 @@ int seam_step(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, cudaS
     int rc = 0;
     if (nch) {
         const int s0 = h->nwin;
-        Scratch base = h->sc, sh = h->sc;
+        Scratch sh = h->sc;    // the window from slot s0 on
         sh.ypart += (size_t)s0 * R * pl.Mf;
         sh.agg += (size_t)s0 * R * nt * 16;
         sh.tile_agg += (size_t)s0 * nt;
         sh.off_tile += (size_t)s0 * (nt + 1);
         sh.gain += s0;
         sh.start += s0;
-        h->sc = sh;
-        rc = launch_chain(h, raw, nch, nullptr, st, PH_MAIN | PH_IQSCAN);
-        h->sc = base;
+        rc = launch_chain(h, sh, raw, nch, nullptr, st, PH_MAIN | PH_IQSCAN);
         if (rc) return rc;
         rc = with_enc(h, h->enc_code, [&](auto enc) {
-            k_seam_edges<decltype(enc)::value><<<(unsigned)nch, 64, 0, st>>>(pl, sd, raw, s0, (int)nch);
+            launch(h, k_seam_edges<decltype(enc)::value>, (unsigned)nch, 64, 0, st, pl, sd, raw, s0, (int)nch);
             return 0;
         });
         if (rc) return rc;
         const size_t items = nch * (size_t)R;
-        k_seam_agg<<<(unsigned)((items + 7) / 8), 256, 0, st>>>(pl, h->sc, sd, s0, (int)nch, h->seen);
-        if (h->seen == 0) k_seam_head<<<(unsigned)R, 32, 0, st>>>(pl, h->sc, sd, s0);
-        k_seam_fscan<<<(unsigned)R, 256, 0, st>>>(pl, sd, s0, (int)nch);
-        h->launches += 3 + (h->seen == 0);
+        launch(h, k_seam_agg, (unsigned)((items + 7) / 8), 256, 0, st, pl, h->sc, sd, s0, (int)nch, h->seen);
+        if (h->seen == 0) launch(h, k_seam_head, (unsigned)R, 32, 0, st, pl, h->sc, sd, s0);
+        launch(h, k_seam_fscan, (unsigned)R, 256, 0, st, pl, sd, s0, (int)nch);
         h->seen += (long long)nch;
         h->nwin += (int)nch;
     }
@@ -853,30 +905,23 @@ int seam_step(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, cudaS
     const int ne = (int)(upto - h->emitted);
     const long long g0 = h->emitted;
     if (ne > 0) {
-        if (end) {
-            k_seam_tail<<<(unsigned)R, 32, 0, st>>>(pl, h->sc, sd, h->nwin - 1, h->seen - 1);
-            h->launches++;
-        }
+        if (end) launch(h, k_seam_tail, (unsigned)R, 32, 0, st, pl, h->sc, sd, h->nwin - 1, h->seen - 1);
         const size_t items = (size_t)ne * R;
         const unsigned wg = (unsigned)((items + 7) / 8);
-        k_seam_carry<<<wg, 256, 0, st>>>(pl, h->sc, sd, ne, h->nwin, g0, end ? 1 : 0);
-        k_seam_y<<<wg, 256, 0, st>>>(pl, h->sc, sd, ne, h->nwin, g0, end ? 1 : 0);
-        const bool ssb = is_ssb(pl.demod);
-        if (ssb) k_seam_demod<true><<<wg, 256, 0, st>>>(pl, sd, out, ne, h->nwin, end ? 1 : 0);
-        else k_seam_demod<false><<<wg, 256, 0, st>>>(pl, sd, out, ne, h->nwin, end ? 1 : 0);
-        h->launches += 3;
-        if (pl.nsec_out) {
-            const size_t total = items * M;
-            const unsigned fg = (unsigned)std::min<size_t>((total + 255) / 256, (size_t)h->num_sms * 16);
-            if (ssb) {
-                k_seam_sscan<double2><<<(unsigned)R, 32, 0, st>>>(pl, sd, ne);
-                k_seam_frame<true><<<fg, 256, 0, st>>>(pl, sd, out, ne);
-            } else {
-                k_seam_sscan<double><<<(unsigned)R, 32, 0, st>>>(pl, sd, ne);
-                k_seam_frame<false><<<fg, 256, 0, st>>>(pl, sd, out, ne);
+        launch(h, k_seam_carry, wg, 256, 0, st, pl, h->sc, sd, ne, h->nwin, g0, end ? 1 : 0);
+        launch(h, k_seam_y, wg, 256, 0, st, pl, h->sc, sd, ne, h->nwin, g0, end ? 1 : 0);
+        with_out(pl.demod, [&](auto ok) {
+            // usb / lsb run the complex SOS state; real and iq rows the real one
+            constexpr bool SSB = decltype(ok)::value == OUT_SSB;
+            launch(h, k_seam_demod<SSB>, wg, 256, 0, st, pl, sd, out, ne, h->nwin, end ? 1 : 0);
+            if (pl.nsec_out) {
+                const size_t total = items * M;
+                const unsigned fg = (unsigned)std::min<size_t>((total + 255) / 256, (size_t)h->num_sms * 16);
+                launch(h, k_seam_sscan<std::conditional_t<SSB, double2, double>>, (unsigned)R, 32, 0, st, pl, sd, ne);
+                launch(h, k_seam_frame<SSB>, fg, 256, 0, st, pl, sd, out, ne);
             }
-            h->launches += 2;
-        }
+            return 0;
+        });
         CK(h, cudaGetLastError());
         // the chunks still held back move to the front of the window
         const int keep = h->nwin - ne;
@@ -907,12 +952,7 @@ int sdrb_stream_device(sdrb_handle *h, const void *raw_dev, size_t nchunks, doub
                        size_t *nchunks_out)
 {
     if (nchunks_out) *nchunks_out = 0;
-    if (!h || (!raw_dev && nchunks) || !out_dev) return fail(h, SDRB_ERR_ARG, "null argument");
-    if (!h->seamless) return fail(h, SDRB_ERR_STATE, "sdrb_stream needs a handle created with cfg.seamless");
-    if (nchunks > h->max_chunks) return fail(h, SDRB_ERR_ARG, "nchunks %zu > max_chunks %zu", nchunks, h->max_chunks);
-    if (h->pl.demod == SDRB_IQ && ((uintptr_t)out_dev & 15))
-        return fail(h, SDRB_ERR_ARG, "iq output is stored as 16-byte (Re, Im) pairs: `out` must be 16-byte aligned");
-    CK(h, cudaSetDevice(h->cfg.device));
+    if (int rc = entry(h, (raw_dev || !nchunks) && out_dev, SEAMLESS, nchunks, UPTO, out_dev)) return rc;
     return seam_step(h, static_cast<const uint8_t *>(raw_dev), nchunks, out_dev, static_cast<cudaStream_t>(stream), false,
                      nchunks_out);
 }
@@ -920,26 +960,17 @@ int sdrb_stream_device(sdrb_handle *h, const void *raw_dev, size_t nchunks, doub
 int sdrb_stream_end_device(sdrb_handle *h, double *out_dev, void *stream, size_t *nchunks_out)
 {
     if (nchunks_out) *nchunks_out = 0;
-    if (!h || !out_dev) return fail(h, SDRB_ERR_ARG, "null argument");
-    if (!h->seamless) return fail(h, SDRB_ERR_STATE, "sdrb_stream_end needs a handle created with cfg.seamless");
-    if (h->pl.demod == SDRB_IQ && ((uintptr_t)out_dev & 15))
-        return fail(h, SDRB_ERR_ARG, "iq output is stored as 16-byte (Re, Im) pairs: `out` must be 16-byte aligned");
-    CK(h, cudaSetDevice(h->cfg.device));
+    if (int rc = entry(h, out_dev, SEAMLESS, 0, UPTO, out_dev)) return rc;
     return seam_step(h, nullptr, 0, out_dev, static_cast<cudaStream_t>(stream), true, nchunks_out);
 }
 
 static int seam_host(sdrb_handle *h, const void *raw_host, size_t nchunks, double *out_host, size_t *nchunks_out, bool end)
 {
     if (nchunks_out) *nchunks_out = 0;
-    if (!h || (!raw_host && nchunks) || !out_host) return fail(h, SDRB_ERR_ARG, "null argument");
-    if (!h->seamless) return fail(h, SDRB_ERR_STATE, "sdrb_stream needs a handle created with cfg.seamless");
-    if (nchunks > h->max_chunks) return fail(h, SDRB_ERR_ARG, "nchunks %zu > max_chunks %zu", nchunks, h->max_chunks);
-    CK(h, cudaSetDevice(h->cfg.device));
-    int rc = ensure_slot(h, 0);
+    int rc = entry(h, (raw_host || !nchunks) && out_host, SEAMLESS, nchunks);
+    if (!rc) rc = stage_in(h, 0, raw_host, nchunks);
     if (rc) return rc;
     Slot &sl = h->slot[0];
-    if (nchunks)
-        CK(h, cudaMemcpyAsync(sl.raw, raw_host, nchunks * sdrb_chunk_bytes(h), cudaMemcpyHostToDevice, sl.stream));
     size_t ne = 0;
     rc = seam_step(h, sl.raw, nchunks, sl.out, sl.stream, end, &ne);
     if (rc) return rc;
@@ -981,10 +1012,9 @@ int sdrb_set_smooth(sdrb_handle *h, int window, int nhead, int ntail, int lo, co
     h->smooth_w = 0;
     if (window == 0) return SDRB_OK;
     const size_t n = (size_t)(nhead + 1 + ntail) * window;
-    double *dS = nullptr;
-    int rc = dalloc(h, n, &dS);
+    const double *dS = nullptr;
+    int rc = upload(h, tab, n, &dS);
     if (rc) return rc;
-    CK(h, cudaMemcpy(dS, tab, n * sizeof(double), cudaMemcpyHostToDevice));
     if (!h->smooth_tmp) {
         rc = dalloc(h, h->max_chunks * (size_t)h->pl.R * h->pl.M, &h->smooth_tmp);
         if (rc) return rc;
@@ -997,23 +1027,19 @@ int sdrb_set_smooth(sdrb_handle *h, int window, int nhead, int ntail, int lo, co
 
 int sdrb_iq_gain(sdrb_handle *h, const void *raw_host, size_t nchunks)
 {
-    if (!h || !raw_host) return fail(h, SDRB_ERR_ARG, "null argument");
-    if (h->seamless) return fail(h, SDRB_ERR_STATE, "seamless handle: the IQ state advances with sdrb_stream");
-    if (nchunks == 0 || !h->pl.correct_iq) return SDRB_OK;
-    if (nchunks > h->max_chunks) return fail(h, SDRB_ERR_ARG, "nchunks %zu > max_chunks %zu", nchunks, h->max_chunks);
-    CK(h, cudaSetDevice(h->cfg.device));
-    int rc = ensure_slot(h, 0);
-    if (rc) return rc;
+    // without the corrector there is no state to advance: a no-op, like zero chunks
+    int rc = entry(h, raw_host, CHUNK_LOCAL, h && h->pl.correct_iq ? nchunks : 0, BATCH);
+    if (rc) return rc == NOTHING_TO_DO ? SDRB_OK : rc;
+    if ((rc = stage_in(h, 0, raw_host, nchunks))) return rc;
     Slot &sl = h->slot[0];
-    CK(h, cudaMemcpyAsync(sl.raw, raw_host, nchunks * sdrb_chunk_bytes(h), cudaMemcpyHostToDevice, sl.stream));
     CK(h, cudaStreamWaitEvent(sl.stream, h->iq_done, 0));
     rc = with_enc(h, h->enc_code, [&](auto enc) {
-        k_iqchunk<decltype(enc)::value><<<(unsigned)((nchunks + 7) / 8), 256, 0, sl.stream>>>(h->pl, h->sc, sl.raw, (int)nchunks);
+        launch(h, k_iqchunk<decltype(enc)::value>, (unsigned)((nchunks + 7) / 8), 256, 0, sl.stream, h->pl, h->sc, sl.raw,
+               (int)nchunks);
         return 0;
     });
     if (rc) return rc;
-    k_iqscan_c<<<1, 1024, 0, sl.stream>>>(h->pl, h->sc, (int)nchunks);
-    h->launches += 2;
+    launch(h, k_iqscan_c, 1, 1024, 0, sl.stream, h->pl, h->sc, (int)nchunks);
     CK(h, cudaGetLastError());
     CK(h, cudaEventRecord(h->iq_done, sl.stream));
     CK(h, cudaStreamSynchronize(sl.stream));
@@ -1022,43 +1048,35 @@ int sdrb_iq_gain(sdrb_handle *h, const void *raw_host, size_t nchunks)
 
 int sdrb_process_device_phases(sdrb_handle *h, const void *raw_dev, size_t nchunks, double *out_dev, void *stream, int phases)
 {
-    if (!h || !raw_dev || (!out_dev && (phases & PH_FINISH))) return fail(h, SDRB_ERR_ARG, "null argument");
-    if (h->seamless) return fail(h, SDRB_ERR_STATE, "seamless handle: time-segment phases are not available");
-    if (nchunks == 0) return SDRB_OK;
-    if (nchunks > h->max_chunks) return fail(h, SDRB_ERR_ARG, "nchunks %zu > max_chunks %zu", nchunks, h->max_chunks);
-    CK(h, cudaSetDevice(h->cfg.device));
+    const bool finish = phases & PH_FINISH;
+    int rc = entry(h, raw_dev && (out_dev || !finish), CHUNK_LOCAL, nchunks, BATCH, finish ? out_dev : nullptr);
+    if (rc) return rc == NOTHING_TO_DO ? SDRB_OK : rc;
     h->last_nchunks = nchunks;
     if (phases & SDRB_PHASE_ZERO_IQ)
         CK(h, cudaMemsetAsync(h->sc.iq_state, 0, sizeof(double2), static_cast<cudaStream_t>(stream)));
-    return launch_chain(h, static_cast<const uint8_t *>(raw_dev), nchunks, out_dev, static_cast<cudaStream_t>(stream), phases & 7);
+    return launch_chain(h, h->sc, static_cast<const uint8_t *>(raw_dev), nchunks, out_dev, static_cast<cudaStream_t>(stream),
+                        phases & 7);
 }
 
 int sdrb_iq_export_device(sdrb_handle *h, double *dst3_dev, double nsamples, void *stream)
 {
-    if (!h || !dst3_dev) return fail(h, SDRB_ERR_ARG, "null argument");
-    if (h->seamless) return fail(h, SDRB_ERR_STATE, "seamless handle: time-segment phases are not available");
-    CK(h, cudaSetDevice(h->cfg.device));
-    k_iq_export<<<1, 32, 0, static_cast<cudaStream_t>(stream)>>>(h->sc, dst3_dev, nsamples);
-    h->launches++;
+    if (int rc = entry(h, dst3_dev, CHUNK_LOCAL)) return rc;
+    launch(h, k_iq_export, 1, 32, 0, static_cast<cudaStream_t>(stream), h->sc, dst3_dev, nsamples);
     CK(h, cudaGetLastError());
     return SDRB_OK;
 }
 
 int sdrb_iq_prefix_device(sdrb_handle *h, const double *gains3_dev, int rank, void *stream)
 {
-    if (!h || !gains3_dev || rank < 0) return fail(h, SDRB_ERR_ARG, "bad argument");
-    if (h->seamless) return fail(h, SDRB_ERR_STATE, "seamless handle: time-segment phases are not available");
-    CK(h, cudaSetDevice(h->cfg.device));
-    k_iq_prefix<<<1, 32, 0, static_cast<cudaStream_t>(stream)>>>(h->sc, gains3_dev, rank, h->pl.lam);
-    h->launches++;
+    if (int rc = entry(h, gains3_dev && rank >= 0, CHUNK_LOCAL)) return rc;
+    launch(h, k_iq_prefix, 1, 32, 0, static_cast<cudaStream_t>(stream), h->sc, gains3_dev, rank, h->pl.lam);
     CK(h, cudaGetLastError());
     return SDRB_OK;
 }
 
 int sdrb_set_profiling(sdrb_handle *h, int on)
 {
-    if (!h) return fail(h, SDRB_ERR_ARG, "null argument");
-    CK(h, cudaSetDevice(h->cfg.device));
+    if (int rc = entry(h, true, EITHER)) return rc;
     if (on) for (int i = 0; i < 5; i++) if (!h->pev[i]) CK(h, cudaEventCreate(&h->pev[i]));
     h->profiling = on != 0;
     return SDRB_OK;
@@ -1075,8 +1093,7 @@ int sdrb_kernel_times(sdrb_handle *h, float ms[4])
 
 int sdrb_get_iq_state(sdrb_handle *h, double off[2])
 {
-    if (!h || !off) return fail(h, SDRB_ERR_ARG, "null argument");
-    CK(h, cudaSetDevice(h->cfg.device));
+    if (int rc = entry(h, off, EITHER)) return rc;
     CK(h, cudaDeviceSynchronize());
     CK(h, cudaMemcpy(off, h->sc.iq_state, sizeof(double2), cudaMemcpyDeviceToHost));
     return SDRB_OK;
@@ -1084,8 +1101,7 @@ int sdrb_get_iq_state(sdrb_handle *h, double off[2])
 
 int sdrb_set_iq_state(sdrb_handle *h, const double off[2])
 {
-    if (!h || !off) return fail(h, SDRB_ERR_ARG, "null argument");
-    CK(h, cudaSetDevice(h->cfg.device));
+    if (int rc = entry(h, off, EITHER)) return rc;
     CK(h, cudaDeviceSynchronize());
     CK(h, cudaMemcpy(h->sc.iq_state, off, sizeof(double2), cudaMemcpyHostToDevice));
     return SDRB_OK;
@@ -1116,10 +1132,9 @@ int sdrb_keep_decimated(sdrb_handle *h, int on)
 
 int sdrb_read_decimated(sdrb_handle *h, size_t nchunks, double *y_host)
 {
-    if (!h || !y_host) return fail(h, SDRB_ERR_ARG, "null argument");
+    if (int rc = entry(h, y_host, EITHER)) return rc;
     if (h->finish_on && !h->keep_y) return fail(h, SDRB_ERR_STATE, "decimator output not kept: call sdrb_keep_decimated(h, 1) first");
     if (nchunks > h->last_nchunks) return fail(h, SDRB_ERR_STATE, "only %zu chunks in the last batch", h->last_nchunks);
-    CK(h, cudaSetDevice(h->cfg.device));
     CK(h, cudaDeviceSynchronize());
     CK(h, cudaMemcpy(y_host, h->sc.y, nchunks * (size_t)h->pl.R * h->pl.M * sizeof(double2), cudaMemcpyDeviceToHost));
     return SDRB_OK;
@@ -1134,6 +1149,13 @@ struct DevBuf {
     void *p = nullptr;
     ~DevBuf() { if (p) cudaFree(p); }
     cudaError_t alloc(size_t bytes) { return cudaMalloc(&p, bytes ? bytes : 1); }
+    // alloc + copy of n host elements; no elements leave the buffer null
+    template <typename T> cudaError_t upload(const T *src, size_t n)
+    {
+        if (n == 0) return cudaSuccess;
+        const cudaError_t e = alloc(n * sizeof(T));
+        return e != cudaSuccess ? e : cudaMemcpy(p, src, n * sizeof(T), cudaMemcpyHostToDevice);
+    }
     template <typename T> T *as() const { return static_cast<T *>(p); }
 };
 
@@ -1149,40 +1171,26 @@ struct FeedWorkspace {
     std::mutex mu;
     cudaError_t get(int device, int slot, size_t bytes, void **out)
     {
-        if (dev_cap[device][slot] < bytes) {
-            if (dev[device][slot]) cudaFree(dev[device][slot]);
-            dev[device][slot] = nullptr; dev_cap[device][slot] = 0;
-            cudaError_t e = cudaMalloc(&dev[device][slot], bytes);
-            if (e != cudaSuccess) return e;
-            dev_cap[device][slot] = bytes;
-        }
-        *out = dev[device][slot];
-        return cudaSuccess;
+        return grow(dev[device][slot], dev_cap[device][slot], bytes, false, out);
     }
     cudaError_t get_host(int device, int slot, size_t bytes, void **out)
     {
-        if (host_cap[device][slot] < bytes) {
-            if (host[device][slot]) cudaFreeHost(host[device][slot]);
-            host[device][slot] = nullptr; host_cap[device][slot] = 0;
-            cudaError_t e = cudaHostAlloc(&host[device][slot], bytes, cudaHostAllocDefault);
+        return grow(host[device][slot], host_cap[device][slot], bytes, true, out);
+    }
+    static cudaError_t grow(void *&buf, size_t &cap, size_t bytes, bool pinned, void **out)
+    {
+        if (cap < bytes) {
+            if (buf) pinned ? cudaFreeHost(buf) : cudaFree(buf);
+            buf = nullptr; cap = 0;
+            const cudaError_t e = pinned ? cudaHostAlloc(&buf, bytes, cudaHostAllocDefault) : cudaMalloc(&buf, bytes);
             if (e != cudaSuccess) return e;
-            host_cap[device][slot] = bytes;
+            cap = bytes;
         }
-        *out = host[device][slot];
+        *out = buf;
         return cudaSuccess;
     }
 };
 FeedWorkspace g_feed;
-
-int need_device(int device)
-{
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        return fail(nullptr, SDRB_ERR_CUDA, "no CUDA device: libsdrterm_b200 has no CPU fallback");
-    if (device < 0 || device >= ndev) return fail(nullptr, SDRB_ERR_ARG, "bad device ordinal");
-    CK(nullptr, cudaSetDevice(device));
-    return 0;
-}
 
 // scipy.signal.resample(r, M) of a real row of h samples as a dense [M][h] matrix (any h, any
 // M >= h): y[k] = sum_m W[k][m] r[m], W[k][m] = (1/h) (1 + 2 sum_{b=1}^{B} c_b cos(b theta)),
@@ -1210,6 +1218,50 @@ std::vector<double> resample_matrix(int h, int M)
         }
     return W;
 }
+
+// The host tables a k_demod operator reads through its plan (empty when unused).
+struct DemodTables {
+    std::vector<double2> tw, rot;    // twiddles; usb / lsb e^{j omega k}
+    std::vector<double> interp, ca;  // fm dense interpolation; usb / lsb c A^i
+};
+
+// One k_demod operator call on the default stream: `pl` holds the scalars, this uploads the tables
+// and the R rows of M decimator outputs (laid out [R][M], run as R rows of a single chunk) and
+// copies the R * pl.W output doubles back.
+int run_demod(DevPlan pl, const DemodTables &t, const double *y, double *out, int demod)
+{
+    const int R = pl.R, M = pl.M;
+    const size_t dsm = (size_t)M * (2 * sizeof(double2) + sizeof(double));
+    pl.demod_in_smem = dsm <= 48 * 1024;
+    DevBuf d_y, d_out, d_fft, d_z, d_tw, d_rot, d_w, d_ca;
+    CK(nullptr, d_y.upload(reinterpret_cast<const double2 *>(y), (size_t)R * M));
+    CK(nullptr, d_out.alloc((size_t)R * pl.W * sizeof(double)));
+    if (!pl.demod_in_smem) {
+        CK(nullptr, d_fft.alloc((size_t)R * 2 * M * sizeof(double2)));
+        CK(nullptr, d_z.alloc((size_t)R * M * sizeof(double)));
+    }
+    CK(nullptr, d_tw.upload(t.tw.data(), t.tw.size()));
+    CK(nullptr, d_rot.upload(t.rot.data(), t.rot.size()));
+    CK(nullptr, d_w.upload(t.interp.data(), t.interp.size()));
+    CK(nullptr, d_ca.upload(t.ca.data(), t.ca.size()));
+    pl.tw = d_tw.as<double2>();
+    pl.ssb_rot = d_rot.as<double2>();
+    pl.fm_interp = d_w.as<double>();
+    pl.sos_CA = d_ca.as<double>();
+    with_out(demod, [&](auto ok) {
+        constexpr int OK = decltype(ok)::value;
+        if constexpr (OK == OUT_IQ)
+            k_demod<OK><<<R, 128, 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), nullptr, nullptr, 1, demod, 0, 0);
+        else
+            k_demod<OK><<<R, 128, pl.demod_in_smem ? dsm : 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), d_fft.as<double2>(),
+                                                               d_z.as<double>(), 1, demod, OK == OUT_SSB, 0);
+        return 0;
+    });
+    CK(nullptr, cudaGetLastError());
+    CK(nullptr, cudaDeviceSynchronize());
+    CK(nullptr, cudaMemcpy(out, d_out.p, (size_t)R * pl.W * sizeof(double), cudaMemcpyDeviceToHost));
+    return SDRB_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -1227,37 +1279,11 @@ static int demod_op(int device, const double *y, int R, int M, double *out, int 
     pl.fft_n = pl.fft_ok ? M : 0;
     if (demod == SDRB_FM && (M & 1))
         return fail(nullptr, SDRB_ERR_ARG, "fmDemod pairs samples: the row length must be even (got %d)", M);
-    std::vector<double2> tw = make_twiddles(pl.fft_n);
-    DevBuf d_tw, d_y, d_out, d_fft, d_z, d_w;
-    const size_t dsm = (size_t)M * (2 * sizeof(double2) + sizeof(double));
-    pl.demod_in_smem = dsm <= 48 * 1024;
-    CK(nullptr, d_tw.alloc(tw.size() * sizeof(double2)));
-    CK(nullptr, d_y.alloc((size_t)R * M * sizeof(double2)));
-    CK(nullptr, d_out.alloc((size_t)R * pl.W * sizeof(double)));
-    if (!pl.demod_in_smem) {
-        CK(nullptr, d_fft.alloc((size_t)R * 2 * M * sizeof(double2)));
-        CK(nullptr, d_z.alloc((size_t)R * M * sizeof(double)));
-    }
-    if (demod == SDRB_FM && !pl.fft_ok) {
-        // any even length: the same dense interpolation the engine uses for non-FFT sizes
-        const std::vector<double> W = resample_matrix(h2, M);
-        CK(nullptr, d_w.alloc(W.size() * sizeof(double)));
-        CK(nullptr, cudaMemcpy(d_w.p, W.data(), W.size() * sizeof(double), cudaMemcpyHostToDevice));
-        pl.fm_interp = d_w.as<double>();
-    }
-    CK(nullptr, cudaMemcpy(d_tw.p, tw.data(), tw.size() * sizeof(double2), cudaMemcpyHostToDevice));
-    CK(nullptr, cudaMemcpy(d_y.p, y, (size_t)R * M * sizeof(double2), cudaMemcpyHostToDevice));
-    pl.tw = d_tw.as<double2>();
-    // rows are laid out [R][M]: run as R "rows" of a single chunk
-    if (demod == SDRB_IQ)
-        k_demod<OUT_IQ><<<R, 128, 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), nullptr, nullptr, 1, demod, 0, 0);
-    else
-        k_demod<OUT_REAL><<<R, 128, pl.demod_in_smem ? dsm : 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), d_fft.as<double2>(),
-                                                                  d_z.as<double>(), 1, demod, 0, 0);
-    CK(nullptr, cudaGetLastError());
-    CK(nullptr, cudaDeviceSynchronize());
-    CK(nullptr, cudaMemcpy(out, d_out.p, (size_t)R * pl.W * sizeof(double), cudaMemcpyDeviceToHost));
-    return SDRB_OK;
+    DemodTables t;
+    t.tw = make_twiddles(pl.fft_n);
+    // any even length: the same dense interpolation the engine uses for non-FFT sizes
+    if (demod == SDRB_FM && !pl.fft_ok) t.interp = resample_matrix(h2, M);
+    return run_demod(pl, t, y, out, demod);
 }
 
 int sdrb_fm_demod(int device, const double *y, int R, int M, double *out) { return demod_op(device, y, R, M, out, SDRB_FM); }
@@ -1321,34 +1347,14 @@ int sdrb_ssb_demod(int device, const double *y, int R, int M, const double *sos,
                 for (int k = 0; k < ns; k++) PP[(size_t)a * ns + b] += P[(size_t)a * ns + k] * P[(size_t)k * ns + b];
         P = PP;
     }
-    std::vector<double2> rot((size_t)M + 1);
+    DemodTables t;
+    t.ca = std::move(ca);
+    t.rot.resize((size_t)M + 1);
     for (int k = 0; k <= M; k++) {
         const long double a = (long double)omega * (long double)k;
-        rot[k] = make_double2((double)cosl(a), (double)sinl(a));
+        t.rot[k] = make_double2((double)cosl(a), (double)sinl(a));
     }
-    DevBuf d_y, d_out, d_fft, d_z, d_ca, d_rot;
-    const size_t dsm = (size_t)M * (2 * sizeof(double2) + sizeof(double));
-    pl.demod_in_smem = dsm <= 48 * 1024;
-    CK(nullptr, d_y.alloc((size_t)R * M * sizeof(double2)));
-    CK(nullptr, d_out.alloc((size_t)R * M * sizeof(double)));
-    CK(nullptr, d_ca.alloc(ca.size() * sizeof(double)));
-    CK(nullptr, d_rot.alloc(rot.size() * sizeof(double2)));
-    if (!pl.demod_in_smem) {
-        CK(nullptr, d_fft.alloc((size_t)R * 2 * M * sizeof(double2)));
-        CK(nullptr, d_z.alloc((size_t)R * M * sizeof(double)));
-    }
-    CK(nullptr, cudaMemcpy(d_y.p, y, (size_t)R * M * sizeof(double2), cudaMemcpyHostToDevice));
-    CK(nullptr, cudaMemcpy(d_ca.p, ca.data(), ca.size() * sizeof(double), cudaMemcpyHostToDevice));
-    CK(nullptr, cudaMemcpy(d_rot.p, rot.data(), rot.size() * sizeof(double2), cudaMemcpyHostToDevice));
-    pl.sos_CA = d_ca.as<double>();
-    pl.ssb_rot = d_rot.as<double2>();
-    // rows are laid out [R][M]: run as R "rows" of a single chunk
-    k_demod<OUT_SSB><<<R, 128, pl.demod_in_smem ? dsm : 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), d_fft.as<double2>(),
-                                                             d_z.as<double>(), 1, SDRB_USB, 1, 0);
-    CK(nullptr, cudaGetLastError());
-    CK(nullptr, cudaDeviceSynchronize());
-    CK(nullptr, cudaMemcpy(out, d_out.p, (size_t)R * M * sizeof(double), cudaMemcpyDeviceToHost));
-    return SDRB_OK;
+    return run_demod(pl, t, y, out, SDRB_USB);
 }
 
 int sdrb_shift_freq(int device, const double *y, const double *shift, int R, int N, double *res)
@@ -1357,11 +1363,9 @@ int sdrb_shift_freq(int device, const double *y, const double *shift, int R, int
     int rc = need_device(device);
     if (rc) return rc;
     DevBuf d_y, d_s, d_r;
-    CK(nullptr, d_y.alloc((size_t)N * sizeof(double2)));
-    CK(nullptr, d_s.alloc((size_t)R * N * sizeof(double2)));
+    CK(nullptr, d_y.upload(reinterpret_cast<const double2 *>(y), (size_t)N));
+    CK(nullptr, d_s.upload(reinterpret_cast<const double2 *>(shift), (size_t)R * N));
     CK(nullptr, d_r.alloc((size_t)R * N * sizeof(double2)));
-    CK(nullptr, cudaMemcpy(d_y.p, y, (size_t)N * sizeof(double2), cudaMemcpyHostToDevice));
-    CK(nullptr, cudaMemcpy(d_s.p, shift, (size_t)R * N * sizeof(double2), cudaMemcpyHostToDevice));
     k_shift<<<148 * 4, 256>>>(d_y.as<double2>(), d_s.as<double2>(), d_r.as<double2>(), R, N);
     CK(nullptr, cudaGetLastError());
     CK(nullptr, cudaDeviceSynchronize());
@@ -1468,9 +1472,8 @@ int sdrb_decode_iq(int device, const void *raw, size_t nsamples, char enc, int s
     if (rc) return rc;
     const size_t nbytes = nsamples * 2 * (size_t)itemsize_of(code);
     DevBuf d_raw, d_z;
-    CK(nullptr, d_raw.alloc(nbytes));
+    CK(nullptr, d_raw.upload(static_cast<const uint8_t *>(raw), nbytes));
     CK(nullptr, d_z.alloc(nsamples * sizeof(double2)));
-    CK(nullptr, cudaMemcpy(d_raw.p, raw, nbytes, cudaMemcpyHostToDevice));
     const unsigned grid = (unsigned)std::min<size_t>((nsamples + 255) / 256, 148 * 8);
     const uint8_t *r8 = d_raw.as<uint8_t>();
     double2 *z = d_z.as<double2>();
@@ -1493,10 +1496,8 @@ int sdrb_correct_iq(int device, double *z_inout, size_t nsamples, double off_ino
     int rc = need_device(device);
     if (rc) return rc;
     DevBuf d_z, d_off;
-    CK(nullptr, d_z.alloc(nsamples * sizeof(double2)));
-    CK(nullptr, d_off.alloc(sizeof(double2)));
-    CK(nullptr, cudaMemcpy(d_z.p, z_inout, nsamples * sizeof(double2), cudaMemcpyHostToDevice));
-    CK(nullptr, cudaMemcpy(d_off.p, off_inout, sizeof(double2), cudaMemcpyHostToDevice));
+    CK(nullptr, d_z.upload(reinterpret_cast<const double2 *>(z_inout), nsamples));
+    CK(nullptr, d_off.upload(reinterpret_cast<const double2 *>(off_inout), 1));
     k_correct_iq<<<1, 1024>>>(d_z.as<double2>(), nsamples, d_off.as<double2>(), L);
     CK(nullptr, cudaGetLastError());
     CK(nullptr, cudaDeviceSynchronize());
@@ -1520,9 +1521,8 @@ int sdrb_host_free(void *ptr)
 
 int sdrb_keep_x0(sdrb_handle *h, int on)
 {
-    if (!h) return fail(h, SDRB_ERR_ARG, "null argument");
+    if (int rc = entry(h, true, EITHER)) return rc;
     if (!h->tc_on) return fail(h, SDRB_ERR_STATE, "block first samples exist only on the tensor-core front end");
-    CK(h, cudaSetDevice(h->cfg.device));
     CK(h, cudaDeviceSynchronize());
     if (on && !h->x0_buf) {
         int rc = dalloc(h, h->max_chunks * (size_t)h->pl.R * h->pl.Mf, &h->x0_buf);
@@ -1534,10 +1534,9 @@ int sdrb_keep_x0(sdrb_handle *h, int on)
 
 int sdrb_read_x0(sdrb_handle *h, size_t nchunks, double *x0_host)
 {
-    if (!h || !x0_host) return fail(h, SDRB_ERR_ARG, "null argument");
+    if (int rc = entry(h, x0_host, EITHER)) return rc;
     if (!h->sc.x0) return fail(h, SDRB_ERR_STATE, "block first samples not kept: call sdrb_keep_x0(h, 1) first");
     if (nchunks > h->last_nchunks) return fail(h, SDRB_ERR_STATE, "only %zu chunks in the last batch", h->last_nchunks);
-    CK(h, cudaSetDevice(h->cfg.device));
     CK(h, cudaDeviceSynchronize());
     CK(h, cudaMemcpy(x0_host, h->sc.x0, nchunks * (size_t)h->pl.R * h->pl.Mf * sizeof(double2), cudaMemcpyDeviceToHost));
     return SDRB_OK;

@@ -59,6 +59,24 @@ def test_no_cpu_fallback():
         dem.amDemod(np.zeros((1, 8), dtype=np.complex128), np.zeros((1, 8)))
 
 
+def test_create_refuses_inconsistent_plans_before_touching_the_device():
+    """sdrb_create checks the whole configuration on the host before any CUDA call: an inconsistent
+    plan is refused with SDRB_ERR_ARG naming the problem, with or without a CUDA device."""
+    import dataclasses
+    from sdrterm_b200.engine import Engine
+    from sdrterm_b200.plan import build_plan
+    kw = dict(correct_iq=True, demod='fm', omega_out=5000)
+    fm = build_plan(1_024_000, 'h', 64, [15000], **kw)
+    fm_d50 = build_plan(1_024_000, 'h', 50, [15000], **kw)        # M = 656: FM needs the dense interpolation
+    seamless = build_plan(1_024_000, 'h', 64, [15000], seamless=True, **kw)
+    assert fm_d50.fm_interp is not None and seamless.lookahead >= 1
+    for pl, problem in ((dataclasses.replace(fm, RL=fm.RL + 1), 'RL'),
+                        (dataclasses.replace(fm_d50, fm_interp=None), 'dense interpolation table'),
+                        (dataclasses.replace(seamless, lookahead=0), 'lookahead')):
+        with pytest.raises(nat.SdrbError, match=f'error -1: .*{problem}'):
+            Engine(pl, max_chunks=1, use_tc=False)
+
+
 def test_product_code_never_imports_the_oracle():
     for dirpath, _, files in os.walk(os.path.join(ROOT, 'sdrterm_b200')):
         for f in files:

@@ -145,21 +145,135 @@ def test_seamless_short_and_empty_streams():
         assert rel_err(out2, ref2) < TOL
 
 
+OK, ARG, STATE = 0, -1, -4     # SDRB_OK, SDRB_ERR_ARG, SDRB_ERR_STATE
+MAXC = 2                       # max_chunks of the handles below
+# Misuse of every handle entry point, called through the C ABI on a chunk-local handle and on a
+# seamless one: (case, demod, call, code on the chunk-local handle, code on the seamless handle).
+# `call(L, h, b)` gets the library, the handle and the buffers of _misuse_buffers; fm handles run
+# the IQ corrector, iq handles do not.  Zero chunks: sdrb_submit refuses them, the other
+# chunk-local calls are a successful no-op, the stream calls run.
+MISUSE = [
+    # null pointers (a null handle is refused first, whatever the call)
+    ('process_device null handle', 'fm', lambda L, h, b: L.sdrb_process_device(None, b.raw_d, 1, b.out_d, None), ARG, ARG),
+    ('process_device null raw', 'fm', lambda L, h, b: L.sdrb_process_device(h, None, 1, b.out_d, None), ARG, ARG),
+    ('process_device null out', 'fm', lambda L, h, b: L.sdrb_process_device(h, b.raw_d, 1, None, None), ARG, ARG),
+    ('submit null handle', 'fm', lambda L, h, b: L.sdrb_submit(None, 0, b.raw_h, 1, b.out_h), ARG, ARG),
+    ('submit null raw', 'fm', lambda L, h, b: L.sdrb_submit(h, 0, None, 1, b.out_h), ARG, ARG),
+    ('submit null out', 'fm', lambda L, h, b: L.sdrb_submit(h, 0, b.raw_h, 1, None), ARG, ARG),
+    ('process null handle', 'fm', lambda L, h, b: L.sdrb_process(None, b.raw_h, 1, b.out_h), ARG, ARG),
+    ('process null raw', 'fm', lambda L, h, b: L.sdrb_process(h, None, 1, b.out_h), ARG, ARG),
+    ('process null out', 'fm', lambda L, h, b: L.sdrb_process(h, b.raw_h, 1, None), ARG, ARG),
+    ('process null buffers 0 chunks', 'fm', lambda L, h, b: L.sdrb_process(h, None, 0, None), OK, STATE),
+    ('stream_device null handle', 'fm', lambda L, h, b: L.sdrb_stream_device(None, b.raw_d, 1, b.out_d, None, b.got), ARG, ARG),
+    ('stream_device null raw', 'fm', lambda L, h, b: L.sdrb_stream_device(h, None, 1, b.out_d, None, b.got), ARG, ARG),
+    ('stream_device null raw 0 chunks', 'fm', lambda L, h, b: L.sdrb_stream_device(h, None, 0, b.out_d, None, b.got), STATE, OK),
+    ('stream_device null out', 'fm', lambda L, h, b: L.sdrb_stream_device(h, b.raw_d, 1, None, None, b.got), ARG, ARG),
+    ('stream_end_device null handle', 'fm', lambda L, h, b: L.sdrb_stream_end_device(None, b.out_d, None, b.got), ARG, ARG),
+    ('stream_end_device null out', 'fm', lambda L, h, b: L.sdrb_stream_end_device(h, None, None, b.got), ARG, ARG),
+    ('stream null handle', 'fm', lambda L, h, b: L.sdrb_stream(None, b.raw_h, 1, b.out_h, b.got), ARG, ARG),
+    ('stream null raw', 'fm', lambda L, h, b: L.sdrb_stream(h, None, 1, b.out_h, b.got), ARG, ARG),
+    ('stream null out', 'fm', lambda L, h, b: L.sdrb_stream(h, b.raw_h, 1, None, b.got), ARG, ARG),
+    ('stream_end null handle', 'fm', lambda L, h, b: L.sdrb_stream_end(None, b.out_h, b.got), ARG, ARG),
+    ('stream_end null out', 'fm', lambda L, h, b: L.sdrb_stream_end(h, None, b.got), ARG, ARG),
+    ('iq_gain null handle', 'fm', lambda L, h, b: L.sdrb_iq_gain(None, b.raw_h, 1), ARG, ARG),
+    ('iq_gain null raw', 'fm', lambda L, h, b: L.sdrb_iq_gain(h, None, 1), ARG, ARG),
+    ('phases null handle', 'fm', lambda L, h, b: L.sdrb_process_device_phases(None, b.raw_d, 1, b.out_d, None, 7), ARG, ARG),
+    ('phases null raw', 'fm', lambda L, h, b: L.sdrb_process_device_phases(h, None, 1, b.out_d, None, 7), ARG, ARG),
+    ('phases null out with finish', 'fm', lambda L, h, b: L.sdrb_process_device_phases(h, b.raw_d, 1, None, None, 7), ARG, ARG),
+    ('phases null out without finish', 'fm', lambda L, h, b: L.sdrb_process_device_phases(h, b.raw_d, 1, None, None, 3), OK, STATE),
+    ('iq_export null handle', 'fm', lambda L, h, b: L.sdrb_iq_export_device(None, b.g3_d, 1.0, None), ARG, ARG),
+    ('iq_export null dst', 'fm', lambda L, h, b: L.sdrb_iq_export_device(h, None, 1.0, None), ARG, ARG),
+    ('iq_prefix null handle', 'fm', lambda L, h, b: L.sdrb_iq_prefix_device(None, b.g3_d, 0, None), ARG, ARG),
+    ('iq_prefix null gains', 'fm', lambda L, h, b: L.sdrb_iq_prefix_device(h, None, 0, None), ARG, ARG),
+    ('iq_prefix rank -1', 'fm', lambda L, h, b: L.sdrb_iq_prefix_device(h, b.g3_d, -1, None), ARG, ARG),
+    # zero chunks
+    ('process_device 0 chunks', 'fm', lambda L, h, b: L.sdrb_process_device(h, b.raw_d, 0, b.out_d, None), OK, STATE),
+    ('submit 0 chunks', 'fm', lambda L, h, b: L.sdrb_submit(h, 0, b.raw_h, 0, b.out_h), ARG, STATE),
+    ('process 0 chunks', 'fm', lambda L, h, b: L.sdrb_process(h, b.raw_h, 0, b.out_h), OK, STATE),
+    ('stream_device 0 chunks', 'fm', lambda L, h, b: L.sdrb_stream_device(h, b.raw_d, 0, b.out_d, None, b.got), STATE, OK),
+    ('stream 0 chunks', 'fm', lambda L, h, b: L.sdrb_stream(h, b.raw_h, 0, b.out_h, b.got), STATE, OK),
+    ('iq_gain 0 chunks', 'fm', lambda L, h, b: L.sdrb_iq_gain(h, b.raw_h, 0), OK, STATE),
+    ('phases 0 chunks', 'fm', lambda L, h, b: L.sdrb_process_device_phases(h, b.raw_d, 0, b.out_d, None, 7), OK, STATE),
+    # max_chunks + 1 (sdrb_process takes any number: it runs them in batches)
+    ('process_device max+1', 'fm', lambda L, h, b: L.sdrb_process_device(h, b.raw_d, MAXC + 1, b.out_d, None), ARG, STATE),
+    ('submit max+1', 'fm', lambda L, h, b: L.sdrb_submit(h, 0, b.raw_h, MAXC + 1, b.out_h), ARG, STATE),
+    ('process max+1', 'fm', lambda L, h, b: L.sdrb_process(h, b.raw_h, MAXC + 1, b.out_h), OK, STATE),
+    ('stream_device max+1', 'fm', lambda L, h, b: L.sdrb_stream_device(h, b.raw_d, MAXC + 1, b.out_d, None, b.got), STATE, ARG),
+    ('stream max+1', 'fm', lambda L, h, b: L.sdrb_stream(h, b.raw_h, MAXC + 1, b.out_h, b.got), STATE, ARG),
+    ('iq_gain max+1', 'fm', lambda L, h, b: L.sdrb_iq_gain(h, b.raw_h, MAXC + 1), ARG, STATE),
+    ('iq_gain max+1 without corrector', 'iq', lambda L, h, b: L.sdrb_iq_gain(h, b.raw_h, MAXC + 1), OK, STATE),
+    ('phases max+1', 'fm', lambda L, h, b: L.sdrb_process_device_phases(h, b.raw_d, MAXC + 1, b.out_d, None, 7), ARG, STATE),
+    # the wrong kind of handle for a valid call
+    ('process_device', 'fm', lambda L, h, b: L.sdrb_process_device(h, b.raw_d, 1, b.out_d, None), OK, STATE),
+    ('submit + wait', 'fm', lambda L, h, b: L.sdrb_submit(h, 1, b.raw_h, 1, b.out_h) or L.sdrb_wait(h, 1), OK, STATE),
+    ('process', 'fm', lambda L, h, b: L.sdrb_process(h, b.raw_h, 1, b.out_h), OK, STATE),
+    ('stream_device', 'fm', lambda L, h, b: L.sdrb_stream_device(h, b.raw_d, 1, b.out_d, None, b.got), STATE, OK),
+    ('stream_end_device', 'fm', lambda L, h, b: L.sdrb_stream_end_device(h, b.out_d, None, b.got), STATE, OK),
+    ('stream', 'fm', lambda L, h, b: L.sdrb_stream(h, b.raw_h, 1, b.out_h, b.got), STATE, OK),
+    ('stream_end', 'fm', lambda L, h, b: L.sdrb_stream_end(h, b.out_h, b.got), STATE, OK),
+    ('iq_gain', 'fm', lambda L, h, b: L.sdrb_iq_gain(h, b.raw_h, 1), OK, STATE),
+    ('phases', 'fm', lambda L, h, b: L.sdrb_process_device_phases(h, b.raw_d, 1, b.out_d, None, 7), OK, STATE),
+    ('iq_export', 'fm', lambda L, h, b: L.sdrb_iq_export_device(h, b.g3_d, 1.0, None), OK, STATE),
+    ('iq_prefix', 'fm', lambda L, h, b: L.sdrb_iq_prefix_device(h, b.g3_d, 0, None), OK, STATE),
+    ('set_smooth', 'fm', lambda L, h, b: L.sdrb_set_smooth(h, 5, 2, 2, -2, b.smooth), OK, ARG),
+    # slots
+    ('submit slot -1', 'fm', lambda L, h, b: L.sdrb_submit(h, -1, b.raw_h, 1, b.out_h), ARG, ARG),
+    ('submit slot 2', 'fm', lambda L, h, b: L.sdrb_submit(h, 2, b.raw_h, 1, b.out_h), ARG, ARG),
+    ('wait slot -1', 'fm', lambda L, h, b: L.sdrb_wait(h, -1), ARG, ARG),
+    ('wait slot 2', 'fm', lambda L, h, b: L.sdrb_wait(h, 2), ARG, ARG),
+    # device outputs 8 bytes off: iq stores 16-byte (Re, Im) pairs, real rows 8-byte doubles
+    ('process_device out+8 iq', 'iq', lambda L, h, b: L.sdrb_process_device(h, b.raw_d, 1, b.out_d + 8, None), ARG, STATE),
+    ('process_device out+8 fm', 'fm', lambda L, h, b: L.sdrb_process_device(h, b.raw_d, 1, b.out_d + 8, None), OK, STATE),
+    ('phases out+8 iq', 'iq', lambda L, h, b: L.sdrb_process_device_phases(h, b.raw_d, 1, b.out_d + 8, None, 7), ARG, STATE),
+    ('phases out+8 iq without finish', 'iq',
+     lambda L, h, b: L.sdrb_process_device_phases(h, b.raw_d, 1, b.out_d + 8, None, 3), OK, STATE),
+    ('stream_device out+8 iq', 'iq', lambda L, h, b: L.sdrb_stream_device(h, b.raw_d, 1, b.out_d + 8, None, b.got), STATE, ARG),
+    ('stream_device out+8 fm', 'fm', lambda L, h, b: L.sdrb_stream_device(h, b.raw_d, 1, b.out_d + 8, None, b.got), STATE, OK),
+    ('stream_end_device out+8 iq', 'iq', lambda L, h, b: L.sdrb_stream_end_device(h, b.out_d + 8, None, b.got), STATE, ARG),
+]
+
+
+def _misuse_buffers(kw, eng):
+    import ctypes as C
+    import torch
+    from types import SimpleNamespace
+    nout = (MAXC + 1 + eng.lookahead + 2) * eng.R * eng.W       # rows of any call above, plus slack for +8
+    raw = np.frombuffer(_body(kw, MAXC + 1, 1), dtype=np.uint8).copy()
+    b = SimpleNamespace(raw=raw, raw_dt=torch.from_numpy(raw).cuda(), out_dt=torch.zeros(nout, dtype=torch.float64, device='cuda'),
+                        g3=torch.zeros(6, dtype=torch.float64, device='cuda'), out=np.zeros(nout), sm=np.zeros(25),
+                        got=C.pointer(C.c_size_t(0)))
+    b.raw_h, b.out_h, b.smooth = b.raw.ctypes.data, b.out.ctypes.data, b.sm.ctypes.data
+    b.raw_d, b.out_d, b.g3_d = b.raw_dt.data_ptr(), b.out_dt.data_ptr(), b.g3.data_ptr()
+    return b
+
+
 @pytest.mark.gpu
-def test_seamless_refuses_chunk_local_entry_points():
+def test_entry_points_refuse_misuse():
+    """Every handle entry point returns the same code for the same misuse, on both kinds of handle."""
+    import torch
     from sdrterm_b200 import _native as nat
     from sdrterm_b200.engine import Engine
-    kw = _kw('h', 64, 'fm', True, 15000)
-    pl = _plan(kw)
-    with Engine(pl, max_chunks=2) as eng:
-        with pytest.raises(nat.SdrbError):
-            eng.process(_body(kw, 1, 1))
-        with pytest.raises(ValueError):
-            eng.set_smooth(5)
-        rc = nat.lib().sdrb_set_smooth(eng._h, 5, 2, 2, -2, np.zeros(25).ctypes.data)
-        assert rc == -1
-        rc = nat.lib().sdrb_iq_gain(eng._h, _body(kw, 1, 1), 1)
-        assert rc == -4
+    L = nat.lib()
+    got = []
+    for demod, iq in (('fm', True), ('iq', False)):
+        kw = _kw('h', 64, demod, iq, 15000)
+        for col in (3, 4):
+            pl = build_plan(kw['fs'], 'h', 64, [15000], correct_iq=iq, demod=demod, omega_out=5000, seamless=col == 4)
+            with Engine(pl, max_chunks=MAXC) as eng:
+                b = _misuse_buffers(kw, eng)
+                for case in MISUSE:
+                    if case[1] == demod:
+                        rc = case[2](L, eng._h, b)
+                        torch.cuda.synchronize()
+                        got.append((case[0], 'seamless' if col == 4 else 'chunk-local', rc, case[col]))
+                if col == 4:
+                    with pytest.raises(nat.SdrbError):
+                        eng.process(_body(kw, 1, 1))
+                    with pytest.raises(ValueError):
+                        eng.set_smooth(5)
+    bad = [g for g in got if g[2] != g[3]]
+    assert not bad, bad
+    assert len(got) == 2 * len(MISUSE)
 
 
 def _edge_error(out, ref, M, halfwidth=8):
