@@ -181,13 +181,17 @@ inline double2 c2(const double *a, size_t i) { return make_double2(a[2 * i], a[2
 inline double2 hmul(double2 a, double2 b) { return make_double2(a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x); }
 
 bool is_pow2(int v) { return v > 0 && (v & (v - 1)) == 0; }
+// FM interpolates a row of M = 2h outputs by the packed FFT when h is a power of two >= 2 (the
+// transform has h/2 points), by the dense resample matrix otherwise.
+int fft_ok(int M) { return M % 2 == 0 && M >= 4 && is_pow2(M / 2) ? 1 : 0; }
 
-std::vector<double2> make_twiddles(int n)
+// The FFT's half table exp(-2 pi i k / M), k < M/2 (sdrb_fft.cuh); one unused entry for M = 0.
+std::vector<double2> make_twiddles(int M)
 {
-    std::vector<double2> tw(n > 0 ? n : 1);
+    std::vector<double2> tw(std::max(1, M / 2));
     const long double two_pi = 6.283185307179586476925286766559005768L;
-    for (int k = 0; k < n; k++) {
-        long double a = -two_pi * (long double)k / (long double)n;
+    for (int k = 0; k < M / 2; k++) {
+        long double a = -two_pi * (long double)k / (long double)M;
         tw[k] = make_double2((double)cosl(a), (double)sinl(a));
     }
     return tw;
@@ -342,10 +346,9 @@ int launch_chain_t(sdrb_handle *h, const Scratch &sc, const uint8_t *raw, size_t
         with_out(pl.demod, [&](auto ok) {
             constexpr int OK = decltype(ok)::value;
             if constexpr (OK == OUT_IQ)
-                launch(h, k_demod<OK>, rows, 128, 0, st, pl, sc.y, out, nullptr, nullptr, (int)nch, pl.demod, 0, pl.be_out);
+                launch(h, k_demod<OK>, rows, 128, 0, st, pl, sc.y, out, nullptr, (int)nch, pl.demod, 0, pl.be_out);
             else
-                launch(h, k_demod<OK>, rows, 128, h->demod_smem, st, pl, sc.y, out, sc.fftbuf, sc.zrow, (int)nch, pl.demod, 1,
-                       pl.be_out);
+                launch(h, k_demod<OK>, rows, 128, h->demod_smem, st, pl, sc.y, out, sc.fftbuf, (int)nch, pl.demod, 1, pl.be_out);
             return 0;
         });
         mark(4);
@@ -422,9 +425,7 @@ DevPlan plan_of(const sdrb_config *cfg, const sdrb_tables *tab)
     for (int i = 0; i < SDRB_NP * SDRB_NP; i++) pl.xi[i] = c2(tab->xi, i);
     for (int i = 0; i < 6 * cfg->n_out_sections; i++) pl.out_sos[i] = tab->out_sos[i];
     for (int i = 0; i < 33; i++) { pl.lam_pw[i] = tab->lam_k[i]; pl.mu_pw[i] = tab->mu_k[i]; }
-    const int h2 = pl.M >> 1;
-    pl.fft_ok = (pl.M == 2 * h2) && is_pow2(h2) ? 1 : 0;
-    pl.fft_n = pl.fft_ok ? pl.M : 0;
+    pl.fft_ok = fft_ok(pl.M);
     return pl;
 }
 
@@ -558,7 +559,7 @@ int plan_tables(sdrb_handle *h, const sdrb_tables *tab)
             rb[(size_t)r * 8 + i] = hmul(pl.rho[i], b); rbT[(size_t)r * 8 + i] = hmul(pl.rho_p[i], bT);
         }
     }
-    const std::vector<double2> tw = make_twiddles(pl.fft_n);
+    const std::vector<double2> tw = make_twiddles(pl.fft_ok ? M : 0);
     auto d2 = [](const double *a) { return reinterpret_cast<const double2 *>(a); };
     int rc;
     if ((rc = upload(h, afrag.data(), afrag.size(), &pl.Afrag)) ||
@@ -609,7 +610,7 @@ int set_geometry(sdrb_handle *h)
                    (pl.nsec_out == 0 || pl.nsec_out == 2);
     h->finish_smem = h->finish_on ? finish_smem_bytes(M, pl.edge) : 0;
     if (h->finish_smem > 227 * 1024) h->finish_on = false;
-    const size_t dsm = (size_t)M * (2 * sizeof(double2) + sizeof(double));
+    const size_t dsm = demod_smem_bytes(M);
     pl.demod_in_smem = dsm <= 96 * 1024 ? 1 : 0;
     h->demod_smem = pl.demod_in_smem ? dsm : 0;
     return with_enc(h, h->enc_code, [&](auto enc) {
@@ -633,7 +634,7 @@ int alloc_scratch(sdrb_handle *h, size_t nch)
         (rc = dalloc(h, nch * R * (nt + 1) * 16, &sc.carry)) ||
         (rc = dalloc(h, nch * R * M, &sc.y)) ||
         (rc = dalloc(h, (size_t)1, &sc.iq_state)) ||
-        (!pl.demod_in_smem && ((rc = dalloc(h, nch * R * 2 * M, &sc.fftbuf)) || (rc = dalloc(h, nch * R * M, &sc.zrow)))) ||
+        (!pl.demod_in_smem && (rc = dalloc(h, nch * R * (demod_smem_bytes(M) / sizeof(double2)), &sc.fftbuf))) ||
         (env_int("SDRB_TC_DEBUG", 0) && (rc = dalloc(h, (size_t)64 * 16, &sc.dbg))))
         return rc;
     CK(h, cudaMemset(sc.iq_state, 0, sizeof(double2)));
@@ -1231,15 +1232,12 @@ struct DemodTables {
 int run_demod(DevPlan pl, const DemodTables &t, const double *y, double *out, int demod)
 {
     const int R = pl.R, M = pl.M;
-    const size_t dsm = (size_t)M * (2 * sizeof(double2) + sizeof(double));
+    const size_t dsm = demod_smem_bytes(M);
     pl.demod_in_smem = dsm <= 48 * 1024;
-    DevBuf d_y, d_out, d_fft, d_z, d_tw, d_rot, d_w, d_ca;
+    DevBuf d_y, d_out, d_fft, d_tw, d_rot, d_w, d_ca;
     CK(nullptr, d_y.upload(reinterpret_cast<const double2 *>(y), (size_t)R * M));
     CK(nullptr, d_out.alloc((size_t)R * pl.W * sizeof(double)));
-    if (!pl.demod_in_smem) {
-        CK(nullptr, d_fft.alloc((size_t)R * 2 * M * sizeof(double2)));
-        CK(nullptr, d_z.alloc((size_t)R * M * sizeof(double)));
-    }
+    if (!pl.demod_in_smem) CK(nullptr, d_fft.alloc((size_t)R * dsm));
     CK(nullptr, d_tw.upload(t.tw.data(), t.tw.size()));
     CK(nullptr, d_rot.upload(t.rot.data(), t.rot.size()));
     CK(nullptr, d_w.upload(t.interp.data(), t.interp.size()));
@@ -1251,10 +1249,10 @@ int run_demod(DevPlan pl, const DemodTables &t, const double *y, double *out, in
     with_out(demod, [&](auto ok) {
         constexpr int OK = decltype(ok)::value;
         if constexpr (OK == OUT_IQ)
-            k_demod<OK><<<R, 128, 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), nullptr, nullptr, 1, demod, 0, 0);
+            k_demod<OK><<<R, 128, 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), nullptr, 1, demod, 0, 0);
         else
-            k_demod<OK><<<R, 128, pl.demod_in_smem ? dsm : 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), d_fft.as<double2>(),
-                                                               d_z.as<double>(), 1, demod, OK == OUT_SSB, 0);
+            k_demod<OK><<<R, 128, pl.demod_in_smem ? dsm : 0>>>(pl, d_y.as<double2>(), d_out.as<double>(), d_fft.as<double2>(), 1,
+                                                               demod, OK == OUT_SSB, 0);
         return 0;
     });
     CK(nullptr, cudaGetLastError());
@@ -1274,15 +1272,13 @@ static int demod_op(int device, const double *y, int R, int M, double *out, int 
     DevPlan pl{};
     pl.M = M; pl.R = R; pl.nsec_out = 0;
     pl.W = demod == SDRB_IQ ? 2 * M : M;
-    const int h2 = M >> 1;
-    pl.fft_ok = (M == 2 * h2) && is_pow2(h2);
-    pl.fft_n = pl.fft_ok ? M : 0;
+    pl.fft_ok = fft_ok(M);
     if (demod == SDRB_FM && (M & 1))
         return fail(nullptr, SDRB_ERR_ARG, "fmDemod pairs samples: the row length must be even (got %d)", M);
     DemodTables t;
-    t.tw = make_twiddles(pl.fft_n);
+    t.tw = make_twiddles(pl.fft_ok ? M : 0);
     // any even length: the same dense interpolation the engine uses for non-FFT sizes
-    if (demod == SDRB_FM && !pl.fft_ok) t.interp = resample_matrix(h2, M);
+    if (demod == SDRB_FM && !pl.fft_ok) t.interp = resample_matrix(M >> 1, M);
     return run_demod(pl, t, y, out, demod);
 }
 

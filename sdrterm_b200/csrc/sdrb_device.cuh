@@ -18,8 +18,7 @@ struct DevPlan {
     int sb;                // bytes per complex sample
     int run_len[8];        // samples per run, sample order (4 ascending + 4 descending)
     int sos_ns, sos_Lseg;  // output SOS evaluated in 32 segments of sos_Lseg samples
-    int fft_ok;            // FM resample by FFT (M == 2h, h power of two)
-    int fft_n;             // twiddle table length (== M when fft_ok)
+    int fft_ok;            // FM resample by FFT (M == 2h, h a power of two >= 2)
     int demod_in_smem;     // FFT / row buffers fit shared memory
     double Liq, lam, lam_q, lam_N, lam_inv, g0, d, norm_xmin, norm_k;
     double lam_run[8];     // lam^run_len
@@ -60,7 +59,7 @@ struct DevPlan {
     const double2 *phE;    // [R]     e^{j w q Mf}
     const double2 *psiY;   // [2][R][TB]  gamma (lam e^{jw})^(q l): tile-start offset -> output of block l
     const double2 *Prot;   // [R][16]  rotating-frame block multipliers (8 forward, 8 backward)
-    const double2 *tw;     // [fft_n]  exp(-2 pi i k / fft_n)
+    const double2 *tw;     // [M/2]  exp(-2 pi i k / M) when fft_ok
     const double *fm_interp;  // [M][M/2] or null
     const double *sos_CA;     // [sos_Lseg][ns]  c A^i
     const unsigned char *use_nco;  // [R]

@@ -4,9 +4,9 @@
 //      extension and zi start-up (head), the tail extension (end), the boundary vector zeta
 //   2. carries of the 8 forward / 8 anticausal modal states across the tiles of the chunk
 //   3. decimated outputs y[k] = partial output of the front end + carry-in response (+ boundary)
-//   4. demodulation: fm (pair phase, 2x trigonometric interpolation by a real-input FFT of half
-//      the length and its inverse) | am | re | im; the iq instance (OUT_IQ) stores y straight from
-//      registers instead, (Re, Im) per output, and skips 3b-5
+//   4. demodulation: fm (pair phase, 2x trigonometric interpolation: sdrb_fft.cuh's fm_interp2x on
+//      the warp) | am | re | im; the iq instance (OUT_IQ) stores y straight from registers
+//      instead, (Re, Im) per output, and skips 3b-5
 //   5. output low-pass (zero initial state per chunk): sdrb_outstage.cuh's output stage, 32 lane
 //      segments composed by a Kogge-Stone scan of the segment maps; framing (native or big-endian)
 //   The usb / lsb instance (OUT_SSB) skips 3b and 4: it stages y in the warp's shared memory (Re in
@@ -20,8 +20,9 @@
 // Reference behaviour reproduced: scipy.signal.decimate's sosfiltfilt boundary handling
 // (src/dsp/dsp_processor.py:147), src/dsp/demodulation.py:25-68, dsp_processor.py:32-36,149,162,
 // src/dsp/vfo_processor.py:84, src/misc/read_file.py:65-77.  tests/emulator.py (emu_fixup,
-// emu_demod, emu_fm_interp_real) is the numpy twin.
+// emu_demod) is the numpy twin.
 #pragma once
+#include "sdrb_fft.cuh"
 #include "sdrb_kernels.cuh"
 #include "sdrb_outstage.cuh"
 
@@ -46,85 +47,6 @@ __host__ __device__ inline size_t finish_smem_bytes(int M, int edge)
     const int nt = M / SDRB_TB;
     const size_t tables = (size_t)(nt + 48 + nt * 8 + 32 + 32 + 64) * sizeof(double2);   // single-row tables
     return (size_t)(M / 2) * sizeof(double2) + (size_t)(edge + 1) * 8 * sizeof(double2) + tables + FIN_WARPS * finish_warp_bytes(M);
-}
-
-// Stockham radix-2 pass over n points by one warp (two butterflies in flight per lane); twiddle
-// exp(-+2 pi i k / (2 Ns)) = tw[k * tstride].
-__device__ __forceinline__ void fin_fft_pass(const double2 *in, double2 *out, int n, int Ns, int tstride,
-                                             bool inverse, const double2 *tw, int lane)
-{
-    const int half = n >> 1;
-    for (int j = lane; j < half; j += 64) {
-        const int jb = j + 32;
-        const bool two = jb < half;
-        const int ka = j & (Ns - 1), kb = jb & (Ns - 1);
-        double2 wa = tw[ka * tstride], wb = tw[kb * tstride];
-        if (inverse) { wa.y = -wa.y; wb.y = -wb.y; }
-        const double2 a0 = in[j], a1 = in[j + half];
-        const double2 b0 = two ? in[jb] : a0, b1 = two ? in[jb + half] : a1;
-        const double2 ta = cmul(wa, a1), tb = cmul(wb, b1);
-        const int ja = ((j - ka) << 1) + ka, jc = ((jb - kb) << 1) + kb;
-        out[ja] = cadd(a0, ta);
-        out[ja + Ns] = csub(a0, ta);
-        if (two) {
-            out[jc] = cadd(b0, tb);
-            out[jc + Ns] = csub(b0, tb);
-        }
-    }
-}
-
-// exp(-+2 pi i m / M) for m < M from the half table tw[m], m < M/2 (tw[m + M/2] = -tw[m]).
-__device__ __forceinline__ double2 fin_tw(const double2 *tw, int m, int Mh, bool inverse)
-{
-    const bool neg = m >= Mh;
-    double2 w = tw[neg ? m - Mh : m];
-    if (neg) { w.x = -w.x; w.y = -w.y; }
-    if (inverse) w.y = -w.y;
-    return w;
-}
-
-// Stockham radix-4 pass over n points by one warp: one butterfly per lane and step; the twiddle
-// exp(-+2 pi i k / (4 Ns)) = table entry k * tstride (table base M = 2 * Mh).  Half the passes of
-// the radix-2 version, and each pass is one shared-memory round trip of dependent latency.
-__device__ __forceinline__ void fin_fft_pass4(const double2 *in, double2 *out, int n, int Ns, int tstride,
-                                              bool inverse, const double2 *tw, int Mh, int lane)
-{
-    const int quarter = n >> 2;
-    for (int j = lane; j < quarter; j += 32) {
-        const int k = j & (Ns - 1);
-        const int m = k * tstride;
-        const double2 a = in[j];
-        const double2 b = cmul(fin_tw(tw, m, Mh, inverse), in[j + quarter]);
-        const double2 c = cmul(fin_tw(tw, 2 * m, Mh, inverse), in[j + 2 * quarter]);
-        const double2 d = cmul(fin_tw(tw, 3 * m, Mh, inverse), in[j + 3 * quarter]);
-        const double2 s0 = cadd(a, c), s1 = csub(a, c), s2 = cadd(b, d), s3 = csub(b, d);
-        // -i (b - d) forward, +i (b - d) inverse
-        const double2 r3 = inverse ? make_double2(-s3.y, s3.x) : make_double2(s3.y, -s3.x);
-        const int j0 = ((j - k) << 2) + k;
-        out[j0] = cadd(s0, s2);
-        out[j0 + Ns] = cadd(s1, r3);
-        out[j0 + 2 * Ns] = csub(s0, s2);
-        out[j0 + 3 * Ns] = csub(s1, r3);
-    }
-}
-
-// n-point FFT (n a power of two >= 4) by radix-4 passes and one radix-2 pass if needed; returns
-// the buffer that holds the result.
-__device__ __forceinline__ double2 *fin_fft(double2 *src, double2 *dst, int n, int M, bool inverse,
-                                            const double2 *tw, int lane)
-{
-    int Ns = 1;
-    for (; Ns * 4 <= n; Ns <<= 2) {
-        fin_fft_pass4(src, dst, n, Ns, M / (4 * Ns), inverse, tw, M >> 1, lane);
-        __syncwarp();
-        double2 *tmp = src; src = dst; dst = tmp;
-    }
-    if (Ns < n) {
-        fin_fft_pass(src, dst, n, Ns, M / (2 * Ns), inverse, tw, lane);
-        __syncwarp();
-        double2 *tmp = src; src = dst; dst = tmp;
-    }
-    return src;
 }
 
 // usb / lsb staging layout: output k of lane segment g = k >> lsh sits at g*Ls + ((k + g) mod Ls), a
@@ -451,44 +373,8 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
         // ---------------------------------------------------------------- 3b. fm: 2x interpolation
         if (OUT == OUT_REAL && pl.demod == 0) {
             // even outputs of scipy.signal.resample(ph, 2h) are the phases themselves (already in
-            // zrow), the odd ones come from the half-sample-shifted spectrum.  Forward FFT of
-            // z[m] = ph[2m] + i ph[2m+1], n2 = h/2 points
-            double2 *src = fin_fft(fa, fb, n2, M, false, tw, lane);
-            double2 *dst = src == fa ? fb : fa;
-            // spectrum of the real row X[k] (k <= h/2) from Z, times the half-sample shift
-            // H[k] = exp(i pi k / h), re-packed for the half-length inverse transform
-            for (int k = lane; k <= (n2 >> 1); k += 32) {
-                if (k == 0) {
-                    const double2 Z0 = src[0];
-                    const double X0 = Z0.x + Z0.y;
-                    dst[0] = make_double2(X0, X0);
-                } else {
-                    const int kp = n2 - k;
-                    const double2 Zk = src[k], Zc = cconj(src[kp]);
-                    const double2 Xe = cscale(0.5, cadd(Zk, Zc));
-                    const double2 dd = csub(Zk, Zc);
-                    const double2 Xo = make_double2(0.5 * dd.y, -0.5 * dd.x);           // -i (Zk - Zc) / 2
-                    const double2 w2 = tw[2 * k];                                       // exp(-2 pi i k / h)
-                    const double2 tX = cmul(w2, Xo);
-                    const double2 Xk = cadd(Xe, tX), Xkp = cconj(csub(Xe, tX));
-                    const double2 Uk = cmul(Xk, cconj(tw[k])), Ukp = cmul(Xkp, cconj(tw[kp]));
-                    // V[k] = (U[k] + conj U[k']) + i (U[k] - conj U[k']) conj(w2)
-                    const double2 s1 = cadd(Uk, cconj(Ukp)), d1 = cmul(csub(Uk, cconj(Ukp)), cconj(w2));
-                    dst[k] = make_double2(s1.x - d1.y, s1.y + d1.x);
-                    // V[k'] = (U[k'] + conj U[k]) + i (U[k'] - conj U[k]) (-w2)
-                    const double2 s2 = cadd(Ukp, cconj(Uk)), d2 = cmul(csub(Ukp, cconj(Uk)), w2);
-                    dst[kp] = make_double2(s2.x + d2.y, s2.y - d2.x);
-                }
-            }
-            __syncwarp();
-            src = fin_fft(dst, src, n2, M, true, tw, lane);
-            const double sc1 = 1.0 / (double)h;
-            for (int m = lane; m < n2; m += 32) {
-                const double2 v = src[m];
-                const int k1 = 4 * m + 1, k3 = 4 * m + 3;
-                zrow[k1 + (k1 >> lsh)] = v.x * sc1;
-                zrow[k3 + (k3 >> lsh)] = v.y * sc1;
-            }
+            // zrow), the odd ones come from the half-sample-shifted spectrum
+            fm_interp2x(fa, fb, M, tw, WarpGroup{lane}, [&](int k, double v) { zrow[k + (k >> lsh)] = v; });
             __syncwarp();
         }
         FIN_DBG(8);

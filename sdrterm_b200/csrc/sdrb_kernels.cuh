@@ -20,6 +20,7 @@
 // tests/emulator.py is the numpy twin of these kernels (same tables, same decomposition).
 #pragma once
 #include "sdrb_device.cuh"
+#include "sdrb_fft.cuh"
 #include "sdrb_outstage.cuh"
 
 // Scratch written by k_main / read by k_fixup, per batch of chunks.
@@ -33,8 +34,7 @@ struct Scratch {
     double2 *carry;     // [nch][R][ntiles+1][16] 0..7 Win[t], 8..15 Tn[t]
     double2 *y;         // [nch][R][M]
     double2 *iq_state;  // [1] offset before the batch (in) / after it (out)
-    double2 *fftbuf;    // [nch*R][2][M] when the demod buffers do not fit shared memory
-    double *zrow;       // [nch*R][M]     "
+    double2 *fftbuf;    // [nch*R] k_demod row scratch of demod_smem_bytes(M) when it does not fit shared memory
     unsigned long long *dbg;  // optional k_tc timeline (SDRB_TC_DEBUG): [64 tiles][16 events] clock64 of CTA 0
     double2 *x0;        // optional [nch][R][Mf]: first raw sample of every block as the tensor-core
                         // front end sees it (exact integers; sdrb_keep_x0, parity tests)
@@ -726,22 +726,10 @@ k_fixup(const __grid_constant__ DevPlan pl, Scratch sc, const uint8_t *__restric
 }
 
 // ----------------------------------------------------------------------------------- k_demod
-// Stockham radix-2 pass over n points, twiddles from the plan's table (stride fft_n / (2 Ns)).
-__device__ __forceinline__ void fft_pass(const double2 *in, double2 *out, int n, int Ns, bool inverse,
-                                         const DevPlan &pl)
-{
-    const int half = n >> 1;
-    const int tstride = pl.fft_n / (2 * Ns);
-    for (int j = threadIdx.x; j < half; j += blockDim.x) {
-        const int k = j & (Ns - 1);
-        double2 w = pl.tw[(size_t)k * tstride];
-        if (inverse) w.y = -w.y;
-        const double2 a = in[j], b = cmul(w, in[j + half]);
-        const int j0 = ((j - k) << 1) + k;
-        out[j0] = cadd(a, b);
-        out[j0 + Ns] = csub(a, b);
-    }
-}
+// k_demod's row scratch (bytes), in shared memory or, when it does not fit, per CTA in global
+// memory: the output row of M doubles, then two FFT buffers of ceil(M/4) complex points (fm: the
+// first holds the M/2 pair phases as doubles).
+__host__ __device__ inline size_t demod_smem_bytes(int M) { return (size_t)4 * ((M + 3) / 4) * sizeof(double2); }
 
 // One CTA per (chunk, row): y[M] complex -> out[row][chunk*M .. +M) doubles.
 // Generic entry used both by the chain (y from sc.y) and by the module-level operators.  The iq
@@ -751,7 +739,7 @@ __device__ __forceinline__ void fft_pass(const double2 *in, double2 *out, int n,
 template <int OUT>
 __global__ void __launch_bounds__(256)
 k_demod(const __grid_constant__ DevPlan pl, const double2 *__restrict__ yall, double *__restrict__ out,
-        double2 *fftglob, double *zglob, int nchunks, int demod, int apply_sos, int be_out)
+        double2 *scratch, int nchunks, int demod, int apply_sos, int be_out)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int chunk = blockIdx.x / pl.R, r = blockIdx.x % pl.R;
@@ -763,52 +751,29 @@ k_demod(const __grid_constant__ DevPlan pl, const double2 *__restrict__ yall, do
         for (int k = threadIdx.x; k < M; k += blockDim.x) frame_store(o2 + k, y[k], be_out);
         return;
     }
-    double2 *bufA, *bufB;
-    double *z;
-    if (pl.demod_in_smem) {
-        bufA = reinterpret_cast<double2 *>(smem_raw);
-        bufB = bufA + M;
-        z = reinterpret_cast<double *>(bufB + M);
-    } else {
-        bufA = fftglob + (size_t)blockIdx.x * 2 * M;
-        bufB = bufA + M;
-        z = zglob + (size_t)blockIdx.x * M;
-    }
+    const int nq = (M + 3) >> 2;
+    double2 *row = pl.demod_in_smem ? reinterpret_cast<double2 *>(smem_raw) : scratch + (size_t)blockIdx.x * 4 * nq;
+    double *z = reinterpret_cast<double *>(row);
+    double2 *fa = row + 2 * nq, *fb = fa + nq;
     if (OUT == OUT_REAL && demod == 0) {   // fm: demodulation.py:25-38
-        for (int i = threadIdx.x; i < h; i += blockDim.x) bufA[i] = make_double2(pair_phase(y[2 * i], y[2 * i + 1]), 0.0);
+        // the pair phases are also the even outputs of the FFT interpolation (the dense matrix
+        // overwrites them)
+        double *ph = reinterpret_cast<double *>(fa);
+        for (int i = threadIdx.x; i < h; i += blockDim.x) {
+            const double v = pair_phase(y[2 * i], y[2 * i + 1]);
+            ph[i] = v;
+            z[2 * i] = v;
+        }
         __syncthreads();
         if (pl.fft_ok) {
-            double2 *src = bufA, *dst = bufB;
-            for (int Ns = 1; Ns < h; Ns <<= 1) {
-                fft_pass(src, dst, h, Ns, false, pl);
-                __syncthreads();
-                double2 *tmp = src; src = dst; dst = tmp;
-            }
-            // spectrum of the 2x interpolated row (scipy.signal.resample: halve the unpaired bin)
-            for (int k = threadIdx.x; k < M; k += blockDim.x) {
-                double2 v = make_double2(0.0, 0.0);
-                const int hh = h >> 1;
-                if (k < hh) v = src[k];
-                else if (k == hh) v = cscale(0.5, (h > 1) ? src[hh] : src[0]);
-                else if (k > M - hh) v = src[h - (M - k)];
-                else if (k == M - hh && hh > 0) v = cscale(0.5, cconj(src[hh]));
-                dst[k] = v;
-            }
-            __syncthreads();
-            double2 *s2 = dst, *d2 = src;
-            for (int Ns = 1; Ns < M; Ns <<= 1) {
-                fft_pass(s2, d2, M, Ns, true, pl);
-                __syncthreads();
-                double2 *tmp = s2; s2 = d2; d2 = tmp;
-            }
-            const double sc1 = 1.0 / (double)h;
-            for (int k = threadIdx.x; k < M; k += blockDim.x) z[k] = s2[k].x * sc1;
+            fm_interp2x(fa, fb, M, pl.tw, CtaGroup{(int)threadIdx.x, (int)blockDim.x},
+                        [&](int k, double v) { z[k] = v; });
         } else {
             // dense interpolation matrix built by the host from scipy.signal.resample
             for (int k = threadIdx.x; k < M; k += blockDim.x) {
-                const double *row = pl.fm_interp + (size_t)k * h;
+                const double *wrow = pl.fm_interp + (size_t)k * h;
                 double acc = 0.0;
-                for (int i = 0; i < h; i++) acc = fma(row[i], bufA[i].x, acc);
+                for (int i = 0; i < h; i++) acc = fma(wrow[i], ph[i], acc);
                 z[k] = acc;
             }
         }

@@ -14,6 +14,7 @@
 // scale_to='magnitude', phase_shift=None)`, `10*log10(abs(stft(y)))`).  The Qt widgets around them
 // are not part of this build.
 #pragma once
+#include "sdrb_fft.cuh"
 #include "sdrb_finish.cuh"
 
 // One radix-4 Stockham pass: butterfly j of transform `blockIdx.y`; twiddle exp(-2 pi i k / (4 Ns)).
@@ -30,21 +31,19 @@ k_gfft4(const double2 *__restrict__ in, double2 *__restrict__ out, const double2
             a = cmul(a, shift[j]); b = cmul(b, shift[j + quarter]);
             c = cmul(c, shift[j + 2 * quarter]); d = cmul(d, shift[j + 3 * quarter]);
         }
+        double2 w1 = make_double2(1.0, 0.0), w2 = w1, w3 = w1;      // k = 0: no sincospi, no products
         if (k) {
             const double x = -(double)k / (double)(2 * Ns);          // angle / pi of w1, exact
-            double2 w1, w2, w3;
             sincospi(x, &w1.y, &w1.x);
             sincospi(2.0 * x, &w2.y, &w2.x);
             sincospi(3.0 * x, &w3.y, &w3.x);
-            b = cmul(w1, b); c = cmul(w2, c); d = cmul(w3, d);
         }
-        const double2 s0 = cadd(a, c), s1 = csub(a, c), s2 = cadd(b, d), s3 = csub(b, d);
-        const double2 r3 = make_double2(s3.y, -s3.x);                // -i (b - d)
+        fft_bfly4(a, b, c, d, w1, w2, w3, false, k != 0);
         const int j0 = ((j - k) << 2) + k;
-        dst[j0] = cadd(s0, s2);
-        dst[j0 + Ns] = cadd(s1, r3);
-        dst[j0 + 2 * Ns] = csub(s0, s2);
-        dst[j0 + 3 * Ns] = csub(s1, r3);
+        dst[j0] = a;
+        dst[j0 + Ns] = b;
+        dst[j0 + 2 * Ns] = c;
+        dst[j0 + 3 * Ns] = d;
     }
 }
 
@@ -59,14 +58,12 @@ k_gfft2(const double2 *__restrict__ in, double2 *__restrict__ out, const double2
         const int k = j & (Ns - 1);
         double2 a = src[j], b = src[j + half];
         if (shift) { a = cmul(a, shift[j]); b = cmul(b, shift[j + half]); }
-        if (k) {
-            double2 w;
-            sincospi(-(double)k / (double)Ns, &w.y, &w.x);
-            b = cmul(w, b);
-        }
+        double2 w = make_double2(1.0, 0.0);                          // k = 0: no sincospi, no product
+        if (k) sincospi(-(double)k / (double)Ns, &w.y, &w.x);
+        fft_bfly2(a, b, w, k != 0);
         const int j0 = ((j - k) << 1) + k;
-        dst[j0] = cadd(a, b);
-        dst[j0 + Ns] = csub(a, b);
+        dst[j0] = a;
+        dst[j0 + Ns] = b;
     }
 }
 
@@ -85,7 +82,7 @@ k_spectrum_db(const double2 *__restrict__ X, double *__restrict__ out, int N)
 }
 
 // Short-time transform, one warp per slice p: seg[m] = y[p hop - mid + m] win[m] (zero outside
-// the signal), zero-padded to mfft points, forward FFT in shared memory (fin_fft), centred
+// the signal), zero-padded to mfft points, forward FFT in shared memory (fft on the warp), centred
 // (out row q = bin (q + mfft/2) mod mfft), out[q][p] = 10 log10 |S|.
 __global__ void __launch_bounds__(128)
 k_stft_db(const double2 *__restrict__ y, const double2 *__restrict__ shift, const double *__restrict__ win, double *__restrict__ out,
@@ -114,7 +111,7 @@ k_stft_db(const double2 *__restrict__ y, const double2 *__restrict__ shift, cons
             fa[m] = v;
         }
         __syncwarp();
-        const double2 *X = fin_fft(fa, fb, mfft, mfft, false, tw, lane);
+        const double2 *X = fft(fa, fb, mfft, mfft, false, tw, WarpGroup{lane});
         for (int qo = lane; qo < mfft; qo += 32) {
             const double2 v = X[(qo + (mfft >> 1)) & (mfft - 1)];
             out[(size_t)qo * p_num + p] = 10.0 * log10(hypot(v.x, v.y));

@@ -468,7 +468,7 @@ def build_plan(fs: int, enc: str, dec: int, rows_hz, *, simo: bool = False, swap
             sm['sos_CAM'] = cam
     fm_interp = None
     h = M >> 1
-    if demod == 'fm' and not (M == 2 * h and h & (h - 1) == 0):
+    if demod == 'fm' and not (M == 2 * h and h >= 2 and h & (h - 1) == 0):   # sdrb_api.cu's fft_ok
         # scipy.signal.resample(r, M) is linear in r: its matrix, column by column
         fm_interp = np.ascontiguousarray(_sig.resample(np.eye(h), M, axis=0))
     return Plan(enc=enc, swap=bool(swap), fs=fs, q=q, N=N, edge=edge, L=L, Mf=Mf, rem=rem, M=M,

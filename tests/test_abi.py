@@ -32,6 +32,13 @@ def test_library_builds_and_exports_every_declared_symbol():
     assert set(names) == set(nat.EXPORTS), set(names) ^ set(nat.EXPORTS)
 
 
+def test_every_csrc_file_is_a_rebuild_dependency():
+    """build() recompiles when a file in SOURCES is newer than the library: a header left out would
+    let an edit to it run against the stale library."""
+    csrc = os.path.join(ROOT, 'sdrterm_b200', 'csrc')
+    assert sorted(os.path.join(csrc, f) for f in os.listdir(csrc)) == sorted(nat.SOURCES)
+
+
 def test_abi_version_matches_header():
     m = re.search(r'#define SDRB_ABI_VERSION (\d+)', open(HEADER).read())
     assert int(m.group(1)) == nat.ABI_VERSION

@@ -153,11 +153,12 @@ def test_module_operators_known_answers():
 
 
 def test_fm_demod_operator_takes_any_even_length():
-    """demodulation.py:35-38 resamples for any n; rows of 2*2^k take the FFT path, everything else
-    the dense resample matrix (ADVICE r1)."""
+    """demodulation.py:35-38 resamples for any n; rows of 2*2^k (k >= 1) take the FFT path,
+    everything else the dense resample matrix (ADVICE r1).  2: the matrix; 4: no FFT pass; 8: one
+    radix-2 pass; 16: one radix-4 pass; 2048 / 4096: shared / global scratch; 16384."""
     import sdrterm_b200.dsp.demodulation as dem
     rng = np.random.default_rng(3)
-    for n in (6, 10, 24, 100, 1310, 512):
+    for n in (2, 4, 6, 8, 10, 16, 24, 100, 1310, 512, 2048, 4096, 16384):
         y = rng.normal(size=(2, n)) + 1j * rng.normal(size=(2, n))
         out = np.empty((2, n))
         dem.fmDemod(y, out)
