@@ -18,7 +18,7 @@
 extern "C" {
 #endif
 
-#define SDRB_ABI_VERSION 10
+#define SDRB_ABI_VERSION 11
 #define SDRB_TILE_BLOCKS 32
 #define SDRB_NPOLES 8
 #define SDRB_MAX_DECIMATION 256
@@ -79,7 +79,7 @@ typedef struct sdrb_tables {
     double g0, d;
     const double *Ec, *Oc;   /* [4][Hq] complex, Hq = ceil(q/2) */
     const double *Ppow;      /* [TILE_BLOCKS+1][8] complex */
-    const double *pk;        /* [edge+1][8] complex: p_i^k */
+    const double *pk;        /* [max(edge+1, edge+rem)][8] complex: p_i^k, rem = N mod q */
     const double *Pt;        /* [ntiles][8] complex: p_i^(q*TILE_BLOCKS*m) */
     const double *bx;        /* [8] complex: p_i^edge / kappa_i */
     const double *bnd;       /* [M][8] complex */

@@ -17,7 +17,7 @@ HEADER = os.path.join(ROOT, 'include', 'sdrterm_b200.h')
 SOURCES = [os.path.join(_HERE, 'csrc', f) for f in ('sdrb_api.cu', 'sdrb_kernels.cuh', 'sdrb_device.cuh', 'sdrb_tc.cuh', 'sdrb_finish.cuh',
                                                     'sdrb_spectrum.cuh', 'sdrb_seamless.cuh', 'sdrb_outstage.cuh', 'sdrb_fft.cuh')]
 
-ABI_VERSION = 10
+ABI_VERSION = 11
 FM, AM, RE, IM, IQ, USB, LSB = 0, 1, 2, 3, 4, 5, 6
 DEMOD_CODE = {'fm': FM, 'am': AM, 're': RE, 'im': IM, 'iq': IQ, 'usb': USB, 'lsb': LSB}
 

@@ -406,7 +406,6 @@ DevPlan plan_of(const sdrb_config *cfg, const sdrb_tables *tab)
     pl.RL = tab->RL;
     pl.sb = 2 * pl.itemsize;
     for (int i = 0; i < 8; i++) { pl.run_len[i] = tab->run_len[i]; pl.lam_run[i] = tab->lam_run[i]; }
-    pl.lam_inv = tab->lam_inv;
     pl.sos_ns = 2 * cfg->n_out_sections; pl.sos_Lseg = tab->sos_Lseg;
     pl.ws = std::min(pl.q * pl.Mf, pl.N - 1 - pl.edge); pl.nend = pl.N - pl.ws;
     pl.k_bnd = tab->k_bnd; pl.nsec_out = cfg->n_out_sections;
@@ -465,9 +464,11 @@ int validate(const sdrb_config *cfg, const sdrb_tables *tab)
     if (cfg->R < 1 || cfg->edge < 1 || cfg->N <= cfg->edge + 1 || cfg->max_chunks < 1 || cfg->n_out_sections < 0 ||
         cfg->n_out_sections > 4)
         return fail(nullptr, SDRB_ERR_ARG, "bad geometry");
-    // k_fixup stages (edge+1) head samples and nend = max(rem, edge+1) window samples in shared memory
-    if (cfg->edge + 1 + std::max(cfg->N % cfg->q, cfg->edge + 1) > SDRB_NEDGE)
-        return fail(nullptr, SDRB_ERR_ARG, "filter pad %d too long for the fix-up kernel", cfg->edge);
+    // the chunk boundary runs the head's edge + 1 samples on one warp, lane <-> sample; the general
+    // kernels stage the head extension (edge), the end window (nend = max(rem, edge + 1)) and the
+    // tail extension (edge) in SDRB_NEDGE samples of shared memory
+    if (cfg->edge + 1 > 32 || 2 * cfg->edge + std::max(cfg->N % cfg->q, cfg->edge + 1) > SDRB_NEDGE)
+        return fail(nullptr, SDRB_ERR_ARG, "filter pad %d too long for the chunk boundary (edge + 1 <= 32 samples)", cfg->edge);
     const void *need[] = {tab->p, tab->P, tab->rho, tab->rho_p, tab->c, tab->zhat, tab->xi, tab->Ec, tab->Oc,
                           tab->Ppow, tab->pk, tab->Pt, tab->bx, tab->bnd, tab->lam_j, tab->lam_k, tab->mu_k,
                           tab->T2, tab->T3, tab->T1, tab->Ehead, tab->Eend, tab->alpha, tab->alphaT, tab->beta,
@@ -565,7 +566,7 @@ int plan_tables(sdrb_handle *h, const sdrb_tables *tab)
     if ((rc = upload(h, afrag.data(), afrag.size(), &pl.Afrag)) ||
         (rc = upload(h, tab->lam_j, (size_t)q + 1, &pl.lam_j)) ||
         (rc = upload(h, d2(tab->Ppow), (size_t)(SDRB_TB + 1) * 8, &pl.Ppow)) ||
-        (rc = upload(h, d2(tab->pk), (size_t)(pl.edge + 1) * 8, &pl.pk)) ||
+        (rc = upload(h, d2(tab->pk), (size_t)std::max(pl.edge + 1, pl.edge + pl.rem) * 8, &pl.pk)) ||
         (rc = upload(h, d2(tab->Pt), (size_t)nt * 8, &pl.Pt)) ||
         (rc = upload(h, rw.data(), rw.size(), &pl.RW)) ||
         (rc = upload(h, rt.data(), rt.size(), &pl.RT)) ||
@@ -606,7 +607,7 @@ int set_geometry(sdrb_handle *h)
     h->main_smem = main_geometry(pl, h->tpc, h->warps);
     const int M = pl.M;
     h->finish_on = !env_int("SDRB_NO_FINISH", 0) && pl.rem == 0 && pl.cnt_last == SDRB_TB && pl.q >= pl.edge + 1 &&
-                   is_pow2(M) && M >= 64 && M <= 1024 && pl.edge + 1 <= 32 && pl.ntiles <= 32 &&
+                   is_pow2(M) && M >= 64 && M <= 1024 && pl.ntiles <= 32 &&
                    (pl.nsec_out == 0 || pl.nsec_out == 2);
     h->finish_smem = h->finish_on ? finish_smem_bytes(M, pl.edge) : 0;
     if (h->finish_smem > 227 * 1024) h->finish_on = false;

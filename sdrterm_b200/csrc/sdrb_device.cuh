@@ -7,7 +7,7 @@
 #define SDRB_TB 32          // blocks per tile == warp width (lane <-> block)
 #define SDRB_NP 8           // poles of the cheby1 order-8 decimation low-pass
 #define SDRB_XSTRIDE 33     // exchange buffer row stride in doubles
-#define SDRB_NEDGE 320      // edge samples a chunk-boundary kernel stages: head (edge+1) + end window (nend)
+#define SDRB_NEDGE 320      // samples k_fixup stages: head extension (edge) + end window (nend) + tail extension (edge)
 
 enum { ENC_b = 0, ENC_B, ENC_h, ENC_H, ENC_i, ENC_I, ENC_f, ENC_d, ENC_Z };
 
@@ -20,11 +20,11 @@ struct DevPlan {
     int sos_ns, sos_Lseg;  // output SOS evaluated in 32 segments of sos_Lseg samples
     int fft_ok;            // FM resample by FFT (M == 2h, h a power of two >= 2)
     int demod_in_smem;     // FFT / row buffers fit shared memory
-    double Liq, lam, lam_q, lam_N, lam_inv, g0, d, norm_xmin, norm_k;
+    double Liq, lam, lam_q, lam_N, g0, d, norm_xmin, norm_k;
     double lam_run[8];     // lam^run_len
     double sos_AP[320];    // [5][ns][ns] (A^Lseg)^(2^lv), ns = sos_ns (packed): the lane scan's segment maps
     double lamq_pow[5];    // lam_q^(1,2,4,8,16)
-    double lam_pw[33];     // lam^k, k = 0..32 (k_finish's IQ scans)
+    double lam_pw[33];     // lam^k, k = 0..32 (the chunk boundary's IQ scans)
     double mu_pw[33];      // lam^-k
     double lam_tile[2];
     double2 p[SDRB_NP], P[SDRB_NP], rho[SDRB_NP], rho_p[SDRB_NP], c[SDRB_NP], zhat[SDRB_NP];
@@ -34,7 +34,7 @@ struct DevPlan {
     const double *Afrag;   // [KS][2][32]  DMMA A fragments: even-part (Ec) and odd-part (Oc)
     const double *lam_j;   // [q+1]
     const double2 *Ppow;   // [TB+1][8]
-    const double2 *pk;     // [edge+1][8]  p_i^k (closed forms of the head / tail recurrences)
+    const double2 *pk;     // [max(edge+1, edge+rem)][8]  p_i^k (closed forms of the head / tail recurrences)
     const double2 *Pt;     // [ntiles][8]  P_i^(32 m): a carry moved m whole tiles
     const double2 *RW;     // [TB+1][8]  rho_i   * P_i^l
     const double2 *RT;     // [TB+1][8]  rho_p_i * P_i^l

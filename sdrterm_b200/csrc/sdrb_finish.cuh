@@ -1,7 +1,8 @@
 // sdrb_finish.cuh -- k_finish: everything after the block front end, one warp per (chunk, row).
 //
 //   1. chunk boundaries: IQ-corrected, NCO-shifted head and end-window samples; sosfiltfilt's odd
-//      extension and zi start-up (head), the tail extension (end), the boundary vector zeta
+//      extension and zi start-up (head), the tail extension (end), the boundary vector zeta -- the
+//      chunk-boundary routines of sdrb_kernels.cuh, which k_fixup and the seamless kernels run too
 //   2. carries of the 8 forward / 8 anticausal modal states across the tiles of the chunk
 //   3. decimated outputs y[k] = partial output of the front end + carry-in response (+ boundary)
 //   4. demodulation: fm (pair phase, 2x trigonometric interpolation: sdrb_fft.cuh's fm_interp2x on
@@ -109,10 +110,8 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
         rt[i] = cscale(2.0, pl.RT[(size_t)(SDRB_TB - lane) * 8 + i]);
     }
     const int i8 = lane & 7, grp = (lane >> 3) & 1, sub = lane >> 3;
-    const double2 p_i = pl.p[i8], P32 = pl.Ppow[(size_t)SDRB_TB * 8 + i8];
+    const double2 P32 = pl.Ppow[(size_t)SDRB_TB * 8 + i8];
     const int Ls = pl.sos_Lseg, lsh = Ls > 0 ? 31 - __clz(Ls) : 31;   // no output SOS (re/im): no padding
-    const int dchunk = (edge + 3) >> 2;                                  // dot-product terms per lane group
-    const double lamn = pl.lam_pw[lane], mun = pl.mu_pw[min(32, max(0, edge + 1 - lane))];
 
     const int gw = blockIdx.x * FIN_WARPS + warp, nw = gridDim.x * FIN_WARPS;
     int nit = -1;
@@ -169,32 +168,21 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
             }
         }
         FIN_DBG(1);
-        // ---------------------------------------------------------------- 1b. IQ correction
-        // read_file.py:72-77 is the linear recurrence off' = lam off + L z; lane <-> sample.  Head:
-        // off_n = lam^n off_0 + L sum_{i<n} lam^(n-1-i) z_i (scan upwards).  End window, from the
-        // offset at q*Mf backwards: off_n = mu^m off_E - L mu sum_{i>=n} mu^(i-n) z_i, mu = 1/lam.
-        if (iq) {
-            const double2 o0 = shfl_c(offr, 0);
-            double2 S = xh, B = xe;
-#pragma unroll
-            for (int lv = 0; lv < 5; lv++) {
-                const double2 tu = shfl_up_c(S, 1 << lv);
-                const double2 td = make_double2(__shfl_down_sync(0xffffffffu, B.x, 1 << lv), __shfl_down_sync(0xffffffffu, B.y, 1 << lv));
-                if (lane >= (1 << lv)) { S.x = fma(pl.lam_pw[1 << lv], tu.x, S.x); S.y = fma(pl.lam_pw[1 << lv], tu.y, S.y); }
-                if (lane + (1 << lv) < 32) { B.x = fma(pl.mu_pw[1 << lv], td.x, B.x); B.y = fma(pl.mu_pw[1 << lv], td.y, B.y); }
+        // ---------------------------------------------------------------- 1b. IQ correction, NCO
+        // head forward from the chunk-start offset; end window (nend = edge + 1 samples: rem = 0)
+        // backward from the offset at q*Mf
+        const double2 o0 = shfl_c(offr, 0);
+        {
+            double2 Eh = make_double2(0.0, 0.0), Ee = Eh;
+            if (lane <= edge) {
+                Eh = R == 1 ? tbEh[lane] : pl.Ehead[(size_t)r * (edge + 1) + lane];
+                Ee = R == 1 ? tbEe[lane] : pl.Eend[(size_t)r * pl.nend + lane];
             }
-            double2 Sx = shfl_up_c(S, 1);
-            if (lane == 0) Sx = make_double2(0.0, 0.0);
-            xh.x -= fma(lamn, o0.x, pl.Liq * Sx.x); xh.y -= fma(lamn, o0.y, pl.Liq * Sx.y);
-            const double lm = pl.Liq * pl.mu_pw[1];
-            xe.x -= fma(mun, oE.x, -lm * B.x); xe.y -= fma(mun, oE.y, -lm * B.y);
+            xh = edge_correct(pl, xh, o0, edge + 1, 0, Eh, lane).x;
+            xe = edge_correct(pl, xe, oE, edge + 1, edge + 1, Ee, lane).x;
         }
         FIN_DBG(2);
-        // ---------------------------------------------------------------- 1c. NCO, odd extensions
-        if (lane <= edge) {
-            xh = cmul(xh, R == 1 ? tbEh[lane] : pl.Ehead[(size_t)r * (edge + 1) + lane]);
-            xe = cmul(xe, R == 1 ? tbEe[lane] : pl.Eend[(size_t)r * pl.nend + lane]);
-        }
+        // ---------------------------------------------------------------- 1c. odd extensions
         {
             const double2 x0 = shfl_c(xh, 0), xN1 = shfl_c(xe, edge);
             const double2 ha = shfl_c(xh, max(0, edge - lane)), eb = shfl_c(xe, max(0, edge - 1 - lane));
@@ -206,41 +194,22 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
         __syncwarp();
         FIN_DBG(3);
         // ---------------------------------------------------------------- 1d. head / tail states
-        // closed forms of the serial recurrences: w(edge) = p^edge zhat ext0 + sum_j p^(edge-1-j) ext_j,
-        // T(end) = sum_k p^k tail_k, and the tail-driven part of w(L-2); lane = (pole, quarter of j)
-        double2 accA = make_double2(0.0, 0.0), accB = accA, accC = accA;
-        {
-            const int j0 = sub * dchunk, j1 = min(edge, j0 + dchunk);
-            for (int j = j0; j < j1; j++) {
-                const double2 a = seqA[j], b = seqB[j];
-                accA = cfma(pk[(edge - 1 - j) * 8 + i8], a, accA);
-                accB = cfma(pk[j * 8 + i8], b, accB);
-                if (j <= edge - 2) accC = cfma(pk[(edge - 2 - j) * 8 + i8], b, accC);
-            }
-#pragma unroll
-            for (int sft = 8; sft < 32; sft <<= 1) {
-                accA = cadd(accA, shfl_xor_c(accA, sft));
-                accB = cadd(accB, shfl_xor_c(accB, sft));
-                accC = cadd(accC, shfl_xor_c(accC, sft));
-            }
-            accA = cfma(pk[edge * 8 + i8], cmul(pl.zhat[i8], seqA[0]), accA);
-        }
+        const BoundarySums bs = boundary_sums(pl, pk, seqA, edge, seqB, edge, lane);
         FIN_DBG(4);
         // ---------------------------------------------------------------- 1e. carries across tiles
         // lanes 0..7: forward modal states (Win[t] = state entering tile t); lanes 8..15: anticausal
         // states (Tn[t] = state entering tile t from above)
         // in the frame of the uncorrected samples (3.3): W~ = (w + alpha s) / beta at n = 0,
         // T~ = (T + alphaT s) / betaT at n = q*Mf, s = off e^{jwn}; stored pre-scaled by beta / betaT
-        double2 st = grp ? accB : accA;
+        double2 st = grp ? bs.B : bs.A;
         double2 qal = make_double2(0.0, 0.0), qbe = make_double2(1.0, 0.0), sE = qal;
-        const double2 o0c = shfl_c(offr, 0);
         if (iq) {
             const int mi = grp * 8 + i8;
             qal = R == 1 ? tbPsi[mi] : (grp ? pl.alphaT : pl.alpha)[(size_t)r * 8 + i8];
             const double2 qbi = R == 1 ? tbPsi[16 + mi] : (grp ? pl.binvT : pl.binv)[(size_t)r * 8 + i8];
             qbe = (grp ? pl.betaT : pl.beta)[(size_t)r * 8 + i8];
             sE = cmul(oE, pl.phE[r]);
-            st = cmul(cfma(qal, grp ? sE : o0c, st), qbi);
+            st = cmul(cfma(qal, grp ? sE : o0, st), qbi);
         }
         // (the chain itself stays in the frame of the uncorrected samples; beta / betaT are applied
         // when the carries are turned into real / imaginary stream states below)
@@ -256,22 +225,10 @@ k_finish(const __grid_constant__ DevPlan pl, const __grid_constant__ Scratch sc,
         FIN_DBG(5);
         // ---------------------------------------------------------------- 1f. boundary vector zeta
         {
-            const double2 Wn = shfl_c(st, i8);                              // forward state at n = edge + q*Mf
-            const double2 last = seqB[edge - 1];
-            const double2 wL1 = cfma(pk[(edge - 1) * 8 + i8], Wn, accC);
-            const double2 wL = cfma(p_i, wL1, last);
-            double2 part = cmul(pl.c[i8], wL1);
-            for (int sft = 1; sft < 8; sft <<= 1) part = cadd(part, shfl_xor_c(part, sft));
-            const double2 yfL1 = make_double2(fma(pl.d, last.x, part.x), fma(pl.d, last.y, part.y));
-            double2 za = cmul(pl.zhat[i8], yfL1), zb = make_double2(0.0, 0.0);
-#pragma unroll
-            for (int l = 0; l < 8; l += 2) {
-                za = csub(za, cmul(pl.xi[i8 * 8 + l], shfl_c(wL, l)));
-                zb = csub(zb, cmul(pl.xi[i8 * 8 + l + 1], shfl_c(wL, l + 1)));
-            }
-            // sosfiltfilt's boundary term c_i p_i^(L-1-n) zeta_i is an anticausal modal response:
-            // it rides on the backward carries as X_i = p_i^edge / kappa_i zeta_i at n = edge + q*Mf
-            double2 X = cmul(pl.bx[i8], cadd(za, zb));
+            // from the forward state at n = edge + q*Mf: sosfiltfilt's boundary term c_i p_i^(L-1-n)
+            // zeta_i is an anticausal modal response: it rides on the backward carries as
+            // X_i = p_i^edge / kappa_i zeta_i at n = edge + q*Mf
+            double2 X = cmul(pl.bx[i8], boundary_zeta(pl, pk, seqB, edge, shfl_c(st, i8), bs.C, lane));
             if (iq) X = cmul(X, R == 1 ? tbPsi[24 + i8] : pl.binvT[(size_t)r * 8 + i8]);   // into the T~ frame
             __syncwarp();
             for (int t = sub; t < nt; t += 4) {

@@ -8,7 +8,8 @@
 //              offsets (warp <-> chunk; k_finish derives them itself); tile_offsets is the one
 //              tile-offset routine of all three and k_finish
 //   k_iqchunk  chunk gains straight from the raw bytes (time-segment sharding)
-//   k_fixup    head / end segments, cross-tile carries, boundary term -> decimated complex y
+//   k_fixup    chunk boundary (head, end window, boundary sums and zeta: the chunk-boundary routines
+//              of k_finish and the seamless kernels too), cross-tile carries -> decimated complex y
 //   k_demod    fm (pair phase + 2x FFT interpolation) | am | re | im, output SOS, framing; iq: y
 //              itself framed as (Re, Im) pairs; usb / lsb: the complex band-pass on y, its real part
 //              framed.  The demodulator scalars and the output SOS (32 lane segments, lane scan,
@@ -530,98 +531,159 @@ __global__ void k_iq_prefix(Scratch sc, const double *gains3, int rank, double l
 }
 
 // ------------------------------------------------------------------------- chunk boundary
-// sosfiltfilt's boundary at a chunk's edges and the modal carries across its tiles, shared by k_fixup
-// and the seamless kernels: one warp stages the edge samples in shared memory, lane <-> mode i runs
-// the modal pieces.  The front ends sum the UNcorrected rotated samples, so their frame has
-// W~ = (w + alpha s) / beta and T~ = (T + alphaT s) / betaT, s = off[n] e^{jwn} (DESIGN.md 3.3).
+// sosfiltfilt's boundary at a chunk's two edges, written once for k_finish, k_fixup and the seamless
+// kernels: lane <-> sample for the edge samples, lane = (mode, quarter of the terms) for the closed
+// forms of the boundary recurrences.  The front ends sum the UNcorrected rotated samples, so their
+// frame has W~ = (w + alpha s) / beta and T~ = (T + alphaT s) / betaT, s = off[n] e^{jwn} (DESIGN.md
+// 3.3); the callers convert.
 
-// Edge samples s[0..n), raw -> IQ-corrected (read_file.py:72-77) from o, the offset at sample nb:
-// s[0..nb) BACKWARD (off[n] = (off[n+1] - L z[n]) / lam), s[nb..n) forward; then times the NCO
-// phases E[0..n).
-__device__ __forceinline__ void stage_edge(const DevPlan &pl, double2 *s, int n, int nb, double2 o,
-                                           const double2 *E, int lane)
-{
-    if (pl.correct_iq) {
-        if (lane == 0) {
-            for (int j = nb - 1; j >= 0; j--) {
-                const double2 z = s[j];
-                o.x = fma(-pl.Liq, z.x, o.x) * pl.lam_inv; o.y = fma(-pl.Liq, z.y, o.y) * pl.lam_inv;
-                s[j] = csub(z, o);
-            }
-        } else if (lane == 1) {
-            for (int j = nb; j < n; j++) {
-                const double2 x = csub(s[j], o);
-                o.x = fma(x.x, pl.Liq, o.x); o.y = fma(x.y, pl.Liq, o.y);
-                s[j] = x;
-            }
-        }
-    }
-    __syncwarp();
-    for (int j = lane; j < n; j += 32) s[j] = cmul(s[j], E[j]);
-    __syncwarp();
-}
-__device__ __forceinline__ void stage_head(const DevPlan &pl, int r, double2 *s_h, double2 off0, int lane)
-{
-    stage_edge(pl, s_h, pl.edge + 1, 0, off0, pl.Ehead + (size_t)r * (pl.edge + 1), lane);
-}
-__device__ __forceinline__ void stage_end(const DevPlan &pl, int r, double2 *s_e, double2 offE, int lane)
-{
-    stage_edge(pl, s_e, pl.nend, pl.nend - pl.rem, offE, pl.Eend + (size_t)r * pl.nend, lane);
-}
-
-// Mode i: the forward state at n = edge from the staged head (odd extension 2 x0 - x[edge-j], zi),
-// as W~ with s = o, the offset at sample 0.
-__device__ __forceinline__ double2 head_state(const DevPlan &pl, int r, const double2 *s_h, double2 o, int i)
-{
-    const int edge = pl.edge;
-    const double2 p = pl.p[i], x0 = s_h[0];
-    double2 w = cmul(pl.zhat[i], csub(cscale(2.0, x0), s_h[edge]));
-    for (int j = 0; j < edge; j++) {
-        const double2 ext = csub(cscale(2.0, x0), s_h[edge - j]);
-        w = cfma(p, w, ext);
-    }
-    if (pl.correct_iq) w = cmul(cfma(pl.alpha[(size_t)r * 8 + i], o, w), pl.binv[(size_t)r * 8 + i]);
-    return w;
-}
-
-struct EndState {
-    double2 w, T, Tt, zeta;     // at q*Mf: the true forward and anticausal states, T~; zeta
+struct EdgeSample {
+    double2 x;      // this lane's sample, IQ-corrected and rotated
+    double2 o;      // the offset after the window when it ends running forward: the next round's o
 };
 
-// Mode i from W~, the forward state at q*Mf, and the staged end window: the partial block then the
-// tail extension 2 x[N-1] - x[N-2-j] run forward (w at the last two samples) and anticausally back to
-// q*Mf (T); zeta from y_f at the last sample.  o is the offset at q*Mf.  All 32 lanes must call it
-// (the cross-mode sums shuffle within groups of 8 lanes); the modes' results are those of lanes 0..7.
-__device__ __forceinline__ EndState end_state(const DevPlan &pl, int r, const double2 *s_e, double2 o, double2 Wt, int i)
+// A window of n <= 32 samples, lane <-> sample; z = this lane's decoded sample (zero past the
+// window).  read_file.py:72-77 is the linear recurrence off' = lam off + L z; from o, the offset at
+// sample n_bwd, lanes below n_bwd run it BACKWARD, off_m = mu^(n_bwd-m) o - L mu sum_{m<=i<n_bwd}
+// mu^(i-m) z_i (mu = 1/lam), lanes from n_bwd on forward, off_m = lam^(m-n_bwd) o + L
+// sum_{n_bwd<=i<m} lam^(m-1-i) z_i: a 5-level warp scan for each direction the window has.  The
+// corrected sample is then rotated by E, this lane's NCO phase.
+__device__ __forceinline__ EdgeSample edge_correct(const DevPlan &pl, double2 z, double2 o, int n, int n_bwd, double2 E,
+                                                   int lane)
 {
-    const bool iq = pl.correct_iq != 0;
-    const int nend = pl.nend, rem = pl.rem, nseq = rem + pl.edge;
-    const double2 p = pl.p[i];
-    const double2 sE = iq ? cmul(o, pl.phE[r]) : make_double2(0.0, 0.0);   // rotated offset at q*Mf
-    EndState e;
-    double2 w = iq ? csub(cmul(pl.beta[(size_t)r * 8 + i], Wt), cmul(pl.alpha[(size_t)r * 8 + i], sE)) : Wt;
-    e.w = w;
-    const double2 xN1 = s_e[nend - 1];
-    auto seq = [&](int k) {
-        return k < rem ? s_e[nend - rem + k] : csub(cscale(2.0, xN1), s_e[nend - 2 - (k - rem)]);
-    };
-    double2 wL1 = w, last = make_double2(0.0, 0.0);
-    for (int k = 0; k < nseq; k++) {
-        const double2 v = seq(k);
-        if (k == nseq - 1) { wL1 = w; last = v; }
-        w = cfma(p, w, v);
+    EdgeSample e{z, o};
+    if (pl.correct_iq) {
+        const double2 zero = make_double2(0.0, 0.0);
+        if (n_bwd > 0) {
+            double2 B = lane < n_bwd ? z : zero;
+#pragma unroll
+            for (int lv = 0; lv < 5; lv++) {
+                const double2 td = make_double2(__shfl_down_sync(0xffffffffu, B.x, 1 << lv), __shfl_down_sync(0xffffffffu, B.y, 1 << lv));
+                if (lane + (1 << lv) < 32) { B.x = fma(pl.mu_pw[1 << lv], td.x, B.x); B.y = fma(pl.mu_pw[1 << lv], td.y, B.y); }
+            }
+            if (lane < n_bwd) {
+                const double mun = pl.mu_pw[n_bwd - lane], lm = pl.Liq * pl.mu_pw[1];
+                e.x.x -= fma(mun, o.x, -lm * B.x); e.x.y -= fma(mun, o.y, -lm * B.y);
+            }
+        }
+        if (n_bwd < n) {
+            double2 S = lane >= n_bwd ? z : zero;
+#pragma unroll
+            for (int lv = 0; lv < 5; lv++) {
+                const double2 tu = shfl_up_c(S, 1 << lv);
+                if (lane >= (1 << lv)) { S.x = fma(pl.lam_pw[1 << lv], tu.x, S.x); S.y = fma(pl.lam_pw[1 << lv], tu.y, S.y); }
+            }
+            double2 Sx = shfl_up_c(S, 1);
+            if (lane == 0) Sx = zero;
+            if (lane >= n_bwd) {
+                const double lamn = pl.lam_pw[lane - n_bwd];
+                e.x.x -= fma(lamn, o.x, pl.Liq * Sx.x); e.x.y -= fma(lamn, o.y, pl.Liq * Sx.y);
+            }
+            const double2 Sn = shfl_c(S, n - 1);
+            const double ln = pl.lam_pw[n - n_bwd];
+            e.o = make_double2(fma(ln, o.x, pl.Liq * Sn.x), fma(ln, o.y, pl.Liq * Sn.y));
+        }
     }
-    double2 T = make_double2(0.0, 0.0);
-    for (int k = nseq - 1; k >= 0; k--) T = cfma(p, T, seq(k));
-    e.T = T;
-    e.Tt = iq ? cmul(cfma(pl.alphaT[(size_t)r * 8 + i], sE, T), pl.binvT[(size_t)r * 8 + i]) : T;
-    // y_f[L-1] = sum_l c_l w_l[L-1] + d ext[L-1]   (reduce over the 8 mode lanes)
-    double2 part = cmul(pl.c[i], wL1);
+    if (lane < n) e.x = cmul(e.x, E);
+    return e;
+}
+
+struct BoundarySums {
+    double2 A, B, C;
+};
+
+// The closed forms of the serial boundary recurrences against pk[k][i] = p_i^k, lane = (mode i =
+// lane & 7, quarter lane >> 3 of the terms); every lane returns its mode's sums.  Head, from its odd
+// extension ha[0..nh): A = w(edge) = p^nh zhat ha[0] + sum_j p^(nh-1-j) ha[j].  End, from the sequence
+// seq[0..nseq) (the partial block, then the tail extension): B = T at q*Mf = sum_k p^k seq[k], and
+// C = sum_{k <= nseq-2} p^(nseq-2-k) seq[k], the sequence's part of w(L-2).  nh = 0 or nseq = 0
+// skips that end.
+__device__ __forceinline__ BoundarySums boundary_sums(const DevPlan &pl, const double2 *pk, const double2 *ha, int nh,
+                                                      const double2 *seq, int nseq, int lane)
+{
+    const int i8 = lane & 7, sub = lane >> 3;
+    const int dh = (nh + 3) >> 2, ds = (nseq + 3) >> 2;     // terms per quarter
+    const int h0 = sub * dh, h1 = min(nh, h0 + dh), s0 = sub * ds, s1 = min(nseq, s0 + ds);
+    BoundarySums s;
+    s.A = s.B = s.C = make_double2(0.0, 0.0);
+    for (int u = 0; u < max(dh, ds); u++) {
+        const int j = h0 + u, k = s0 + u;
+        if (j < h1) s.A = cfma(pk[(nh - 1 - j) * 8 + i8], ha[j], s.A);
+        if (k < s1) {
+            const double2 b = seq[k];
+            s.B = cfma(pk[k * 8 + i8], b, s.B);
+            if (k <= nseq - 2) s.C = cfma(pk[(nseq - 2 - k) * 8 + i8], b, s.C);
+        }
+    }
+#pragma unroll
+    for (int sft = 8; sft < 32; sft <<= 1) {
+        s.A = cadd(s.A, shfl_xor_c(s.A, sft));
+        s.B = cadd(s.B, shfl_xor_c(s.B, sft));
+        s.C = cadd(s.C, shfl_xor_c(s.C, sft));
+    }
+    if (nh > 0) s.A = cfma(pk[nh * 8 + i8], cmul(pl.zhat[i8], ha[0]), s.A);
+    return s;
+}
+
+// sosfiltfilt's boundary vector zeta_i (mode i = lane & 7) from W, the true forward state of mode i at
+// q*Mf, and C of boundary_sums over seq[0..nseq): w(L-2) = p^(nseq-1) W + C, w(L-1) one step on, and
+// zeta = zhat y_f(L-1) - xi w(L-1), y_f(L-1) = sum_l c_l w_l(L-2) + d seq[nseq-1].  The modes' values
+// are those of lanes 0..7; all 32 lanes must call it.
+__device__ __forceinline__ double2 boundary_zeta(const DevPlan &pl, const double2 *pk, const double2 *seq, int nseq,
+                                                 double2 W, double2 C, int lane)
+{
+    const int i8 = lane & 7;
+    const double2 last = seq[nseq - 1];
+    const double2 wL1 = cfma(pk[(nseq - 1) * 8 + i8], W, C);
+    const double2 wL = cfma(pl.p[i8], wL1, last);
+    double2 part = cmul(pl.c[i8], wL1);
     for (int sft = 1; sft < 8; sft <<= 1) part = cadd(part, shfl_xor_c(part, sft));
     const double2 yfL1 = make_double2(fma(pl.d, last.x, part.x), fma(pl.d, last.y, part.y));
-    e.zeta = cmul(pl.zhat[i], yfL1);
-    for (int l = 0; l < 8; l++) e.zeta = csub(e.zeta, cmul(pl.xi[i * 8 + l], shfl_c(w, l)));
-    return e;
+    double2 za = cmul(pl.zhat[i8], yfL1), zb = make_double2(0.0, 0.0);
+#pragma unroll
+    for (int l = 0; l < 8; l += 2) {
+        za = csub(za, cmul(pl.xi[i8 * 8 + l], shfl_c(wL, l)));
+        zb = csub(zb, cmul(pl.xi[i8 * 8 + l + 1], shfl_c(wL, l + 1)));
+    }
+    return cadd(za, zb);
+}
+
+// The general kernels' head: z = lane n's decoded sample n <= edge, o = the offset at sample 0; the
+// odd extension 2 x[0] - x[edge-j], j < edge, of the corrected rotated samples -> ha.
+__device__ __forceinline__ void head_window(const DevPlan &pl, int r, double2 z, double2 o, double2 *ha, int lane)
+{
+    const int edge = pl.edge;
+    const double2 E = lane <= edge ? pl.Ehead[(size_t)r * (edge + 1) + lane] : make_double2(0.0, 0.0);
+    const double2 x = edge_correct(pl, z, o, edge + 1, 0, E, lane).x;
+    const double2 x0 = shfl_c(x, 0), xa = shfl_c(x, max(0, edge - lane));
+    if (lane < edge) ha[lane] = make_double2(fma(2.0, x0.x, -xa.x), fma(2.0, x0.y, -xa.y));
+    __syncwarp();
+}
+
+// The general kernels' end window: samples ws..N-1 -> s[0..nend), corrected from o, the offset at
+// q*Mf (backward below nend - rem, forward from there), in rounds of 32 that carry the offset, then
+// the tail extension 2 x[N-1] - x[N-2-j], j < edge -> s[nend..nend+edge).  load(j) decodes window
+// sample j.  The end sequence of boundary_sums is s + nend - rem, rem + edge samples long.
+template <class Load>
+__device__ __forceinline__ void end_window(const DevPlan &pl, int r, Load load, double2 o, double2 *s, int lane)
+{
+    const int nend = pl.nend;
+    // a window longer than one round has rem = nend: forward throughout
+    for (int j0 = 0; j0 < nend; j0 += 32) {
+        const int j = j0 + lane;
+        double2 z = make_double2(0.0, 0.0), E = z;
+        if (j < nend) { z = load(j); E = pl.Eend[(size_t)r * nend + j]; }
+        const EdgeSample e = edge_correct(pl, z, o, min(32, nend - j0), nend - pl.rem, E, lane);
+        if (j < nend) s[j] = e.x;
+        o = e.o;
+    }
+    __syncwarp();
+    const double2 xN1 = s[nend - 1];
+    for (int k = lane; k < pl.edge; k += 32) {
+        const double2 b = s[nend - 2 - k];
+        s[nend + k] = make_double2(fma(2.0, xN1.x, -b.x), fma(2.0, xN1.y, -b.y));
+    }
+    __syncwarp();
 }
 
 // Mode i's carries across a chunk's tiles from the state w at one end: forward from tile 0 (the
@@ -676,14 +738,14 @@ __device__ __forceinline__ void block_outputs(const DevPlan &pl, int r, const do
 }
 
 // ----------------------------------------------------------------------------------- k_fixup
-// One CTA per (chunk, row).  Warp 0 stages the head and end-window samples; lanes 0..7 <-> modes run
-// the head, the forward carries, the end segment and zeta, the partial block's output and the
-// backward carries; then all threads emit the outputs at the full-block starts.
+// One CTA per (chunk, row).  Warp 0 runs the chunk boundary: the head and the end window lane <->
+// sample, the boundary sums; lanes 0..7 <-> modes run the forward carries, zeta, the partial block's
+// output and the backward carries; then all threads emit the outputs at the full-block starts.
 template <int ENC>
 __global__ void __launch_bounds__(128)
 k_fixup(const __grid_constant__ DevPlan pl, Scratch sc, const uint8_t *__restrict__ raw, int nchunks)
 {
-    __shared__ double2 s_x[SDRB_NEDGE];    // head samples (edge+1) then end-window samples (nend)
+    __shared__ double2 s_x[SDRB_NEDGE];    // head extension (edge), then end window (nend) + tail extension (edge)
     __shared__ double2 s_zeta[SDRB_NP];
     const int chunk = blockIdx.x / pl.R, r = blockIdx.x % pl.R;
     if (chunk >= nchunks) return;
@@ -694,31 +756,33 @@ k_fixup(const __grid_constant__ DevPlan pl, Scratch sc, const uint8_t *__restric
     double2 *carry = sc.carry + ((size_t)chunk * pl.R + r) * (nt + 1) * 16;
     double2 *yrow = sc.y + ((size_t)chunk * pl.R + r) * pl.M;
     const double2 *T1r = pl.T1 + (size_t)r * nt;
-    double2 *s_h = s_x, *s_e = s_x + (edge + 1);
+    double2 *s_ha = s_x, *s_e = s_x + edge;
 
     if (threadIdx.x < 32) {
         const int lane = threadIdx.x, i = lane & 7;
-        // fetch: raw head samples and the raw end window; every load is independent
-        for (int n = lane; n <= edge; n += 32) s_h[n] = decode_sample<ENC>(pl, rawc, n);
-        for (int j = lane; j < pl.nend; j += 32) s_e[j] = decode_sample<ENC>(pl, rawc, (long)pl.ws + j);
-        __syncwarp();
-        stage_head(pl, r, s_h, offt[0], lane);
-        stage_end(pl, r, s_e, offt[nt], lane);
-        double2 w = head_state(pl, r, s_h, offt[0], i);
+        const bool iq = pl.correct_iq != 0;
+        const double2 o0 = offt[0], oE = offt[nt];
+        head_window(pl, r, lane <= edge ? decode_sample<ENC>(pl, rawc, lane) : make_double2(0.0, 0.0), o0, s_ha, lane);
+        end_window(pl, r, [&](int j) { return decode_sample<ENC>(pl, rawc, (long)pl.ws + j); }, oE, s_e, lane);
+        const double2 *seq = s_e + pl.nend - pl.rem;
+        const int nseq = pl.rem + edge;
+        const BoundarySums bs = boundary_sums(pl, pl.pk, s_ha, edge, seq, nseq, lane);
+        double2 w = iq ? cmul(cfma(pl.alpha[(size_t)r * 8 + i], o0, bs.A), pl.binv[(size_t)r * 8 + i]) : bs.A;
         auto keep = [&](size_t j, double2 v) { carry[j] = v; };
         if (lane < 8) w = tile_carries(pl, T1r, aggr, i, true, pl.beta[(size_t)r * 8 + i], w, keep);
-        const EndState e = end_state(pl, r, s_e, offt[nt], w, i);
-        if (lane < 8) s_zeta[i] = e.zeta;
+        // at q*Mf: the true forward state, and the anticausal state into the T~ frame
+        const double2 sE = iq ? cmul(oE, pl.phE[r]) : make_double2(0.0, 0.0);
+        if (iq) w = csub(cmul(pl.beta[(size_t)r * 8 + i], w), cmul(pl.alpha[(size_t)r * 8 + i], sE));
+        const double2 Tt = iq ? cmul(cfma(pl.alphaT[(size_t)r * 8 + i], sE, bs.B), pl.binvT[(size_t)r * 8 + i]) : bs.B;
+        const double2 zeta = boundary_zeta(pl, pl.pk, seq, nseq, w, bs.C, lane);
+        if (lane < 8) s_zeta[i] = zeta;
         if (pl.rem) {       // the output at the partial block
-            double2 v = cfma(pl.rho[i], e.w, cmul(pl.rho_p[i], e.T));
-            v = cfma(pl.bnd[(size_t)pl.Mf * 8 + i], e.zeta, v);
+            double2 v = cfma(pl.rho[i], w, cmul(pl.rho_p[i], bs.B));
+            v = cfma(pl.bnd[(size_t)pl.Mf * 8 + i], zeta, v);
             for (int sft = 1; sft < 8; sft <<= 1) v = cadd(v, shfl_xor_c(v, sft));
-            if (lane == 0) {
-                const double2 xp = s_e[pl.nend - pl.rem];
-                yrow[pl.Mf] = make_double2(fma(pl.g0, xp.x, v.x), fma(pl.g0, xp.y, v.y));
-            }
+            if (lane == 0) yrow[pl.Mf] = make_double2(fma(pl.g0, seq[0].x, v.x), fma(pl.g0, seq[0].y, v.y));
         }
-        if (lane < 8) tile_carries(pl, T1r, aggr, i, false, pl.betaT[(size_t)r * 8 + i], e.Tt, keep);
+        if (lane < 8) tile_carries(pl, T1r, aggr, i, false, pl.betaT[(size_t)r * 8 + i], Tt, keep);
     }
     __syncthreads();
     block_outputs(pl, r, sc.ypart + ((size_t)chunk * pl.R + r) * pl.Mf, offt, T1r, carry, s_zeta, pl.k_bnd,

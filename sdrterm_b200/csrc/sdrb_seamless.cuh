@@ -10,7 +10,8 @@
 //   k_seam_head    the stream's real start: odd extension and zi, forward state at sample 0
 //   k_seam_fscan   forward modal state across chunks: affine scan with multiplier p^N per mode
 //   k_seam_tail    the stream's real end: anticausal state after the last chunk and zeta
-//                  (k_seam_agg / head / tail / y run k_fixup's chunk-boundary functions, sdrb_kernels.cuh)
+//                  (k_seam_head / tail run the chunk-boundary routines of k_fixup and k_finish, and
+//                  k_seam_agg / y k_fixup's tile carries and outputs, sdrb_kernels.cuh)
 //   k_seam_carry   per emitted chunk: carry-ins in its own frame (forward state, anticausal window
 //                  over the next D chunks or the real end, zeta) and the fm halo y[k+1]
 //   k_seam_y       per emitted chunk: tile carries and the decimated outputs, global frame
@@ -98,14 +99,13 @@ k_seam_agg(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int slot0
 __global__ void __launch_bounds__(32)
 k_seam_head(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int slot)
 {
-    __shared__ double2 s_h[SDRB_NEDGE];
+    __shared__ double2 s_ha[32];           // head extension (edge < 32)
     const int r = blockIdx.x, lane = threadIdx.x;
     const double2 *z = sd.edges + (size_t)slot * sd.nedge;
     const double2 off0 = sc.off_tile[(size_t)slot * (pl.ntiles + 1)];
-    for (int n = lane; n <= pl.edge; n += 32) s_h[n] = z[n];
-    __syncwarp();
-    stage_head(pl, r, s_h, off0, lane);
-    const double2 w = head_state(pl, r, s_h, off0, lane & 7);
+    head_window(pl, r, lane <= pl.edge ? z[lane] : make_double2(0.0, 0.0), off0, s_ha, lane);
+    double2 w = boundary_sums(pl, pl.pk, s_ha, pl.edge, s_ha, 0, lane).A;
+    if (pl.correct_iq) w = cmul(cfma(pl.alpha[(size_t)r * 8 + (lane & 7)], off0, w), pl.binv[(size_t)r * 8 + (lane & 7)]);
     if (lane < 8) sd.fwd[(size_t)r * 8 + lane] = w;
 }
 
@@ -139,18 +139,24 @@ k_seam_fscan(const __grid_constant__ DevPlan pl, SeamDev sd, int slot0, int nch)
 __global__ void __launch_bounds__(32)
 k_seam_tail(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int slot, long long g)
 {
-    __shared__ double2 s_e[SDRB_NEDGE];
+    __shared__ double2 s_e[SDRB_NEDGE];    // end window (nend) + tail extension (edge)
     const int r = blockIdx.x, lane = threadIdx.x, m = lane & 7;
+    const bool iq = pl.correct_iq != 0;
     const double2 *z = sd.edges + (size_t)slot * sd.nedge + pl.edge + 1;
     const double2 offE = sc.off_tile[(size_t)slot * (pl.ntiles + 1) + pl.ntiles];
-    for (int j = lane; j < pl.nend; j += 32) s_e[j] = z[j];
-    __syncwarp();
-    stage_end(pl, r, s_e, offE, lane);
-    const double2 ph = seam_phasor(sd, r, g);
-    const EndState e = end_state(pl, r, s_e, offE, cmul(cconj(ph), sd.fwd[(size_t)r * 8 + m]), m);
+    end_window(pl, r, [&](int j) { return z[j]; }, offE, s_e, lane);
+    const double2 *seq = s_e + pl.nend - pl.rem;
+    const int nseq = pl.rem + pl.edge;
+    const BoundarySums bs = boundary_sums(pl, pl.pk, seq, 0, seq, nseq, lane);
+    // at q*Mf: the true forward state, and the anticausal state into the T~ frame
+    const double2 ph = seam_phasor(sd, r, g), sE = iq ? cmul(offE, pl.phE[r]) : make_double2(0.0, 0.0);
+    double2 w = cmul(cconj(ph), sd.fwd[(size_t)r * 8 + m]);
+    if (iq) w = csub(cmul(pl.beta[(size_t)r * 8 + m], w), cmul(pl.alpha[(size_t)r * 8 + m], sE));
+    const double2 Tt = iq ? cmul(cfma(pl.alphaT[(size_t)r * 8 + m], sE, bs.B), pl.binvT[(size_t)r * 8 + m]) : bs.B;
+    const double2 zeta = boundary_zeta(pl, pl.pk, seq, nseq, w, bs.C, lane);
     if (lane < 8) {
-        sd.endv[(size_t)r * 16 + m] = cmul(ph, e.Tt);
-        sd.endv[(size_t)r * 16 + 8 + m] = cmul(ph, e.zeta);
+        sd.endv[(size_t)r * 16 + m] = cmul(ph, Tt);
+        sd.endv[(size_t)r * 16 + 8 + m] = cmul(ph, zeta);
     }
 }
 

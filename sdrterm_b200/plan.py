@@ -167,7 +167,7 @@ class Plan:
     Ec: np.ndarray         # (4, Hq) complex: even-part coefficients, upper poles
     Oc: np.ndarray         # (4, Hq) complex: odd-part coefficients
     Ppow: np.ndarray       # (TILE_BLOCKS+1, 8) P^l
-    Pk: np.ndarray         # (edge+1, 8) p^k
+    Pk: np.ndarray         # (max(edge+1, edge+rem), 8) p^k
     Pt: np.ndarray         # (ntiles, 8) p^(q*TILE_BLOCKS*m)
     bx: np.ndarray         # (8,) p^edge / kappa
     bnd: np.ndarray        # (M, 8) c_i p_i^(L-1-n_k)
@@ -312,7 +312,7 @@ def build_plan(fs: int, enc: str, dec: int, rows_hz, *, simo: bool = False, swap
                 Ec[m, j] = _c((pm[m] ** (q - 1 - j) + pm[m] ** j) / 2)
                 Oc[m, j] = _c((pm[m] ** (q - 1 - j) - pm[m] ** j) / 2)
     Ppow = np.array([[_c(pm[i] ** (q * l)) for i in range(n8)] for l in range(TILE_BLOCKS + 1)])
-    Pk = np.array([[_c(pm[i] ** k) for i in range(n8)] for k in range(edge + 1)])
+    Pk = np.array([[_c(pm[i] ** k) for i in range(n8)] for k in range(max(edge + 1, edge + rem))])
     Pt = np.array([[_c(pm[i] ** (q * TILE_BLOCKS * m_)) for i in range(n8)] for m_ in range(ntiles)])
     bx = np.array([_c(pm[i] ** edge / mp.mpc(modes.kappa[i])) for i in range(n8)])
     # boundary weights c_i p_i^(L-1-n_k), n_k = edge + q k

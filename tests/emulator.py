@@ -6,7 +6,8 @@ algorithm and every table against the oracle without a GPU.  Structure mirrors t
                             UNcorrected samples, IQ-EMA block aggregates, tile-local scans, partial
                             outputs + tile aggregates; the IQ corrector enters only through the
                             decoupled terms of DESIGN.md 3.3)
-  emu_fixup   <-> k_fixup  (head / end segments, cross-tile carries, boundary term -> decimated y)
+  emu_fixup   <-> k_fixup  (head / end segments, cross-tile carries, boundary term -> decimated y);
+                emu_head / emu_end: the chunk boundary, also the seamless twin's stream ends
   emu_demod   <-> k_demod  (fm pair-phase + 2x FFT interpolation | am | re | im, output SOS)
 """
 import numpy as np
@@ -139,89 +140,107 @@ def emu_main(pl: Plan, z: np.ndarray):
     return dict(ypart=ypart, Wout=Wout, Tin=Tin, tile_agg=tile_agg)
 
 
+def emu_head(pl: Plan, z: np.ndarray, off0: complex) -> np.ndarray:
+    """(R, 8) forward state at n = edge from the head samples z[0..edge] (IQ-corrected forward from
+    off0, the offset at sample 0; odd extension, zi), in the frame of the uncorrected samples:
+    W~ = (w + alpha s) / beta with s = off0."""
+    m, edge = pl.modes, pl.edge
+    o = off0
+    xh = np.empty(edge + 1, dtype=np.complex128)
+    for n in range(edge + 1):
+        xh[n] = z[n] - o
+        o = o + xh[n] * pl.Liq
+    W = np.zeros((pl.R, 8), dtype=np.complex128)
+    for r in range(pl.R):
+        xs = xh * pl.Ehead[r]
+        ext = 2 * xs[0] - xs[edge:0:-1]
+        w = m.zhat * ext[0]
+        for j in range(edge):
+            w = m.p * w + ext[j]
+        W[r] = (w + pl.alpha[r] * off0) / pl.beta[r]
+    return W
+
+
+def emu_end(pl: Plan, z: np.ndarray, offE: complex, Wt: np.ndarray) -> dict:
+    """The chunk's end from the samples z[ws..N-1], offE, the offset at q*Mf, and Wt (R, 8), the
+    forward state at q*Mf as W~.  Per row (R, 8): the true forward state w at q*Mf, the anticausal
+    state T there and T~ = (T + alphaT s) / betaT, zeta; x0 (R,), the first sample of the partial
+    block, corrected and rotated; off, the offset after the chunk."""
+    q, Mf, N, edge = pl.q, pl.Mf, pl.N, pl.edge
+    m, p = pl.modes, pl.modes.p
+    # corrected end-window samples ws..N-1: inside full blocks BACKWARD from the offset at q*Mf
+    # (off[n] = (off[n+1] - L z[n]) / lam), in the partial block forward from it
+    xe = np.empty(pl.nend, dtype=np.complex128)
+    o = offE
+    for n in range(q * Mf - 1, pl.ws - 1, -1):
+        o = (o - pl.Liq * z[n]) * pl.lam_inv
+        xe[n - pl.ws] = z[n] - o
+    o = offE
+    for n in range(q * Mf, N):
+        xe[n - pl.ws] = z[n] - o
+        o = o + xe[n - pl.ws] * pl.Liq
+    e = {k: np.zeros((pl.R, 8), dtype=np.complex128) for k in ('w', 'T', 'Tt', 'zeta')}
+    e['x0'] = np.zeros(pl.R, dtype=np.complex128)
+    e['off'] = o
+    for r in range(pl.R):
+        xs_e = xe * pl.Eend[r]
+        sE = offE * pl.phE[r]                      # rotated offset at sample q*Mf
+        w = pl.beta[r] * Wt[r] - pl.alpha[r] * sE
+        e['w'][r] = w
+        # end segment: partial block (rem samples) + tail extension
+        tail = 2 * xs_e[-1] - xs_e[-2:-(edge + 2):-1]
+        part = xs_e[pl.nend - pl.rem:] if pl.rem else xs_e[:0]
+        seq = np.concatenate([part, tail])
+        e['x0'][r] = seq[0]
+        for v in seq[:-1]:
+            w = p * w + v
+        wL1 = w
+        wL = p * w + seq[-1]
+        e['zeta'][r] = m.zhat * (np.sum(m.c * wL1) + m.d * seq[-1]) - m.xi @ wL
+        T = np.zeros(8, dtype=np.complex128)
+        for v in seq[::-1]:
+            T = p * T + v
+        e['T'][r] = T                              # anticausal state at n = edge + q*Mf
+        e['Tt'][r] = (T + pl.alphaT[r] * sE) / pl.betaT[r]
+    return e
+
+
 def emu_fixup(pl: Plan, z: np.ndarray, mo: dict, off_chunk: complex):
     """One chunk, all rows: (R, M) decimated complex + offset after the chunk."""
-    q, Mf, nt, edge, N = pl.q, pl.Mf, pl.ntiles, pl.edge, pl.N
+    Mf, nt = pl.Mf, pl.ntiles
     m = pl.modes
-    p, P = m.p, pl.P
     # offsets at tile starts
     off_tile = np.zeros(nt + 1, dtype=np.complex128)
     off_tile[0] = off_chunk
     for t in range(nt):
         kind = 1 if t == nt - 1 else 0
-        cnt = pl.cnt_last if kind else TILE_BLOCKS
         off_tile[t + 1] = pl.lam_tile[kind] * off_tile[t] + mo['tile_agg'][t] if Mf else off_chunk
-        _ = cnt
-    # corrected head samples 0..edge (reference recurrence from the chunk-start offset)
-    o = off_chunk
-    xh = np.empty(edge + 1, dtype=np.complex128)
-    for n in range(edge + 1):
-        xh[n] = z[n] - o
-        o = o + xh[n] * pl.Liq
-    # corrected end-window samples ws..N-1: inside full blocks BACKWARD from the offset at q*Mf
-    # (off[n] = (off[n+1] - L z[n]) / lam), in the partial block forward from it
-    xe = np.empty(pl.nend, dtype=np.complex128)
-    o = off_tile[nt]
-    for n in range(q * Mf - 1, pl.ws - 1, -1):
-        o = (o - pl.Liq * z[n]) * pl.lam_inv
-        xe[n - pl.ws] = z[n] - o
-    o = off_tile[nt]                       # offset at sample q*Mf
-    for n in range(q * Mf, N):
-        xe[n - pl.ws] = z[n] - o
-        o = o + xe[n - pl.ws] * pl.Liq
-    off_after = o
-    if pl.rem == 0:
-        off_after = off_tile[nt]
+    W0 = emu_head(pl, z, off_chunk)
+    s = -off_tile[:nt]
+    # forward across tiles, in the frame of the uncorrected samples (W~)
+    Win = np.zeros((pl.R, nt + 1, 8), dtype=np.complex128)
+    Win[:, 0] = W0
+    for r in range(pl.R):
+        for t in range(nt):
+            cnt = pl.cnt_last if t == nt - 1 else TILE_BLOCKS
+            Win[r, t + 1] = pl.Ppow[cnt] * Win[r, t] + pl.T1[r, t] * mo['Wout'][r, t]
+    e = emu_end(pl, z, off_tile[nt], Win[:, nt])
+    off_after = e['off'] if pl.rem else off_tile[nt]
     y = np.zeros((pl.R, pl.M), dtype=np.complex128)
     for r in range(pl.R):
-        xs_h = xh * pl.Ehead[r]
-        xs_e = xe * pl.Eend[r]
-        # head: odd extension, zi, edge samples
-        ext = 2 * xs_h[0] - xs_h[edge:0:-1]
-        w = m.zhat * ext[0]
-        for j in range(edge):
-            w = p * w + ext[j]
-        # forward across tiles, in the frame of the uncorrected samples: W~ = (w + alpha s) / beta
-        # with s = off e^{jwn} (n = 0: the chunk-start offset itself)
-        Win = np.zeros((nt + 1, 8), dtype=np.complex128)
-        Win[0] = (w + pl.alpha[r] * off_chunk) / pl.beta[r]
-        s = -off_tile[:nt]
-        for t in range(nt):
-            kind = 1 if t == nt - 1 else 0
-            cnt = pl.cnt_last if kind else TILE_BLOCKS
-            Win[t + 1] = pl.Ppow[cnt] * Win[t] + pl.T1[r, t] * mo['Wout'][r, t]
-        sE = off_tile[nt] * pl.phE[r]              # rotated offset at sample q*Mf
-        w_end = pl.beta[r] * Win[nt] - pl.alpha[r] * sE
-        # end segment: partial block (rem samples) + tail extension
-        xN1 = xs_e[-1]
-        tail = 2 * xN1 - xs_e[-2:-(edge + 2):-1]
-        part = xs_e[pl.nend - pl.rem:] if pl.rem else xs_e[:0]
-        seq = np.concatenate([part, tail])
-        w = w_end.copy()
-        wL1 = None
-        for i, v in enumerate(seq):
-            if i == len(seq) - 1:
-                wL1 = w.copy()
-            w = p * w + v
-        wL = w
-        yfL1 = np.sum(m.c * wL1) + m.d * seq[-1]
-        zeta = m.zhat * yfL1 - m.xi @ wL
-        T = np.zeros(8, dtype=np.complex128)
-        for v in seq[::-1]:
-            T = p * T + v
-        Tend = T                                   # anticausal state at n = edge + q*Mf
+        zeta = e['zeta'][r]
         if pl.rem:
             k = Mf
-            y[r, k] = (np.sum(m.rho * w_end) + np.sum(m.rho_p * Tend) + m.g0 * part[0]
+            y[r, k] = (np.sum(m.rho * e['w'][r]) + np.sum(m.rho_p * e['T'][r]) + m.g0 * e['x0'][r]
                        + np.sum(pl.bnd[k] * zeta))
         # backward across tiles
         Tn = np.zeros((nt + 1, 8), dtype=np.complex128)
-        Tn[nt] = (Tend + pl.alphaT[r] * sE) / pl.betaT[r]
+        Tn[nt] = e['Tt'][r]
         for t in range(nt - 1, -1, -1):
             kind = 1 if t == nt - 1 else 0
             cnt = pl.cnt_last if kind else TILE_BLOCKS
             Tn[t] = pl.Ppow[cnt] * Tn[t + 1] + pl.T1[r, t] * mo['Tin'][r, t]
-        Wc, Tc = pl.beta[r][None, :] * Win, pl.betaT[r][None, :] * Tn      # carries as the kernels keep them
+        Wc, Tc = pl.beta[r][None, :] * Win[r], pl.betaT[r][None, :] * Tn      # carries as the kernels keep them
         for t in range(nt):
             kind = 1 if t == nt - 1 else 0
             cnt = pl.cnt_last if kind else TILE_BLOCKS

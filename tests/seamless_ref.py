@@ -112,51 +112,12 @@ class SeamlessTwin:
 
     def _head(self, c) -> np.ndarray:
         """Forward state at sample 0 of the stream (odd extension, zi), frame of the uncorrected samples."""
-        pl, m = self.pl, self.pl.modes
-        edge = pl.edge
-        o = c['offt'][0]
-        xh = np.empty(edge + 1, dtype=np.complex128)
-        for n in range(edge + 1):
-            xh[n] = c['z'][n] - o
-            o = o + xh[n] * pl.Liq
-        G = np.zeros((pl.R, 8), dtype=np.complex128)
-        for r in range(pl.R):
-            xs = xh * pl.Ehead[r]
-            ext = 2 * xs[0] - xs[edge:0:-1]
-            w = m.zhat * ext[0]
-            for j in range(edge):
-                w = m.p * w + ext[j]
-            G[r] = (w + pl.alpha[r] * c['offt'][0]) / pl.beta[r]
-        return G
+        return emu.emu_head(self.pl, c['z'], c['offt'][0])
 
     def _tail(self, c, Gend):
         """True end of the stream: anticausal state after the last chunk and zeta (global frame)."""
-        pl, m = self.pl, self.pl.modes
-        q, Mf, edge = pl.q, pl.Mf, pl.edge
-        z = c['z']
-        xe = np.empty(pl.nend, dtype=np.complex128)
-        o = c['offt'][pl.ntiles]
-        for n in range(q * Mf - 1, pl.ws - 1, -1):
-            o = (o - pl.Liq * z[n]) * pl.lam_inv
-            xe[n - pl.ws] = z[n] - o
-        E = np.zeros((pl.R, 8), dtype=np.complex128)
-        Z = np.zeros((pl.R, 8), dtype=np.complex128)
-        for r in range(pl.R):
-            xs = xe * pl.Eend[r]
-            sE = c['offt'][pl.ntiles] * pl.phE[r]
-            w = pl.beta[r] * (np.conj(c['phi'][r]) * Gend[r]) - pl.alpha[r] * sE
-            seq = 2 * xs[-1] - xs[-2:-(edge + 2):-1]
-            for v in seq[:-1]:
-                w = m.p * w + v
-            wL1 = w
-            wL = m.p * w + seq[-1]
-            zeta = m.zhat * (np.sum(m.c * wL1) + m.d * seq[-1]) - m.xi @ wL
-            T = np.zeros(8, dtype=np.complex128)
-            for v in seq[::-1]:
-                T = m.p * T + v
-            E[r] = c['phi'][r] * (T + pl.alphaT[r] * sE) / pl.betaT[r]
-            Z[r] = c['phi'][r] * zeta
-        return E, Z
+        e = emu.emu_end(self.pl, c['z'], c['offt'][self.pl.ntiles], np.conj(c['phi'])[:, None] * Gend)
+        return c['phi'][:, None] * e['Tt'], c['phi'][:, None] * e['zeta']
 
     # -- one chunk's decimated output (global frame) with its carry-ins, plus the halo sample
     def _y(self, i, end):

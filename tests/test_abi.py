@@ -79,7 +79,8 @@ def test_create_refuses_inconsistent_plans_before_touching_the_device():
     assert fm_d50.fm_interp is not None and seamless.lookahead >= 1
     for pl, problem in ((dataclasses.replace(fm, RL=fm.RL + 1), 'RL'),
                         (dataclasses.replace(fm_d50, fm_interp=None), 'dense interpolation table'),
-                        (dataclasses.replace(seamless, lookahead=0), 'lookahead')):
+                        (dataclasses.replace(seamless, lookahead=0), 'lookahead'),
+                        (dataclasses.replace(fm, edge=32), 'filter pad 32')):     # the head is one warp of samples
         with pytest.raises(nat.SdrbError, match=f'error -1: .*{problem}'):
             Engine(pl, max_chunks=1, use_tc=False)
 

@@ -234,6 +234,7 @@ def test_file_sharded_entry_point_single_process(tmp_path):
     ('b', 3, 're', True, False, 10000),      # the smallest odd block
     ('i', 50, 'fm', True, False, 15000),     # even but ragged (rem != 0), 32-bit integers
     ('d', 10, 'am', False, False, 5000),     # float64 samples (16 bytes per sample)
+    ('h', 200, 're', True, False, 20000),    # rem = 168: the IQ-corrected end window runs in rounds of 32
 ])
 def test_fp64_block_kernel_odd_and_ragged_blocks(enc, q, demod, iq, norm, center):
     """k_main keeps the raw tile in fragment order (sample j beside its mirror q-1-j, DESIGN 3.5):
