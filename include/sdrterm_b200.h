@@ -319,6 +319,37 @@ int sdrb_stream_device(sdrb_handle *h, const void *raw_dev, size_t nchunks, doub
 int sdrb_stream_end(sdrb_handle *h, double *out_host, size_t *nchunks_out);
 int sdrb_stream_end_device(sdrb_handle *h, double *out_dev, void *stream, size_t *nchunks_out);
 int sdrb_stream_lookahead(const sdrb_handle *h);
+/* Sample-granular seamless streaming: any whole number of complex samples per call, for every q.
+ * The handle's "chunk" (cfg.N) is then the seamless FRAME, a whole number of tiles (plan.py
+ * seamless_frame_samples: 32 q floor(N_reader / (32 q)); the reader's chunk itself for a power-of-two
+ * q).  The handle keeps the samples that do not fill a frame (fewer than N) on the device, in front
+ * of the next call's samples; whole frames go through the sdrb_stream machinery.  Outputs are
+ * counted per row: *nout outputs per row, `out` is [row][*nout * W / M] doubles, contiguous per row
+ * (for whole frames exactly the [row][chunk][W] layout of sdrb_stream).
+ *   sdrb_stream_samples         host `raw` of nsamples samples (at most max_chunks * N), synchronous
+ *   sdrb_stream_samples_device  the same from a device buffer (one device-to-device copy into the
+ *                               handle's window), only enqueued on `stream`
+ *   sdrb_stream_samples_end     end of stream: the frames still held back and the partial last frame
+ *                               (ceil(Lp / q) outputs from its Lp samples; scipy.signal.decimate's last
+ *                               output of a ragged stream), then a reset.  A stream of 27 samples or
+ *                               fewer (the decimator's pad length) is refused with SDRB_ERR_ARG.
+ *   sdrb_stream_samples_end_device  the same into a device buffer
+ *   sdrb_stream_capacity        the most outputs per row that a sdrb_stream_samples* call with
+ *                               `nsamples` new samples, or an end call, can emit (size `out` by it)
+ * A stream takes its input either in chunks (sdrb_stream*) or in samples (sdrb_stream_samples*): an
+ * input call of the other kind returns SDRB_ERR_STATE until the stream ends, and so does
+ * sdrb_stream_end while samples of a partial frame are pending.  An fm stream of at most q samples
+ * (one output, no discriminator pair) is refused with SDRB_ERR_ARG at its end.
+ * The first sample call allocates the handle's two raw windows ((max_chunks + 1) * N samples each).
+ * An end call with a partial frame derives that frame's tables on the host and copies them from
+ * pageable memory, which synchronises `stream` before the copy; the other sample calls only
+ * enqueue. */
+int sdrb_stream_samples(sdrb_handle *h, const void *raw_host, size_t nsamples, double *out_host, size_t *nout);
+int sdrb_stream_samples_device(sdrb_handle *h, const void *raw_dev, size_t nsamples, double *out_dev, void *stream,
+                               size_t *nout);
+int sdrb_stream_samples_end(sdrb_handle *h, double *out_host, size_t *nout);
+int sdrb_stream_samples_end_device(sdrb_handle *h, double *out_dev, void *stream, size_t *nout);
+size_t sdrb_stream_capacity(const sdrb_handle *h, size_t nsamples);
 
 const char *sdrb_global_error(void);
 

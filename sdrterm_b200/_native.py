@@ -67,7 +67,9 @@ EXPORTS = ['sdrb_create', 'sdrb_destroy', 'sdrb_last_error', 'sdrb_outputs_per_c
            'sdrb_set_profiling', 'sdrb_kernel_times', 'sdrb_keep_decimated', 'sdrb_read_debug', 'sdrb_iq_export_device',
            'sdrb_iq_prefix_device', 'sdrb_decode_iq', 'sdrb_correct_iq', 'sdrb_keep_x0', 'sdrb_read_x0', 'sdrb_iq_gain', 'sdrb_set_smooth', 'sdrb_host_alloc', 'sdrb_host_free', 'sdrb_reserve_sms',
            'sdrb_stream', 'sdrb_stream_device', 'sdrb_stream_end', 'sdrb_stream_end_device', 'sdrb_stream_lookahead',
-           'sdrb_row_doubles', 'sdrb_iq_output', 'sdrb_ssb_demod']
+           'sdrb_row_doubles', 'sdrb_iq_output', 'sdrb_ssb_demod',
+           'sdrb_stream_samples', 'sdrb_stream_samples_device', 'sdrb_stream_samples_end',
+           'sdrb_stream_samples_end_device', 'sdrb_stream_capacity']
 
 
 def nvcc_command(out: str = LIB_PATH) -> list[str]:
@@ -145,6 +147,12 @@ def lib():
         L.sdrb_stream_end.argtypes = [vp, vp, szp]
         L.sdrb_stream_end_device.argtypes = [vp, vp, vp, szp]
         L.sdrb_stream_lookahead.argtypes = [vp]
+        L.sdrb_stream_samples.argtypes = [vp, vp, sz, vp, szp]
+        L.sdrb_stream_samples_device.argtypes = [vp, vp, sz, vp, vp, szp]
+        L.sdrb_stream_samples_end.argtypes = [vp, vp, szp]
+        L.sdrb_stream_samples_end_device.argtypes = [vp, vp, vp, szp]
+        L.sdrb_stream_capacity.argtypes = [vp, sz]
+        L.sdrb_stream_capacity.restype = sz
         _lib = L
     return _lib
 

@@ -69,6 +69,17 @@ struct sdrb_handle {
     SeamDev sd{};
     long long seen = 0, emitted = 0;   // chunks of the current stream taken in / emitted
     int nwin = 0;
+    // sample-granular input (sdrb_stream_samples*): two raw windows, each `hist` samples of the
+    // stream before the frame start (a short last frame's end window reaches back into them), then
+    // the `pend` samples of the partial frame, then a call's new samples
+    uint8_t *rawwin[2] = {nullptr, nullptr};
+    int wsel = 0, hist = 0;
+    size_t pend = 0;
+    int feed = 0;                   // input kind of the current stream: 0 none yet, FEED_CHUNKS, FEED_SAMPLES
+    // host copies of the tables a ragged last frame derives its own from, and that frame's tables
+    std::vector<double2> h_pk, h_Ppow, h_Pt, h_bnd, h_T1, h_T2, h_T3, h_rag;
+    std::vector<double> h_lamj;
+    double2 *d_rag = nullptr;       // [16] p^Lp, p^(q Mf); [R] phE; [R][nend] Eend; [M][8] bnd; [R][ntiles] T1
 };
 
 namespace {
@@ -301,9 +312,8 @@ int setup_tc(sdrb_handle *h, const sdrb_tables *tab)
 
 template <int ENC, bool IQ>
 int launch_chain_t(sdrb_handle *h, const Scratch &sc, const uint8_t *raw, size_t nch, double *out, cudaStream_t st,
-                   int phases)
+                   int phases, const DevPlan &pl)
 {
-    const DevPlan &pl = h->pl;
     const bool prof = h->profiling && phases == PH_ALL;
     auto mark = [&](int i) {
         if (prof) { cudaEventRecord(h->pev[i], st); h->pev_valid[i] = true; }
@@ -311,7 +321,7 @@ int launch_chain_t(sdrb_handle *h, const Scratch &sc, const uint8_t *raw, size_t
     if (prof) for (int i = 0; i < 5; i++) h->pev_valid[i] = false;
     mark(0);
     if (phases & PH_MAIN) {
-        if (h->tc_on && ((uintptr_t)raw & 15) == 0) {
+        if (h->tc_on && &pl == &h->pl && ((uintptr_t)raw & 15) == 0) {
             int rc = launch_tc<IQ>(h, sc, raw, nch, st);
             if (rc) return rc;
         } else {
@@ -364,13 +374,15 @@ int launch_chain_t(sdrb_handle *h, const Scratch &sc, const uint8_t *raw, size_t
 }
 
 // The kernel chain over `nch` chunks on the scratch view `sc` (seamless mode: a window of h->sc).
+// `plan` other than the handle's: a seamless stream's ragged last frame, on the FP64 front end.
 int launch_chain(sdrb_handle *h, const Scratch &sc, const uint8_t *raw, size_t nch, double *out, cudaStream_t st,
-                 int phases = PH_ALL)
+                 int phases = PH_ALL, const DevPlan *plan = nullptr)
 {
+    const DevPlan &pl = plan ? *plan : h->pl;
     return with_enc(h, h->enc_code, [&](auto enc) {
         constexpr int E = decltype(enc)::value;
-        return h->pl.correct_iq ? launch_chain_t<E, true>(h, sc, raw, nch, out, st, phases)
-                                : launch_chain_t<E, false>(h, sc, raw, nch, out, st, phases);
+        return h->pl.correct_iq ? launch_chain_t<E, true>(h, sc, raw, nch, out, st, phases, pl)
+                                : launch_chain_t<E, false>(h, sc, raw, nch, out, st, phases, pl);
     });
 }
 
@@ -649,7 +661,29 @@ int seam_setup(sdrb_handle *h, const sdrb_tables *tab, size_t nch)
     SeamDev &sd = h->sd;
     const size_t R = pl.R, M = pl.M;
     const size_t sn = (size_t)SEAM_NS * (is_ssb(pl.demod) ? 2 : 1);   // doubles per SOS state (usb / lsb: complex)
-    sd.D = tab->lookahead; sd.fs = tab->fs; sd.nedge = pl.edge + 1 + pl.nend;
+    sd.D = tab->lookahead; sd.fs = tab->fs; sd.nedge = pl.edge + 1 + std::max(pl.nend, pl.q - 1);
+    // what a ragged last frame derives its tables from (seam_ragged_plan)
+    auto keep = [](const double *a, size_t n) {
+        std::vector<double2> v(n);
+        for (size_t i = 0; i < n; i++) v[i] = c2(a, i);
+        return v;
+    };
+    // pk up to edge + q - 1 (a ragged last frame's partial block): p^k = p^(k-edge) p^edge for k > edge
+    const size_t npk = (size_t)pl.edge + pl.q;
+    h->h_pk = keep(tab->pk, (size_t)(pl.edge + 1) * 8);
+    h->h_pk.resize(npk * 8);
+    for (size_t k = pl.edge + 1; k < npk; k++)
+        for (int i = 0; i < 8; i++)
+            h->h_pk[k * 8 + i] = hmul(h->h_pk[(k - pl.edge) * 8 + i], h->h_pk[(size_t)pl.edge * 8 + i]);
+    h->h_Ppow = keep(tab->Ppow, (size_t)(SDRB_TB + 1) * 8);
+    h->h_Pt = keep(tab->Pt, (size_t)pl.ntiles * 8);
+    h->h_bnd = keep(tab->bnd, M * 8);
+    h->h_T1 = keep(tab->T1, R * pl.ntiles);
+    h->h_T2 = keep(tab->T2, R * pl.q);
+    h->h_T3 = keep(tab->T3, R * (SDRB_TB + 1));
+    h->h_lamj.assign(tab->lam_j, tab->lam_j + pl.q + 1);
+    h->h_rag.resize(16 + R + R * (size_t)(sd.nedge - pl.edge - 1) + M * 8 + R * pl.ntiles);
+    h->hist = (pl.edge + 1 + 15) / 16 * 16;     // keeps the frames 16-byte aligned (k_tc)
     if (pl.nsec_out)
         for (int i = 0; i < SEAM_NS * SEAM_NS; i++) sd.AM[i] = tab->sos_AM[i];
     int rc;
@@ -665,7 +699,9 @@ int seam_setup(sdrb_handle *h, const sdrb_tables *tab, size_t nch)
         (rc = dalloc(h, nch * R * sn, &sd.sst)) ||
         (rc = dalloc(h, R * 8, &sd.fwd)) ||
         (rc = dalloc(h, R * sn, &sd.sos)) ||
-        (rc = dalloc(h, R * 16, &sd.endv)))
+        (rc = dalloc(h, R * 16, &sd.endv)) ||
+        (rc = dalloc(h, h->h_rag.size(), &h->d_rag)) ||
+        (rc = upload(h, h->h_pk.data(), h->h_pk.size(), &h->pl.pk)))
         return rc;
     CK(h, cudaMemset(sd.sos, 0, R * sn * sizeof(double)));
     return 0;
@@ -747,6 +783,7 @@ int sdrb_destroy(sdrb_handle *h)
     cudaDeviceSynchronize();
     for (void *p : h->owned) cudaFree(p);
     for (int s = 0; s < 2; s++) {
+        if (h->rawwin[s]) cudaFree(h->rawwin[s]);
         if (h->slot[s].raw) cudaFree(h->slot[s].raw);
         if (h->slot[s].out) cudaFree(h->slot[s].out);
         if (h->slot[s].stream) cudaStreamDestroy(h->slot[s].stream);
@@ -871,6 +908,62 @@ int seam_shift(sdrb_handle *h, T *buf, size_t per, int from, int n, cudaStream_t
     return 0;
 }
 
+// A new stream starts from scratch: counters, pending samples, output filter and IQ corrector.
+enum { FEED_CHUNKS = 1, FEED_SAMPLES = 2 };
+
+// One input kind per stream: chunks and samples keep different raw windows (the ragged end reads
+// the samples before the pending ones from the sample window).
+int seam_feed(sdrb_handle *h, int kind, size_t n)
+{
+    if (!n) return 0;
+    if (h->feed && h->feed != kind)
+        return fail(h, SDRB_ERR_STATE, "this stream takes its input in %s: end it before feeding %s",
+                    h->feed == FEED_CHUNKS ? "chunks (sdrb_stream*)" : "samples (sdrb_stream_samples*)",
+                    kind == FEED_CHUNKS ? "chunks" : "samples");
+    h->feed = kind;
+    return 0;
+}
+
+int seam_reset(sdrb_handle *h, cudaStream_t st)
+{
+    h->seen = h->emitted = 0;
+    h->nwin = 0;
+    h->pend = 0;
+    h->feed = 0;
+    CK(h, cudaMemsetAsync(h->sd.sos, 0, (size_t)h->pl.R * SEAM_NS * (is_ssb(h->pl.demod) ? 2 : 1) * sizeof(double), st));
+    CK(h, cudaMemsetAsync(h->sc.iq_state, 0, sizeof(double2), st));
+    return 0;
+}
+
+// The scratch and the seamless buffers seen from window slot s on (whole-frame strides).
+Scratch seam_scratch_at(const sdrb_handle *h, int s)
+{
+    const DevPlan &pl = h->pl;
+    const size_t R = pl.R, nt = pl.ntiles;
+    Scratch v = h->sc;
+    v.ypart += (size_t)s * R * pl.Mf;
+    v.agg += (size_t)s * R * nt * 16;
+    v.tile_agg += (size_t)s * nt;
+    v.off_tile += (size_t)s * (nt + 1);
+    v.gain += s;
+    v.start += s;
+    v.carry += (size_t)s * R * (nt + 1) * 16;
+    return v;
+}
+SeamDev seam_dev_at(const sdrb_handle *h, int s)
+{
+    const size_t R = h->pl.R, M = h->pl.M, sn = (size_t)SEAM_NS * (is_ssb(h->pl.demod) ? 2 : 1);
+    SeamDev v = h->sd;
+    v.edges += (size_t)s * v.nedge;
+    v.cagg += (size_t)s * R * 16;
+    v.G += (size_t)s * R * 8;
+    v.cin += (size_t)s * R * 24;
+    v.ybuf += (size_t)s * R * (M + 1);
+    v.echunk += (size_t)s * R * sn;
+    v.sst += (size_t)s * R * sn;
+    return v;
+}
+
 // One seamless step: the front end and the IQ kernels over `nch` new chunks (into the window slots
 // after the held-back ones), the chunk aggregates and the forward scan; then every chunk that is
 // final (all of them when `end`) goes through carry / outputs / demodulation / SOS into `out`.
@@ -882,14 +975,7 @@ int seam_step(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, cudaS
     int rc = 0;
     if (nch) {
         const int s0 = h->nwin;
-        Scratch sh = h->sc;    // the window from slot s0 on
-        sh.ypart += (size_t)s0 * R * pl.Mf;
-        sh.agg += (size_t)s0 * R * nt * 16;
-        sh.tile_agg += (size_t)s0 * nt;
-        sh.off_tile += (size_t)s0 * (nt + 1);
-        sh.gain += s0;
-        sh.start += s0;
-        rc = launch_chain(h, sh, raw, nch, nullptr, st, PH_MAIN | PH_IQSCAN);
+        rc = launch_chain(h, seam_scratch_at(h, s0), raw, nch, nullptr, st, PH_MAIN | PH_IQSCAN);
         if (rc) return rc;
         rc = with_enc(h, h->enc_code, [&](auto enc) {
             launch(h, k_seam_edges<decltype(enc)::value>, (unsigned)nch, 64, 0, st, pl, sd, raw, s0, (int)nch);
@@ -915,12 +1001,12 @@ int seam_step(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, cudaS
         with_out(pl.demod, [&](auto ok) {
             // usb / lsb run the complex SOS state; real and iq rows the real one
             constexpr bool SSB = decltype(ok)::value == OUT_SSB;
-            launch(h, k_seam_demod<SSB>, wg, 256, 0, st, pl, sd, out, ne, h->nwin, end ? 1 : 0);
+            launch(h, k_seam_demod<SSB>, wg, 256, 0, st, pl, sd, out, ne, h->nwin, end ? 1 : 0, (size_t)ne * M);
             if (pl.nsec_out) {
                 const size_t total = items * M;
                 const unsigned fg = (unsigned)std::min<size_t>((total + 255) / 256, (size_t)h->num_sms * 16);
                 launch(h, k_seam_sscan<std::conditional_t<SSB, double2, double>>, (unsigned)R, 32, 0, st, pl, sd, ne);
-                launch(h, k_seam_frame<SSB>, fg, 256, 0, st, pl, sd, out, ne);
+                launch(h, k_seam_frame<SSB>, fg, 256, 0, st, pl, sd, out, (size_t)ne * M);
             }
             return 0;
         });
@@ -939,22 +1025,191 @@ int seam_step(sdrb_handle *h, const uint8_t *raw, size_t nch, double *out, cudaS
     }
     CK(h, cudaGetLastError());
     if (nout) *nout = (size_t)std::max(ne, 0);
-    if (end) {   // a new stream starts from scratch: counters, output filter and IQ corrector
-        h->seen = h->emitted = 0;
-        h->nwin = 0;
-        CK(h, cudaMemsetAsync(sd.sos, 0, (size_t)R * SEAM_NS * (is_ssb(pl.demod) ? 2 : 1) * sizeof(double), st));
-        CK(h, cudaMemsetAsync(h->sc.iq_state, 0, sizeof(double2), st));
+    return end ? seam_reset(h, st) : 0;
+}
+
+// The plan of a ragged last frame of Lp samples (0 < Lp < N): the handle's, with that frame's
+// geometry and the tables that depend on its length, derived from the handle's tables (host copies)
+// into d_rag: [0..8) p^Lp, [8..16) p^(q Mf), then phE [R], Eend [R][nend], bnd [M][8] and T1 [R][ntiles]
+// (the rows of T1 are ntiles long).
+int seam_ragged_plan(sdrb_handle *h, int Lp, DevPlan &pp, cudaStream_t st)
+{
+    const DevPlan &pl = h->pl;
+    const int q = pl.q, R = pl.R, edge = pl.edge, nt = pl.ntiles;
+    pp = pl;
+    pp.N = Lp; pp.L = Lp + 2 * edge;
+    pp.Mf = Lp / q; pp.rem = Lp - pp.Mf * q; pp.M = pp.Mf + (pp.rem ? 1 : 0);
+    pp.W = pl.demod == SDRB_IQ ? 2 * pp.M : pp.M;
+    pp.ntiles = std::max(1, (pp.Mf + SDRB_TB - 1) / SDRB_TB);     // Mf = 0: one empty tile
+    pp.cnt_last = pp.Mf - (pp.ntiles - 1) * SDRB_TB;
+    pp.ws = std::min(q * pp.Mf, Lp - 1 - edge);                    // < 0: the window reaches into the frame before
+    pp.nend = Lp - pp.ws;
+    pp.k_bnd = std::max(0, pl.k_bnd - (pl.M - pp.M));
+    pp.lam_N = std::pow(pl.lam_q, pp.Mf) * h->h_lamj[pp.rem];
+    pp.lam_tile[1] = std::pow(pl.lam_q, pp.cnt_last);
+    // p_i^n (0 <= n < N) and the in-frame NCO phase of sample n (|n| < N), from the whole-frame tables
+    auto pw_of = [&](long n, int i) {
+        const long b = n / q, j = n % q;
+        return hmul(hmul(h->h_Pt[(size_t)(b / SDRB_TB) * 8 + i], h->h_Ppow[(size_t)(b % SDRB_TB) * 8 + i]),
+                    h->h_pk[(size_t)j * 8 + i]);
+    };
+    auto phase = [&](int r, long n) {
+        const long a = n < 0 ? -n : n, b = a / q, j = a % q;
+        const double2 e = hmul(hmul(h->h_T1[(size_t)r * nt + b / SDRB_TB], h->h_T3[(size_t)r * (SDRB_TB + 1) + b % SDRB_TB]),
+                               h->h_T2[(size_t)r * q + j]);
+        return n < 0 ? make_double2(e.x, -e.y) : e;
+    };
+    std::vector<double2> &g = h->h_rag;
+    for (int i = 0; i < 8; i++) { g[i] = pw_of(Lp, i); g[8 + i] = pw_of((long)q * pp.Mf, i); }
+    double2 *phE = g.data() + 16, *Eend = phE + R, *bnd = Eend + (size_t)R * pp.nend;
+    for (int r = 0; r < R; r++) {
+        phE[r] = phase(r, (long)q * pp.Mf);
+        for (int j = 0; j < pp.nend; j++) Eend[(size_t)r * pp.nend + j] = phase(r, (long)pp.ws + j);
     }
+    // bnd[k] = c p^(Lp-1-q k): the whole frame's row M-M'+k, over p^(q-rem) when the last block is partial
+    for (int k = 0; k < pp.M; k++)
+        for (int i = 0; i < 8; i++) {
+            const double2 b = h->h_bnd[(size_t)(pl.M - pp.M + k) * 8 + i], d = h->h_pk[(size_t)(q - pp.rem) * 8 + i];
+            const double dd = d.x * d.x + d.y * d.y;
+            bnd[(size_t)k * 8 + i] = pp.rem ? make_double2((b.x * d.x + b.y * d.y) / dd, (b.y * d.x - b.x * d.y) / dd) : b;
+        }
+    double2 *T1 = bnd + (size_t)pp.M * 8;
+    for (int r = 0; r < R; r++)
+        for (int t = 0; t < pp.ntiles; t++) T1[(size_t)r * pp.ntiles + t] = h->h_T1[(size_t)r * nt + t];
+    const size_t n = 16 + (size_t)R * (1 + pp.nend) + (size_t)pp.M * 8 + (size_t)R * pp.ntiles;
+    CK(h, cudaMemcpyAsync(h->d_rag, g.data(), n * sizeof(double2), cudaMemcpyHostToDevice, st));
+    pp.phE = h->d_rag + 16;
+    pp.Eend = pp.phE + R;
+    pp.bnd = pp.Eend + (size_t)R * pp.nend;
+    pp.T1 = pp.bnd + (size_t)pp.M * 8;
     return 0;
+}
+
+// The end of a stream whose last frame is ragged: Lp samples at rawp (0 < Lp < N; h->hist samples
+// of the stream before them readable).  That frame goes through the front end, the IQ kernels and
+// the seamless kernels on its own plan, in window slot s = nwin after the whole frames still held
+// back, as the stream's real end.  k_seam_fold then moves the end to the last whole frame, which
+// are emitted as by seam_step; the ragged frame's M' outputs follow theirs in every row.
+int seam_end_ragged(sdrb_handle *h, const uint8_t *rawp, int Lp, double *out, cudaStream_t st, size_t *nout)
+{
+    const DevPlan &pl = h->pl;
+    const SeamDev &sd = h->sd;
+    const int R = pl.R, M = pl.M, ne = h->nwin;
+    DevPlan pp;
+    int rc = seam_ragged_plan(h, Lp, pp, st);
+    if (rc) return rc;
+    const double2 *pw = h->d_rag;
+    const Scratch sv = seam_scratch_at(h, ne);
+    const SeamDev sdv = seam_dev_at(h, ne);
+    const long long g = h->seen, g0 = h->emitted;
+    if (pp.Mf == 0) {   // a partial block only: no front end, zero tile aggregates
+        CK(h, cudaMemsetAsync(sv.agg, 0, (size_t)R * 16 * sizeof(*sv.agg), st));
+        CK(h, cudaMemsetAsync(sv.tile_agg, 0, sizeof(*sv.tile_agg), st));
+    }
+    if ((rc = launch_chain(h, sv, rawp, 1, nullptr, st, (pp.Mf ? PH_MAIN : 0) | PH_IQSCAN, &pp))) return rc;
+    rc = with_enc(h, h->enc_code, [&](auto enc) {
+        launch(h, k_seam_edges<decltype(enc)::value>, 1u, 64, 0, st, pp, sdv, rawp, 0, 1);
+        return 0;
+    });
+    if (rc) return rc;
+    const unsigned w1 = (unsigned)((R + 7) / 8);
+    launch(h, k_seam_agg, w1, 256, 0, st, pp, sv, sdv, 0, 1, g);
+    if (g == 0) launch(h, k_seam_head, (unsigned)R, 32, 0, st, pp, sv, sdv, 0);
+    SeamDev sdq = sdv;
+    sdq.PN = pw;        // the forward state crosses the frame's full blocks: p^(q Mf) in PN's row 1
+    launch(h, k_seam_fscan, (unsigned)R, 256, 0, st, pp, sdq, 0, 1);
+    launch(h, k_seam_tail, (unsigned)R, 32, 0, st, pp, sv, sdv, 0, g);
+    launch(h, k_seam_carry, w1, 256, 0, st, pp, sv, sdv, 1, 1, g, 1);
+    launch(h, k_seam_y, w1, 256, 0, st, pp, sv, sdv, 1, 1, g, 1);
+    const unsigned wg = (unsigned)(((size_t)ne * R + 7) / 8);
+    if (ne) {
+        launch(h, k_seam_fold, (unsigned)R, 32, 0, st, sdv, pw);
+        launch(h, k_seam_carry, wg, 256, 0, st, pl, h->sc, sd, ne, ne, g0, 1);
+        launch(h, k_seam_y, wg, 256, 0, st, pl, h->sc, sd, ne, ne, g0, 1);
+        // the last whole frame's fm halo is the ragged frame's first output; a one-output ragged
+        // frame's fm pairs that output with the last whole frame's last one
+        double2 *ylast = sd.ybuf + (size_t)(ne - 1) * R * (M + 1);
+        CK(h, cudaMemcpy2DAsync(ylast + M, (M + 1) * sizeof(double2), sdv.ybuf, (pp.M + 1) * sizeof(double2),
+                                sizeof(double2), R, cudaMemcpyDeviceToDevice, st));
+        if (pp.M == 1)
+            CK(h, cudaMemcpy2DAsync(sdv.ybuf + 1, 2 * sizeof(double2), ylast + M - 1, (M + 1) * sizeof(double2),
+                                    sizeof(double2), R, cudaMemcpyDeviceToDevice, st));
+    }
+    const size_t rs = (size_t)ne * M + pp.M, dpo = (size_t)(pl.W / M);
+    with_out(pl.demod, [&](auto ok) {
+        constexpr bool SSB = decltype(ok)::value == OUT_SSB;
+        if (ne) launch(h, k_seam_demod<SSB>, wg, 256, 0, st, pl, sd, out, ne, ne, 0, rs);
+        launch(h, k_seam_demod<SSB, true>, w1, 256, 0, st, pp, sdv, out + (size_t)ne * M * dpo, 1, 1, 1, rs);
+        if (pl.nsec_out) {
+            const unsigned fg = (unsigned)std::min<size_t>((R * rs + 255) / 256, (size_t)h->num_sms * 16);
+            launch(h, k_seam_sscan<std::conditional_t<SSB, double2, double>>, (unsigned)R, 32, 0, st, pl, sd, ne + 1);
+            launch(h, k_seam_frame<SSB>, fg, 256, 0, st, pl, sd, out, rs);
+        }
+        return 0;
+    });
+    CK(h, cudaGetLastError());
+    if (nout) *nout = rs;
+    return seam_reset(h, st);
+}
+
+// Sample-granular input: `ns` samples behind the pending ones in the current raw window, the whole
+// frames through seam_step, then the samples left over (with the h->hist before them) to the front
+// of the other window.  *nout = outputs per row.
+int seam_samples(sdrb_handle *h, const void *src, size_t ns, bool host, double *out, cudaStream_t st, size_t *nout)
+{
+    const size_t sb = h->pl.sb, N = h->pl.N, hist = h->hist;
+    for (uint8_t *&w : h->rawwin)
+        if (!w) CK(h, cudaMalloc(&w, (hist + (h->max_chunks + 1) * N) * sb));
+    const uint8_t *base = h->rawwin[h->wsel] + hist * sb;
+    if (ns)
+        CK(h, cudaMemcpyAsync(h->rawwin[h->wsel] + (hist + h->pend) * sb, src, ns * sb,
+                              host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, st));
+    const size_t avail = h->pend + ns, nf = avail / N, left = avail - nf * N;
+    size_t ne = 0;
+    if (int rc = seam_step(h, base, nf, out, st, false, &ne)) return rc;
+    if (nf) {
+        h->wsel ^= 1;
+        CK(h, cudaMemcpyAsync(h->rawwin[h->wsel], base + (nf * N - hist) * sb, (hist + left) * sb, cudaMemcpyDeviceToDevice,
+                              st));
+    }
+    h->pend = left;
+    *nout = ne * (size_t)h->pl.M;
+    return 0;
+}
+
+// The end of a sample-granular stream: the whole frames held back and the pending partial frame.
+int seam_samples_end(sdrb_handle *h, double *out, cudaStream_t st, size_t *nout)
+{
+    const long long L = h->seen * h->pl.N + (long long)h->pend;
+    if (L > 0 && L <= h->pl.edge) {
+        seam_reset(h, st);
+        return fail(h, SDRB_ERR_ARG, "a stream of %lld samples is not longer than the decimator's pad (%d)", L, h->pl.edge);
+    }
+    if (h->pl.demod == SDRB_FM && L > 0 && L <= h->pl.q) {
+        seam_reset(h, st);
+        return fail(h, SDRB_ERR_ARG, "fm needs two decimated outputs: a stream of %lld samples at -d %d gives one", L,
+                    h->pl.q);
+    }
+    if (!h->pend) {
+        size_t ne = 0;
+        if (int rc = seam_step(h, nullptr, 0, out, st, true, &ne)) return rc;
+        *nout = ne * (size_t)h->pl.M;
+        return 0;
+    }
+    return seam_end_ragged(h, h->rawwin[h->wsel] + (size_t)h->hist * h->pl.sb, (int)h->pend, out, st, nout);
 }
 }  // namespace
 extern "C" {
+
+static const char *pending_msg = "samples of a partial frame are pending: continue and end the stream with sdrb_stream_samples*";
 
 int sdrb_stream_device(sdrb_handle *h, const void *raw_dev, size_t nchunks, double *out_dev, void *stream,
                        size_t *nchunks_out)
 {
     if (nchunks_out) *nchunks_out = 0;
     if (int rc = entry(h, (raw_dev || !nchunks) && out_dev, SEAMLESS, nchunks, UPTO, out_dev)) return rc;
+    if (h->pend) return fail(h, SDRB_ERR_STATE, pending_msg);
+    if (int rc = seam_feed(h, FEED_CHUNKS, nchunks)) return rc;
     return seam_step(h, static_cast<const uint8_t *>(raw_dev), nchunks, out_dev, static_cast<cudaStream_t>(stream), false,
                      nchunks_out);
 }
@@ -963,6 +1218,7 @@ int sdrb_stream_end_device(sdrb_handle *h, double *out_dev, void *stream, size_t
 {
     if (nchunks_out) *nchunks_out = 0;
     if (int rc = entry(h, out_dev, SEAMLESS, 0, UPTO, out_dev)) return rc;
+    if (h->pend) return fail(h, SDRB_ERR_STATE, pending_msg);
     return seam_step(h, nullptr, 0, out_dev, static_cast<cudaStream_t>(stream), true, nchunks_out);
 }
 
@@ -970,6 +1226,8 @@ static int seam_host(sdrb_handle *h, const void *raw_host, size_t nchunks, doubl
 {
     if (nchunks_out) *nchunks_out = 0;
     int rc = entry(h, (raw_host || !nchunks) && out_host, SEAMLESS, nchunks);
+    if (!rc && h->pend) rc = fail(h, SDRB_ERR_STATE, pending_msg);
+    if (!rc) rc = seam_feed(h, FEED_CHUNKS, nchunks);
     if (!rc) rc = stage_in(h, 0, raw_host, nchunks);
     if (rc) return rc;
     Slot &sl = h->slot[0];
@@ -992,6 +1250,64 @@ int sdrb_stream(sdrb_handle *h, const void *raw_host, size_t nchunks, double *ou
 int sdrb_stream_end(sdrb_handle *h, double *out_host, size_t *nchunks_out)
 {
     return seam_host(h, nullptr, 0, out_host, nchunks_out, true);
+}
+
+int sdrb_stream_samples_device(sdrb_handle *h, const void *raw_dev, size_t nsamples, double *out_dev, void *stream,
+                               size_t *nout)
+{
+    if (nout) *nout = 0;
+    if (int rc = entry(h, (raw_dev || !nsamples) && out_dev && nout, SEAMLESS, 0, UPTO, out_dev)) return rc;
+    if (nsamples > h->max_chunks * (size_t)h->pl.N)
+        return fail(h, SDRB_ERR_ARG, "nsamples %zu above max_chunks * N = %zu", nsamples, h->max_chunks * (size_t)h->pl.N);
+    if (int rc = seam_feed(h, FEED_SAMPLES, nsamples)) return rc;
+    return seam_samples(h, raw_dev, nsamples, false, out_dev, static_cast<cudaStream_t>(stream), nout);
+}
+
+int sdrb_stream_samples_end_device(sdrb_handle *h, double *out_dev, void *stream, size_t *nout)
+{
+    if (nout) *nout = 0;
+    if (int rc = entry(h, out_dev && nout, SEAMLESS, 0, UPTO, out_dev)) return rc;
+    return seam_samples_end(h, out_dev, static_cast<cudaStream_t>(stream), nout);
+}
+
+// The host forms: through slot 0's device output staging, synchronously.
+static int seam_samples_host(sdrb_handle *h, const void *raw_host, size_t nsamples, double *out_host, size_t *nout, bool end)
+{
+    if (nout) *nout = 0;
+    if (int rc = entry(h, (raw_host || !nsamples) && out_host && nout, SEAMLESS)) return rc;
+    if (nsamples > h->max_chunks * (size_t)h->pl.N)
+        return fail(h, SDRB_ERR_ARG, "nsamples %zu above max_chunks * N = %zu", nsamples, h->max_chunks * (size_t)h->pl.N);
+    if (int rc = seam_feed(h, FEED_SAMPLES, nsamples)) return rc;
+    Slot &sl = h->slot[0];
+    const size_t och = h->max_chunks + (size_t)h->sd.D;
+    if (!sl.out) CK(h, cudaMalloc(&sl.out, och * (size_t)h->pl.R * h->pl.W * sizeof(double)));
+    size_t n = 0;
+    int rc = end ? seam_samples_end(h, sl.out, sl.stream, &n) : seam_samples(h, raw_host, nsamples, true, sl.out, sl.stream, &n);
+    if (rc) return rc;
+    if (n)
+        CK(h, cudaMemcpyAsync(out_host, sl.out, n * (size_t)h->pl.R * (h->pl.W / h->pl.M) * sizeof(double),
+                              cudaMemcpyDeviceToHost, sl.stream));
+    CK(h, cudaStreamSynchronize(sl.stream));
+    *nout = n;
+    return SDRB_OK;
+}
+
+int sdrb_stream_samples(sdrb_handle *h, const void *raw_host, size_t nsamples, double *out_host, size_t *nout)
+{
+    return seam_samples_host(h, raw_host, nsamples, out_host, nout, false);
+}
+
+int sdrb_stream_samples_end(sdrb_handle *h, double *out_host, size_t *nout)
+{
+    return seam_samples_host(h, nullptr, 0, out_host, nout, true);
+}
+
+size_t sdrb_stream_capacity(const sdrb_handle *h, size_t nsamples)
+{
+    if (!h || !h->seamless) return 0;
+    // a call emits at most its whole frames; an end call the D frames held back and one partial frame
+    const size_t N = (size_t)h->pl.N;
+    return std::max((N - 1 + nsamples) / N, (size_t)h->sd.D + 1) * (size_t)h->pl.M;
 }
 
 int sdrb_stream_lookahead(const sdrb_handle *h)

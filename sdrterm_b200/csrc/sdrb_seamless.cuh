@@ -33,7 +33,8 @@
 
 struct SeamDev {
     int D;                     // lookahead in chunks
-    int nedge;                 // decoded samples kept per chunk: head (edge+1) + end window (nend)
+    int nedge;                 // decoded samples kept per chunk: head (edge+1) + end window (nend); the
+                               // stride holds a ragged last frame's longer window (max(edge+1, q-1))
     long long fs;
     const long long *step;     // [R] (f_r N) mod fs
     const double2 *PN;         // [D+1][8] p_i^(N j)
@@ -75,7 +76,7 @@ k_seam_edges(const __grid_constant__ DevPlan pl, SeamDev sd, const uint8_t *__re
     if (c >= nch) return;
     const uint8_t *rawc = raw + (size_t)c * pl.N * pl.sb;
     double2 *e = sd.edges + (size_t)(slot0 + c) * sd.nedge;
-    for (int j = threadIdx.x; j < sd.nedge; j += blockDim.x) {
+    for (int j = threadIdx.x; j < pl.edge + 1 + pl.nend; j += blockDim.x) {
         const long n = j <= pl.edge ? j : (long)pl.ws + (j - pl.edge - 1);
         e[j] = decode_sample<ENC>(pl, rawc, n);
     }
@@ -158,6 +159,28 @@ k_seam_tail(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int slot
         sd.endv[(size_t)r * 16 + m] = cmul(ph, Tt);
         sd.endv[(size_t)r * 16 + 8 + m] = cmul(ph, zeta);
     }
+    if (pl.rem) {       // a ragged last frame: the output at its partial block, as k_fixup's
+        double2 v = cfma(pl.rho[m], w, cmul(pl.rho_p[m], bs.B));
+        v = cfma(pl.bnd[(size_t)pl.Mf * 8 + m], zeta, v);
+        for (int sft = 1; sft < 8; sft <<= 1) v = cadd(v, shfl_xor_c(v, sft));
+        if (lane == 0)
+            sd.ybuf[((size_t)slot * pl.R + r) * (pl.M + 1) + pl.Mf] =
+                cmul(ph, make_double2(fma(pl.g0, seq[0].x, v.x), fma(pl.g0, seq[0].y, v.y)));
+    }
+}
+
+// warp <-> row: a ragged last frame (its slot in `sd`) moves the real end to the last whole frame,
+// so that k_seam_carry runs over the whole frames unchanged: the anticausal state crosses the
+// frame's full blocks (pw[8..15] = p^(q Mf)) and takes its backward aggregate, zeta is referred to
+// Lp samples earlier (pw[0..7] = p^Lp).
+__global__ void __launch_bounds__(32)
+k_seam_fold(SeamDev sd, const double2 *pw)
+{
+    const int r = blockIdx.x, m = threadIdx.x;
+    if (m >= 8) return;
+    double2 *e = sd.endv + (size_t)r * 16;
+    e[m] = cfma(pw[8 + m], e[m], sd.cagg[(size_t)r * 16 + 8 + m]);
+    e[8 + m] = cmul(pw[m], e[8 + m]);
 }
 
 // warp <-> (emitted chunk i, row), lane <-> mode.  Window slots 0..nwin-1 hold global chunks g0..;
@@ -231,18 +254,24 @@ k_seam_y(const __grid_constant__ DevPlan pl, Scratch sc, SeamDev sd, int ne, int
 __device__ __forceinline__ double seam_demod_at(const double2 *y, int k, int M, bool last, int demod)
 {
     if (demod != SDRB_FM) return demod_scalar(y[k], demod);
-    if (last && k == M - 1) k = M - 2;
+    if (last && k == M - 1) {
+        if (M == 1) return pair_phase(y[1], y[0]);    // a one-output last frame: y[1] holds the output before it
+        k = M - 2;
+    }
     return pair_phase(y[k], y[k + 1]);
 }
 
-// warp <-> (emitted chunk, row), lane <-> segment of Lseg = M/32 outputs.  Without an output
+// warp <-> (emitted chunk, row), lane <-> segment of Lseg = ceil(M/32) outputs.  Without an output
 // filter the demodulated values are framed and stored; with it the output stage runs the cascade
 // from the chunk's zero state (sdrb_outstage.cuh) and the chunk's zero-state end state goes to
 // echunk.  The response to the state carried from earlier chunks is k_seam_frame's.  The SSB
-// instance runs the complex band-pass on y, its end state complex.
-template <bool SSB>
+// instance runs the complex band-pass on y, its end state complex.  Rows of `out` are rs outputs
+// long (W / M doubles each).  A ragged last frame comes in its own launch of the SHORT instance
+// (M < 32 Lseg): its lanes stop at M (a short or empty segment only feeds the states of the lanes
+// after it, whose outputs lie past M; its end state is not used, the stream ends there).
+template <bool SSB, bool SHORT = false>
 __global__ void __launch_bounds__(256)
-k_seam_demod(const __grid_constant__ DevPlan pl, SeamDev sd, double *out, int ne, int nwin, int end)
+k_seam_demod(const __grid_constant__ DevPlan pl, SeamDev sd, double *out, int ne, int nwin, int end, size_t rs)
 {
     using T = std::conditional_t<SSB, double2, double>;
     const int lane = threadIdx.x & 31;
@@ -251,9 +280,9 @@ k_seam_demod(const __grid_constant__ DevPlan pl, SeamDev sd, double *out, int ne
     const int i = (int)(item / pl.R), r = (int)(item % pl.R), M = pl.M, lo = lane * pl.sos_Lseg;
     const bool last = end && i == nwin - 1;
     const double2 *y = sd.ybuf + ((size_t)i * pl.R + r) * (M + 1);
-    double *o = out + (size_t)r * ne * M + (size_t)i * M;
-    if (!SSB && pl.demod == SDRB_IQ) {     // rows of ne * 2M doubles, no output low-pass
-        double2 *o2 = reinterpret_cast<double2 *>(out + ((size_t)r * ne + i) * pl.W);
+    double *o = out + (size_t)r * rs + (size_t)i * M;
+    if (!SSB && pl.demod == SDRB_IQ) {     // rows of rs (Re, Im) pairs, no output low-pass
+        double2 *o2 = reinterpret_cast<double2 *>(out) + (size_t)r * rs + (size_t)i * M;
         for (int k = lane; k < M; k += 32) frame_store(o2 + k, y[k], pl.be_out);
         return;
     }
@@ -263,7 +292,7 @@ k_seam_demod(const __grid_constant__ DevPlan pl, SeamDev sd, double *out, int ne
     }
     T st[SEAM_NS];
     sos_segments(
-        pl, SEAM_NS / 2, lo, pl.sos_Lseg, lane,
+        pl, SEAM_NS / 2, lo, SHORT ? max(0, min(pl.sos_Lseg, M - lo)) : pl.sos_Lseg, lane,
         [&](int j) {
             if constexpr (SSB) return y[lo + j];
             else return seam_demod_at(y, lo + j, M, last, pl.demod);
@@ -374,15 +403,16 @@ k_seam_sscan(const __grid_constant__ DevPlan pl, SeamDev sd, int ne)
     }
 }
 
-// thread <-> output: out += c A^k s[chunk], then framing; SSB: out += Re(e^{j Omega k} c A^k s[chunk])
+// thread <-> output: out += c A^k s[chunk], then framing; SSB: out += Re(e^{j Omega k} c A^k s[chunk]).
+// Rows of rs outputs: M per chunk, the last chunk possibly shorter (a ragged last frame).
 template <bool SSB>
 __global__ void __launch_bounds__(256)
-k_seam_frame(const __grid_constant__ DevPlan pl, SeamDev sd, double *out, int ne)
+k_seam_frame(const __grid_constant__ DevPlan pl, SeamDev sd, double *out, size_t rs)
 {
     using T = std::conditional_t<SSB, double2, double>;
-    const size_t M = pl.M, total = (size_t)pl.R * ne * M;
+    const size_t M = pl.M, total = (size_t)pl.R * rs;
     for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (size_t)gridDim.x * blockDim.x) {
-        const size_t r = e / ((size_t)ne * M), rest = e % ((size_t)ne * M), i = rest / M, k = rest % M;
+        const size_t r = e / rs, rest = e % rs, i = rest / M, k = rest % M;
         const T *s = reinterpret_cast<const T *>(sd.sst) + (i * pl.R + r) * SEAM_NS;
         const double2 ph = SSB ? pl.ssb_rot[k] : make_double2(1.0, 0.0);
         frame_store(out + e, add_response<SEAM_NS>(out[e], sd.CAM + k * SEAM_NS, SEAM_NS, s, ph), pl.be_out);

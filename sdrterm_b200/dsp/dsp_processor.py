@@ -195,7 +195,7 @@ class DspProcessor(DataProcessor):
 
     def _makeEngine(self, first):
         from ..engine import Engine
-        from ..plan import cached_plan
+        from ..plan import _ITEMSIZE, cached_plan, seamless_frame_samples
         if isinstance(first, np.ndarray) and np.iscomplexobj(first):
             enc, swap, ciq, norm = 'Z', False, False, False       # producer already did these
             chunk_bytes = first.size * 16
@@ -216,9 +216,13 @@ class DspProcessor(DataProcessor):
             ciq, norm = self._correctIq, self._normalize
             nb = len(first) if not isinstance(first, np.ndarray) else first.nbytes
             chunk_bytes = 131072 if nb % 131072 == 0 else nb     # the reader may hand over several chunks at once
+        plan_bytes = chunk_bytes
+        if self._seamless:     # the seamless pipeline runs on frames of whole tiles (DESIGN.md section 11)
+            sb = 2 * _ITEMSIZE[enc]
+            plan_bytes = seamless_frame_samples(chunk_bytes // sb, self._decimationFactor) * sb
         plan, tc = cached_plan(self.__fs, enc, self._decimationFactor, self._rowsHz(), simo=self._simo(),
                                swap=swap, correct_iq=ciq, normalize=norm, demod=self._demodName(),
-                               omega_out=self.omegaOut, chunk_bytes=chunk_bytes,
+                               omega_out=self.omegaOut, chunk_bytes=plan_bytes,
                                **({'seamless': True} if self._seamless else {}))
         self._chunkBytes = chunk_bytes
         # --smooth-output (dsp_processor.py:159-160): standard mode only, the SIMO override of
@@ -238,8 +242,9 @@ class DspProcessor(DataProcessor):
             return np.ascontiguousarray(chunk).view(np.uint8).reshape(-1)
         return np.frombuffer(chunk, dtype=np.uint8)
 
-    def _emit(self, out: np.ndarray, nchunks: int, file) -> None:
-        """Standard mode: one stream, native doubles, chunk after chunk (:162)."""
+    def _emit(self, out: np.ndarray, noutputs: int, file) -> None:
+        """Standard mode: one stream, native doubles, chunk after chunk (:162); ``noutputs`` outputs
+        per row."""
         file.write(out[0].tobytes())
 
     def _staging(self):
@@ -333,8 +338,9 @@ class DspProcessor(DataProcessor):
 
     def _processSeamless(self, isDead, buffer, file) -> None:
         """The consumer loop of the seamless mode, synchronous: every batch goes through
-        ``Engine.stream`` (which emits the chunks that have become final), and at end of stream or on
-        halt ``Engine.stream_end`` emits the chunks still held back, so no tail is lost."""
+        ``Engine.stream_samples`` (which emits the outputs of the frames that have become final), and
+        at end of stream or on halt ``Engine.stream_samples_end`` emits the frames still held back and
+        the partial last frame, so no tail is lost."""
         eof = False
         pool = self._inputPool
         while not (self._isDead or isDead.value or eof):
@@ -358,16 +364,16 @@ class DspProcessor(DataProcessor):
                 a = self._asBytes(c)
                 if a.size % self._chunkBytes:
                     raise ValueError('queue items must be whole chunks of the size of the first one')
-                out = self._engine.stream(a)
+                out = self._engine.stream_samples(a)
                 home = pool.owner(a) if pool is not None else None
                 if home is not None:
-                    pool.release(home)                   # stream() has copied the bytes to the device
+                    pool.release(home)                   # the bytes are on the device, behind the pending ones
                 if out.shape[1]:
-                    self._emit(out, out.shape[1] // self._rowDoubles(), file)
+                    self._emit(out, out.shape[1] * self._engine.M // self._rowDoubles(), file)
         if self._engine is not None:
-            out = self._engine.stream_end()
+            out = self._engine.stream_samples_end()
             if out.shape[1]:
-                self._emit(out, out.shape[1] // self._rowDoubles(), file)
+                self._emit(out, out.shape[1] * self._engine.M // self._rowDoubles(), file)
 
     def useInputPool(self, pool) -> None:
         """Queue items that are views of ``pool``'s buffers (misc.read_file.ChunkPool) are sent to
@@ -402,7 +408,7 @@ class DspProcessor(DataProcessor):
         out = self._hout[slot].view(np.float64)[:eng.R * n * W].reshape(eng.R, n * W)
         if eng.plan.big_endian_out:
             out = out.view('>f8')
-        self._emit(out, n, file)
+        self._emit(out, n * eng.M, file)
 
     def processData(self, isDead, buffer, f: str | None, *args, **kwargs) -> None:
         with open(f, 'wb') if f is not None else open(stdout.fileno(), 'wb', closefd=False) as file:

@@ -64,14 +64,13 @@ class VfoProcessor(DspProcessor):
             # example_simo.sh waits for this line before it starts the stream (:165-170)
             print('Connection(s) established', file=sys.stderr, flush=True)
 
-    def _emit(self, out: np.ndarray, nchunks: int, file) -> None:
-        """Row r goes to client r; ``out`` rows already hold big-endian doubles (:84)."""
+    def _emit(self, out: np.ndarray, noutputs: int, file) -> None:
+        """Row r (``noutputs`` outputs) goes to client r; ``out`` rows already hold big-endian
+        doubles (:84)."""
         if self._shift is None:
             self._generateShift(1)
-        M = out.shape[1] // nchunks
         for r in range(self._nFreq):
             self._clients[r].write(out[r].tobytes())
-        _ = M
 
     def processData(self, isDead, buffer, *args, **kwargs) -> None:
         self._rowQueue = _queue.Queue()

@@ -211,6 +211,63 @@ class Engine:
         nat.check(nat.lib().sdrb_stream_end(self._h, out.ctypes.data, C.byref(got)), self._h)
         return self._rows(out, got.value)
 
+    def stream_capacity(self, nsamples: int) -> int:
+        """The most outputs per row a ``stream_samples`` call with ``nsamples`` new samples, or a
+        ``stream_samples_end`` call, can emit."""
+        return int(nat.lib().sdrb_stream_capacity(self._h, nsamples))
+
+    def _out_outputs(self, nout: int) -> np.ndarray:
+        dt = np.dtype('>f8') if self.plan.big_endian_out else np.dtype('=f8')
+        return np.empty(self.R * nout * (self.W // self.M), dtype=dt)
+
+    def stream_samples(self, raw) -> np.ndarray:
+        """Seamless mode, any whole number of complex samples (the plan's chunk is the seamless frame,
+        ``plan.seamless_frame_samples``): returns (R, n) doubles for the n outputs per row that have
+        become final (2n for iq).  Samples that do not fill a frame wait on the device for the next
+        call.  Inputs larger than ``max_chunks`` frames are fed in pieces."""
+        if not self.seamless:
+            raise nat.SdrbError('stream_samples() needs a plan built with seamless=True')
+        buf = np.frombuffer(raw, dtype=np.uint8) if not isinstance(raw, np.ndarray) else raw
+        buf = np.ascontiguousarray(buf).view(np.uint8).reshape(-1)
+        sb = self.chunk_bytes // self.plan.N
+        if buf.size % sb:
+            raise ValueError(f'{buf.size} bytes are not whole samples of {sb} bytes')
+        ns, step = buf.size // sb, self.max_chunks * self.plan.N
+        parts = []
+        for s0 in range(0, ns, step):
+            k = min(step, ns - s0)
+            out = self._out_outputs(self.stream_capacity(k))
+            got = C.c_size_t(0)
+            nat.check(nat.lib().sdrb_stream_samples(self._h, buf[s0 * sb:].ctypes.data, k, out.ctypes.data,
+                                                    C.byref(got)), self._h)
+            parts.append(out[:self.R * got.value * (self.W // self.M)].reshape(self.R, -1))
+        if not parts:
+            return self._out_outputs(0).reshape(self.R, 0)
+        return np.concatenate(parts, axis=1) if len(parts) > 1 else parts[0]
+
+    def stream_samples_end(self) -> np.ndarray:
+        """Seamless mode: end of a ``stream_samples`` stream.  Returns the outputs still held back,
+        the partial last frame's included (ceil(L/q) outputs per row over the whole stream), and
+        resets the stream."""
+        if not self.seamless:
+            raise nat.SdrbError('stream_samples_end() needs a plan built with seamless=True')
+        out = self._out_outputs(self.stream_capacity(0))
+        got = C.c_size_t(0)
+        nat.check(nat.lib().sdrb_stream_samples_end(self._h, out.ctypes.data, C.byref(got)), self._h)
+        return out[:self.R * got.value * (self.W // self.M)].reshape(self.R, -1)
+
+    def stream_samples_device(self, raw_ptr: int, nsamples: int, out_ptr: int, stream: int = 0) -> int:
+        """Device pointers in/out, only enqueued on ``stream``; returns the outputs per row emitted."""
+        got = C.c_size_t(0)
+        nat.check(nat.lib().sdrb_stream_samples_device(self._h, raw_ptr, nsamples, out_ptr, stream, C.byref(got)),
+                  self._h)
+        return got.value
+
+    def stream_samples_end_device(self, out_ptr: int, stream: int = 0) -> int:
+        got = C.c_size_t(0)
+        nat.check(nat.lib().sdrb_stream_samples_end_device(self._h, out_ptr, stream, C.byref(got)), self._h)
+        return got.value
+
     def stream_device(self, raw_ptr: int, nchunks: int, out_ptr: int, stream: int = 0) -> int:
         """Device pointers in/out, only enqueued on ``stream``; returns the number of chunks emitted."""
         got = C.c_size_t(0)

@@ -270,6 +270,14 @@ def lookahead_chunks(p, rho_p, N: int, tol: float = LOOKAHEAD_TOL) -> int:
     return D
 
 
+def seamless_frame_samples(N: int, q: int) -> int:
+    """Samples per frame of the seamless mode for chunks of N samples at decimation q: the most
+    whole tiles (32 blocks of q samples) that fit a chunk, 32 q floor(N / (32 q)).  Equal to N for
+    every power-of-two q that divides N/32.  The seamless pipeline runs on frames, not on the reader's
+    chunks, so any q works (DESIGN.md section 11)."""
+    return TILE_BLOCKS * q * (N // (TILE_BLOCKS * q))
+
+
 def build_plan(fs: int, enc: str, dec: int, rows_hz, *, simo: bool = False, swap: bool = False,
                correct_iq: bool = False, normalize: bool = False, impedance: int = 50,
                demod: str = 'fm', omega_out: int = 12500, chunk_bytes: int = CHUNK_BYTES,

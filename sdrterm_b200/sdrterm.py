@@ -46,7 +46,7 @@ def buildParser() -> argparse.ArgumentParser:
     ap.add_argument('--seamless', dest='seamless', action='store_true',
                     help='not a reference option: filter and demodulate the whole stream as one signal '
                          'instead of each 131072-byte chunk (no transient at chunk edges; output '
-                         'delayed by a few chunks; needs a power-of-two -d; no --smooth-output)')
+                         'delayed by a few chunks; any -d; no --smooth-output)')
     ap.add_argument('--no-seamless', dest='seamless', action='store_false')
     ap.add_argument('--normalize-input', dest='normalize', action='store_true')
     ap.add_argument('--no-normalize-input', dest='normalize', action='store_false')
